@@ -93,6 +93,17 @@ __device__ inline void cov_pose_row(const float* __restrict__ t3, const float* _
     row[5] = make_float4(t3[0], t3[1], t3[2], 0.f);
 }
 
+// Normalisation constants of a pose row from its extrema a = min_j m and mx = max_j m: row[4] = (b/2, b, 1/b, a),
+// b = mx - a, and the conservative gate threshold thr = (a + b/2)(1 - 2^-20) (no pair below it is gated), which goes
+// where the caller's table layout keeps it.  thr is written before row[4] (not returned): for a row in shared memory
+// the other store order costs the dense sweep kernel 4 more registers.
+__device__ __forceinline__ void cov_norm_row(float4* row, float a, float mx, float& thr) {
+    const float b = __fsub_rn(mx, a);
+    const float hb = 0.5f * b;
+    thr = (a + hb) * (1.f - 9.5367431640625e-07f);
+    row[4] = make_float4(hb, b, __frcp_rn(b), a);
+}
+
 // |x - td|^2 exactly as cov_vis computes it (same three instructions per component), for the pruning
 // pre-filter:  m = s * 2^-(kd q2 + ...) <= 2^-(kd q2) * (1 + 1.3e-5)   (s <= 1 up to the rcp rounding).
 __device__ __forceinline__ float cov_q2(float x, float y, float z, const float4& v3) {
@@ -126,6 +137,16 @@ __device__ __forceinline__ float cov_vis(float x, float y, float z, const float4
         ev->zi = zi; ev->s = s; ev->e2z = e2z; ev->du = du; ev->dv = dv;
     }
     return __fmul_rn(E, s);
+}
+
+// Log-odds term of a gated (point, pose) with v4 = (b/2, b, 1/b, a) (cov_norm_row): the pair is gated exactly when
+// p = d/b >= 1/2 for d = m - a, i.e. when d >= b/2, and then adds logit(min(p, hi)) to the point's log-odds sum.  The
+// gate test stays with the callers: the dense pass B takes a warp ballot of it before it branches to the log-odds and
+// the tie test, and folding the test in here would split that branch in two (more instructions in its hot loop).
+__device__ __forceinline__ float cov_logodds(float d, const float4& v4, const CovConst& C) {
+    const float p = __fmul_rn(d, v4.z);
+    const float qc = (p > C.hi) ? C.hi : p;  // upper clip; a NaN p (pose that sees nothing: 0/0) stays NaN, as torch.clip
+    return COV_LN2_F * cov_lg2(qc * cov_rcp(1.f - qc));
 }
 
 // ---- packed fp32 pairs (sm_100: fma/mul/add/sub.rn.f32x2 -> FFMA2 / FMUL2 / FADD2) --------------------------------
@@ -252,6 +273,36 @@ __device__ __forceinline__ double cov_warp_sum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
+}
+
+// ---- TMA bulk copies (global -> shared) completing on an mbarrier ------------------------------------------------
+__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void tma_copy(void* dst_smem, const void* src_gmem, unsigned bytes, unsigned long long* bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                     smem_u32(dst_smem)),
+                 "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
+                 : "memory");
+}
+// the labels live inside the { } scope, so every inlined copy of the loop has its own
+__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "WAIT_LOOP:\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
+        "@p bra WAIT_DONE;\n"
+        "bra WAIT_LOOP;\n"
+        "WAIT_DONE:\n"
+        "}\n" ::"r"(smem_u32(bar)),
+        "r"(parity)
+        : "memory");
 }
 
 // ---- host-side helpers (cov_api.cu) ----

@@ -18,6 +18,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "cov_common.cuh"  // TMA bulk copies and their mbarriers
+
 namespace covradix {
 
 constexpr int kThreads = 256;
@@ -147,34 +149,6 @@ __global__ void __launch_bounds__(1024) scan_small_kernel(unsigned* __restrict__
     }
 }
 
-// ---- TMA bulk copies (global -> shared) completing on an mbarrier ----
-__device__ __forceinline__ unsigned rs_smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void rs_mbar_init(unsigned long long* bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(rs_smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void rs_mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(rs_smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void rs_tma_copy(void* dst_smem, const void* src_gmem, unsigned bytes, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     rs_smem_u32(dst_smem)),
-                 "l"(src_gmem), "r"(bytes), "r"(rs_smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void rs_mbar_wait(unsigned long long* bar, unsigned parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "RS_WAIT_LOOP:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra RS_WAIT_DONE;\n"
-        "bra RS_WAIT_LOOP;\n"
-        "RS_WAIT_DONE:\n"
-        "}\n" ::"r"(rs_smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-
 // dynamic shared memory of the downsweep kernel: [stage keys][stage vals][tile keys][tile vals][warp counters][base][doff]
 constexpr size_t kDownSmemBytes = 4 * (size_t)kTile * 4 + ((size_t)kWarps * kBins + 2 * kBins) * 4;
 
@@ -205,20 +179,20 @@ __global__ void __launch_bounds__(kThreads, 3) downsweep_kernel(const unsigned* 
     // thread 0 stages whole tiles only; every thread derives the same predicate when it consumes them
     auto stage_keys = [&](int64_t tile) {
         if (tile < tile1 && (tile + 1) * kTile <= n) {
-            rs_mbar_expect_tx(&bar_k, kTile * 4u);
-            rs_tma_copy(st_keys, keys_in + tile * kTile, kTile * 4u, &bar_k);
+            mbar_expect_tx(&bar_k, kTile * 4u);
+            tma_copy(st_keys, keys_in + tile * kTile, kTile * 4u, &bar_k);
         }
     };
     auto stage_vals = [&](int64_t tile) {
         if (tile < tile1 && (tile + 1) * kTile <= n) {
-            rs_mbar_expect_tx(&bar_v, kTile * 4u);
-            rs_tma_copy(st_vals, vals_in + tile * kTile, kTile * 4u, &bar_v);
+            mbar_expect_tx(&bar_v, kTile * 4u);
+            tma_copy(st_vals, vals_in + tile * kTile, kTile * 4u, &bar_v);
         }
     };
     if (t == 0) {
-        rs_mbar_init(&bar_k, 1);
-        rs_mbar_init(&bar_v, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(&bar_k, 1);
+        mbar_init(&bar_v, 1);
+        mbar_fence_init();
         stage_keys(tile0);
         stage_vals(tile0);
     }
@@ -234,7 +208,7 @@ __global__ void __launch_bounds__(kThreads, 3) downsweep_kernel(const unsigned* 
         unsigned key[kIpt];
         unsigned rank[kIpt];
         if (whole) {
-            rs_mbar_wait(&bar_k, par_k);
+            mbar_wait(&bar_k, par_k);
             par_k ^= 1u;
 #pragma unroll
             for (int r = 0; r < kIpt; ++r) key[r] = st_keys[warp * (32 * kIpt) + r * 32 + lane];
@@ -299,7 +273,7 @@ __global__ void __launch_bounds__(kThreads, 3) downsweep_kernel(const unsigned* 
 
         // reorder the tile by digit in shared memory (stable)
         if (whole) {
-            rs_mbar_wait(&bar_v, par_v);
+            mbar_wait(&bar_v, par_v);
             par_v ^= 1u;
         }
 #pragma unroll

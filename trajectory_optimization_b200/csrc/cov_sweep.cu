@@ -32,11 +32,7 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
     for (int w = tid; w < W; w += COV_THREADS) {
         float4* row = ptab + (size_t)w * COV_ROW_F4;
         cov_pose_row(poses + 3 * w, quats + 4 * w, K9, C, row);
-        const float a = mins[w];
-        const float b = __fsub_rn(maxs[w], a);
-        const float hb = 0.5f * b;
-        row[3].w = (a + hb) * (1.f - 9.5367431640625e-07f);  // conservative gate threshold
-        row[4] = make_float4(hb, b, __frcp_rn(b), a);
+        cov_norm_row(row, mins[w], maxs[w], row[3].w);  // conservative gate threshold in v3.w
     }
     for (int t = tid; t < n_traj; t += COV_THREADS) ssum[t] = 0.0;
     __syncthreads();
@@ -72,11 +68,7 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
 #pragma unroll
                     for (int s = 0; s < PPT; ++s) {
                         const float d = __fsub_rn(m[s], v4.w);
-                        if (d >= v4.x) {
-                            const float pn = __fmul_rn(d, v4.z);
-                            const float qc = (pn > C.hi) ? C.hi : pn;  // NaN (pose that sees nothing) stays NaN, as torch.clip
-                            L[s] += COV_LN2_F * cov_lg2(qc * cov_rcp(1.f - qc));
-                        }
+                        if (d >= v4.x) L[s] += cov_logodds(d, v4, C);  // exactly p >= 0.5
                     }
                 }
             }

@@ -33,10 +33,12 @@
 //                        ascending work list of the tiles with a non-empty mask, positions from a decoupled
 //                        look-back scan over the blocks' counts (deterministic; no second kernel); in pass B the
 //                        same blocks pre-fill the rewards with 1/2 (what every unlisted point gets, exactly)
-//   *_tiles_kernel       persistent blocks walk the work list; tile points, boxes and mask arrive together through a
-//                        double-buffered TMA bulk copy (one mbarrier per buffer); a warp evaluates a listed pose only
-//                        if its own 128-point box and then one of its points pass the same test.  Pass B queues its
-//                        gated (point, pose) pairs per warp and differentiates them 32 at a time with every lane busy.
+//   *_tiles_kernel       persistent WARPS (for_each_item): a warp draws 128-point items of the listed tiles from a
+//                        ticket counter; the next item's points, box and the tile's pose mask arrive by TMA bulk copy
+//                        in the warp's other stage (double-buffered, one mbarrier per stage) while it works on the
+//                        current one.  A warp evaluates a listed pose only if its own 128-point box (in pass A, then
+//                        also one of its points) passes the same test.  Pass B's backward re-evaluates: the warp walks
+//                        the poses it gated and recomputes m and dm/dx for its own points, with every lane busy.
 //   Tiles that are not listed are never read: their rewards are the pre-filled 1/2 (exact), their sum is 0.5 * count.
 //
 // Block accumulators are added to the caller's fp64 accumulator rows with fp64 atomics (the order of those additions is
@@ -77,16 +79,12 @@ size_t fused_smem_bytes(int W, int ppt) {  // dense pass B: pose table | tile po
 }
 
 // Unweighted dm/dy and dm/dy x y of one (point, pose) into a tie-set accumulator (7 doubles: F, T, count).  Rare (one
-// point per pose and step), so these are real calls; they take the pose INDEX (or its row in the global table) and find
-// the constants themselves — passing loaded rows would keep them live across the callers' hot loops.
-// The dense pass B keeps its table in pose PAIRS at the start of dynamic shared memory (COV_PAIR_F4, cov_common.cuh).
-__device__ __noinline__ void tie_accumulate_pair(float x, float y, float z, int w, CovConst C, double* acc, int slot) {
-    extern __shared__ float4 smem4[];
-    const float4* pair = smem4 + (size_t)(w >> 1) * COV_PAIR_F4;
-    const int h = w & 1;
-    const float4 v0 = cov_pair_row(pair, h, 0), v1 = cov_pair_row(pair, h, 1), v2 = cov_pair_row(pair, h, 2),
-                 v3 = cov_pair_row(pair, h, 3), v5 = pair[10 + h];
-    double* dst = acc + slot;
+// point per pose and step), so the two entry points below are real calls; they take the pose INDEX (or its row in the
+// global table) and find the constants themselves — passing loaded rows would keep them live across the callers' hot
+// loops.
+__device__ __forceinline__ void tie_accumulate(float x, float y, float z, const float4& v0, const float4& v1,
+                                               const float4& v2, const float4& v3, const float4& v5, const CovConst& C,
+                                               double* dst) {
     CovEval ev;
     const float m = cov_vis<true>(x, y, z, v0, v1, v2, v3, C, &ev);
     float gx, gy, gz;
@@ -101,22 +99,19 @@ __device__ __noinline__ void tie_accumulate_pair(float x, float y, float z, int 
     atomicAdd(dst + 6, 1.0);
 }
 
-// Same for the pruned pass B, whose pose table stays in global memory (read through L1, a handful of rows per tile).
+// The dense pass B keeps its table in pose PAIRS at the start of dynamic shared memory (COV_PAIR_F4, cov_common.cuh).
+__device__ __noinline__ void tie_accumulate_pair(float x, float y, float z, int w, CovConst C, double* acc, int slot) {
+    extern __shared__ float4 smem4[];
+    const float4* pair = smem4 + (size_t)(w >> 1) * COV_PAIR_F4;
+    const int h = w & 1;
+    tie_accumulate(x, y, z, cov_pair_row(pair, h, 0), cov_pair_row(pair, h, 1), cov_pair_row(pair, h, 2),
+                   cov_pair_row(pair, h, 3), pair[10 + h], C, acc + slot);
+}
+
+// The pruned pass B, whose pose table stays in global memory (read through L1, a handful of rows per tile).
 __device__ __noinline__ void tie_accumulate_g(float x, float y, float z, const float4* __restrict__ row, CovConst C,
                                               double* dst) {
-    const float4 v0 = __ldg(row), v1 = __ldg(row + 1), v2 = __ldg(row + 2), v3 = __ldg(row + 3), v5 = __ldg(row + 5);
-    CovEval ev;
-    const float m = cov_vis<true>(x, y, z, v0, v1, v2, v3, C, &ev);
-    float gx, gy, gz;
-    cov_vis_grad(m, ev, v0, v1, v2, C, gx, gy, gz);
-    const float yx = x - v5.x, yy = y - v5.y, yz = z - v5.z;
-    atomicAdd(dst + 0, (double)gx);
-    atomicAdd(dst + 1, (double)gy);
-    atomicAdd(dst + 2, (double)gz);
-    atomicAdd(dst + 3, (double)(gy * yz - gz * yy));
-    atomicAdd(dst + 4, (double)(gz * yx - gx * yz));
-    atomicAdd(dst + 5, (double)(gx * yy - gy * yx));
-    atomicAdd(dst + 6, 1.0);
+    tie_accumulate(x, y, z, __ldg(row), __ldg(row + 1), __ldg(row + 2), __ldg(row + 3), __ldg(row + 5), C, dst);
 }
 
 // ---- pruning helpers ------------------------------------------------------------------------------------------
@@ -148,35 +143,6 @@ __device__ __forceinline__ float minmax_qcap(unsigned mn, unsigned mx, float inv
     float cap = __uint_as_float(0x7f800000u);
     if (mn == 0u && mx != 0u) cap = (1e-4f - __log2f(__uint_as_float(mx))) * inv_kd * 1.000001f;
     return cap;
-}
-
-// ---- TMA bulk copies (global -> shared) completing on an mbarrier ------------------------------------------------
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void tma_copy(void* dst_smem, const void* src_gmem, unsigned bytes, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     smem_u32(dst_smem)),
-                 "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_LOOP:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra WAIT_DONE;\n"
-        "bra WAIT_LOOP;\n"
-        "WAIT_DONE:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
 }
 
 // =============================================== pass A, dense ===============================================
@@ -364,14 +330,12 @@ cov_traj_table_kernel(const float* __restrict__ poses, const float* __restrict__
     float4 row[COV_ROW_F4];
     cov_pose_row(poses + 3 * w, quats + 4 * w, K9, C, row);
     const float a = minmax[w];
-    const float b = __fsub_rn(minmax[W + w], a);
-    const float hb = 0.5f * b;
-    const float thr = (a + hb) * (1.f - 9.5367431640625e-07f);  // conservative gate threshold
+    float thr;
+    cov_norm_row(row, a, minmax[W + w], thr);
     row[5].w = thr;
     // q2 above qthr cannot reach thr (thr <= 0 or NaN, or a > 0 — arg-min points carry gradient: never prune)
     row[3].w = (thr > 0.f && !(a > 0.f)) ? (float)((1e-4 - log2((double)thr)) / (double)C.kd * 1.000001)
                                          : __uint_as_float(0x7f800000u);
-    row[4] = make_float4(hb, b, __frcp_rn(b), a);
 #pragma unroll
     for (int i = 0; i < COV_ROW_F4; ++i) table[(size_t)w * COV_ROW_F4 + i] = row[i];
 }
@@ -556,19 +520,134 @@ cov_cull_kernel(const float4* __restrict__ boxes, int boxes_per_tile, int64_t nt
     if (lane == 0 && npairs) atomicAdd(reinterpret_cast<unsigned long long*>(ctrl + 4), npairs);
 }
 
-// =============================================== pass A, pruned ===============================================
-// Persistent WARPS over the work list, like pass B below: the unit of work is one box of 128 consecutive points of a
-// listed tile, drawn by a warp from a global ticket counter; lane 0 stages the next item (points, box, the tile's pose
-// mask) by TMA into the warp's other private stage while the warp works on the current one.  A listed pose is evaluated
-// when the cap ball (from the seed's extrema; any later value is tighter and valid) meets the warp's box and one of its
-// points.  Extrema meet per block in shared memory, then in the zero-initialised encoded arrays; the last block decodes
-// them into the caller's floats.
+// ================================= pruned evaluation: the persistent-warp item loop =================================
+// The three *_tiles_kernel below run persistent WARPS over the work list.  The unit of work is one box of 128
+// consecutive points (one eighth of a listed tile), taken by ONE WARP from a global ticket counter: warps never wait for
+// each other (no block barrier, no static assignment), so neither the uneven cost of neighbouring boxes nor a heavy tile
+// at the end of the list leaves lanes idle.  A warp keeps two private stages in shared memory; its lane 0 draws the next
+// ticket and issues the TMA bulk copies for it (points, the box, the tile's pose mask, and in pass B the slice of the
+// permutation — one mbarrier per stage) before the warp starts on the current item.  The pose table stays in global
+// memory (a box touches ~5 rows: L1 hits).
 constexpr int kItemPts = 128;                 // points per work item = one warp's registers = one precomputed box
 constexpr int kItemsPerTile = 8;              // a listed tile (1024 points) is eight items
 constexpr int kItemPpt = kItemPts / 32;
-constexpr int kItemStageWordsA = kItemPts * 3 + 8 + kMaskWords;               // points | box | pose mask
-constexpr int kItemStageWords = kItemStageWordsA + kItemPts;                  // ... | permutation (pass B)
 
+// One work item as the loop body sees it: points [j0, j0 + 128) of the cloud.
+struct Item {
+    int64_t j0;
+    bool whole;             // j0 + 128 <= n: the points (and the permutation slice) were staged
+    const float* pts;       // the staged points, xyz interleaved
+    const float4* box;      // the item's bounding box (lo, hi); the sweep copies it to registers once per item, the
+                            // two passes read it from the stage at each pose: the faster choice for each kernel
+    const unsigned* mask;   // the tile's pose mask
+    const int32_t* perm;    // the staged slice of the permutation (WITH_PERM, whole, permutation given)
+};
+
+// Draws items until the work list is exhausted; `pre_wait(it)` runs after the next item was issued and before the wait
+// for the current one, `body(item)` once the current one has arrived.  Every lane of the warp calls it.
+template <bool WITH_PERM, typename PreWait, typename Body>
+__device__ __forceinline__ void for_each_item(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ boxes,
+                                              const unsigned* __restrict__ amask_g, int mask_stride,
+                                              const int32_t* __restrict__ perm, const int* __restrict__ worklist,
+                                              int n_items, int* ticket, PreWait pre_wait, Body body) {
+    constexpr int kStageWords = kItemPts * 3 + 8 + kMaskWords + (WITH_PERM ? kItemPts : 0);  // points|box|mask|perm
+    __shared__ __align__(128) float stages[kWarps][2][kStageWords];
+    __shared__ __align__(8) unsigned long long mbar[kWarps][2];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    unsigned long long* bar = mbar[warp];
+    if (lane == 0) {
+        mbar_init(&bar[0], 1);
+        mbar_init(&bar[1], 1);
+        mbar_fence_init();
+    }
+    __syncwarp();
+    // lane 0: stage item `it` (tile = worklist[it / 8], box k = it % 8); a ragged item's points are loaded by hand
+    auto issue = [&](int it, int b) {
+        if (it >= n_items) return;
+        const int64_t tile = worklist[it >> 3];
+        const int64_t j0 = tile * (kItemsPerTile * kItemPts) + (int64_t)(it & 7) * kItemPts;
+        float* st = stages[warp][b];
+        const bool whole = j0 + kItemPts <= n;
+        const bool with_perm = WITH_PERM && whole && perm != nullptr;
+        mbar_expect_tx(&bar[b], (whole ? kItemPts * 12u : 0u) + 32u + (unsigned)mask_stride * 4u + (with_perm ? kItemPts * 4u : 0u));
+        if (whole) tma_copy(st, xyz + j0 * 3, kItemPts * 12u, &bar[b]);
+        tma_copy(st + kItemPts * 3, boxes + (j0 / kBoxPts) * 2, 32u, &bar[b]);
+        tma_copy(st + kItemPts * 3 + 8, amask_g + tile * mask_stride, (unsigned)mask_stride * 4u, &bar[b]);
+        if (with_perm) tma_copy(st + kItemPts * 3 + 8 + kMaskWords, perm + j0, kItemPts * 4u, &bar[b]);
+    };
+    unsigned uses0 = 0, uses1 = 0;
+    int cur = 0;
+    if (lane == 0) {
+        cur = atomicAdd(ticket, 1);
+        issue(cur, 0);
+    }
+    cur = __shfl_sync(kFull, cur, 0);
+    int buf = 0;
+    while (cur < n_items) {
+        int nxt = 0;
+        if (lane == 0) {  // the other stage was last read before the __syncwarp that ended the previous item
+            nxt = atomicAdd(ticket, 1);
+            issue(nxt, buf ^ 1);
+        }
+        nxt = __shfl_sync(kFull, nxt, 0);
+        pre_wait(cur);
+        if (buf == 0) mbar_wait(&bar[0], uses0++ & 1u);
+        else mbar_wait(&bar[1], uses1++ & 1u);
+        const float* st = stages[warp][buf];
+        Item item;
+        item.j0 = (int64_t)worklist[cur >> 3] * (kItemsPerTile * kItemPts) + (int64_t)(cur & 7) * kItemPts;
+        item.whole = item.j0 + kItemPts <= n;
+        item.pts = st;
+        item.box = reinterpret_cast<const float4*>(st + kItemPts * 3);
+        item.mask = reinterpret_cast<const unsigned*>(st + kItemPts * 3 + 8);
+        item.perm = reinterpret_cast<const int32_t*>(st + kItemPts * 3 + 8 + kMaskWords);
+        body(item);
+        __syncwarp();  // every lane is done with this stage before lane 0 refills it
+        cur = nxt;
+        buf ^= 1;
+    }
+}
+
+// The item's points into registers, point s * 32 + lane in slot s: from the stage, or by hand at the ragged end of the
+// cloud, where the slots past the end get one of two fillers that are not interchangeable:
+//   CLAMP   point n - 1 again (pass A: a duplicate cannot change a min or a max; a sentinel would make the min 0)
+//   !CLAMP  a point 3e18 m away, valid = false (pass B, sweep: m = 0 exactly, never gated, never a tie; a duplicate
+//           would be counted twice)
+template <bool CLAMP>
+__device__ __forceinline__ void load_item_points(const Item& item, const float* __restrict__ xyz, int64_t n, int lane,
+                                                 float (&px)[kItemPpt], float (&py)[kItemPpt], float (&pz)[kItemPpt],
+                                                 bool (&valid)[kItemPpt]) {
+    if (item.whole) {
+#pragma unroll
+        for (int s = 0; s < kItemPpt; ++s) {
+            valid[s] = true;
+            px[s] = item.pts[(s * 32 + lane) * 3];
+            py[s] = item.pts[(s * 32 + lane) * 3 + 1];
+            pz[s] = item.pts[(s * 32 + lane) * 3 + 2];
+        }
+    } else {
+#pragma unroll
+        for (int s = 0; s < kItemPpt; ++s) {
+            const int64_t j = item.j0 + s * 32 + lane;
+            valid[s] = j < n;
+            if (CLAMP) {
+                const int64_t jc = valid[s] ? j : n - 1;
+                px[s] = __ldg(xyz + jc * 3);
+                py[s] = __ldg(xyz + jc * 3 + 1);
+                pz[s] = __ldg(xyz + jc * 3 + 2);
+            } else {
+                px[s] = valid[s] ? __ldg(xyz + j * 3) : 3.0e18f;
+                py[s] = valid[s] ? __ldg(xyz + j * 3 + 1) : 3.0e18f;
+                pz[s] = valid[s] ? __ldg(xyz + j * 3 + 2) : 3.0e18f;
+            }
+        }
+    }
+}
+
+// =============================================== pass A, pruned ===============================================
+// A listed pose is evaluated when the cap ball (from the seed's extrema; any later value is tighter and valid) meets
+// the warp's box and one of its points.  Extrema meet per block in shared memory, then in the zero-initialised encoded
+// arrays; the last block decodes them into the caller's floats.
 __global__ void __launch_bounds__(COV_THREADS, 3)
 cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, CovConst C,
                              unsigned* __restrict__ enc, float* __restrict__ minmax_out, const float4* __restrict__ boxes,
@@ -580,16 +659,8 @@ cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
     unsigned* smin = reinterpret_cast<unsigned*>(smem4);
     unsigned* smax = smin + W;
     float* sqcap = reinterpret_cast<float*>(smax + W);
-    __shared__ __align__(128) float stages[kWarps][2][kItemStageWordsA];
-    __shared__ __align__(8) unsigned long long mbar[kWarps][2];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const float inv_kd = 1.f / C.kd;
-    unsigned long long* bar = mbar[warp];
-    if (lane == 0) {
-        mbar_init(&bar[0], 1);
-        mbar_init(&bar[1], 1);
-        mbar_fence_init();
-    }
     for (int w = tid; w < W; w += COV_THREADS) {
         smin[w] = 0x7f800000u;
         smax[w] = 0u;
@@ -598,7 +669,6 @@ cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
     __syncthreads();
     const int n_items = ctrl[0] * kItemsPerTile;
     const int nwords = (W + 31) >> 5;
-    int* ticket = ctrl + 3;
     // Pre-fill of pass B's rewards with 1/2 under this kernel's idle memory bandwidth (cov_traj_opts.prefill_dev): the
     // warp that takes item i also writes slice i of the buffer (fire-and-forget streaming stores), in 16-byte units.
     const int64_t fill_q = (fill_n + 3) / 4;                                          // float4 slots (tail handled below)
@@ -615,100 +685,51 @@ cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
         const int64_t per = (fill_q + nw - 1) / nw;
         fill_slice(gw * per, (gw + 1) * per);
     }
-    auto issue = [&](int it, int b) {
-        if (it >= n_items) return;
-        const int64_t tile = worklist[it >> 3];
-        const int64_t j0 = tile * (kItemsPerTile * kItemPts) + (int64_t)(it & 7) * kItemPts;
-        float* st = stages[warp][b];
-        const bool whole = j0 + kItemPts <= n;
-        mbar_expect_tx(&bar[b], (whole ? kItemPts * 12u : 0u) + 32u + (unsigned)mask_stride * 4u);
-        if (whole) tma_copy(st, xyz + j0 * 3, kItemPts * 12u, &bar[b]);
-        tma_copy(st + kItemPts * 3, boxes + (j0 / kBoxPts) * 2, 32u, &bar[b]);
-        tma_copy(st + kItemPts * 3 + 8, amask_g + tile * mask_stride, (unsigned)mask_stride * 4u, &bar[b]);
-    };
     unsigned n_box = 0, n_pre = 0, n_full = 0;
-    unsigned uses0 = 0, uses1 = 0;
-    int cur = 0;
-    if (lane == 0) {
-        cur = atomicAdd(ticket, 1);
-        issue(cur, 0);
-    }
-    cur = __shfl_sync(kFull, cur, 0);
-    int buf = 0;
-    while (cur < n_items) {
-        int nxt = 0;
-        if (lane == 0) {  // the other stage was last read before the __syncwarp that ended the previous item
-            nxt = atomicAdd(ticket, 1);
-            issue(nxt, buf ^ 1);
-        }
-        nxt = __shfl_sync(kFull, nxt, 0);
-        if (fill_dst) fill_slice((int64_t)cur * fill_per_item, (int64_t)(cur + 1) * fill_per_item);
-        if (buf == 0) mbar_wait(&bar[0], uses0++ & 1u);
-        else mbar_wait(&bar[1], uses1++ & 1u);
-        const float* st = stages[warp][buf];
-        const int64_t tile = worklist[cur >> 3];
-        const int64_t j0 = tile * (kItemsPerTile * kItemPts) + (int64_t)(cur & 7) * kItemPts;
+    auto fill_item = [&](int it) {
+        if (fill_dst) fill_slice((int64_t)it * fill_per_item, (int64_t)(it + 1) * fill_per_item);
+    };
+    for_each_item<false>(xyz, n, boxes, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 3, fill_item,
+                         [&](const Item& item) {
         float px[PPT], py[PPT], pz[PPT];
-        if (j0 + kItemPts <= n) {
+        bool valid[PPT];
+        load_item_points<true>(item, xyz, n, lane, px, py, pz, valid);
+        if (item.j0 >= n) return;  // a listed tile's items past the end of the cloud
+        for (int c = 0; c < nwords; ++c) {
+            unsigned word = item.mask[c];
+            while (word) {
+                const int w = c * 32 + __ffs(word) - 1;
+                word &= word - 1;
+                const float4* row = table + (size_t)w * COV_ROW_F4;
+                const float4 v3 = __ldg(row + 3);
+                const float cap = sqcap[w];
+                ++n_box;
+                if (box_q2lb(item.box[0], item.box[1], v3) > cap) continue;
+                ++n_pre;
+                float qmin = cov_q2(px[0], py[0], pz[0], v3);
 #pragma unroll
-            for (int s = 0; s < PPT; ++s) {
-                px[s] = st[(s * 32 + lane) * 3];
-                py[s] = st[(s * 32 + lane) * 3 + 1];
-                pz[s] = st[(s * 32 + lane) * 3 + 2];
-            }
-        } else {
+                for (int s = 1; s < PPT; ++s) qmin = fminf(qmin, cov_q2(px[s], py[s], pz[s], v3));
+                if (!__any_sync(kFull, !(qmin > cap))) continue;
+                ++n_full;
+                const float4 v0 = __ldg(row), v1 = __ldg(row + 1), v2 = __ldg(row + 2);
+                float m[PPT];
 #pragma unroll
-            for (int s = 0; s < PPT; ++s) {
-                int64_t j = j0 + s * 32 + lane;
-                j = j < n ? j : n - 1;  // a duplicate cannot change a min or a max (j0 < n: the item holds a real point)
-                px[s] = __ldg(xyz + j * 3);
-                py[s] = __ldg(xyz + j * 3 + 1);
-                pz[s] = __ldg(xyz + j * 3 + 2);
-            }
-        }
-        const float4* tb = reinterpret_cast<const float4*>(st + kItemPts * 3);
-        const float4 wlo = tb[0], whi = tb[1];
-        const unsigned* am = reinterpret_cast<const unsigned*>(st + kItemPts * 3 + 8);
-        if (j0 < n) {
-            for (int c = 0; c < nwords; ++c) {
-                unsigned word = am[c];
-                while (word) {
-                    const int w = c * 32 + __ffs(word) - 1;
-                    word &= word - 1;
-                    const float4* row = table + (size_t)w * COV_ROW_F4;
-                    const float4 v3 = __ldg(row + 3);
-                    const float cap = sqcap[w];
-                    ++n_box;
-                    if (box_q2lb(wlo, whi, v3) > cap) continue;
-                    ++n_pre;
-                    float qmin = cov_q2(px[0], py[0], pz[0], v3);
+                for (int s = 0; s < PPT; ++s) m[s] = cov_vis<false>(px[s], py[s], pz[s], v0, v1, v2, v3, C, nullptr);
+                float mn = m[0], mx = m[0];
 #pragma unroll
-                    for (int s = 1; s < PPT; ++s) qmin = fminf(qmin, cov_q2(px[s], py[s], pz[s], v3));
-                    if (!__any_sync(kFull, !(qmin > cap))) continue;
-                    ++n_full;
-                    const float4 v0 = __ldg(row), v1 = __ldg(row + 1), v2 = __ldg(row + 2);
-                    float m[PPT];
-#pragma unroll
-                    for (int s = 0; s < PPT; ++s) m[s] = cov_vis<false>(px[s], py[s], pz[s], v0, v1, v2, v3, C, nullptr);
-                    float mn = m[0], mx = m[0];
-#pragma unroll
-                    for (int s = 1; s < PPT; ++s) {
-                        mn = fminf(mn, m[s]);
-                        mx = fmaxf(mx, m[s]);
-                    }
-                    const unsigned umn = __reduce_min_sync(kFull, __float_as_uint(mn));
-                    const unsigned umx = __reduce_max_sync(kFull, __float_as_uint(mx));
-                    if (lane == 0) {
-                        atomicMin(smin + w, umn);
-                        atomicMax(smax + w, umx);
-                    }
+                for (int s = 1; s < PPT; ++s) {
+                    mn = fminf(mn, m[s]);
+                    mx = fmaxf(mx, m[s]);
+                }
+                const unsigned umn = __reduce_min_sync(kFull, __float_as_uint(mn));
+                const unsigned umx = __reduce_max_sync(kFull, __float_as_uint(mx));
+                if (lane == 0) {
+                    atomicMin(smin + w, umn);
+                    atomicMax(smax + w, umx);
                 }
             }
         }
-        __syncwarp();  // every lane is done with this stage before lane 0 refills it
-        cur = nxt;
-        buf ^= 1;
-    }
+    });
     __syncthreads();
     for (int w = tid; w < W; w += COV_THREADS) {
         if (smax[w] != 0u || smin[w] != 0x7f800000u) {
@@ -794,9 +815,7 @@ __device__ __forceinline__ bool dense_pair_iter(int pair, int W, unsigned ptab_s
             bal[s] = __ballot_sync(kFull, act);
             any_h |= bal[s];
             if (act) {
-                const float p = __fmul_rn(d, v4.z);
-                const float qc = (p > C.hi) ? C.hi : p;  // upper clip; a NaN p (pose that sees nothing: 0/0) stays NaN, as torch.clip
-                L[s] += COV_LN2_F * cov_lg2(qc * cov_rcp(1.f - qc));
+                L[s] += cov_logodds(d, v4, C);
                 if (d == v4.y) {
                     float x, y, z, t;
                     f2_unpack(X[s], x, t); f2_unpack(Y[s], y, t); f2_unpack(Z[s], z, t);
@@ -851,9 +870,7 @@ __device__ __forceinline__ bool tiles_pose_iter(const float4* __restrict__ row, 
             const bool act = d >= v4.x;  // exactly p >= 0.5
             any |= act;
             if (act) {
-                const float p = __fmul_rn(d, v4.z);
-                const float qc = (p > C.hi) ? C.hi : p;  // upper clip; a NaN p (pose that sees nothing: 0/0) stays NaN, as torch.clip
-                L[s] += COV_LN2_F * cov_lg2(qc * cov_rcp(1.f - qc));
+                L[s] += cov_logodds(d, v4, C);
                 if (acc_row && d == v4.y) tie_accumulate_g(px[s], py[s], pz[s], row, C, acc_row + 8);
             }
         }
@@ -960,7 +977,7 @@ __device__ __forceinline__ void fused_block_flush(const T* accs, int W, double* 
 }
 
 // ---- dense ----
-template <int PPT, bool HAS_UP, int U>
+template <int PPT, bool HAS_UP>
 __global__ void __launch_bounds__(COV_THREADS, 2)
 cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __restrict__ poses,
                       const float* __restrict__ quats, int W, const float* __restrict__ K9, CovConst C,
@@ -988,10 +1005,7 @@ cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __r
         float4 row[COV_ROW_F4];
         cov_pose_row(poses + 3 * ws, quats + 4 * ws, K9, C, row);
         const float a = minmax[ws];
-        const float b = __fsub_rn(minmax[W + ws], a);
-        const float hb = 0.5f * b;
-        row[3].w = (a + hb) * (1.f - 9.5367431640625e-07f);  // conservative gate threshold (exact test in the rare path)
-        row[4] = make_float4(hb, b, __frcp_rn(b), a);
+        cov_norm_row(row, a, minmax[W + ws], row[3].w);  // conservative gate threshold (exact test in the rare path)
         cov_pair_store(ptab + (size_t)(w >> 1) * COV_PAIR_F4, w & 1, row);
         if (a > 0.f) amin_pos = 1;  // benign race: every writer stores 1
     }
@@ -1053,12 +1067,7 @@ cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __r
     fused_block_flush(accs, W, acc, sum_r, red, tid);
 }
 
-// ---- pruned: persistent WARPS over the work list of tiles with a non-empty pose mask ----
-// The unit of work is one box of 128 consecutive points (one eighth of a listed tile), taken by ONE WARP from a global
-// ticket counter: warps never wait for each other (no block barrier, no static assignment), so neither the uneven cost
-// of neighbouring boxes nor a heavy tile at the end of the list leaves lanes idle.  A warp keeps two private stages in
-// shared memory; its lane 0 draws the next ticket and issues the TMA bulk copies for it (points, the box, the tile's pose
-// mask, the slice of the permutation — one mbarrier per stage) before the warp starts on the current item.
+// ---- pruned: persistent warps over the work list (for_each_item), per 128-point item ----
 //   forward   walk the tile's pose mask; a listed pose is evaluated when its qthr-ball meets the warp's box; gated lanes
 //             add their log-odds; the warp notes (one bit per pose) whether it had a gated pair.  Then r_j,
 //             G_j = r_j (1 - r_j) per point; rewards stored.
@@ -1066,7 +1075,7 @@ cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __r
 //             sums in registers; a fixed 9-shuffle tree reduces them over the warp and one lane per component adds the
 //             result to the caller's fp64 accumulator row (fire-and-forget RED.F64).
 // On the bench cloud ~58 % of the point slots of an evaluated (warp, pose) are gated (profiles/r02_*), so the
-// re-evaluation keeps most lanes busy.  The pose table stays in global memory (a box touches ~5 rows: L1 hits).
+// re-evaluation keeps most lanes busy.
 // `rewards` was pre-filled with 1/2, only other values are stored; the warps add sum_j (r_j - 1/2) of the listed
 // tiles to acc[W * STRIDE], which starts at 0.5 * n.
 constexpr int kTilesMinBlocks = 3;            // resident blocks per SM the register allocation aims at
@@ -1080,93 +1089,25 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
                             const int* __restrict__ worklist, int* __restrict__ ctrl, int64_t ntiles,
                             unsigned long long* __restrict__ stats) {
     constexpr int PPT = kItemPpt;
-    __shared__ __align__(128) float stages[kWarps][2][kItemStageWords];
     __shared__ unsigned wgate[kWarps][kMaskWords];   // per warp: poses with a gated pair among its points (this item)
-    __shared__ __align__(8) unsigned long long mbar[kWarps][2];
-
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned long long* bar = mbar[warp];
-    if (lane == 0) {
-        mbar_init(&bar[0], 1);
-        mbar_init(&bar[1], 1);
-        mbar_fence_init();
-    }
-    __syncwarp();
     const bool check_amin = ctrl[1] != 0;  // some pose has min_j m > 0
     const int n_items = ctrl[0] * kItemsPerTile;
     const int nwords = (W + 31) >> 5;
-    unsigned* wg = wgate[warp];
-    int* ticket = ctrl + 3;
-
-    // lane 0: stage item `it` (tile = worklist[it / 8], box k = it % 8) unless it is past the end or ragged
-    auto issue = [&](int it, int b) {
-        if (it >= n_items) return;
-        const int64_t tile = worklist[it >> 3];
-        const int64_t j0 = tile * (kItemsPerTile * kItemPts) + (int64_t)(it & 7) * kItemPts;
-        float* st = stages[warp][b];
-        const bool whole = j0 + kItemPts <= n;
-        const bool with_perm = whole && out_index != nullptr;
-        mbar_expect_tx(&bar[b], (whole ? kItemPts * 12u : 0u) + 32u + (unsigned)mask_stride * 4u + (with_perm ? kItemPts * 4u : 0u));
-        if (whole) tma_copy(st, xyz + j0 * 3, kItemPts * 12u, &bar[b]);
-        tma_copy(st + kItemPts * 3, boxes + (j0 / kBoxPts) * 2, 32u, &bar[b]);
-        tma_copy(st + kItemPts * 3 + 8, amask_g + tile * mask_stride, (unsigned)mask_stride * 4u, &bar[b]);
-        if (with_perm) tma_copy(st + kItemPts * 3 + 8 + kMaskWords, out_index + j0, kItemPts * 4u, &bar[b]);
-    };
-
+    unsigned* wg = wgate[warp];  // lane 0 rewrites it for the next item only after the closing __syncwarp of this one
     double sum_r = 0.0;
     unsigned n_box = 0, n_full = 0, n_bwd = 0;
-    unsigned uses0 = 0, uses1 = 0;
-    int cur = 0;
-    if (lane == 0) {
-        cur = atomicAdd(ticket, 1);
-        issue(cur, 0);
-    }
-    cur = __shfl_sync(kFull, cur, 0);
-    int buf = 0;
-    while (cur < n_items) {
-        int nxt = 0;
-        if (lane == 0) {  // the other stage was last read before the __syncwarp that ended the previous item
-            nxt = atomicAdd(ticket, 1);
-            issue(nxt, buf ^ 1);
-        }
-        nxt = __shfl_sync(kFull, nxt, 0);
-        if (buf == 0) mbar_wait(&bar[0], uses0++ & 1u);
-        else mbar_wait(&bar[1], uses1++ & 1u);
-        const float* st = stages[warp][buf];
-        const int64_t tile = worklist[cur >> 3];
-        const int64_t j0 = tile * (kItemsPerTile * kItemPts) + (int64_t)(cur & 7) * kItemPts;
-        const bool whole = j0 + kItemPts <= n;
+    for_each_item<true>(xyz, n, boxes, amask_g, mask_stride, out_index, worklist, n_items, ctrl + 3, [](int) {},
+                        [&](const Item& item) {
         // ------------------------------ forward ------------------------------
         float px[PPT], py[PPT], pz[PPT], L[PPT];
         bool valid[PPT];
-        if (whole) {
+        load_item_points<false>(item, xyz, n, lane, px, py, pz, valid);
 #pragma unroll
-            for (int s = 0; s < PPT; ++s) {
-                valid[s] = true;
-                px[s] = st[(s * 32 + lane) * 3];
-                py[s] = st[(s * 32 + lane) * 3 + 1];
-                pz[s] = st[(s * 32 + lane) * 3 + 2];
-                L[s] = 0.f;
-            }
-        } else {  // the ragged end of the cloud: loaded by hand
-#pragma unroll
-            for (int s = 0; s < PPT; ++s) {
-                const int64_t j = j0 + s * 32 + lane;
-                valid[s] = j < n;
-                // a point past the end sits 3e18 m away: m = 0 exactly, never gated, never a tie
-                px[s] = valid[s] ? __ldg(xyz + j * 3) : 3.0e18f;
-                py[s] = valid[s] ? __ldg(xyz + j * 3 + 1) : 3.0e18f;
-                pz[s] = valid[s] ? __ldg(xyz + j * 3 + 2) : 3.0e18f;
-                L[s] = 0.f;
-            }
-        }
-        const float4* tb = reinterpret_cast<const float4*>(st + kItemPts * 3);
-        const float4 wlo = tb[0], whi = tb[1];
-        const unsigned* am = reinterpret_cast<const unsigned*>(st + kItemPts * 3 + 8);
-        const int32_t* sperm = reinterpret_cast<const int32_t*>(st + kItemPts * 3 + 8 + kMaskWords);
+        for (int s = 0; s < PPT; ++s) L[s] = 0.f;
         bool warp_gated = false;
         for (int c = 0; c < nwords; ++c) {
-            unsigned word = am[c];
+            unsigned word = item.mask[c];
             unsigned gbits = 0u;
             while (word) {
                 const int b = __ffs(word) - 1;
@@ -1177,7 +1118,7 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
                 ++n_box;
                 // the warp's own box against the pose's qthr-ball; no per-point pre-filter here: it rejected only 11 % of
                 // what the box test let through and cost a fifth of the evaluation it saved
-                if (box_q2lb(wlo, whi, v3) > v3.w) continue;
+                if (box_q2lb(item.box[0], item.box[1], v3) > v3.w) continue;
                 ++n_full;
                 double* acc_row = acc + (size_t)w * COV_ACC_STRIDE;
                 const bool g = check_amin ? tiles_pose_iter<PPT, true>(row, v3, px, py, pz, L, C, acc_row)
@@ -1197,12 +1138,12 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
                 G[s] = r * (1.f - r);
             }
             if (valid[s]) {
-                const int64_t j = j0 + s * 32 + lane;
+                const int64_t j = item.j0 + s * 32 + lane;
                 sum_r += (double)(r - 0.5f);
                 const bool store = r != 0.5f;
                 int64_t jo = j;
                 if (out_index && (store || HAS_UP))
-                    jo = whole ? (int64_t)sperm[s * 32 + lane] : (int64_t)out_index[j];  // staged with the item
+                    jo = item.whole ? (int64_t)item.perm[s * 32 + lane] : (int64_t)out_index[j];  // staged with the item
                 if (store) rewards[jo] = r;
                 if (HAS_UP) G[s] *= upstream[jo];
             }
@@ -1275,10 +1216,7 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
                 }
             }
         }
-        __syncwarp();  // every lane is done with this stage (and with wg) before lane 0 refills it
-        cur = nxt;
-        buf ^= 1;
-    }
+    });
     {
         const double ws = cov_warp_sum(sum_r);
         if (lane == 0 && ws != 0.0) atomicAdd(acc + (size_t)W * COV_ACC_STRIDE, ws);
@@ -1292,12 +1230,11 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
 }
 
 // ---- candidate sweep, pruned (BASELINE config 5): forward only, per-trajectory sum_j r_j ----
-// Persistent warps as in the two passes above (128-point items from a ticket counter, private double-buffered TMA
-// stages, pose table read through L1).  Poses are trajectory-major (pose = traj * per_traj + i), so walking a tile's pose
-// mask in ascending order visits the trajectories one after the other: a warp keeps the log-odds sums of its points for
-// the current trajectory, and when the trajectory changes it adds sum_j (sigmoid(L_j) - 1/2) to that trajectory's total
-// (fp64 shared atomic; the block adds its totals to the output at the end).  Trajectories no pose of which is listed for
-// an item contribute exactly 1/2 per point: 0.5 * n is added once.
+// Persistent warps as in the two passes above (for_each_item).  Poses are trajectory-major (pose = traj * per_traj + i),
+// so walking a tile's pose mask in ascending order visits the trajectories one after the other: a warp keeps the log-odds
+// sums of its points for the current trajectory, and when the trajectory changes it adds sum_j (sigmoid(L_j) - 1/2) to
+// that trajectory's total (fp64 shared atomic; the block adds its totals to the output at the end).  Trajectories no
+// pose of which is listed for an item contribute exactly 1/2 per point: 0.5 * n is added once.
 __global__ void __launch_bounds__(COV_THREADS, 3)
 cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, int per_traj,
                        int n_traj, CovConst C, const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g,
@@ -1306,74 +1243,17 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
     constexpr int PPT = kItemPpt;
     extern __shared__ float4 smem4[];
     double* ssum = reinterpret_cast<double*>(smem4);   // per-trajectory totals of this block
-    __shared__ __align__(128) float stages[kWarps][2][kItemStageWordsA];
-    __shared__ __align__(8) unsigned long long mbar[kWarps][2];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    unsigned long long* bar = mbar[warp];
-    if (lane == 0) {
-        mbar_init(&bar[0], 1);
-        mbar_init(&bar[1], 1);
-        mbar_fence_init();
-    }
+    const int tid = threadIdx.x, lane = tid & 31;
     for (int t = tid; t < n_traj; t += COV_THREADS) ssum[t] = 0.0;
     __syncthreads();
     const int n_items = ctrl[0] * kItemsPerTile;
     const int nwords = (W + 31) >> 5;
-    int* ticket = ctrl + 3;
-    auto issue = [&](int it, int b) {
-        if (it >= n_items) return;
-        const int64_t tile = worklist[it >> 3];
-        const int64_t j0 = tile * (kItemsPerTile * kItemPts) + (int64_t)(it & 7) * kItemPts;
-        float* st = stages[warp][b];
-        const bool whole = j0 + kItemPts <= n;
-        mbar_expect_tx(&bar[b], (whole ? kItemPts * 12u : 0u) + 32u + (unsigned)mask_stride * 4u);
-        if (whole) tma_copy(st, xyz + j0 * 3, kItemPts * 12u, &bar[b]);
-        tma_copy(st + kItemPts * 3, boxes + (j0 / kBoxPts) * 2, 32u, &bar[b]);
-        tma_copy(st + kItemPts * 3 + 8, amask_g + tile * mask_stride, (unsigned)mask_stride * 4u, &bar[b]);
-    };
-    unsigned uses0 = 0, uses1 = 0;
-    int cur_it = 0;
-    if (lane == 0) {
-        cur_it = atomicAdd(ticket, 1);
-        issue(cur_it, 0);
-    }
-    cur_it = __shfl_sync(kFull, cur_it, 0);
-    int buf = 0;
-    while (cur_it < n_items) {
-        int nxt = 0;
-        if (lane == 0) {
-            nxt = atomicAdd(ticket, 1);
-            issue(nxt, buf ^ 1);
-        }
-        nxt = __shfl_sync(kFull, nxt, 0);
-        if (buf == 0) mbar_wait(&bar[0], uses0++ & 1u);
-        else mbar_wait(&bar[1], uses1++ & 1u);
-        const float* st = stages[warp][buf];
-        const int64_t tile = worklist[cur_it >> 3];
-        const int64_t j0 = tile * (kItemsPerTile * kItemPts) + (int64_t)(cur_it & 7) * kItemPts;
+    for_each_item<false>(xyz, n, boxes, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 3, [](int) {},
+                         [&](const Item& item) {
         float px[PPT], py[PPT], pz[PPT], L[PPT];
         bool valid[PPT];
-        if (j0 + kItemPts <= n) {
-#pragma unroll
-            for (int s = 0; s < PPT; ++s) {
-                valid[s] = true;
-                px[s] = st[(s * 32 + lane) * 3];
-                py[s] = st[(s * 32 + lane) * 3 + 1];
-                pz[s] = st[(s * 32 + lane) * 3 + 2];
-            }
-        } else {
-#pragma unroll
-            for (int s = 0; s < PPT; ++s) {
-                const int64_t j = j0 + s * 32 + lane;
-                valid[s] = j < n;
-                px[s] = valid[s] ? __ldg(xyz + j * 3) : 3.0e18f;  // past the end: m = 0 exactly, never gated
-                py[s] = valid[s] ? __ldg(xyz + j * 3 + 1) : 3.0e18f;
-                pz[s] = valid[s] ? __ldg(xyz + j * 3 + 2) : 3.0e18f;
-            }
-        }
-        const float4* tb = reinterpret_cast<const float4*>(st + kItemPts * 3);
-        const float4 wlo = tb[0], whi = tb[1];
-        const unsigned* am = reinterpret_cast<const unsigned*>(st + kItemPts * 3 + 8);
+        load_item_points<false>(item, xyz, n, lane, px, py, pz, valid);
+        const float4 lo = item.box[0], hi = item.box[1];
         int cur = -1;      // trajectory whose log-odds sums are in L
         bool touched = false;
         auto flush = [&]() {
@@ -1387,13 +1267,13 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
             }
         };
         for (int c = 0; c < nwords; ++c) {
-            unsigned word = am[c];
+            unsigned word = item.mask[c];
             while (word) {
                 const int w = c * 32 + __ffs(word) - 1;
                 word &= word - 1;
                 const float4* row = table + (size_t)w * COV_ROW_F4;
                 const float4 v3 = __ldg(row + 3);
-                if (box_q2lb(wlo, whi, v3) > v3.w) continue;
+                if (box_q2lb(lo, hi, v3) > v3.w) continue;
                 const int t = w / per_traj;
                 if (t != cur) {
                     flush();
@@ -1406,10 +1286,7 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
             }
         }
         flush();
-        __syncwarp();  // every lane is done with this stage before lane 0 refills it
-        cur_it = nxt;
-        buf ^= 1;
-    }
+    });
     __syncthreads();
     for (int t = tid; t < n_traj; t += COV_THREADS) {
         double v = ssum[t];
@@ -1500,12 +1377,16 @@ int blocks_per_sm(Kern kern, int threads, size_t smem) {
     return per_sm;
 }
 
+// Grid of a persistent kernel: as many blocks as are resident at once, but no more than there are tiles.
 template <typename Kern>
-int grid_for(Kern kern, size_t smem, int64_t ntiles) {
-    int64_t g = (int64_t)blocks_per_sm(kern, COV_THREADS, smem) * cov_sm_count_cached();
-    if (g > ntiles) g = ntiles;
-    if (g > COV_MAX_GRID) g = COV_MAX_GRID;
-    return g < 1 ? 1 : (int)g;
+unsigned persistent_grid(Kern kern, size_t smem, int64_t ntiles) {
+    const int64_t g = (int64_t)blocks_per_sm(kern, COV_THREADS, smem) * cov_sm_count_cached();
+    return (unsigned)std::max<int64_t>(1, std::min<int64_t>(g, ntiles));
+}
+// the dense kernels: a block-stride loop over the tiles, at most COV_MAX_GRID blocks
+template <typename Kern>
+unsigned grid_for(Kern kern, size_t smem, int64_t ntiles) {
+    return std::min(persistent_grid(kern, smem, ntiles), (unsigned)COV_MAX_GRID);
 }
 
 // points per thread of the DENSE kernels: the largest tile that still gives every SM two tiles and fits shared memory
@@ -1591,12 +1472,16 @@ int check_traj_args(const char* who, const float* xyz, int64_t n, const float* p
     return COV_OK;
 }
 
+void launch_tile_boxes(const float* xyz, int64_t n, float4* boxes, cudaStream_t s) {
+    const int64_t nb = boxes_padded(n);
+    const int grid = (int)std::min<int64_t>((nb + 7) / 8, (int64_t)cov_sm_count_cached() * 16);
+    cov_tile_boxes_kernel<<<grid, 256, 0, s>>>(xyz, n, nb, boxes);
+}
+
 // boxes for this call: the caller's (cov_tile_boxes, once per cloud) or built into the workspace now
 const float4* boxes_for_call(const float* xyz, int64_t n, const float* boxes_dev, const TrajWorkspace& t, cudaStream_t s) {
     if (boxes_dev) return reinterpret_cast<const float4*>(boxes_dev);
-    const int64_t nb = boxes_padded(n);
-    const int grid = (int)std::min<int64_t>((nb + 7) / 8, (int64_t)cov_sm_count_cached() * 16);
-    cov_tile_boxes_kernel<<<grid, 256, 0, s>>>(xyz, n, nb, t.boxes);
+    launch_tile_boxes(xyz, n, t.boxes, s);
     return t.boxes;
 }
 
@@ -1656,9 +1541,7 @@ extern "C" int cov_tile_boxes(const float* xyz, int64_t n, float* boxes, void* s
         cov_set_error("cov_tile_boxes: boxes must be 16-byte aligned");
         return COV_ERR_ALIGN;
     }
-    const int64_t nb = boxes_padded(n);
-    const int grid = (int)std::min<int64_t>((nb + 7) / 8, (int64_t)cov_sm_count_cached() * 16);
-    cov_tile_boxes_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(xyz, n, nb, reinterpret_cast<float4*>(boxes));
+    launch_tile_boxes(xyz, n, reinterpret_cast<float4*>(boxes), (cudaStream_t)stream);
     return cov_check_launch("cov_tile_boxes");
 }
 
@@ -1716,14 +1599,10 @@ extern "C" int cov_traj_minmax(const float* xyz, int64_t n, const float* poses, 
         cov_traj_prepare_kernel<<<sgrid, COV_THREADS, 0, s>>>(xyz, nsamples, stride, poses, quats, W, K, C, t.table, t.enc);
     }
     if ((rc = launch_cull(boxes, ppt_t, ntiles_t, t, W, t.enc, 1.f / C.kd, nullptr, 0, s)) != COV_OK) return rc;
-    {
-        const size_t smem_t = (size_t)W * 12;
-        int64_t grid = (int64_t)blocks_per_sm(cov_traj_minmax_tiles_kernel, COV_THREADS, smem_t) * cov_sm_count_cached();
-        grid = std::max<int64_t>(1, std::min<int64_t>(grid, ntiles_t));
-        cov_traj_minmax_tiles_kernel<<<(unsigned)grid, COV_THREADS, smem_t, s>>>(
-            xyz, n, t.table, W, C, t.enc, minmax, boxes, t.amask, mask_stride_words(W), t.worklist, t.ctrl, ntiles_t,
-            opts ? opts->stats_dev : nullptr, opts ? opts->prefill_dev : nullptr, n);
-    }
+    const size_t smem_t = (size_t)W * 12;
+    cov_traj_minmax_tiles_kernel<<<persistent_grid(cov_traj_minmax_tiles_kernel, smem_t, ntiles_t), COV_THREADS, smem_t, s>>>(
+        xyz, n, t.table, W, C, t.enc, minmax, boxes, t.amask, mask_stride_words(W), t.worklist, t.ctrl, ntiles_t,
+        opts ? opts->stats_dev : nullptr, opts ? opts->prefill_dev : nullptr, n);
     return cov_check_launch("cov_traj_minmax");
 }
 
@@ -1759,9 +1638,9 @@ extern "C" int cov_traj_fused(const float* xyz, int64_t n, const float* poses, c
         while ((W << seg_log2) < 2 * COV_THREADS && (2 << seg_log2) <= bit_words(ppt_d) && seg_log2 < 5) ++seg_log2;
 #define LAUNCH_F(P, UP)                                                                                           \
     {                                                                                                             \
-        const int grid = grid_for(cov_traj_fused_kernel<P, UP, 1>, smem, ntiles);                                 \
-        cov_traj_fused_kernel<P, UP, 1><<<grid, COV_THREADS, smem, s>>>(xyz, n, poses, quats, W, K, C, minmax,    \
-                                                                        upstream, reward_index, rewards, acc, seg_log2); \
+        const int grid = grid_for(cov_traj_fused_kernel<P, UP>, smem, ntiles);                                    \
+        cov_traj_fused_kernel<P, UP><<<grid, COV_THREADS, smem, s>>>(xyz, n, poses, quats, W, K, C, minmax, upstream, \
+                                                                     reward_index, rewards, acc, seg_log2);        \
     }
         if (upstream) {
             if (ppt_d == 4) LAUNCH_F(4, true) else if (ppt_d == 2) LAUNCH_F(2, true) else LAUNCH_F(1, true)
@@ -1780,22 +1659,11 @@ extern "C" int cov_traj_fused(const float* xyz, int64_t n, const float* poses, c
                                                        (int)(t.ctrl_bytes / sizeof(int)), acc, 0.5 * (double)n);
     const bool prefilled = opts && opts->rewards_prefilled;
     if ((rc = launch_cull(boxes, ppt, ntiles, t, W, nullptr, 0.f, prefilled ? nullptr : rewards, n, s)) != COV_OK) return rc;
-    unsigned long long* stats = opts ? opts->stats_dev : nullptr;
-    {
-        // persistent warps: as many blocks as are resident; every warp draws 128-point items from a ticket counter
-        int64_t grid = 0;
-        if (upstream) grid = (int64_t)blocks_per_sm(cov_traj_fused_tiles_kernel<true>, COV_THREADS, 0) * cov_sm_count_cached();
-        else grid = (int64_t)blocks_per_sm(cov_traj_fused_tiles_kernel<false>, COV_THREADS, 0) * cov_sm_count_cached();
-        grid = std::max<int64_t>(1, std::min<int64_t>(grid, ntiles));
-        if (upstream)
-            cov_traj_fused_tiles_kernel<true><<<(unsigned)grid, COV_THREADS, 0, s>>>(
-                xyz, n, t.table, W, C, upstream, reward_index, rewards, acc, boxes, t.amask, mask_stride_words(W),
-                t.worklist, t.ctrl, ntiles, stats);
-        else
-            cov_traj_fused_tiles_kernel<false><<<(unsigned)grid, COV_THREADS, 0, s>>>(
-                xyz, n, t.table, W, C, upstream, reward_index, rewards, acc, boxes, t.amask, mask_stride_words(W),
-                t.worklist, t.ctrl, ntiles, stats);
-    }
+    // persistent warps: as many blocks as are resident; every warp draws 128-point items from a ticket counter
+    const auto tiles_kern = upstream ? cov_traj_fused_tiles_kernel<true> : cov_traj_fused_tiles_kernel<false>;
+    tiles_kern<<<persistent_grid(tiles_kern, 0, ntiles), COV_THREADS, 0, s>>>(
+        xyz, n, t.table, W, C, upstream, reward_index, rewards, acc, boxes, t.amask, mask_stride_words(W), t.worklist,
+        t.ctrl, ntiles, opts ? opts->stats_dev : nullptr);
     return cov_check_launch("cov_traj_fused");
 }
 
@@ -1840,11 +1708,8 @@ extern "C" int cov_sweep_rewards(const float* xyz, int64_t n, const float* poses
                                                             t.ctrl, (int)(t.ctrl_bytes / sizeof(int)), nullptr, 0.0);
         if (launch_cull(boxes, ppt, ntiles, t, Wn, nullptr, 0.f, nullptr, 0, s) != COV_OK) return COV_ERR_UNSUPPORTED;
         const size_t smem = (size_t)nt * sizeof(double);
-        int64_t grid = (int64_t)blocks_per_sm(cov_sweep_tiles_kernel, COV_THREADS, smem) * cov_sm_count_cached();
-        grid = std::max<int64_t>(1, std::min<int64_t>(grid, ntiles));
-        cov_sweep_tiles_kernel<<<(unsigned)grid, COV_THREADS, smem, s>>>(xyz, n, t.table, Wn, per_traj, nt, C, boxes, t.amask,
-                                                                        mask_stride_words(Wn), t.worklist, t.ctrl,
-                                                                        sum_rewards + t0);
+        cov_sweep_tiles_kernel<<<persistent_grid(cov_sweep_tiles_kernel, smem, ntiles), COV_THREADS, smem, s>>>(
+            xyz, n, t.table, Wn, per_traj, nt, C, boxes, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, sum_rewards + t0);
     }
     return cov_check_launch("cov_sweep_rewards");
 }
