@@ -152,6 +152,31 @@ int cov_sweep_rewards(const float* xyz_dev, int64_t n, const float* poses_dev, c
                       const float* minmax_dev, double* sum_rewards_dev, const cov_traj_opts* opts, void* workspace_dev,
                       size_t workspace_bytes, void* stream);
 
+/* Differentiable candidate sweep: for each of n_traj trajectories x poses_per_traj (= P) poses sharing one cloud, the
+ * accumulators cov_traj_fused computes for that trajectory alone (W = P, no upstream), in one pass over the cloud per
+ * chunk of cov_traj_max_poses_pruned() poses.
+ * ref: no reference implementation; semantics = ModelTraj.forward + backward of mean(rewards) per trajectory with every
+ * pose evaluated.  No per-point rewards are written.
+ *   acc_dev: n_traj blocks of COV_SWEEP_ACC_BLOCK(P) doubles; block t = P rows of COV_ACC_STRIDE doubles then sum_j r_j(t),
+ *   exactly what cov_traj_fused writes for trajectory t.  The call initialises every block itself.  Shard-additive: with
+ *   a sharded cloud, SUM the blocks over the ranks, then run cov_sweep_epilogue.
+ *   minmax_dev (2, n_traj*P): the global normalisers (cov_traj_minmax per chunk of poses, MIN/MAX over the ranks).
+ *   opts: dense (or n < 65536) runs the dense cov_traj_fused once per trajectory (P <= cov_traj_max_poses()); the pruned
+ *   path takes P <= cov_traj_max_poses_pruned().  stats_dev: on the pruned path the evaluation kernel adds the pass B
+ *   counters [0], [1], [4], [6]; the dense path adds nothing (its kernels count no work).
+ *   workspace_dev: cov_sweep_fused_workspace_bytes(n, n_traj, P, opts) bytes for the same n, P and opts, 256-byte aligned
+ *   (the dense path's size includes n floats of reward scratch; the pruned path's does not). */
+#define COV_SWEEP_ACC_BLOCK(P) ((size_t)(P) * COV_ACC_STRIDE + 1)
+size_t cov_sweep_fused_workspace_bytes(int64_t n, int n_traj, int poses_per_traj, const cov_traj_opts* opts);
+int cov_sweep_fused(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev, int n_traj,
+                    int poses_per_traj, const float* K_dev, const cov_camera* cam, const float* boxes_dev,
+                    const float* minmax_dev, double* acc_dev, const cov_traj_opts* opts, void* workspace_dev,
+                    size_t workspace_bytes, void* stream);
+/* out_dev (fp32): [n_traj means | n_traj*P*3 d mean_t/d poses | n_traj*P*4 d mean_t/d quats]; trajectory t's part is
+ * what cov_traj_epilogue (upstream_mode 0) gives for block t with minmax [min_t | max_t] and quats_t, bit for bit. */
+int cov_sweep_epilogue(const double* acc_dev, const float* minmax_dev, const float* quats_dev, int n_traj,
+                       int poses_per_traj, int64_t n_total, float* out_dev, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * The two exchange steps of the point-sharded objective (MAX of the 2 W normalisers, SUM of the 22 W + 1 accumulator
  * doubles) as ONE small kernel each over NVLink peer memory, in place of a collective-library launch.

@@ -60,6 +60,9 @@ PROTOTYPES = {
     "cov_traj_regularizers": (_int, [_vp, _vp, _int, _f, _f, _f, _vp, _vp]),
     "cov_sweep_workspace_bytes": (_sz, [_i64, _int, _int]),
     "cov_sweep_rewards": (_int, [_vp, _i64, _vp, _vp, _int, _int, _vp, _cam, _vp, _vp, _vp, _opts, _vp, _sz, _vp]),
+    "cov_sweep_fused_workspace_bytes": (_sz, [_i64, _int, _int, _opts]),
+    "cov_sweep_fused": (_int, [_vp, _i64, _vp, _vp, _int, _int, _vp, _cam, _vp, _vp, _vp, _opts, _vp, _sz, _vp]),
+    "cov_sweep_epilogue": (_int, [_vp, _vp, _vp, _int, _int, _i64, _vp, _vp]),
     "cov_peer_region_bytes": (_sz, [_int, _i64, _int]),
     "cov_peer_allreduce": (_int, [_int, _vp, _i64, C.POINTER(Peers), _sz, _vp]),
     "cov_rig_poses": (_int, [_vp, _int, _vp, _int, _vp, _vp, _vp]),

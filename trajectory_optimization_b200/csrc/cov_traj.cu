@@ -41,6 +41,11 @@
 //                        the poses it gated and recomputes m and dm/dx for its own points, with every lane busy.
 //   Tiles that are not listed are never read: their rewards are the pre-filled 1/2 (exact), their sum is 0.5 * count.
 //
+// CANDIDATE SWEEPS (many trajectories, one cloud; pose tables of up to 2048 trajectory-major poses per launch):
+//   cov_sweep_tiles_kernel        forward only: per-trajectory sum_j r_j
+//   cov_sweep_fused_tiles_kernel  per trajectory, pass B's accumulators (its forward and its backward, shared with the
+//                                 pass B kernel through tiles_pose_iter and tiles_pose_backward)
+//
 // Block accumulators are added to the caller's fp64 accumulator rows with fp64 atomics (the order of those additions is
 // the only thing that differs between runs: ~1e-16 relative).  The arg-max / arg-min tie sets of the normalisation
 // backward are rare (one point per pose unless the minimum underflowed to 0, in which case their gradient is exactly
@@ -887,6 +892,71 @@ __device__ __forceinline__ bool tiles_pose_iter(const float4* __restrict__ row, 
     return any;
 }
 
+// Backward of one gated pose for a warp of the pruned kernels (pass B, the differentiable sweep): m again for the warp's
+// points (bit-identical to the forward), the gate, dm/dx, the 8 weighted sums in registers; a fixed 9-shuffle tree reduces
+// them over the warp and one lane per component adds the result to the pose's fp64 accumulator row (fire-and-forget
+// RED.F64).  G = the points' dr/dL (times the upstream gradient, if any).
+template <int PPT>
+__device__ __forceinline__ void tiles_pose_backward(const float4* __restrict__ row, const float (&px)[PPT],
+                                                    const float (&py)[PPT], const float (&pz)[PPT], const float (&G)[PPT],
+                                                    const CovConst& C, double* __restrict__ acc_row, int lane) {
+    const float4 v0 = __ldg(row), v1 = __ldg(row + 1), v2 = __ldg(row + 2), v3 = __ldg(row + 3), v4 = __ldg(row + 4),
+                 v5 = __ldg(row + 5);
+    float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+    for (int s = 0; s < PPT; ++s) {
+        CovEval ev;
+        const float m = cov_vis<true>(px[s], py[s], pz[s], v0, v1, v2, v3, C, &ev);
+        const float d = __fsub_rn(m, v4.w);
+        if (d >= v4.x) {  // exactly p >= 0.5, as in the forward
+            const float p = __fdiv_rn(d, v4.y);
+            if (p <= C.hi) {  // clamp backward gate (inclusive)
+                float gx, gy, gz;
+                cov_vis_grad(m, ev, v0, v1, v2, C, gx, gy, gz);
+                const float yx = px[s] - v5.x, yy = py[s] - v5.y, yz = pz[s] - v5.z;
+                const float e = G[s] * cov_rcp(p * (1.f - p));
+                const float om = e * v4.z;
+                v[0] += om * gx; v[1] += om * gy; v[2] += om * gz;
+                v[3] += om * (gy * yz - gz * yy);
+                v[4] += om * (gz * yx - gx * yz);
+                v[5] += om * (gx * yy - gy * yx);
+                v[6] += e;
+                v[7] += e * p;
+            }
+        }
+    }
+    // 8 sums over 32 lanes in 9 shuffles: halve the number of values a lane carries at offsets 16, 8, 4 (a lane keeps the
+    // half its lane bit selects and hands the other half over), then two plain steps; lanes with (lane & 3) == 0 end with
+    // component (lane bits 4,3,2)
+    {
+        const bool up = (lane & 16) != 0;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const float keep = up ? v[q + 4] : v[q], send = up ? v[q] : v[q + 4];
+            v[q] = keep + __shfl_xor_sync(kFull, send, 16);
+        }
+    }
+    {
+        const bool up = (lane & 8) != 0;
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+            const float keep = up ? v[q + 2] : v[q], send = up ? v[q] : v[q + 2];
+            v[q] = keep + __shfl_xor_sync(kFull, send, 8);
+        }
+    }
+    {
+        const bool up = (lane & 4) != 0;
+        const float keep = up ? v[1] : v[0], send = up ? v[0] : v[1];
+        v[0] = keep + __shfl_xor_sync(kFull, send, 4);
+    }
+    v[0] += __shfl_xor_sync(kFull, v[0], 2);
+    v[0] += __shfl_xor_sync(kFull, v[0], 1);
+    if ((lane & 3) == 0 && v[0] != 0.f) {  // one fire-and-forget fp64 RED per component
+        const int comp = ((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1);
+        atomicAdd(acc_row + comp, (double)v[0]);
+    }
+}
+
 // Phase 2 of the dense kernel: the gated pairs of all W bit rows, each row split over 2^seg_log2 lanes.  A lane pops
 // its set bits in ascending point order, recomputes m (bit-identical) and dm/dx, and accumulates in registers;
 // segments are combined with xor-shuffles; one owner lane adds into accs.
@@ -1157,62 +1227,8 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
                     const int w = c * 32 + __ffs(word) - 1;
                     word &= word - 1;
                     ++n_bwd;
-                    const float4* row = table + (size_t)w * COV_ROW_F4;
-                    const float4 v0 = __ldg(row), v1 = __ldg(row + 1), v2 = __ldg(row + 2), v3 = __ldg(row + 3),
-                                 v4 = __ldg(row + 4), v5 = __ldg(row + 5);
-                    float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-                    for (int s = 0; s < PPT; ++s) {
-                        CovEval ev;
-                        const float m = cov_vis<true>(px[s], py[s], pz[s], v0, v1, v2, v3, C, &ev);
-                        const float d = __fsub_rn(m, v4.w);
-                        if (d >= v4.x) {  // exactly p >= 0.5, as in the forward
-                            const float p = __fdiv_rn(d, v4.y);
-                            if (p <= C.hi) {  // clamp backward gate (inclusive)
-                                float gx, gy, gz;
-                                cov_vis_grad(m, ev, v0, v1, v2, C, gx, gy, gz);
-                                const float yx = px[s] - v5.x, yy = py[s] - v5.y, yz = pz[s] - v5.z;
-                                const float e = G[s] * cov_rcp(p * (1.f - p));
-                                const float om = e * v4.z;
-                                v[0] += om * gx; v[1] += om * gy; v[2] += om * gz;
-                                v[3] += om * (gy * yz - gz * yy);
-                                v[4] += om * (gz * yx - gx * yz);
-                                v[5] += om * (gx * yy - gy * yx);
-                                v[6] += e;
-                                v[7] += e * p;
-                            }
-                        }
-                    }
-                    // 8 sums over 32 lanes in 9 shuffles: halve the number of values a lane carries at offsets 16, 8, 4
-                    // (a lane keeps the half its lane bit selects and hands the other half over), then two plain steps;
-                    // lanes with (lane & 3) == 0 end with component (lane bits 4,3,2)
-                    {
-                        const bool up = (lane & 16) != 0;
-#pragma unroll
-                        for (int q = 0; q < 4; ++q) {
-                            const float keep = up ? v[q + 4] : v[q], send = up ? v[q] : v[q + 4];
-                            v[q] = keep + __shfl_xor_sync(kFull, send, 16);
-                        }
-                    }
-                    {
-                        const bool up = (lane & 8) != 0;
-#pragma unroll
-                        for (int q = 0; q < 2; ++q) {
-                            const float keep = up ? v[q + 2] : v[q], send = up ? v[q] : v[q + 2];
-                            v[q] = keep + __shfl_xor_sync(kFull, send, 8);
-                        }
-                    }
-                    {
-                        const bool up = (lane & 4) != 0;
-                        const float keep = up ? v[1] : v[0], send = up ? v[0] : v[1];
-                        v[0] = keep + __shfl_xor_sync(kFull, send, 4);
-                    }
-                    v[0] += __shfl_xor_sync(kFull, v[0], 2);
-                    v[0] += __shfl_xor_sync(kFull, v[0], 1);
-                    if ((lane & 3) == 0 && v[0] != 0.f) {  // one fire-and-forget fp64 RED per component
-                        const int comp = ((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1);
-                        atomicAdd(acc + (size_t)w * COV_ACC_STRIDE + comp, (double)v[0]);
-                    }
+                    tiles_pose_backward<PPT>(table + (size_t)w * COV_ROW_F4, px, py, pz, G, C,
+                                             acc + (size_t)w * COV_ACC_STRIDE, lane);
                 }
             }
         }
@@ -1295,16 +1311,123 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
     }
 }
 
-// SURVEY.md App. A.2: fold the min/max-path terms in and map (F, T) to (d/dt, d/dq~).
-__global__ void cov_traj_epilogue_kernel(const double* __restrict__ acc, const float* __restrict__ minmax,
-                                         const float* __restrict__ quats, int W, double n_total, int upstream_mode,
-                                         float* __restrict__ out) {
-    const int w = blockIdx.x * blockDim.x + threadIdx.x;
-    if (w == 0) out[0] = (float)(acc[(size_t)W * COV_ACC_STRIDE] / n_total);
-    if (w >= W) return;
-    const double* A = acc + (size_t)w * COV_ACC_STRIDE;
-    const float a = minmax[w];
-    const double b = (double)__fsub_rn(minmax[W + w], a);
+// ---- differentiable candidate sweep, pruned: per trajectory what pass B computes for it alone ----
+// The walk of cov_sweep_tiles_kernel (trajectory-major poses, one trajectory's log-odds sums in L at a time) with pass B's
+// bookkeeping: while it walks the poses of the current trajectory, lane 0 notes in the warp's shared mask which of them had
+// a gated pair.  At each trajectory boundary and at the end of the item the warp computes r_j and G_j = dr/dL with pass B's
+// expressions, adds sum_j (r_j - 1/2) to the trajectory's reward sum and runs pass B's backward (tiles_pose_backward) over
+// the noted poses, then clears the notes.  Pose w of trajectory t owns row (w - t P) of block t of the accumulators,
+// `acc + t * COV_SWEEP_ACC_BLOCK(P)`: the layout cov_traj_fused writes for that trajectory alone (rows, then sum_j r_j).
+// The forward of a trajectory visits the same poses in the same order as pass B with W = P on the same item (same cull,
+// same box test), so its L, r_j and G_j — and the re-evaluated m of the backward — are bit-identical to pass B's.
+__global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
+cov_sweep_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, int per_traj,
+                             CovConst C, const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g,
+                             int mask_stride, const int* __restrict__ worklist, int* __restrict__ ctrl, int64_t ntiles,
+                             double* __restrict__ acc, unsigned long long* __restrict__ stats) {
+    constexpr int PPT = kItemPpt;
+    __shared__ unsigned wgate[kWarps][kMaskWords];   // per warp: poses of the current trajectory with a gated pair
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const bool check_amin = ctrl[1] != 0;  // some pose has min_j m > 0
+    const int n_items = ctrl[0] * kItemsPerTile;
+    const int nwords = (W + 31) >> 5;
+    const size_t block = COV_SWEEP_ACC_BLOCK(per_traj);
+    unsigned* wg = wgate[warp];
+    for (int c = lane; c < kMaskWords; c += 32) wg[c] = 0u;  // afterwards every flush clears the words it walked
+    __syncwarp();
+    unsigned n_box = 0, n_full = 0, n_bwd = 0;
+    for_each_item<false>(xyz, n, boxes, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 3, [](int) {},
+                         [&](const Item& item) {
+        float px[PPT], py[PPT], pz[PPT], L[PPT];
+        bool valid[PPT];
+        load_item_points<false>(item, xyz, n, lane, px, py, pz, valid);
+        int cur = -1;          // trajectory whose log-odds sums are in L
+        bool gated = false;    // warp-uniform: some pose of `cur` had a gated pair (otherwise r_j = 1/2, nothing to add)
+        auto flush = [&]() {
+            if (cur < 0 || !gated) return;
+            double* A = acc + (size_t)cur * block;
+            float G[PPT];
+            float a = 0.f;
+#pragma unroll
+            for (int s = 0; s < PPT; ++s) {
+                float r = 0.5f;
+                G[s] = 0.25f;  // exactly what the formulas below give for L = 0
+                if (L[s] != 0.f) {
+                    r = 1.f / (1.f + expf(-L[s]));
+                    G[s] = r * (1.f - r);
+                }
+                if (valid[s]) a += r - 0.5f;
+            }
+            a = cov_warp_sum(a);
+            if (lane == 0 && a != 0.f) atomicAdd(A + (size_t)per_traj * COV_ACC_STRIDE, (double)a);
+            __syncwarp();  // lane 0's notes are visible to the warp
+            const int p0 = cur * per_traj;
+            const int c1 = (p0 + per_traj - 1) >> 5;
+            for (int c = p0 >> 5; c <= c1; ++c) {  // only this trajectory's poses are noted
+                unsigned word = wg[c];
+                while (word) {
+                    const int w = c * 32 + __ffs(word) - 1;
+                    word &= word - 1;
+                    ++n_bwd;
+                    tiles_pose_backward<PPT>(table + (size_t)w * COV_ROW_F4, px, py, pz, G, C,
+                                             A + (size_t)(w - p0) * COV_ACC_STRIDE, lane);
+                }
+            }
+            __syncwarp();  // every lane has read the notes
+            if (lane == 0)
+                for (int c = p0 >> 5; c <= c1; ++c) wg[c] = 0u;
+        };
+        for (int c = 0; c < nwords; ++c) {
+            unsigned word = item.mask[c];
+            while (word) {
+                const int b = __ffs(word) - 1;
+                const int w = c * 32 + b;
+                word &= word - 1;
+                const float4* row = table + (size_t)w * COV_ROW_F4;
+                const float4 v3 = __ldg(row + 3);
+                ++n_box;
+                if (box_q2lb(item.box[0], item.box[1], v3) > v3.w) continue;
+                ++n_full;
+                const int t = w / per_traj;
+                if (t != cur) {
+                    flush();
+                    cur = t;
+                    gated = false;
+#pragma unroll
+                    for (int s = 0; s < PPT; ++s) L[s] = 0.f;
+                }
+                double* acc_row = acc + (size_t)t * block + (size_t)(w - t * per_traj) * COV_ACC_STRIDE;
+                const bool g = check_amin ? tiles_pose_iter<PPT, true>(row, v3, px, py, pz, L, C, acc_row)
+                                          : tiles_pose_iter<PPT, false>(row, v3, px, py, pz, L, C, acc_row);
+                if (g) {
+                    gated = true;
+                    if (lane == 0) wg[c] |= 1u << b;
+                }
+            }
+        }
+        flush();
+    });
+    if (stats && lane == 0) {
+        if (threadIdx.x == 0 && blockIdx.x == 0) atomicAdd(stats + 0, (unsigned long long)ntiles * kWarps * W);
+        atomicAdd(stats + 1, (unsigned long long)n_full);
+        atomicAdd(stats + 4, (unsigned long long)n_bwd);
+        atomicAdd(stats + 6, (unsigned long long)n_box);
+    }
+}
+
+// Every trajectory's accumulator block as pass B starts it: rows zero, the reward sum at `sum_base` (0.5 * n: what the
+// points no listed pose reaches add).
+__global__ void cov_sweep_acc_init_kernel(double* __restrict__ acc, int64_t count, int64_t block, double sum_base) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (int64_t)gridDim.x * blockDim.x)
+        acc[i] = (i % block == block - 1) ? sum_base : 0.0;
+}
+
+// SURVEY.md App. A.2, one pose: fold the min/max-path terms into the accumulator row A and map (F, T) to (d/dt, d/dq~).
+// a, mx: the pose's normalisers; q: its raw quaternion; c0: the scale of the gradient (1/N for the mean).
+__device__ __forceinline__ void traj_epilogue_pose(const double* __restrict__ A, float a, float mx,
+                                                   const float* __restrict__ q, double c0, float* __restrict__ gp,
+                                                   float* __restrict__ gq) {
+    const double b = (double)__fsub_rn(mx, a);
     const double dLdb = -A[7] / b;
     const double dLda = -A[6] / b - dLdb;
     double F[3] = {A[0], A[1], A[2]}, Tq[3] = {A[3], A[4], A[5]};
@@ -1316,19 +1439,42 @@ __global__ void cov_traj_epilogue_kernel(const double* __restrict__ acc, const f
         const double c = dLda / A[21];
         for (int k = 0; k < 3; ++k) { F[k] += c * A[15 + k]; Tq[k] += c * A[18 + k]; }
     }
-    const double c0 = upstream_mode ? 1.0 : 1.0 / n_total;
-    double qw = quats[4 * w], qx = quats[4 * w + 1], qy = quats[4 * w + 2], qz = quats[4 * w + 3];
+    double qw = q[0], qx = q[1], qy = q[2], qz = q[3];
     double qn = sqrt(qw * qw + qx * qx + qy * qy + qz * qz);
     qn = qn > 1e-12 ? qn : 1e-12;
     qw /= qn; qx /= qn; qy /= qn; qz /= qn;
-    float* gp = out + 1 + 3 * w;
-    float* gq = out + 1 + 3 * W + 4 * w;
     for (int k = 0; k < 3; ++k) gp[k] = (float)(-c0 * F[k]);
     const double s = 2.0 * c0 / qn;
     gq[0] = (float)(s * (-Tq[0] * qx - Tq[1] * qy - Tq[2] * qz));
     gq[1] = (float)(s * (Tq[0] * qw + Tq[1] * qz - Tq[2] * qy));
     gq[2] = (float)(s * (Tq[1] * qw - Tq[0] * qz + Tq[2] * qx));
     gq[3] = (float)(s * (Tq[2] * qw + Tq[0] * qy - Tq[1] * qx));
+}
+
+__global__ void cov_traj_epilogue_kernel(const double* __restrict__ acc, const float* __restrict__ minmax,
+                                         const float* __restrict__ quats, int W, double n_total, int upstream_mode,
+                                         float* __restrict__ out) {
+    const int w = blockIdx.x * blockDim.x + threadIdx.x;
+    if (w == 0) out[0] = (float)(acc[(size_t)W * COV_ACC_STRIDE] / n_total);
+    if (w >= W) return;
+    const double c0 = upstream_mode ? 1.0 : 1.0 / n_total;
+    traj_epilogue_pose(acc + (size_t)w * COV_ACC_STRIDE, minmax[w], minmax[W + w], quats + 4 * w, c0, out + 1 + 3 * w,
+                       out + 1 + 3 * W + 4 * w);
+}
+
+// The sweep's epilogue: trajectory t's mean and the gradient of that mean, from block t of the accumulators.
+// minmax (2, T P): all minima, then all maxima.  out = [T means | T P (d/dt) | T P (d/dq~)].
+__global__ void cov_sweep_epilogue_kernel(const double* __restrict__ acc, const float* __restrict__ minmax,
+                                          const float* __restrict__ quats, int n_traj, int per_traj, double n_total,
+                                          float* __restrict__ out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;  // pose t * P + k
+    const int TP = n_traj * per_traj;
+    const size_t block = COV_SWEEP_ACC_BLOCK(per_traj);
+    if (i < n_traj) out[i] = (float)(acc[(size_t)i * block + (size_t)per_traj * COV_ACC_STRIDE] / n_total);
+    if (i >= TP) return;
+    const int t = i / per_traj, k = i - t * per_traj;
+    traj_epilogue_pose(acc + (size_t)t * block + (size_t)k * COV_ACC_STRIDE, minmax[i], minmax[TP + i], quats + 4 * (size_t)i,
+                       1.0 / n_total, out + n_traj + 3 * (size_t)i, out + n_traj + 3 * (size_t)TP + 4 * (size_t)i);
 }
 
 // ==================================================== host ====================================================
@@ -1720,6 +1866,117 @@ extern "C" size_t cov_sweep_workspace_bytes(int64_t n, int n_traj, int per_traj)
     if (W > 32 * kMaskWords) W = 32 * kMaskWords;
     if (W < 1) W = 1;
     return cov_traj_workspace_bytes(n, W) + align256(2 * (size_t)W * sizeof(float));
+}
+
+// The dense path of cov_sweep_fused: [cov_traj_fused workspace for P poses][n rewards (scratch)][2 P normalisers]
+static size_t sweep_fused_dense_bytes(int64_t n, int per_traj) {
+    return cov_traj_workspace_bytes(n, per_traj) + align256((size_t)n * sizeof(float)) +
+           align256(2 * (size_t)per_traj * sizeof(float));
+}
+
+// the path a cov_sweep_fused call with these options takes on n points
+static bool sweep_fused_prunes(int64_t n, const cov_traj_opts* opts) { return !(opts && opts->dense) && n >= kDenseBelow; }
+
+extern "C" size_t cov_sweep_fused_workspace_bytes(int64_t n, int n_traj, int per_traj, const cov_traj_opts* opts) {
+    if (n < 1) n = 1;
+    if (n_traj < 1) n_traj = 1;
+    per_traj = std::min(std::max(per_traj, 1), 32 * kMaskWords);
+    return sweep_fused_prunes(n, opts) ? cov_sweep_workspace_bytes(n, n_traj, per_traj) : sweep_fused_dense_bytes(n, per_traj);
+}
+
+extern "C" int cov_sweep_fused(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
+                               int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
+                               const float* minmax, double* acc, const cov_traj_opts* opts, void* ws, size_t ws_bytes,
+                               void* stream) {
+    if (!xyz || n <= 0 || !poses || !quats || n_traj <= 0 || per_traj <= 0 || !K || !cam || !minmax || !acc || !ws) {
+        cov_set_error("cov_sweep_fused: null pointer, empty cloud or no poses (n=%lld, n_traj=%d, poses_per_traj=%d)",
+                      (long long)n, n_traj, per_traj);
+        return COV_ERR_ARG;
+    }
+    const bool prune = sweep_fused_prunes(n, opts);
+    const int max_p = prune ? cov_traj_max_poses_pruned() : cov_traj_max_poses();
+    if (per_traj > max_p) {
+        cov_set_error("cov_sweep_fused: %d poses per trajectory exceed what one call takes on this path (max %d)", per_traj,
+                      max_p);
+        return COV_ERR_UNSUPPORTED;
+    }
+    if ((int64_t)n_traj * per_traj > INT32_MAX / 8 || n >= ((int64_t)1 << 31) * 256) {
+        cov_set_error("cov_sweep_fused: %d x %d poses or %lld points exceed the index range", n_traj, per_traj, (long long)n);
+        return COV_ERR_UNSUPPORTED;
+    }
+    const size_t need = cov_sweep_fused_workspace_bytes(n, n_traj, per_traj, opts);
+    if (ws_bytes < need) {
+        cov_set_error("cov_sweep_fused: workspace %zu < cov_sweep_fused_workspace_bytes(n, %d, %d, opts) = %zu", ws_bytes,
+                      n_traj, per_traj, need);
+        return COV_ERR_WORKSPACE;
+    }
+    if ((((uintptr_t)ws) & 255) || (((uintptr_t)xyz) & 15) || (boxes_dev && (((uintptr_t)boxes_dev) & 15))) {
+        cov_set_error("cov_sweep_fused: workspace must be 256-byte aligned, the cloud and boxes 16-byte aligned");
+        return COV_ERR_ALIGN;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t block = COV_SWEEP_ACC_BLOCK(per_traj);
+    const int TP = n_traj * per_traj;
+    if (!prune) {  // the reference path: the dense cov_traj_fused once per trajectory, into that trajectory's block
+                   // (the dense kernels count no work: stats_dev is left as it is)
+        const size_t tws = cov_traj_workspace_bytes(n, per_traj);
+        float* rewards = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + tws);
+        float* mm = reinterpret_cast<float*>(reinterpret_cast<char*>(rewards) + align256((size_t)n * sizeof(float)));
+        cov_traj_opts dense{};
+        dense.dense = 1;
+        for (int t = 0; t < n_traj; ++t) {
+            const size_t w0 = (size_t)t * per_traj;
+            cudaMemcpyAsync(mm, minmax + w0, (size_t)per_traj * sizeof(float), cudaMemcpyDeviceToDevice, s);
+            cudaMemcpyAsync(mm + per_traj, minmax + TP + w0, (size_t)per_traj * sizeof(float), cudaMemcpyDeviceToDevice, s);
+            const int rc = cov_traj_fused(xyz, n, poses + 3 * w0, quats + 4 * w0, per_traj, K, cam, nullptr, mm, nullptr,
+                                          nullptr, rewards, acc + (size_t)t * block, &dense, ws, tws, stream);
+            if (rc) return rc;
+        }
+        return COV_OK;
+    }
+    // pruned: the chunking of cov_sweep_rewards (as many trajectories per launch as the tile pose mask holds); per chunk
+    // pose table, cull + work list, evaluation of the listed tiles
+    const int chunk = std::min((32 * kMaskWords) / per_traj, n_traj);
+    const CovConst C = cov_make_const(cam);
+    const TrajWorkspace t = carve_workspace(ws, n, chunk * per_traj);
+    const float4* boxes = boxes_for_call(xyz, n, boxes_dev, t, s);
+    constexpr int ppt = 4;  // tiles of 1024 points, eight 128-point items each
+    const int64_t ntiles = (n + tile_points(ppt) - 1) / tile_points(ppt);
+    float* mm = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + t.bytes);  // the chunk's minima and maxima, contiguous
+    {
+        const int64_t count = (int64_t)n_traj * (int64_t)block;
+        const int grid = (int)std::min<int64_t>((count + 255) / 256, (int64_t)cov_sm_count_cached() * 8);
+        cov_sweep_acc_init_kernel<<<grid, 256, 0, s>>>(acc, count, (int64_t)block, 0.5 * (double)n);
+    }
+    unsigned long long* stats = opts ? opts->stats_dev : nullptr;
+    for (int t0 = 0; t0 < n_traj; t0 += chunk) {
+        const int nt = std::min(n_traj - t0, chunk);
+        const int w0 = t0 * per_traj, Wn = nt * per_traj;
+        cudaMemcpyAsync(mm, minmax + w0, (size_t)Wn * sizeof(float), cudaMemcpyDeviceToDevice, s);
+        cudaMemcpyAsync(mm + Wn, minmax + TP + w0, (size_t)Wn * sizeof(float), cudaMemcpyDeviceToDevice, s);
+        cov_traj_table_kernel<<<(Wn + 63) / 64, 64, 0, s>>>(poses + 3 * (size_t)w0, quats + 4 * (size_t)w0, Wn, K, C, mm,
+                                                            t.table, t.ctrl, (int)(t.ctrl_bytes / sizeof(int)), nullptr, 0.0);
+        int rc = launch_cull(boxes, ppt, ntiles, t, Wn, nullptr, 0.f, nullptr, 0, s);
+        if (rc != COV_OK) return rc;
+        cov_sweep_fused_tiles_kernel<<<persistent_grid(cov_sweep_fused_tiles_kernel, 0, ntiles), COV_THREADS, 0, s>>>(
+            xyz, n, t.table, Wn, per_traj, C, boxes, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, ntiles,
+            acc + (size_t)t0 * block, stats);
+    }
+    return cov_check_launch("cov_sweep_fused");
+}
+
+extern "C" int cov_sweep_epilogue(const double* acc, const float* minmax, const float* quats, int n_traj, int per_traj,
+                                  int64_t n_total, float* out, void* stream) {
+    if (!acc || !minmax || !quats || !out || n_traj <= 0 || per_traj <= 0 || n_total <= 0 ||
+        (int64_t)n_traj * per_traj > INT32_MAX / 8) {
+        cov_set_error("cov_sweep_epilogue: bad argument (n_traj=%d, poses_per_traj=%d, n_total=%lld)", n_traj, per_traj,
+                      (long long)n_total);
+        return COV_ERR_ARG;
+    }
+    const int TP = n_traj * per_traj;
+    cov_sweep_epilogue_kernel<<<(TP + 127) / 128, 128, 0, (cudaStream_t)stream>>>(acc, minmax, quats, n_traj, per_traj,
+                                                                                 (double)n_total, out);
+    return cov_check_launch("cov_sweep_epilogue");
 }
 
 extern "C" int cov_traj_epilogue(const double* acc, const float* minmax, const float* quats, int W, int64_t n_total,

@@ -167,7 +167,81 @@ def mean_angle_calc(traj_wps, eps=1e-6):
     return torch.arccos(cosang).sum() / (n_wps - 2)
 
 
-class ModelTraj(nn.Module):
+def _wps_quotient(poses0, vis_wps_dist):
+    """src/model.py:214: vis_wps_dist over the mean waypoint spacing of (W, 3) `poses0`, as a 0-d tensor of poses0's
+    dtype (the reference divides by an fp32 tensor: when the spacing divides the distance, the rounded quotient can land
+    on the integer that an fp64 division would miss, and the stride int(quotient) + 1 depends on it)."""
+    mean_wps_dist = (poses0[1:, :] - poses0[:-1, :]).norm(dim=1).mean()
+    return vis_wps_dist / mean_wps_dist
+
+
+class _OrderedCloudModel(nn.Module):
+    """What ModelTraj and ModelTrajBatch share: the Morton-ordered copy of `self.points` with its permutation and tile
+    boxes (made once per state of the cloud), the kept workspace, and the release of the last autograd graph.
+    Subclasses set `points`, `spatial_sort`, `_pts32`, `_perm`, `_boxes`, `_ws` and `_mean` in their constructor."""
+
+    def _cloud(self):
+        # The ordered copy, its permutation and the tile boxes belong to ONE state of `self.points`: the cache is keyed
+        # on identity and on torch's version counter, so both `model.points = new` and an in-place `model.points.copy_()`
+        # trigger a re-sort (the exact pruning relies on the boxes bounding the points the kernels read).
+        key = (id(self.points), self.points._version)
+        if self._pts32 is None or self._pts32_key != key:
+            pts = ops._BACKEND.prepare(self.points, what="points")
+            self._pts32, self._perm, self._boxes = ops._BACKEND.order_cloud(pts, self.spatial_sort)
+            self._pts32_key = key
+        return self._pts32
+
+    def set_points(self, points):
+        """Replace the cloud; the Morton-ordered copy, permutation and boxes are rebuilt on the next forward.  Inside a
+        captured CUDA graph use `refresh_points_()` instead (same shapes, buffers rewritten in place)."""
+        self.points = torch.as_tensor(points, dtype=torch.float32).to(self.device)
+        self._pts32 = None
+
+    def detach_state(self):
+        """Drop the references this model keeps into the last autograd graph (`loss[...]`, `_mean`) so that the graph —
+        and the gradient-accumulation nodes bound to the stream it ran on — can be freed (graphs.GraphedStep calls this
+        before it warms up on its capture stream)."""
+        self._mean = None
+        for name in ("loss", "losses"):
+            terms = getattr(self, name, None) or {}
+            for k, v in list(terms.items()):
+                if isinstance(v, torch.Tensor):
+                    terms[k] = v.detach()
+        for name in ("rewards", "means"):
+            v = getattr(self, name, None)
+            if isinstance(v, torch.Tensor):
+                setattr(self, name, v.detach())
+
+    @torch.no_grad()
+    def refresh_points_(self, points):
+        """In-place cloud update for CUDA-graph replays (graphs.GraphedStep): `points` must have the shape of the
+        current cloud; `self.points`, the ordered copy, the permutation and the boxes keep their addresses and are
+        rewritten, so a graph captured earlier evaluates the NEW cloud on its next replay."""
+        if self._pts32 is None:
+            self._cloud()
+        if tuple(points.shape) != tuple(self.points.shape):
+            raise ValueError("refresh_points_ needs a cloud of the same shape; use set_points() and re-capture")
+        self.points.copy_(points)
+        pts = ops._BACKEND.prepare(self.points, what="points")
+        new_pts, new_perm, new_boxes = ops._BACKEND.order_cloud(pts, self.spatial_sort)
+        if self._pts32.data_ptr() != self.points.data_ptr():
+            self._pts32.copy_(new_pts)
+        if self._perm is not None:
+            self._perm.copy_(new_perm)
+        if self._boxes is not None and new_boxes is not None:
+            self._boxes.copy_(new_boxes)
+        self._pts32_key = (id(self.points), self.points._version)
+
+    def _kept_workspace(self, cloud, need):
+        # one workspace per (cloud, size), kept across steps: nothing in it outlives a call
+        if not cloud.is_cuda:
+            return None
+        if self._ws is None or self._ws.numel() < need or self._ws.device != cloud.device:
+            self._ws = torch.empty(need, dtype=torch.uint8, device=cloud.device)
+        return self._ws
+
+
+class ModelTraj(_OrderedCloudModel):
     def __init__(self, points, wps_poses, wps_quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0,
                  smoothness_weight=14.0, traj_length_weight=0.02, device=torch.device("cuda"), group=None,
                  n_total=None, spatial_sort=True, fused_regularizers=False):
@@ -212,69 +286,16 @@ class ModelTraj(nn.Module):
         self._ws = None
         self.to(self.device)
 
-    def _cloud(self):
-        # The ordered copy, its permutation and the tile boxes belong to ONE state of `self.points`: the cache is keyed
-        # on identity and on torch's version counter, so both `model.points = new` and an in-place `model.points.copy_()`
-        # trigger a re-sort (the exact pruning relies on the boxes bounding the points the kernels read).
-        key = (id(self.points), self.points._version)
-        if self._pts32 is None or self._pts32_key != key:
-            pts = ops._BACKEND.prepare(self.points, what="points")
-            self._pts32, self._perm, self._boxes = ops._BACKEND.order_cloud(pts, self.spatial_sort)
-            self._pts32_key = key
-        return self._pts32
-
-    def set_points(self, points):
-        """Replace the cloud; the Morton-ordered copy, permutation and boxes are rebuilt on the next forward.  Inside a
-        captured CUDA graph use `refresh_points_()` instead (same shapes, buffers rewritten in place)."""
-        self.points = torch.as_tensor(points, dtype=torch.float32).to(self.device)
-        self._pts32 = None
-
-    def detach_state(self):
-        """Drop the references this model keeps into the last autograd graph (`loss[...]`, `_mean`) so that the graph —
-        and the gradient-accumulation nodes bound to the stream it ran on — can be freed (graphs.GraphedStep calls this
-        before it warms up on its capture stream)."""
-        self._mean = None
-        for k, v in list(self.loss.items()):
-            if isinstance(v, torch.Tensor):
-                self.loss[k] = v.detach()
-        if self.rewards is not None:
-            self.rewards = self.rewards.detach()
-
-    @torch.no_grad()
-    def refresh_points_(self, points):
-        """In-place cloud update for CUDA-graph replays (graphs.GraphedStep): `points` must have the shape of the
-        current cloud; `self.points`, the ordered copy, the permutation and the boxes keep their addresses and are
-        rewritten, so a graph captured earlier evaluates the NEW cloud on its next replay."""
-        if self._pts32 is None:
-            self._cloud()
-        if tuple(points.shape) != tuple(self.points.shape):
-            raise ValueError("refresh_points_ needs a cloud of the same shape; use set_points() and re-capture")
-        self.points.copy_(points)
-        pts = ops._BACKEND.prepare(self.points, what="points")
-        new_pts, new_perm, new_boxes = ops._BACKEND.order_cloud(pts, self.spatial_sort)
-        if self._pts32.data_ptr() != self.points.data_ptr():
-            self._pts32.copy_(new_pts)
-        if self._perm is not None:
-            self._perm.copy_(new_perm)
-        if self._boxes is not None and new_boxes is not None:
-            self._boxes.copy_(new_boxes)
-        self._pts32_key = (id(self.points), self.points._version)
-
     def _workspace(self, cloud):
-        # one workspace per (cloud, pose count), kept across steps: nothing in it outlives a call
         if not cloud.is_cuda:
             return None
-        need = ops._BACKEND.traj_workspace_bytes(cloud, max(1, self.poses.shape[0]))
-        if self._ws is None or self._ws.numel() < need or self._ws.device != cloud.device:
-            self._ws = torch.empty(need, dtype=torch.uint8, device=cloud.device)
-        return self._ws
+        return self._kept_workspace(cloud, ops._BACKEND.traj_workspace_bytes(cloud, max(1, self.poses.shape[0])))
 
     def _wps_step(self, vis_wps_dist):
         # src/model.py:214-215.  poses0 never changes, so the host sync happens once per distance
         key = float(vis_wps_dist)
         if key not in self._step_cache:
-            mean_wps_dist = (self.poses0[1:, :] - self.poses0[:-1, :]).norm(dim=1).mean()
-            self._step_cache[key] = int(vis_wps_dist / mean_wps_dist) + 1
+            self._step_cache[key] = int(_wps_quotient(self.poses0, vis_wps_dist)) + 1
         return self._step_cache[key]
 
     def forward(self, vis_wps_dist=0.5, debug=False):
@@ -317,3 +338,90 @@ class ModelTraj(nn.Module):
         self.loss["smooth"] = self.smoothness_weight / (mean_angle_calc(self.poses, self.eps) + self.eps)
         self.loss["length"] = self.traj_length_weight * torch.abs(length_calc(self.poses) - length_calc(self.poses0))
         return self.loss["vis"] + self.loss["l2"] + self.loss["length"] + self.loss["smooth"]
+
+
+# ------------------------------------------------------------------------------------------
+# T trajectories optimised at once (no reference counterpart: multi-start refinement of sweep candidates)
+# ------------------------------------------------------------------------------------------
+class ModelTrajBatch(_OrderedCloudModel):
+    """T independent ModelTraj objectives on one cloud, evaluated together: the visibility terms of all trajectories
+    and their gradients come from one differentiable sweep (ops.coverage_sweep) instead of T coverage_traj calls.
+    Parameters `poses` (T, W, 3) and `quats` (T, W, 4); `forward()` returns sum_t loss_t, where loss_t is
+    ModelTraj.criterion's loss of trajectory t.  The per-trajectory terms are kept as (T,) tensors in `self.losses`
+    ("vis", "l2", "smooth", "length"), the (T,) mean rewards in `self.means`."""
+
+    def __init__(self, points, wps_poses, wps_quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0,
+                 smoothness_weight=14.0, traj_length_weight=0.02, device=torch.device("cuda"), group=None,
+                 n_total=None, spatial_sort=True):
+        super().__init__()
+        wps_poses = torch.as_tensor(wps_poses, dtype=torch.float32)
+        wps_quats = torch.as_tensor(wps_quats, dtype=torch.float32)
+        if (wps_poses.dim() != 3 or wps_quats.dim() != 3 or wps_poses.shape[2] != 3 or wps_quats.shape[2] != 4
+                or wps_poses.shape[:2] != wps_quats.shape[:2]):
+            raise ValueError("ModelTrajBatch: wps_poses must be (T, W, 3) and wps_quats (T, W, 4) with the same T and W")
+        if wps_poses.shape[1] < 3:
+            raise ValueError("ModelTrajBatch: the smoothness term needs W >= 3 waypoints per trajectory")
+        self.device = device
+        self.points = torch.as_tensor(points, dtype=torch.float32).to(self.device)
+        self.poses0 = wps_poses.to(self.device)
+        self.quats0 = wps_quats.to(self.device)
+        self.poses = nn.Parameter(deepcopy(self.poses0))
+        self.quats = nn.Parameter(deepcopy(self.quats0))
+        self.K = torch.as_tensor(intrins, dtype=torch.float32).to(self.device)
+        self.img_width, self.img_height = float(img_width), float(img_height)
+        self.eps = 1e-6
+        self.pc_clip_limits = [min_dist, max_dist]
+        self.smoothness_weight = smoothness_weight
+        self.traj_length_weight = traj_length_weight
+        self.group = group        # torch.distributed group when `points` is this rank's shard
+        self.n_total = n_total    # global point count in that case
+        self.spatial_sort = spatial_sort
+        self.losses = {}
+        self.means = None
+        self._mean = None
+        self._step_cache = {}
+        self._pts32 = None
+        self._perm = None
+        self._boxes = None
+        self._ws = None
+        self.to(self.device)
+
+    def _wps_step(self, vis_wps_dist):
+        # ModelTraj._wps_step for every trajectory's poses0, with the same arithmetic; one host sync per distance
+        key = float(vis_wps_dist)
+        if key not in self._step_cache:
+            quot = torch.stack([_wps_quotient(p0, vis_wps_dist) for p0 in self.poses0]).cpu()
+            steps = sorted({int(q) + 1 for q in quot})
+            if len(steps) != 1:
+                raise ValueError(f"ModelTrajBatch: the trajectories' visibility strides differ ({steps}) at "
+                                 f"vis_wps_dist={vis_wps_dist}: every trajectory must be evaluated on the same waypoints")
+            self._step_cache[key] = steps[0]
+        return self._step_cache[key]
+
+    def forward(self, vis_wps_dist=0.5):
+        wps_step = self._wps_step(vis_wps_dist)
+        cloud = self._cloud()
+        P, Q = self.poses[:, ::wps_step], self.quats[:, ::wps_step]
+        with ops.evaluation(dense=None if self.spatial_sort else True):
+            ws = self._kept_workspace(cloud, ops._BACKEND.sweep_fused_workspace_bytes(cloud, P.shape[0], P.shape[1]))
+            means = ops.coverage_sweep(cloud, P, Q, self.K, self.img_width, self.img_height, self.pc_clip_limits[0],
+                                       self.pc_clip_limits[1], self.eps, n_total=self.n_total, group=self.group,
+                                       boxes=self._boxes, presorted=True, workspace=ws)
+        self.means = means
+        return self.criterion(means)
+
+    def criterion(self, means):
+        # ModelTraj.criterion per trajectory; length_calc and mean_angle_calc restated over the batch dimension
+        p, p0 = self.poses, self.poses0
+        self.losses["vis"] = 1.0 / (means + self.eps)
+        self.losses["l2"] = torch.linalg.norm(p[:, 0] - p0[:, 0], dim=-1)
+        ab = p[:, :-2] - p[:, 1:-1]
+        ac = p[:, 2:] - p[:, 1:-1]
+        cosang = (ab * ac).sum(dim=2) / (torch.linalg.norm(ab, dim=2) * torch.linalg.norm(ac, dim=2) + self.eps)
+        mean_angle = torch.arccos(cosang).sum(dim=1) / (p.shape[1] - 2)
+        self.losses["smooth"] = self.smoothness_weight / (mean_angle + self.eps)
+        length = torch.linalg.norm(p[:, 1:] - p[:, :-1], dim=-1).sum(dim=1)
+        length0 = torch.linalg.norm(p0[:, 1:] - p0[:, :-1], dim=-1).sum(dim=1)
+        self.losses["length"] = self.traj_length_weight * torch.abs(length - length0)
+        loss = self.losses["vis"] + self.losses["l2"] + self.losses["length"] + self.losses["smooth"]
+        return loss.sum()

@@ -285,6 +285,29 @@ class CudaBackend:
         _call("cov_traj_epilogue", acc, _ptr(acc), _ptr(minmax), _ptr(Q), W, n_total, upstream_mode, _ptr(out))
         return out
 
+    def sweep_fused_workspace_bytes(self, pts, T, Pn, dense=None):
+        """Workspace of a cov_sweep_fused call on this cloud with the current (or the given) dense mode."""
+        opts = _opts(dense)
+        return _lib.lib().cov_sweep_fused_workspace_bytes(pts.shape[0], T, Pn, ctypes.byref(opts))
+
+    def sweep_fused(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, ws=None):
+        """This cloud's pass-B accumulators of every trajectory: T blocks of 22 Pn + 1 doubles (cov_sweep_fused)."""
+        n, dev = pts.shape[0], pts.device
+        ws_bytes = self.sweep_fused_workspace_bytes(pts, T, Pn)
+        if ws is None or ws.numel() < ws_bytes or ws.device != dev:
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        acc = torch.empty(T * (Pn * _lib.ACC_STRIDE + 1), dtype=torch.float64, device=dev)
+        opts = _opts()
+        _call("cov_sweep_fused", pts, _ptr(pts), n, _ptr(P), _ptr(Q), T, Pn, _ptr(Kd), ctypes.byref(cam), _ptr(boxes),
+              _ptr(minmax), _ptr(acc), ctypes.byref(opts), _ptr(ws), ws.numel())
+        return acc
+
+    def sweep_epilogue(self, acc, minmax, Q, T, Pn, n_total):
+        """[T means | T Pn 3 d mean_t/d poses | T Pn 4 d mean_t/d quats] (fp32) from the summed accumulators."""
+        out = torch.empty(T * (1 + 7 * Pn), dtype=torch.float32, device=acc.device)
+        _call("cov_sweep_epilogue", acc, _ptr(acc), _ptr(minmax), _ptr(Q), T, Pn, n_total, _ptr(out))
+        return out
+
 
 _BACKEND = CudaBackend()
 
@@ -402,6 +425,67 @@ class CoverageTrajFn(torch.autograd.Function):
         ps, qs = ctx.shapes
         return (None, None if g_p is None else g_p.reshape(ps), None if g_q is None else g_q.reshape(qs),
                 None, None, None, None, None, None, None, None)
+
+
+class CoverageSweepFn(torch.autograd.Function):
+    """means_t = mean_j rewards_j(t) of T candidate trajectories on one cloud, each trajectory's poses evaluated as
+    CoverageTrajFn evaluates them, and d means_t / d (poses_t, quats_t) from the same pass (cov_sweep_fused)."""
+
+    @staticmethod
+    def forward(ctx, pts, poses, quats, K, cam, n_total, group, boxes, shard, workspace):
+        B = _BACKEND
+        dev = pts.device
+        T, Pn = poses.shape[0], poses.shape[1]
+        Kd = B.prepare(K, dev, "intrins").reshape(9)
+        if group is not None and shard == "trajectories":
+            # every rank holds the whole cloud and evaluates its contiguous block of trajectories; the per-rank outputs
+            # [means | d/dposes | d/dquats] are gathered and reassembled in the layout of one unsharded call
+            import torch.distributed as dist
+            world, rank = dist.get_world_size(group), dist.get_rank(group)
+            per = (T + world - 1) // world
+            t0, t1 = min(T, rank * per), min(T, (rank + 1) * per)
+            nt = t1 - t0
+            mine = torch.zeros(per * (1 + 7 * Pn), dtype=torch.float32, device=dev)
+            if nt > 0:
+                o = CoverageSweepFn._run(pts, poses[t0:t1], quats[t0:t1], Kd, cam, n_total, None, boxes, workspace)
+                mine[:nt] = o[:nt]
+                mine[per:per + 3 * nt * Pn] = o[nt:nt + 3 * nt * Pn]
+                mine[per + 3 * per * Pn:per + 3 * per * Pn + 4 * nt * Pn] = o[nt + 3 * nt * Pn:]
+            every = torch.empty(world * mine.numel(), dtype=mine.dtype, device=dev)
+            dist.all_gather_into_tensor(every, mine, group=group)
+            every = every.view(world, -1)
+            out = torch.cat([every[:, :per].reshape(-1)[:T], every[:, per:per + 3 * per * Pn].reshape(-1)[:3 * T * Pn],
+                             every[:, per + 3 * per * Pn:].reshape(-1)[:4 * T * Pn]])
+        else:
+            out = CoverageSweepFn._run(pts, poses, quats, Kd, cam, n_total, group, boxes, workspace)
+        ctx.shapes = (poses.shape, quats.shape)
+        ctx.save_for_backward(out)
+        return out[:T].clone()
+
+    @staticmethod
+    def _run(pts, poses, quats, Kd, cam, n_total, group, boxes, workspace):
+        B = _BACKEND
+        dev = pts.device
+        T, Pn = poses.shape[0], poses.shape[1]
+        P = B.prepare(poses, dev, "poses").reshape(-1, 3)
+        Q = B.prepare(quats, dev, "quats").reshape(-1, 4)
+        minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)     # pass A on this shard, (2, T Pn)
+        _all_reduce_minmax(minmax, T * Pn, group)
+        acc = B.sweep_fused(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, workspace)
+        if group is not None:
+            # plain all-reduce: the in-kernel exchange buffers are sized for the 22 W + 1 doubles of one trajectory
+            _all_reduce(acc, _reduce_ops()[2], group)
+        return B.sweep_epilogue(acc, minmax, Q, T, Pn, n_total)
+
+    @staticmethod
+    def backward(ctx, g_means):
+        (out,) = ctx.saved_tensors
+        ps, qs = ctx.shapes
+        T, Pn = ps[0], ps[1]
+        g = g_means.reshape(T, 1).to(out.dtype)
+        g_p = (g * out[T:T + 3 * T * Pn].reshape(T, 3 * Pn)).reshape(ps)
+        g_q = (g * out[T + 3 * T * Pn:].reshape(T, 4 * Pn)).reshape(qs)
+        return None, g_p, g_q, None, None, None, None, None, None, None
 
 
 class TrajRegularizersFn(torch.autograd.Function):
@@ -546,6 +630,33 @@ def sweep_rewards(points, poses, quats, intrins, img_width, img_height, min_dist
     if group is not None:
         _all_reduce(sums, _reduce_ops()[2], group)
     return sums / float(n if n_total is None else n_total)
+
+
+def coverage_sweep(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
+                   n_total=None, group=None, boxes=None, presorted=False, shard="points", workspace=None):
+    """Differentiable candidate sweep: poses (T, P, 3), quats (T, P, 4) -> means (T,) fp32, where means[t] is the mean
+    reward of trajectory t as `coverage_traj(points, poses[t], quats[t])` computes it.  `means` is differentiable w.r.t.
+    `poses` and `quats`; each trajectory's gradient comes from the same pass over the cloud (cov_sweep_fused), so a
+    backward of any weighted sum of the means costs no further pass.
+    The cloud is ordered as in `sweep_rewards` (Morton order, unless `presorted` or `boxes` are given); dense mode comes
+    from `evaluation(dense=True)`.  No host synchronisation: capturable in a CUDA graph.  `workspace`: a uint8 CUDA tensor
+    kept by the caller across calls (grown when too small).
+    Sharding as in `sweep_rewards`: shard="points" (this rank's slice of the cloud; normalisers and accumulators are
+    all-reduced) or shard="trajectories" (the whole cloud on every rank; means and gradients are all-gathered)."""
+    B = _BACKEND
+    if shard not in ("points", "trajectories"):
+        raise ValueError("shard must be 'points' or 'trajectories'")
+    if (not isinstance(poses, torch.Tensor) or not isinstance(quats, torch.Tensor) or poses.dim() != 3
+            or quats.dim() != 3 or poses.shape[2] != 3 or quats.shape[2] != 4 or poses.shape[:2] != quats.shape[:2]
+            or poses.shape[0] == 0 or poses.shape[1] == 0):
+        raise ValueError("coverage_sweep: poses must be (T, P, 3) and quats (T, P, 4) with the same T, P >= 1; got "
+                         f"{tuple(getattr(poses, 'shape', ()))} and {tuple(getattr(quats, 'shape', ()))}")
+    pts = B.prepare(points, what="points")
+    if not presorted and boxes is None and pts.shape[0] > 0:
+        pts, _, boxes = B.order_cloud(pts, True)
+    n_total = int(pts.shape[0] if n_total is None else n_total)
+    cam = _lib.camera(img_width, img_height, min_dist, max_dist, eps)
+    return CoverageSweepFn.apply(pts, poses, quats, intrins, cam, n_total, group, boxes, shard, workspace)
 
 
 @torch.no_grad()
