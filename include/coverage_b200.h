@@ -178,6 +178,27 @@ int cov_sweep_epilogue(const double* acc_dev, const float* minmax_dev, const flo
                        int poses_per_traj, int64_t n_total, float* out_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Batched ModelPose: K candidate poses (t_k, q~_k) on one cloud, for every k the COV_POSE_ACC sums cov_pose_fused
+ * computes for pose k alone ([0] sum m, [1..3] F, [4..6] T, [7] 0), in one pass over the cloud per chunk of poses.
+ * ref: src/model.py:98-127 per pose (multi-start pose optimisation, scoring of candidate views); no per-point output.
+ *   weight_dev (n) or NULL: one weight per point shared by all poses.  trans_dev (K,3), quats_dev (K,4) fp32.
+ *   boxes_dev: NULL, or cov_tile_boxes of this cloud: a warp then skips a (128-point box, pose) pair whose distance
+ *   Gaussian bound is below 2^-128, where every pair is exactly 0 (exact; pays on clouds much larger than the
+ *   ~27 m reach of the default clip limits).  No boxes are built inside the call: with NULL every pair is evaluated.
+ *   acc_dev: K blocks of COV_POSE_ACC doubles, initialised by the call.  Shard-additive: with a sharded cloud, SUM the
+ *   blocks over the ranks, then run cov_pose_batch_epilogue.  Sums are fp32 within one (box, pose), fp64 above.
+ *   opts: honours `dense` (ignore boxes_dev) and `stats_dev` ([0] (warp box, pose) pairs, [1] pairs evaluated).
+ *   workspace_dev: cov_pose_batch_workspace_bytes(n, K, opts) bytes, 16-byte aligned (xyz and weight likewise).
+ * ------------------------------------------------------------------------------------------ */
+size_t cov_pose_batch_workspace_bytes(int64_t n, int n_poses, const cov_traj_opts* opts);
+int cov_pose_batch_fused(const float* xyz_dev, int64_t n, const float* weight_dev, const float* trans_dev,
+                         const float* quats_dev, int n_poses, const float* K_dev, const cov_camera* cam,
+                         const float* boxes_dev, double* acc_dev, const cov_traj_opts* opts, void* workspace_dev,
+                         size_t workspace_bytes, void* stream);
+/* out_dev (K, 8) fp32: row k is what cov_pose_epilogue gives for acc block k and quat k, bit for bit. */
+int cov_pose_batch_epilogue(const double* acc_dev, const float* quats_dev, int n_poses, float* out_dev, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * The two exchange steps of the point-sharded objective (MAX of the 2 W normalisers, SUM of the 22 W + 1 accumulator
  * doubles) as ONE small kernel each over NVLink peer memory, in place of a collective-library launch.
  * ref: no reference code (the reference is single-process); replaces the dist.all_reduce calls of SURVEY.md 8e.

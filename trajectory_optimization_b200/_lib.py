@@ -50,6 +50,9 @@ PROTOTYPES = {
     "cov_pose_workspace_bytes": (_sz, [_i64]),
     "cov_pose_fused": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _cam, _vp, _vp, _vp, _sz, _vp]),
     "cov_pose_epilogue": (_int, [_vp, _vp, _vp, _vp, _vp]),
+    "cov_pose_batch_workspace_bytes": (_sz, [_i64, _int, _opts]),
+    "cov_pose_batch_fused": (_int, [_vp, _i64, _vp, _vp, _vp, _int, _vp, _cam, _vp, _vp, _opts, _vp, _sz, _vp]),
+    "cov_pose_batch_epilogue": (_int, [_vp, _vp, _int, _vp, _vp]),
     "cov_traj_max_poses": (_int, []),
     "cov_traj_max_poses_pruned": (_int, []),
     "cov_traj_workspace_bytes": (_sz, [_i64, _int]),

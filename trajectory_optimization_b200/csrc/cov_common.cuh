@@ -111,6 +111,16 @@ __device__ __forceinline__ float cov_q2(float x, float y, float z, const float4&
     return __fmaf_rn(ez, ez, __fmaf_rn(ey, ey, __fmul_rn(ex, ex)));
 }
 
+// Lower bound of cov_q2(x, y, z, v3) over every point of the box [lo, hi].  Rounding is monotone, so with the same
+// operation sequence as cov_q2 (fsub, then fmul/fma/fma) the bound holds for the COMPUTED q2 of each point, exactly:
+// |fl(x - td)| >= max(fl(lo - td), fl(td - hi), 0) for lo <= x <= hi.  An empty box (lo = +inf) gives +inf.
+__device__ __forceinline__ float box_q2lb(const float4& lo, const float4& hi, const float4& v3) {
+    const float dx = fmaxf(fmaxf(__fsub_rn(lo.x, v3.x), __fsub_rn(v3.x, hi.x)), 0.f);
+    const float dy = fmaxf(fmaxf(__fsub_rn(lo.y, v3.y), __fsub_rn(v3.y, hi.y)), 0.f);
+    const float dz = fmaxf(fmaxf(__fsub_rn(lo.z, v3.z), __fsub_rn(v3.z, hi.z)), 0.f);
+    return __fmaf_rn(dz, dz, __fmaf_rn(dy, dy, __fmul_rn(dx, dx)));
+}
+
 struct CovEval {  // intermediates the gradient needs
     float ex, ey, ez, zi, s, e2z, du, dv;
 };
@@ -273,6 +283,35 @@ __device__ __forceinline__ double cov_warp_sum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
+}
+
+// 8 sums over 32 lanes in 9 shuffles, in a fixed order: halve the number of values a lane carries at offsets 16, 8, 4 (a
+// lane keeps the half its lane bit selects and hands the other half over), then two plain steps.  Afterwards the lanes
+// with (lane & 3) == 0 hold in v[0] the warp sum of component (lane bits 4,3,2); v[1..7] are left as scratch.
+__device__ __forceinline__ void cov_warp_sum8(float (&v)[8], int lane) {
+    {
+        const bool up = (lane & 16) != 0;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const float keep = up ? v[q + 4] : v[q], send = up ? v[q] : v[q + 4];
+            v[q] = keep + __shfl_xor_sync(0xffffffffu, send, 16);
+        }
+    }
+    {
+        const bool up = (lane & 8) != 0;
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+            const float keep = up ? v[q + 2] : v[q], send = up ? v[q] : v[q + 2];
+            v[q] = keep + __shfl_xor_sync(0xffffffffu, send, 8);
+        }
+    }
+    {
+        const bool up = (lane & 4) != 0;
+        const float keep = up ? v[1] : v[0], send = up ? v[0] : v[1];
+        v[0] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
+    }
+    v[0] += __shfl_xor_sync(0xffffffffu, v[0], 2);
+    v[0] += __shfl_xor_sync(0xffffffffu, v[0], 1);
 }
 
 // ---- TMA bulk copies (global -> shared) completing on an mbarrier ------------------------------------------------

@@ -129,15 +129,7 @@ __device__ __forceinline__ float ord2f(unsigned u) {
     return __uint_as_float((u & 0x80000000u) ? (u ^ 0x80000000u) : ~u);
 }
 
-// Lower bound of cov_q2(x, y, z, v3) over every point of the box [lo, hi].  Rounding is monotone, so with the same
-// operation sequence as cov_q2 (fsub, then fmul/fma/fma) the bound holds for the COMPUTED q2 of each point, exactly:
-// |fl(x - td)| >= max(fl(lo - td), fl(td - hi), 0) for lo <= x <= hi.  An empty box (lo = +inf) gives +inf.
-__device__ __forceinline__ float box_q2lb(const float4& lo, const float4& hi, const float4& v3) {
-    const float dx = fmaxf(fmaxf(__fsub_rn(lo.x, v3.x), __fsub_rn(v3.x, hi.x)), 0.f);
-    const float dy = fmaxf(fmaxf(__fsub_rn(lo.y, v3.y), __fsub_rn(v3.y, hi.y)), 0.f);
-    const float dz = fmaxf(fmaxf(__fsub_rn(lo.z, v3.z), __fsub_rn(v3.z, hi.z)), 0.f);
-    return __fmaf_rn(dz, dz, __fmaf_rn(dy, dy, __fmul_rn(dx, dx)));
-}
+// (box_q2lb, the box bound the pruned kernels test against, is in cov_common.cuh)
 __device__ __forceinline__ void box_union(float4& lo, float4& hi, const float4& lo2, const float4& hi2) {
     lo.x = fminf(lo.x, lo2.x); lo.y = fminf(lo.y, lo2.y); lo.z = fminf(lo.z, lo2.z);
     hi.x = fmaxf(hi.x, hi2.x); hi.y = fmaxf(hi.y, hi2.y); hi.z = fmaxf(hi.z, hi2.z);
@@ -925,32 +917,7 @@ __device__ __forceinline__ void tiles_pose_backward(const float4* __restrict__ r
             }
         }
     }
-    // 8 sums over 32 lanes in 9 shuffles: halve the number of values a lane carries at offsets 16, 8, 4 (a lane keeps the
-    // half its lane bit selects and hands the other half over), then two plain steps; lanes with (lane & 3) == 0 end with
-    // component (lane bits 4,3,2)
-    {
-        const bool up = (lane & 16) != 0;
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const float keep = up ? v[q + 4] : v[q], send = up ? v[q] : v[q + 4];
-            v[q] = keep + __shfl_xor_sync(kFull, send, 16);
-        }
-    }
-    {
-        const bool up = (lane & 8) != 0;
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-            const float keep = up ? v[q + 2] : v[q], send = up ? v[q] : v[q + 2];
-            v[q] = keep + __shfl_xor_sync(kFull, send, 8);
-        }
-    }
-    {
-        const bool up = (lane & 4) != 0;
-        const float keep = up ? v[1] : v[0], send = up ? v[0] : v[1];
-        v[0] = keep + __shfl_xor_sync(kFull, send, 4);
-    }
-    v[0] += __shfl_xor_sync(kFull, v[0], 2);
-    v[0] += __shfl_xor_sync(kFull, v[0], 1);
+    cov_warp_sum8(v, lane);
     if ((lane & 3) == 0 && v[0] != 0.f) {  // one fire-and-forget fp64 RED per component
         const int comp = ((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1);
         atomicAdd(acc_row + comp, (double)v[0]);

@@ -176,7 +176,7 @@ def _wps_quotient(poses0, vis_wps_dist):
 
 
 class _OrderedCloudModel(nn.Module):
-    """What ModelTraj and ModelTrajBatch share: the Morton-ordered copy of `self.points` with its permutation and tile
+    """What ModelTraj, ModelTrajBatch and ModelPoseBatch share: the Morton-ordered copy of `self.points` with its permutation and tile
     boxes (made once per state of the cloud), the kept workspace, and the release of the last autograd graph.
     Subclasses set `points`, `spatial_sort`, `_pts32`, `_perm`, `_boxes`, `_ws` and `_mean` in their constructor."""
 
@@ -198,19 +198,18 @@ class _OrderedCloudModel(nn.Module):
         self._pts32 = None
 
     def detach_state(self):
-        """Drop the references this model keeps into the last autograd graph (`loss[...]`, `_mean`) so that the graph —
-        and the gradient-accumulation nodes bound to the stream it ran on — can be freed (graphs.GraphedStep calls this
-        before it warms up on its capture stream)."""
+        """Drop the references this model keeps into the last autograd graph (`loss[...]`, `losses`, `_mean`, the
+        per-point or per-candidate outputs) so that the graph — and the gradient-accumulation nodes bound to the stream it
+        ran on — can be freed (graphs.GraphedStep calls this before it warms up on its capture stream)."""
         self._mean = None
-        for name in ("loss", "losses"):
-            terms = getattr(self, name, None) or {}
-            for k, v in list(terms.items()):
-                if isinstance(v, torch.Tensor):
-                    terms[k] = v.detach()
-        for name in ("rewards", "means"):
+        for name in ("loss", "losses", "rewards", "means", "totals"):
             v = getattr(self, name, None)
             if isinstance(v, torch.Tensor):
                 setattr(self, name, v.detach())
+            elif isinstance(v, dict):
+                for k, t in list(v.items()):
+                    if isinstance(t, torch.Tensor):
+                        v[k] = t.detach()
 
     @torch.no_grad()
     def refresh_points_(self, points):
@@ -425,3 +424,70 @@ class ModelTrajBatch(_OrderedCloudModel):
         self.losses["length"] = self.traj_length_weight * torch.abs(length - length0)
         loss = self.losses["vis"] + self.losses["l2"] + self.losses["length"] + self.losses["smooth"]
         return loss.sum()
+
+
+# ------------------------------------------------------------------------------------------
+# K camera poses optimised at once (no reference counterpart: multi-start ModelPose, scoring of candidate views)
+# ------------------------------------------------------------------------------------------
+class ModelPoseBatch(_OrderedCloudModel):
+    """K independent ModelPose objectives on one cloud, evaluated together: the totals of all candidates and their
+    gradients come from one pass over the cloud (ops.coverage_pose_batch) instead of K coverage_pose calls.
+    Parameters `trans` (K, 3) and `quat` (K, 4); `forward()` returns sum_k 1/(total_k + eps), i.e. ModelPose.criterion
+    per candidate, summed.  Adam is elementwise, so one Adam over both parameters is K independent ModelPose
+    optimisations.  The (K,) totals are kept in `self.totals`, the (K,) per-candidate losses in `self.losses`."""
+
+    def __init__(self, points, trans0, q0, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0,
+                 device=torch.device("cuda:0"), group=None, spatial_sort=True):
+        super().__init__()
+        trans0 = torch.as_tensor(trans0, dtype=torch.float32)
+        q0 = torch.as_tensor(q0, dtype=torch.float32)
+        if (trans0.dim() != 2 or q0.dim() != 2 or trans0.shape[1] != 3 or q0.shape[1] != 4
+                or trans0.shape[0] != q0.shape[0] or trans0.shape[0] == 0):
+            raise ValueError("ModelPoseBatch: trans0 must be (K, 3) and q0 (K, 4) with the same K >= 1; got "
+                             f"{tuple(trans0.shape)} and {tuple(q0.shape)}")
+        assert intrins.size() == torch.Size([3, 3])
+        self.device = device
+        self.points = torch.as_tensor(points, dtype=torch.float32).to(self.device)
+        self.trans = nn.Parameter(trans0.to(self.device))
+        self.quat = nn.Parameter(q0.to(self.device))
+        self.K = torch.as_tensor(intrins, dtype=torch.float32).to(self.device)
+        self.img_width, self.img_height = float(img_width), float(img_height)
+        self.eps = 1e-6
+        self.pc_clip_limits = [min_dist, max_dist]
+        self.group = group            # torch.distributed group when `points` is this rank's shard
+        # the objective is a sum over the points, so their order is free: the kernels read a Morton-ordered copy made
+        # once per cloud, whose tile boxes let them skip (box, pose) pairs that are exactly zero
+        self.spatial_sort = spatial_sort
+        self.totals = None
+        self.losses = None
+        self._mean = None
+        self._pts32 = None
+        self._perm = None
+        self._boxes = None
+        self._ws = None
+        self.to(self.device)
+
+    def forward(self, debug=False, hpr=False):
+        t0 = time()
+        cloud = self._cloud()
+        weight = None
+        if hpr:  # ModelPose's mask: HPR of the untransformed cloud, in the caller's order, then into the cloud's order
+            weight = hidden_pts_removal(self.points.detach(), device=self.device)[1]
+            weight = ops._BACKEND.prepare(weight, cloud.device, "weight").reshape(-1)
+            if self._perm is not None:
+                weight = weight.index_select(0, self._perm.long())
+        with ops.evaluation(dense=None if self.spatial_sort else True):
+            ws = self._kept_workspace(cloud, ops._BACKEND.pose_batch_workspace_bytes(cloud, self.trans.shape[0]))
+            totals = ops.coverage_pose_batch(cloud, self.trans, self.quat, self.K, self.img_width, self.img_height,
+                                             self.pc_clip_limits[0], self.pc_clip_limits[1], self.eps, weight=weight,
+                                             group=self.group, boxes=self._boxes, presorted=True, workspace=ws)
+        self.totals = totals
+        if debug:
+            if totals.is_cuda:
+                torch.cuda.synchronize(totals.device)
+            print(f"\nBatched visibility estimation of {totals.shape[0]} poses took: {1000 * (time() - t0)} msec")
+        return self.criterion(totals)
+
+    def criterion(self, totals):
+        self.losses = 1.0 / (totals + self.eps)
+        return self.losses.sum()

@@ -218,6 +218,29 @@ class CudaBackend:
         _call("cov_pose_epilogue", acc, _ptr(acc), _ptr(t), _ptr(q), _ptr(out))
         return out
 
+    def pose_batch_workspace_bytes(self, pts, K):
+        opts = _opts()
+        return _lib.lib().cov_pose_batch_workspace_bytes(pts.shape[0], K, ctypes.byref(opts))
+
+    def pose_batch_fused(self, pts, T, Q, Kd, cam, w, boxes=None, ws=None):
+        """This cloud's COV_POSE_ACC sums of each of the K poses: (K * 8) fp64 (cov_pose_batch_fused)."""
+        K, n, dev = T.shape[0], pts.shape[0], pts.device
+        ws_bytes = self.pose_batch_workspace_bytes(pts, K)
+        if ws is None or ws.numel() < ws_bytes or ws.device != dev:
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        acc = torch.empty(K * _lib.POSE_ACC, dtype=torch.float64, device=dev)
+        opts = _opts()
+        _call("cov_pose_batch_fused", pts, _ptr(pts), n, _ptr(w), _ptr(T), _ptr(Q), K, _ptr(Kd), ctypes.byref(cam),
+              _ptr(boxes), _ptr(acc), ctypes.byref(opts), _ptr(ws), ws.numel())
+        return acc
+
+    def pose_batch_epilogue(self, acc, Q):
+        """(K, 8) fp32: per pose [total | d total/d trans (3) | d total/d quat (4)] from the summed sums."""
+        K = Q.shape[0]
+        out = torch.empty(K, 8, dtype=torch.float32, device=acc.device)
+        _call("cov_pose_batch_epilogue", acc, _ptr(acc), _ptr(Q), K, _ptr(out))
+        return out
+
     def traj_workspace_bytes(self, pts, W):
         return _lib.lib().cov_traj_workspace_bytes(pts.shape[0], W)
 
@@ -359,6 +382,34 @@ class CoveragePoseFn(torch.autograd.Function):
         ts, qs = ctx.shapes
         return (None, None if g_t is None else g_t.reshape(ts), None if g_q is None else g_q.reshape(qs),
                 None, None, None, None)
+
+
+class CoveragePoseBatchFn(torch.autograd.Function):
+    """totals_k = sum_j obs_j(pose k) for K candidate poses on one cloud, each as CoveragePoseFn computes its total, and
+    d totals_k / d (trans_k, quat_k) from the same pass (cov_pose_batch_fused).  No per-point output exists, so the
+    backward is g_k times the stored gradient rows: no second pass."""
+
+    @staticmethod
+    def forward(ctx, pts, trans, quats, K, cam, weight, group, boxes, workspace):
+        B = _BACKEND
+        dev = pts.device
+        T = B.prepare(trans, dev, "trans").reshape(-1, 3)
+        Q = B.prepare(quats, dev, "quats").reshape(-1, 4)
+        Kd = B.prepare(K, dev, "intrins").reshape(9)
+        acc = B.pose_batch_fused(pts, T, Q, Kd, cam, weight, boxes, workspace)   # this shard's sums, K x 8 doubles
+        if group is not None:
+            _all_reduce(acc, _reduce_ops()[2], group)
+        out = B.pose_batch_epilogue(acc, Q)
+        ctx.shapes = (trans.shape, quats.shape)
+        ctx.save_for_backward(out)
+        return out[:, 0].clone()
+
+    @staticmethod
+    def backward(ctx, g_totals):
+        (out,) = ctx.saved_tensors
+        ts, qs = ctx.shapes
+        g = g_totals.reshape(-1, 1).to(out.dtype)
+        return None, (g * out[:, 1:4]).reshape(ts), (g * out[:, 4:8]).reshape(qs), None, None, None, None, None, None
 
 
 class CoverageTrajFn(torch.autograd.Function):
@@ -523,6 +574,38 @@ def coverage_pose(points, trans, quat, intrins, img_width, img_height, min_dist=
     differentiable w.r.t. trans (.., 3) and quat (.., 4) (w, x, y, z)."""
     cam = _lib.camera(img_width, img_height, min_dist, max_dist, eps)
     return CoveragePoseFn.apply(points, trans, quat, intrins, cam, weight, group)
+
+
+def coverage_pose_batch(points, trans, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
+                        weight=None, group=None, boxes=None, presorted=False, workspace=None):
+    """The ModelPose objective of K candidate poses on one cloud: trans (K, 3), quats (K, 4) -> totals (K,) fp32, where
+    totals[k] is the total `coverage_pose(points, trans[k], quats[k], weight=weight)` returns.  `totals` is differentiable
+    w.r.t. `trans` and `quats`; all K totals and their gradients come from one pass over the cloud (cov_pose_batch_fused),
+    so a backward of any weighted sum of the totals costs no further pass.
+    The cloud is Morton-ordered first (no per-point output exists, so the order is free) unless `presorted` or `boxes`
+    are given; `weight` (N,) is in the order of `points` as passed.  Callers that evaluate the same cloud repeatedly order
+    it once (`spatial_sort`, `tile_boxes`), permute their weight with the same permutation and pass `presorted=True`
+    and the boxes.  The boxes let the kernel skip (128-point box, pose) pairs that are exactly zero: that pays on clouds
+    much larger than the ~27 m reach of the default clip limits.  Dense mode comes from `evaluation(dense=True)`.
+    `group`: `points` (and `weight`) are THIS RANK'S slice of the cloud; the K x 8 sums are all-reduced.  No host
+    synchronisation: capturable in a CUDA graph.  `workspace`: a uint8 CUDA tensor kept by the caller across calls."""
+    B = _BACKEND
+    if (not isinstance(trans, torch.Tensor) or not isinstance(quats, torch.Tensor) or trans.dim() != 2
+            or quats.dim() != 2 or trans.shape[1] != 3 or quats.shape[1] != 4 or trans.shape[0] != quats.shape[0]
+            or trans.shape[0] == 0):
+        raise ValueError("coverage_pose_batch: trans must be (K, 3) and quats (K, 4) with the same K >= 1; got "
+                         f"{tuple(getattr(trans, 'shape', ()))} and {tuple(getattr(quats, 'shape', ()))}")
+    pts = B.prepare(points, what="points")
+    dev = pts.device
+    w = None if weight is None else B.prepare(weight, dev, "weight").reshape(-1)
+    if w is not None and w.shape[0] != pts.shape[0]:
+        raise ValueError(f"coverage_pose_batch: weight has {w.shape[0]} entries for {pts.shape[0]} points")
+    if not presorted and boxes is None and pts.shape[0] > 0:
+        pts, perm, boxes = B.order_cloud(pts, True)
+        if w is not None and perm is not None:
+            w = B.prepare(w.index_select(0, perm.long()), dev, "weight")   # weight[j] belongs to point perm[j]
+    cam = _lib.camera(img_width, img_height, min_dist, max_dist, eps)
+    return CoveragePoseBatchFn.apply(pts, trans, quats, intrins, cam, w, group, boxes, workspace)
 
 
 def coverage_traj(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
