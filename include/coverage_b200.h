@@ -178,6 +178,51 @@ int cov_sweep_epilogue(const double* acc_dev, const float* minmax_dev, const flo
                        int poses_per_traj, int64_t n_total, float* out_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Prior log-odds (map memory): score coverage on top of what earlier, executed paths observed.
+ * ref: no reference implementation; the fusion is OctoMap's: a point's fused log-odds x_j = prior_j + L_j, with
+ * L_j = sum_w lo_jw formed in fp32 in pose order exactly as without a prior (one fp32 add), and r_j = 1/(1 + expf(-x_j)).
+ * The min/max normalisers, the gate, the pruning and the per-pose terms do not change; a point no gated pair reaches
+ * gets sigmoid(prior_j), and G_j = r_j (1 - r_j) uses the shifted r_j.  A prior of all zeros gives the rewards of the
+ * entry points without a prior bit for bit (sigmoid(0) = 1/2 exactly).  Non-finite priors propagate; nothing checks them.
+ *   prior_dev      (n) fp32, 16-byte aligned, one per point, shared by every pose and trajectory of the call.
+ *                  cov_traj_*: indexed like rewards_dev and upstream_dev, i.e. in the CALLER'S order when
+ *                  reward_index_dev is given.  cov_sweep_*: indexed like xyz_dev (the cloud's order).
+ *   prior_sum_dev  1 double: sum_j sigmoid(prior_j) over this shard (cov_prior_reward_sum, once per prior state); it is
+ *                  the reward sum of the points no listed pose reaches, read on the device (no host synchronisation).
+ * With a sharded cloud each rank passes its slice of the prior and its own sum; the SUM all-reduce of the accumulators
+ * makes the sums global as before.
+ * cov_traj_minmax_prior: cov_traj_minmax whose pre-fill (opts->prefill_dev) writes sigmoid(prior_i), the value the
+ *   pruned pass B leaves in place for the points it does not store (pass rewards_prefilled = 1 to cov_traj_fused_prior).
+ * cov_traj_logodds: pass B's forward without the backward.  logodds_dev (n) fp32, indexed like rewards_dev, must hold
+ *   the prior (or zeros) on entry; the call adds L_j where L_j != 0, so that it holds x_j: sigmoid of it is the reward
+ *   cov_traj_fused_prior computes, bit for bit.  Folding an executed path into the map is prior := logodds.
+ *   Takes cov_traj_workspace_bytes(n, n_poses) of workspace and the same options and paths as cov_traj_fused.
+ * ------------------------------------------------------------------------------------------ */
+int cov_prior_reward_sum(const float* prior_dev, int64_t n, double* prior_sum_dev, void* stream);
+int cov_traj_minmax_prior(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev, int n_poses,
+                          const float* K_dev, const cov_camera* cam, const float* boxes_dev, float* minmax_dev,
+                          const float* prior_dev, const cov_traj_opts* opts, void* workspace_dev, size_t workspace_bytes,
+                          void* stream);
+int cov_traj_fused_prior(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev, int n_poses,
+                         const float* K_dev, const cov_camera* cam, const float* boxes_dev, const float* minmax_dev,
+                         const float* upstream_dev, const int32_t* reward_index_dev, float* rewards_dev, double* acc_dev,
+                         const float* prior_dev, const double* prior_sum_dev, const cov_traj_opts* opts,
+                         void* workspace_dev, size_t workspace_bytes, void* stream);
+int cov_traj_logodds(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev, int n_poses,
+                     const float* K_dev, const cov_camera* cam, const float* boxes_dev, const float* minmax_dev,
+                     const int32_t* reward_index_dev, float* logodds_dev, const cov_traj_opts* opts, void* workspace_dev,
+                     size_t workspace_bytes, void* stream);
+int cov_sweep_rewards_prior(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev, int n_traj,
+                            int poses_per_traj, const float* K_dev, const cov_camera* cam, const float* boxes_dev,
+                            const float* minmax_dev, double* sum_rewards_dev, const float* prior_dev,
+                            const double* prior_sum_dev, const cov_traj_opts* opts, void* workspace_dev,
+                            size_t workspace_bytes, void* stream);
+int cov_sweep_fused_prior(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev, int n_traj,
+                          int poses_per_traj, const float* K_dev, const cov_camera* cam, const float* boxes_dev,
+                          const float* minmax_dev, double* acc_dev, const float* prior_dev, const double* prior_sum_dev,
+                          const cov_traj_opts* opts, void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Batched ModelPose: K candidate poses (t_k, q~_k) on one cloud, for every k the COV_POSE_ACC sums cov_pose_fused
  * computes for pose k alone ([0] sum m, [1..3] F, [4..6] T, [7] 0), in one pass over the cloud per chunk of poses.
  * ref: src/model.py:98-127 per pose (multi-start pose optimisation, scoring of candidate views); no per-point output.

@@ -7,7 +7,7 @@ There is no CPU fallback: without the library or without a CUDA device the ops r
 """
 from . import _lib  # noqa: F401
 from .ops import (coverage_pose, coverage_traj, frustum_cull, spherical_flip, hpr_hull_mask,  # noqa: F401
-                  sweep_rewards, coverage_sweep, coverage_pose_batch)
+                  sweep_rewards, coverage_sweep, coverage_pose_batch, traj_logodds)
 
 __all__ = ["coverage_pose", "coverage_traj", "frustum_cull", "spherical_flip", "hpr_hull_mask", "sweep_rewards",
-           "coverage_sweep", "coverage_pose_batch"]
+           "coverage_sweep", "coverage_pose_batch", "traj_logodds"]

@@ -66,6 +66,15 @@ PROTOTYPES = {
     "cov_sweep_fused_workspace_bytes": (_sz, [_i64, _int, _int, _opts]),
     "cov_sweep_fused": (_int, [_vp, _i64, _vp, _vp, _int, _int, _vp, _cam, _vp, _vp, _vp, _opts, _vp, _sz, _vp]),
     "cov_sweep_epilogue": (_int, [_vp, _vp, _vp, _int, _int, _i64, _vp, _vp]),
+    "cov_prior_reward_sum": (_int, [_vp, _i64, _vp, _vp]),
+    "cov_traj_minmax_prior": (_int, [_vp, _i64, _vp, _vp, _int, _vp, _cam, _vp, _vp, _vp, _opts, _vp, _sz, _vp]),
+    "cov_traj_fused_prior": (_int, [_vp, _i64, _vp, _vp, _int, _vp, _cam, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _opts,
+                                    _vp, _sz, _vp]),
+    "cov_traj_logodds": (_int, [_vp, _i64, _vp, _vp, _int, _vp, _cam, _vp, _vp, _vp, _vp, _opts, _vp, _sz, _vp]),
+    "cov_sweep_rewards_prior": (_int, [_vp, _i64, _vp, _vp, _int, _int, _vp, _cam, _vp, _vp, _vp, _vp, _vp, _opts, _vp,
+                                       _sz, _vp]),
+    "cov_sweep_fused_prior": (_int, [_vp, _i64, _vp, _vp, _int, _int, _vp, _cam, _vp, _vp, _vp, _vp, _vp, _opts, _vp, _sz,
+                                     _vp]),
     "cov_peer_region_bytes": (_sz, [_int, _i64, _int]),
     "cov_peer_allreduce": (_int, [_int, _vp, _i64, C.POINTER(Peers), _sz, _vp]),
     "cov_rig_poses": (_int, [_vp, _int, _vp, _int, _vp, _vp, _vp]),

@@ -159,6 +159,15 @@ __device__ __forceinline__ float cov_logodds(float d, const float4& v4, const Co
     return COV_LN2_F * cov_lg2(qc * cov_rcp(1.f - qc));
 }
 
+// A point's reward from its fused log-odds x (prior + L): the expression every pass B and sweep kernel uses, so that a
+// reward computed anywhere (pre-fill, pass B, sweeps, sigma of the fused log-odds output) is the same float.
+__device__ __forceinline__ float cov_sigmoid(float x) { return 1.f / (1.f + expf(-x)); }
+__device__ __forceinline__ float4 cov_sigmoid4(float4 x) {
+    return make_float4(cov_sigmoid(x.x), cov_sigmoid(x.y), cov_sigmoid(x.z), cov_sigmoid(x.w));
+}
+// x = prior + L, one IEEE add (the fused log-odds output writes the same float)
+__device__ __forceinline__ float cov_fuse_prior(float prior, float L) { return __fadd_rn(prior, L); }
+
 // ---- packed fp32 pairs (sm_100: fma/mul/add/sub.rn.f32x2 -> FFMA2 / FMUL2 / FADD2) --------------------------------
 // One instruction does the IEEE round-to-nearest operation on both halves of a 64-bit register pair, at half the issue
 // rate of the scalar instruction: the same flop/s, HALF THE ISSUE SLOTS.  The evaluation is issue-bound (26 FP32-pipe
@@ -351,4 +360,4 @@ CovConst cov_make_const(const struct cov_camera* cam);
 int cov_sm_count_cached();
 int cov_sweep_rewards_dense(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj, int per_traj,
                             const float* K, const struct cov_camera* cam, const float* minmax, double* sum_rewards,
-                            void* stream);
+                            const float* prior, const double* prior_sum, void* stream);

@@ -19,11 +19,14 @@ size_t sweep_smem_bytes(int n_traj, int ppt_poses) {
     return (size_t)n_traj * ppt_poses * COV_ROW_F4 * sizeof(float4) + (size_t)n_traj * sizeof(double);
 }
 
-template <int PPT>
+// HAS_PRIOR: sum_j (sigmoid(prior_j + L_j) - sigmoid(prior_j)) per trajectory (the prior indexed like xyz), and
+// *prior_sum = sum_j sigmoid(prior_j) in place of 0.5 * n.
+template <int PPT, bool HAS_PRIOR>
 __global__ void __launch_bounds__(COV_THREADS, 2)
 cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restrict__ poses,
                  const float* __restrict__ quats, int n_traj, int per_traj, const float* __restrict__ K9, CovConst C,
-                 const float* __restrict__ mins, const float* __restrict__ maxs, double* __restrict__ sum_out) {
+                 const float* __restrict__ mins, const float* __restrict__ maxs, double* __restrict__ sum_out,
+                 const float* __restrict__ prior, const double* __restrict__ prior_sum) {
     extern __shared__ float4 smem4[];
     float4* ptab = smem4;
     const int W = n_traj * per_traj;
@@ -39,7 +42,7 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
     constexpr int T = COV_THREADS * PPT;
     const int64_t ntiles = (n + T - 1) / T;
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        float px[PPT], py[PPT], pz[PPT];
+        float px[PPT], py[PPT], pz[PPT], pr[PPT], r0[PPT];
         bool valid[PPT];
 #pragma unroll
         for (int s = 0; s < PPT; ++s) {
@@ -49,6 +52,10 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
             px[s] = valid[s] ? __ldg(xyz + j * 3) : 3.0e18f;  // past the end: m = 0 exactly, never gated
             py[s] = valid[s] ? __ldg(xyz + j * 3 + 1) : 3.0e18f;
             pz[s] = valid[s] ? __ldg(xyz + j * 3 + 2) : 3.0e18f;
+            if (HAS_PRIOR) {
+                pr[s] = __ldg(prior + j);
+                r0[s] = cov_sigmoid(pr[s]);
+            }
         }
         for (int t = 0; t < n_traj; ++t) {
             float L[PPT];
@@ -78,8 +85,13 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
             for (int s = 0; s < PPT; ++s) any_nz |= (valid[s] && L[s] != 0.f);
             if (__any_sync(kFull, any_nz)) {
 #pragma unroll
-                for (int s = 0; s < PPT; ++s)
-                    if (valid[s] && L[s] != 0.f) acc += 1.f / (1.f + expf(-L[s])) - 0.5f;
+                for (int s = 0; s < PPT; ++s) {
+                    if (HAS_PRIOR) {
+                        if (valid[s] && L[s] != 0.f) acc += cov_sigmoid(cov_fuse_prior(pr[s], L[s])) - r0[s];
+                    } else if (valid[s] && L[s] != 0.f) {
+                        acc += 1.f / (1.f + expf(-L[s])) - 0.5f;
+                    }
+                }
                 acc = cov_warp_sum(acc);
                 if (lane == 0 && acc != 0.f) atomicAdd(ssum + t, (double)acc);
             }
@@ -88,7 +100,7 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
     __syncthreads();
     for (int t = tid; t < n_traj; t += COV_THREADS) {
         double v = ssum[t];
-        if (blockIdx.x == 0) v += 0.5 * (double)n;
+        if (blockIdx.x == 0) v += HAS_PRIOR ? *prior_sum : 0.5 * (double)n;
         if (v != 0.0) atomicAdd(sum_out + t, v);
     }
 }
@@ -98,7 +110,7 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
 // Dense sweep (cov_traj_opts.dense); the pruned pipeline and the C entry point are in cov_traj.cu.
 int cov_sweep_rewards_dense(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
                             int per_traj, const float* K, const cov_camera* cam, const float* minmax,
-                            double* sum_rewards, void* stream) {
+                            double* sum_rewards, const float* prior, const double* prior_sum, void* stream) {
     if (!xyz || n <= 0 || !poses || !quats || n_traj <= 0 || per_traj <= 0 || !K || !cam || !minmax || !sum_rewards) {
         cov_set_error("cov_sweep_rewards: bad argument");
         return COV_ERR_ARG;
@@ -115,11 +127,11 @@ int cov_sweep_rewards_dense(const float* xyz, int64_t n, const float* poses, con
     constexpr int T = COV_THREADS * kSweepPpt;
     const int64_t ntiles = (n + T - 1) / T;
     const size_t smem_max = sweep_smem_bytes(chunk, per_traj);
+    const auto kern = prior ? cov_sweep_kernel<kSweepPpt, true> : cov_sweep_kernel<kSweepPpt, false>;
     // always the same value: two host threads with different trajectory counts cannot race between set and launch
-    cudaFuncSetAttribute(cov_sweep_kernel<kSweepPpt>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 256);
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 256);
     int per_sm = 1;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, cov_sweep_kernel<kSweepPpt>, COV_THREADS, smem_max) !=
-            cudaSuccess || per_sm < 1)
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, COV_THREADS, smem_max) != cudaSuccess || per_sm < 1)
         per_sm = 1;
     int64_t grid = (int64_t)per_sm * cov_sm_count_cached();
     if (grid > ntiles) grid = ntiles;
@@ -127,9 +139,9 @@ int cov_sweep_rewards_dense(const float* xyz, int64_t n, const float* poses, con
     for (int t0 = 0; t0 < n_traj; t0 += chunk) {
         const int nt = (n_traj - t0 < chunk) ? n_traj - t0 : chunk;
         const int w0 = t0 * per_traj;
-        cov_sweep_kernel<kSweepPpt><<<(unsigned)grid, COV_THREADS, sweep_smem_bytes(nt, per_traj), s>>>(
+        kern<<<(unsigned)grid, COV_THREADS, sweep_smem_bytes(nt, per_traj), s>>>(
             xyz, n, poses + 3 * (size_t)w0, quats + 4 * (size_t)w0, nt, per_traj, K, C, minmax + w0, minmax + W + w0,
-            sum_rewards + t0);
+            sum_rewards + t0, prior, prior_sum);
     }
     return cov_check_launch("cov_sweep_rewards");
 }

@@ -306,11 +306,13 @@ cov_traj_prepare_kernel(const float* __restrict__ xyz, int64_t nsamples, int64_t
 // (acc[W * STRIDE] starts at `sum_base` = 0.5 * n: what the unlisted points add to the reward sum) and sets ctrl[1] when
 // some pose has min_j m > 0; every block builds 64 rows of the pose table with the normalisation constants:
 // v3.w = qthr, v4 = (b/2, b, 1/b, a), v5.w = thr.
+// SUM_DEV: the sum starts at *sum_base_dev instead (sum_j sigmoid(prior_j), cov_prior_reward_sum).
+template <bool SUM_DEV>
 __global__ void __launch_bounds__(64)
 cov_traj_table_kernel(const float* __restrict__ poses, const float* __restrict__ quats, int W,
                       const float* __restrict__ K9, CovConst C, const float* __restrict__ minmax,
                       float4* __restrict__ table, int* __restrict__ ctrl, int ctrl_words, double* __restrict__ acc,
-                      double sum_base) {
+                      double sum_base, const double* __restrict__ sum_base_dev) {
     const int tid = threadIdx.x;
     if (blockIdx.x == 0) {
         int amin = 0;
@@ -319,7 +321,7 @@ cov_traj_table_kernel(const float* __restrict__ poses, const float* __restrict__
         for (int i = tid; i < ctrl_words; i += blockDim.x) ctrl[i] = (i == 1) ? amin : 0;
         if (acc) {
             for (int i = tid; i < W * COV_ACC_STRIDE; i += blockDim.x) acc[i] = 0.0;
-            if (tid == 0) acc[(size_t)W * COV_ACC_STRIDE] = sum_base;
+            if (tid == 0) acc[(size_t)W * COV_ACC_STRIDE] = SUM_DEV ? *sum_base_dev : sum_base;
         }
     }
     const int w = blockIdx.x * blockDim.x + tid;
@@ -374,14 +376,15 @@ __global__ void __launch_bounds__(256) cov_tile_boxes_kernel(const float* __rest
 // the own aggregates, then sum predecessors until one carries an inclusive prefix).  The list is a pure function of the
 // masks (deterministic).  Grid <= resident capacity, and every block publishes its aggregates before it waits for
 // anybody's, so every predecessor a block waits for has been (or is being) published.  `fill_dst` (pass B): the same
-// blocks write 1/2 to every reward.
+// blocks write 1/2 to every reward (HAS_PRIOR: sigmoid(prior_i), with pass B's expression).
 constexpr int kCullMaxIter = 32;  // chunks per block at most (the host sizes the grid accordingly)
 
+template <bool HAS_PRIOR>
 __global__ void __launch_bounds__(256)
 cov_cull_kernel(const float4* __restrict__ boxes, int boxes_per_tile, int64_t ntiles, const float4* __restrict__ table,
                 int W, const unsigned* __restrict__ enc, float inv_kd, unsigned* __restrict__ amask_g, int mask_stride,
                 int* __restrict__ worklist, int* __restrict__ ctrl, unsigned long long* __restrict__ desc,
-                float* __restrict__ fill_dst, int64_t fill_n) {
+                float* __restrict__ fill_dst, int64_t fill_n, const float* __restrict__ fill_prior) {
     extern __shared__ float4 v3s[];
     __shared__ unsigned char listed_s[kCullMaxIter][8];  // per own chunk and warp: which of the warp's 8 tiles are listed
     __shared__ int chunk_base[kCullMaxIter];
@@ -394,7 +397,14 @@ cov_cull_kernel(const float4* __restrict__ boxes, int boxes_per_tile, int64_t nt
     if (fill_dst) {  // fire-and-forget stores: they drain while the blocks cull
         const int64_t stride = (int64_t)gridDim.x * blockDim.x * 4;
         for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + tid) * 4; i < fill_n; i += stride) {
-            if (i + 4 <= fill_n && ((reinterpret_cast<uintptr_t>(fill_dst + i) & 15) == 0)) {
+            if (HAS_PRIOR) {
+                if (i + 4 <= fill_n && ((reinterpret_cast<uintptr_t>(fill_dst + i) & 15) == 0) &&
+                    ((reinterpret_cast<uintptr_t>(fill_prior + i) & 15) == 0)) {
+                    __stcs(reinterpret_cast<float4*>(fill_dst + i), cov_sigmoid4(__ldcs(reinterpret_cast<const float4*>(fill_prior + i))));
+                } else {
+                    for (int64_t k = i; k < fill_n && k < i + 4; ++k) fill_dst[k] = cov_sigmoid(fill_prior[k]);
+                }
+            } else if (i + 4 <= fill_n && ((reinterpret_cast<uintptr_t>(fill_dst + i) & 15) == 0)) {
                 __stcs(reinterpret_cast<float4*>(fill_dst + i), make_float4(0.5f, 0.5f, 0.5f, 0.5f));
             } else {
                 for (int64_t k = i; k < fill_n && k < i + 4; ++k) fill_dst[k] = 0.5f;
@@ -645,12 +655,13 @@ __device__ __forceinline__ void load_item_points(const Item& item, const float* 
 // A listed pose is evaluated when the cap ball (from the seed's extrema; any later value is tighter and valid) meets
 // the warp's box and one of its points.  Extrema meet per block in shared memory, then in the zero-initialised encoded
 // arrays; the last block decodes them into the caller's floats.
+template <bool HAS_PRIOR>
 __global__ void __launch_bounds__(COV_THREADS, 3)
 cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, CovConst C,
                              unsigned* __restrict__ enc, float* __restrict__ minmax_out, const float4* __restrict__ boxes,
                              const unsigned* __restrict__ amask_g, int mask_stride, const int* __restrict__ worklist,
                              int* __restrict__ ctrl, int64_t ntiles, unsigned long long* __restrict__ stats,
-                             float* __restrict__ fill_dst, int64_t fill_n) {
+                             float* __restrict__ fill_dst, int64_t fill_n, const float* __restrict__ fill_prior) {
     constexpr int PPT = kItemPpt;
     extern __shared__ float4 smem4[];                      // block minima | maxima (uint) | per-pose caps
     unsigned* smin = reinterpret_cast<unsigned*>(smem4);
@@ -668,13 +679,21 @@ cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
     const int nwords = (W + 31) >> 5;
     // Pre-fill of pass B's rewards with 1/2 under this kernel's idle memory bandwidth (cov_traj_opts.prefill_dev): the
     // warp that takes item i also writes slice i of the buffer (fire-and-forget streaming stores), in 16-byte units.
+    // HAS_PRIOR: sigmoid(prior_i) instead, from streaming 16-byte loads of the prior (same index as the buffer).
     const int64_t fill_q = (fill_n + 3) / 4;                                          // float4 slots (tail handled below)
     const int64_t fill_per_item = fill_dst ? (fill_q + (n_items > 0 ? n_items : 1) - 1) / (n_items > 0 ? n_items : 1) : 0;
     auto fill_slice = [&](int64_t q0, int64_t q1) {
         if (q1 > fill_q) q1 = fill_q;
         for (int64_t q = q0 + lane; q < q1; q += 32) {
-            if (q * 4 + 4 <= fill_n) __stcs(reinterpret_cast<float4*>(fill_dst) + q, make_float4(0.5f, 0.5f, 0.5f, 0.5f));
-            else for (int64_t k = q * 4; k < fill_n; ++k) fill_dst[k] = 0.5f;
+            if (HAS_PRIOR) {
+                if (q * 4 + 4 <= fill_n)
+                    __stcs(reinterpret_cast<float4*>(fill_dst) + q, cov_sigmoid4(__ldcs(reinterpret_cast<const float4*>(fill_prior) + q)));
+                else for (int64_t k = q * 4; k < fill_n; ++k) fill_dst[k] = cov_sigmoid(fill_prior[k]);
+            } else if (q * 4 + 4 <= fill_n) {
+                __stcs(reinterpret_cast<float4*>(fill_dst) + q, make_float4(0.5f, 0.5f, 0.5f, 0.5f));
+            } else {
+                for (int64_t k = q * 4; k < fill_n; ++k) fill_dst[k] = 0.5f;
+            }
         }
     };
     if (fill_dst && n_items == 0) {  // nothing listed: the warps of the grid share the whole buffer
@@ -1014,13 +1033,14 @@ __device__ __forceinline__ void fused_block_flush(const T* accs, int W, double* 
 }
 
 // ---- dense ----
-template <int PPT, bool HAS_UP>
+// HAS_PRIOR: r_j = sigmoid(prior_j + L_j), prior indexed like `rewards` (through out_index).
+template <int PPT, bool HAS_UP, bool HAS_PRIOR>
 __global__ void __launch_bounds__(COV_THREADS, 2)
 cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __restrict__ poses,
                       const float* __restrict__ quats, int W, const float* __restrict__ K9, CovConst C,
                       const float* __restrict__ minmax, const float* __restrict__ upstream,
                       const int32_t* __restrict__ out_index, float* __restrict__ rewards, double* __restrict__ acc,
-                      int seg_log2) {
+                      int seg_log2, const float* __restrict__ prior) {
     constexpr int T = tile_points(PPT);
     constexpr int RS = bit_stride(PPT);
     // shared memory: pose table | the tile's points (xyz interleaved) | G_j | gate bits | block accumulators
@@ -1084,7 +1104,12 @@ cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __r
         }
 #pragma unroll
         for (int s = 0; s < PPT; ++s) {
-            const float r = 1.f / (1.f + expf(-L[s]));
+            float x = L[s];
+            if (HAS_PRIOR && valid[s]) {
+                const int64_t j = tile * T + lbase + s * 32;
+                x = cov_fuse_prior(__ldg(prior + (out_index ? (int64_t)out_index[j] : j)), x);
+            }
+            const float r = 1.f / (1.f + expf(-x));
             float g = r * (1.f - r);
             if (valid[s]) {
                 const int64_t j = tile * T + lbase + s * 32;
@@ -1115,16 +1140,20 @@ cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __r
 // re-evaluation keeps most lanes busy.
 // `rewards` was pre-filled with 1/2, only other values are stored; the warps add sum_j (r_j - 1/2) of the listed
 // tiles to acc[W * STRIDE], which starts at 0.5 * n.
+// HAS_PRIOR: the pre-fill is sigmoid(prior_j) and the sum starts at sum_j sigmoid(prior_j); a listed point reads its
+// prior at the index its reward goes to (the gather HAS_UP makes for upstream_j), r_j = sigmoid(prior_j + L_j) is stored
+// where L_j != 0 and r_j - sigmoid(prior_j) is added.  G_j = r_j (1 - r_j) for every point, L_j = 0 included (a gated
+// pair with p exactly 1/2 adds nothing to L_j but still enters the backward).
 constexpr int kTilesMinBlocks = 3;            // resident blocks per SM the register allocation aims at
 
-template <bool HAS_UP>
+template <bool HAS_UP, bool HAS_PRIOR>
 __global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
 cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, CovConst C,
                             const float* __restrict__ upstream, const int32_t* __restrict__ out_index,
                             float* __restrict__ rewards, double* __restrict__ acc,
                             const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g, int mask_stride,
                             const int* __restrict__ worklist, int* __restrict__ ctrl, int64_t ntiles,
-                            unsigned long long* __restrict__ stats) {
+                            unsigned long long* __restrict__ stats, const float* __restrict__ prior) {
     constexpr int PPT = kItemPpt;
     __shared__ unsigned wgate[kWarps][kMaskWords];   // per warp: poses with a gated pair among its points (this item)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1168,6 +1197,25 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
         float G[PPT];
 #pragma unroll
         for (int s = 0; s < PPT; ++s) {
+            if (HAS_PRIOR) {
+                if (!valid[s]) {  // past the end of the cloud: never gated, G unused
+                    G[s] = 0.f;
+                    continue;
+                }
+                const int64_t j = item.j0 + s * 32 + lane;
+                const int64_t jo = out_index ? (item.whole ? (int64_t)item.perm[s * 32 + lane] : (int64_t)out_index[j]) : j;
+                const float pr = __ldg(prior + jo);
+                const float r0 = cov_sigmoid(pr);
+                float r = r0;
+                if (L[s] != 0.f) {
+                    r = cov_sigmoid(cov_fuse_prior(pr, L[s]));
+                    rewards[jo] = r;
+                }
+                G[s] = r * (1.f - r);
+                sum_r += (double)(r - r0);
+                if (HAS_UP) G[s] *= upstream[jo];
+                continue;
+            }
             float r = 0.5f;
             G[s] = 0.25f;  // exactly what the formulas below give for L = 0
             if (L[s] != 0.f) {
@@ -1218,11 +1266,14 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
 // sums of its points for the current trajectory, and when the trajectory changes it adds sum_j (sigmoid(L_j) - 1/2) to
 // that trajectory's total (fp64 shared atomic; the block adds its totals to the output at the end).  Trajectories no
 // pose of which is listed for an item contribute exactly 1/2 per point: 0.5 * n is added once.
+// HAS_PRIOR: sum_j (sigmoid(prior_j + L_j) - sigmoid(prior_j)) at a flush (the item's 128 priors, in the cloud's order,
+// read there), and *prior_sum = sum_j sigmoid(prior_j) in place of 0.5 * n.
+template <bool HAS_PRIOR>
 __global__ void __launch_bounds__(COV_THREADS, 3)
 cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, int per_traj,
                        int n_traj, CovConst C, const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g,
                        int mask_stride, const int* __restrict__ worklist, int* __restrict__ ctrl,
-                       double* __restrict__ sum_out) {
+                       double* __restrict__ sum_out, const float* __restrict__ prior, const double* __restrict__ prior_sum) {
     constexpr int PPT = kItemPpt;
     extern __shared__ float4 smem4[];
     double* ssum = reinterpret_cast<double*>(smem4);   // per-trajectory totals of this block
@@ -1243,8 +1294,16 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
             if (cur >= 0 && touched) {
                 float a = 0.f;
 #pragma unroll
-                for (int s = 0; s < PPT; ++s)
-                    if (valid[s] && L[s] != 0.f) a += 1.f / (1.f + expf(-L[s])) - 0.5f;
+                for (int s = 0; s < PPT; ++s) {
+                    if (HAS_PRIOR) {
+                        if (valid[s] && L[s] != 0.f) {
+                            const float pr = __ldg(prior + item.j0 + s * 32 + lane);
+                            a += cov_sigmoid(cov_fuse_prior(pr, L[s])) - cov_sigmoid(pr);
+                        }
+                    } else if (valid[s] && L[s] != 0.f) {
+                        a += 1.f / (1.f + expf(-L[s])) - 0.5f;
+                    }
+                }
                 a = cov_warp_sum(a);
                 if (lane == 0 && a != 0.f) atomicAdd(ssum + cur, (double)a);
             }
@@ -1273,7 +1332,7 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
     __syncthreads();
     for (int t = tid; t < n_traj; t += COV_THREADS) {
         double v = ssum[t];
-        if (blockIdx.x == 0) v += 0.5 * (double)n;
+        if (blockIdx.x == 0) v += HAS_PRIOR ? *prior_sum : 0.5 * (double)n;
         if (v != 0.0) atomicAdd(sum_out + t, v);
     }
 }
@@ -1287,11 +1346,15 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
 // `acc + t * COV_SWEEP_ACC_BLOCK(P)`: the layout cov_traj_fused writes for that trajectory alone (rows, then sum_j r_j).
 // The forward of a trajectory visits the same poses in the same order as pass B with W = P on the same item (same cull,
 // same box test), so its L, r_j and G_j — and the re-evaluated m of the backward — are bit-identical to pass B's.
+// HAS_PRIOR: at a flush r_j = sigmoid(prior_j + L_j) and r_j - sigmoid(prior_j) is added, with the item's 128 priors (in
+// the cloud's order) read there; the blocks start at sum_j sigmoid(prior_j) (cov_sweep_acc_init_kernel).
+template <bool HAS_PRIOR>
 __global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
 cov_sweep_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, int per_traj,
                              CovConst C, const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g,
                              int mask_stride, const int* __restrict__ worklist, int* __restrict__ ctrl, int64_t ntiles,
-                             double* __restrict__ acc, unsigned long long* __restrict__ stats) {
+                             double* __restrict__ acc, unsigned long long* __restrict__ stats,
+                             const float* __restrict__ prior) {
     constexpr int PPT = kItemPpt;
     __shared__ unsigned wgate[kWarps][kMaskWords];   // per warp: poses of the current trajectory with a gated pair
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1317,6 +1380,14 @@ cov_sweep_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
             float a = 0.f;
 #pragma unroll
             for (int s = 0; s < PPT; ++s) {
+                if (HAS_PRIOR) {
+                    const float pr = valid[s] ? __ldg(prior + item.j0 + s * 32 + lane) : 0.f;
+                    const float r0 = cov_sigmoid(pr);
+                    const float r = L[s] != 0.f ? cov_sigmoid(cov_fuse_prior(pr, L[s])) : r0;
+                    G[s] = r * (1.f - r);
+                    if (valid[s]) a += r - r0;
+                    continue;
+                }
                 float r = 0.5f;
                 G[s] = 0.25f;  // exactly what the formulas below give for L = 0
                 if (L[s] != 0.f) {
@@ -1383,10 +1454,16 @@ cov_sweep_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
 }
 
 // Every trajectory's accumulator block as pass B starts it: rows zero, the reward sum at `sum_base` (0.5 * n: what the
-// points no listed pose reaches add).
+// points no listed pose reaches add), or at *sum_base_dev (sum_j sigmoid(prior_j)) when that is given.
 __global__ void cov_sweep_acc_init_kernel(double* __restrict__ acc, int64_t count, int64_t block, double sum_base) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (int64_t)gridDim.x * blockDim.x)
         acc[i] = (i % block == block - 1) ? sum_base : 0.0;
+}
+__global__ void cov_sweep_acc_init_dev_kernel(double* __restrict__ acc, int64_t count, int64_t block,
+                                              const double* __restrict__ sum_base_dev) {
+    const double base = *sum_base_dev;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (int64_t)gridDim.x * blockDim.x)
+        acc[i] = (i % block == block - 1) ? base : 0.0;
 }
 
 // SURVEY.md App. A.2, one pose: fold the min/max-path terms into the accumulator row A and map (F, T) to (d/dt, d/dq~).
@@ -1442,6 +1519,124 @@ __global__ void cov_sweep_epilogue_kernel(const double* __restrict__ acc, const 
     const int t = i / per_traj, k = i - t * per_traj;
     traj_epilogue_pose(acc + (size_t)t * block + (size_t)k * COV_ACC_STRIDE, minmax[i], minmax[TP + i], quats + 4 * (size_t)i,
                        1.0 / n_total, out + n_traj + 3 * (size_t)i, out + n_traj + 3 * (size_t)TP + 4 * (size_t)i);
+}
+
+// ============================================ prior log-odds (map memory) ============================================
+// sum_j sigmoid(prior_j) in fp64 (the reward-sum base of the prior paths): grid-stride, warp and block sums, one fp64
+// atomic per block into the zeroed output.
+__global__ void __launch_bounds__(256) cov_prior_sum_kernel(const float* __restrict__ prior, int64_t n,
+                                                            double* __restrict__ out) {
+    __shared__ double red[8];
+    double v = 0.0;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+        v += (double)cov_sigmoid(__ldg(prior + i));
+    v = cov_warp_sum(v);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = 0.0;
+        for (int i = 0; i < 8; ++i) t += red[i];
+        atomicAdd(out, t);
+    }
+}
+
+// Fused log-odds output, pruned: pass B's forward (same work list, same box test, same pose order, hence the same L_j)
+// without the backward; out[jo] = out[jo] + L_j for the points with L_j != 0 (the caller pre-filled `out` with the prior,
+// indexed like the rewards), the x that pass B's sigmoid takes.
+__global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
+cov_traj_logodds_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, CovConst C,
+                              const int32_t* __restrict__ out_index, float* __restrict__ out,
+                              const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g, int mask_stride,
+                              const int* __restrict__ worklist, int* __restrict__ ctrl) {
+    constexpr int PPT = kItemPpt;
+    const int lane = threadIdx.x & 31;
+    const int n_items = ctrl[0] * kItemsPerTile;
+    const int nwords = (W + 31) >> 5;
+    for_each_item<true>(xyz, n, boxes, amask_g, mask_stride, out_index, worklist, n_items, ctrl + 3, [](int) {},
+                        [&](const Item& item) {
+        float px[PPT], py[PPT], pz[PPT], L[PPT];
+        bool valid[PPT];
+        load_item_points<false>(item, xyz, n, lane, px, py, pz, valid);
+#pragma unroll
+        for (int s = 0; s < PPT; ++s) L[s] = 0.f;
+        for (int c = 0; c < nwords; ++c) {
+            unsigned word = item.mask[c];
+            while (word) {
+                const int w = c * 32 + __ffs(word) - 1;
+                word &= word - 1;
+                const float4* row = table + (size_t)w * COV_ROW_F4;
+                const float4 v3 = __ldg(row + 3);
+                if (box_q2lb(item.box[0], item.box[1], v3) > v3.w) continue;
+                tiles_pose_iter<PPT, false>(row, v3, px, py, pz, L, C, nullptr);
+            }
+        }
+#pragma unroll
+        for (int s = 0; s < PPT; ++s) {
+            if (valid[s] && L[s] != 0.f) {
+                const int64_t j = item.j0 + s * 32 + lane;
+                const int64_t jo = out_index ? (item.whole ? (int64_t)item.perm[s * 32 + lane] : (int64_t)out_index[j]) : j;
+                out[jo] = cov_fuse_prior(out[jo], L[s]);
+            }
+        }
+    });
+}
+
+// Fused log-odds output, dense: every (point, pose) pair, the pose rows (with the normalisers, cov_norm_row) in shared
+// memory; the same gate and log-odds terms in pose order as the dense pass B, hence the same L_j.
+template <int PPT>
+__global__ void __launch_bounds__(COV_THREADS, 2)
+cov_traj_logodds_kernel(const float* __restrict__ xyz, int64_t n, const float* __restrict__ poses,
+                        const float* __restrict__ quats, int W, const float* __restrict__ K9, CovConst C,
+                        const float* __restrict__ minmax, const int32_t* __restrict__ out_index, float* __restrict__ out) {
+    extern __shared__ float4 smem4[];
+    const int tid = threadIdx.x;
+    for (int w = tid; w < W; w += COV_THREADS) {
+        float4* row = smem4 + (size_t)w * COV_ROW_F4;
+        cov_pose_row(poses + 3 * w, quats + 4 * w, K9, C, row);
+        cov_norm_row(row, minmax[w], minmax[W + w], row[3].w);  // conservative gate threshold in v3.w
+    }
+    __syncthreads();
+    constexpr int T = COV_THREADS * PPT;
+    const int64_t ntiles = (n + T - 1) / T;
+    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+        float px[PPT], py[PPT], pz[PPT], L[PPT];
+        bool valid[PPT];
+#pragma unroll
+        for (int s = 0; s < PPT; ++s) {
+            const int64_t j = tile * T + s * COV_THREADS + tid;
+            valid[s] = j < n;
+            px[s] = valid[s] ? __ldg(xyz + j * 3) : 3.0e18f;  // past the end: m = 0 exactly, never gated
+            py[s] = valid[s] ? __ldg(xyz + j * 3 + 1) : 3.0e18f;
+            pz[s] = valid[s] ? __ldg(xyz + j * 3 + 2) : 3.0e18f;
+            L[s] = 0.f;
+        }
+        for (int w = 0; w < W; ++w) {
+            const float4* row = smem4 + (size_t)w * COV_ROW_F4;
+            const float4 v0 = row[0], v1 = row[1], v2 = row[2], v3 = row[3];
+            float m[PPT];
+#pragma unroll
+            for (int s = 0; s < PPT; ++s) m[s] = cov_vis<false>(px[s], py[s], pz[s], v0, v1, v2, v3, C, nullptr);
+            float mmax = m[0];
+#pragma unroll
+            for (int s = 1; s < PPT; ++s) mmax = fmaxf(mmax, m[s]);
+            if (__any_sync(kFull, mmax >= v3.w)) {
+                const float4 v4 = row[4];
+#pragma unroll
+                for (int s = 0; s < PPT; ++s) {
+                    const float d = __fsub_rn(m[s], v4.w);
+                    if (d >= v4.x) L[s] += cov_logodds(d, v4, C);  // exactly p >= 0.5
+                }
+            }
+        }
+#pragma unroll
+        for (int s = 0; s < PPT; ++s) {
+            if (valid[s] && L[s] != 0.f) {
+                const int64_t j = tile * T + s * COV_THREADS + tid;
+                const int64_t jo = out_index ? (int64_t)out_index[j] : j;
+                out[jo] = cov_fuse_prior(out[jo], L[s]);
+            }
+        }
+    }
 }
 
 // ==================================================== host ====================================================
@@ -1600,10 +1795,11 @@ const float4* boxes_for_call(const float* xyz, int64_t n, const float* boxes_dev
 
 // cull + work list in one launch; every block must be resident (the blocks wait on one another's descriptors)
 int launch_cull(const float4* boxes, int ppt, int64_t ntiles, const TrajWorkspace& t, int W, const unsigned* enc,
-                float inv_kd, float* fill_dst, int64_t fill_n, cudaStream_t s) {
+                float inv_kd, float* fill_dst, int64_t fill_n, cudaStream_t s, const float* fill_prior = nullptr) {
     const size_t smem = (size_t)W * sizeof(float4);
+    const auto cull = fill_prior ? cov_cull_kernel<true> : cov_cull_kernel<false>;
     const int64_t nchunks = (ntiles + kChunkTiles - 1) / kChunkTiles;
-    const int64_t resident = (int64_t)blocks_per_sm(cov_cull_kernel, 256, smem) * cov_sm_count_cached();
+    const int64_t resident = (int64_t)blocks_per_sm(cull, 256, smem) * cov_sm_count_cached();
     int64_t want = nchunks;
     if (fill_dst) want = std::max<int64_t>(want, (int64_t)cov_sm_count_cached() * 4);  // enough stores in flight for the fill
     int64_t g = std::max<int64_t>(1, std::min<int64_t>(want, resident));
@@ -1613,8 +1809,8 @@ int launch_cull(const float4* boxes, int ppt, int64_t ntiles, const TrajWorkspac
         return COV_ERR_UNSUPPORTED;
     }
     const int grid = (int)g;
-    cov_cull_kernel<<<grid, 256, smem, s>>>(boxes, tile_boxes(ppt), ntiles, t.table, W, enc, inv_kd, t.amask,
-                                            mask_stride_words(W), t.worklist, t.ctrl, t.desc, fill_dst, fill_n);
+    cull<<<grid, 256, smem, s>>>(boxes, tile_boxes(ppt), ntiles, t.table, W, enc, inv_kd, t.amask, mask_stride_words(W),
+                                 t.worklist, t.ctrl, t.desc, fill_dst, fill_n, fill_prior);
     return COV_OK;
 }
 
@@ -1658,9 +1854,22 @@ extern "C" int cov_tile_boxes(const float* xyz, int64_t n, float* boxes, void* s
     return cov_check_launch("cov_tile_boxes");
 }
 
-extern "C" int cov_traj_minmax(const float* xyz, int64_t n, const float* poses, const float* quats, int W,
-                               const float* K, const cov_camera* cam, const float* boxes_dev, float* minmax,
-                               const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+// The prior (16-byte aligned, indexed like the rewards buffer) of the _prior entry points: present and aligned.
+static int check_prior(const char* who, const float* prior, const double* prior_sum, bool need_sum) {
+    if (!prior || (need_sum && !prior_sum)) {
+        cov_set_error("%s: null prior_dev or prior_sum_dev", who);
+        return COV_ERR_ARG;
+    }
+    if (((uintptr_t)prior) & 15) {
+        cov_set_error("%s: prior_dev must be 16-byte aligned", who);
+        return COV_ERR_ALIGN;
+    }
+    return COV_OK;
+}
+
+static int traj_minmax_impl(const float* xyz, int64_t n, const float* poses, const float* quats, int W, const float* K,
+                            const cov_camera* cam, const float* boxes_dev, float* minmax, const float* prior,
+                            const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
     const bool prune = !(opts && opts->dense) && n >= kDenseBelow;
     int rc = check_traj_args("cov_traj_minmax", xyz, n, poses, quats, W, K, cam, ws, ws_bytes, prune);
     if (rc) return rc;
@@ -1713,16 +1922,33 @@ extern "C" int cov_traj_minmax(const float* xyz, int64_t n, const float* poses, 
     }
     if ((rc = launch_cull(boxes, ppt_t, ntiles_t, t, W, t.enc, 1.f / C.kd, nullptr, 0, s)) != COV_OK) return rc;
     const size_t smem_t = (size_t)W * 12;
-    cov_traj_minmax_tiles_kernel<<<persistent_grid(cov_traj_minmax_tiles_kernel, smem_t, ntiles_t), COV_THREADS, smem_t, s>>>(
+    float* prefill = opts ? opts->prefill_dev : nullptr;
+    const auto tiles_kern = (prior && prefill) ? cov_traj_minmax_tiles_kernel<true> : cov_traj_minmax_tiles_kernel<false>;
+    tiles_kern<<<persistent_grid(tiles_kern, smem_t, ntiles_t), COV_THREADS, smem_t, s>>>(
         xyz, n, t.table, W, C, t.enc, minmax, boxes, t.amask, mask_stride_words(W), t.worklist, t.ctrl, ntiles_t,
-        opts ? opts->stats_dev : nullptr, opts ? opts->prefill_dev : nullptr, n);
+        opts ? opts->stats_dev : nullptr, prefill, n, prior);
     return cov_check_launch("cov_traj_minmax");
 }
 
-extern "C" int cov_traj_fused(const float* xyz, int64_t n, const float* poses, const float* quats, int W,
-                              const float* K, const cov_camera* cam, const float* boxes_dev, const float* minmax,
-                              const float* upstream, const int32_t* reward_index, float* rewards, double* acc,
-                              const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+extern "C" int cov_traj_minmax(const float* xyz, int64_t n, const float* poses, const float* quats, int W,
+                               const float* K, const cov_camera* cam, const float* boxes_dev, float* minmax,
+                               const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+    return traj_minmax_impl(xyz, n, poses, quats, W, K, cam, boxes_dev, minmax, nullptr, opts, ws, ws_bytes, stream);
+}
+
+extern "C" int cov_traj_minmax_prior(const float* xyz, int64_t n, const float* poses, const float* quats, int W,
+                                     const float* K, const cov_camera* cam, const float* boxes_dev, float* minmax,
+                                     const float* prior, const cov_traj_opts* opts, void* ws, size_t ws_bytes,
+                                     void* stream) {
+    const int rc = check_prior("cov_traj_minmax_prior", prior, nullptr, false);
+    if (rc) return rc;
+    return traj_minmax_impl(xyz, n, poses, quats, W, K, cam, boxes_dev, minmax, prior, opts, ws, ws_bytes, stream);
+}
+
+static int traj_fused_impl(const float* xyz, int64_t n, const float* poses, const float* quats, int W, const float* K,
+                           const cov_camera* cam, const float* boxes_dev, const float* minmax, const float* upstream,
+                           const int32_t* reward_index, float* rewards, double* acc, const float* prior,
+                           const double* prior_sum, const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
     const bool prune = !(opts && opts->dense) && n >= kDenseBelow;
     int rc = check_traj_args("cov_traj_fused", xyz, n, poses, quats, W, K, cam, ws, ws_bytes, prune);
     if (rc) return rc;
@@ -1749,17 +1975,21 @@ extern "C" int cov_traj_fused(const float* xyz, int64_t n, const float* poses, c
         // phase-2 parallelism: split each pose row over 2^seg_log2 lanes until there are >= 2 tasks per thread
         int seg_log2 = 0;
         while ((W << seg_log2) < 2 * COV_THREADS && (2 << seg_log2) <= bit_words(ppt_d) && seg_log2 < 5) ++seg_log2;
-#define LAUNCH_F(P, UP)                                                                                           \
-    {                                                                                                             \
-        const int grid = grid_for(cov_traj_fused_kernel<P, UP>, smem, ntiles);                                    \
-        cov_traj_fused_kernel<P, UP><<<grid, COV_THREADS, smem, s>>>(xyz, n, poses, quats, W, K, C, minmax, upstream, \
-                                                                     reward_index, rewards, acc, seg_log2);        \
+#define LAUNCH_F(P, UP, PR)                                                                                        \
+    {                                                                                                              \
+        const int grid = grid_for(cov_traj_fused_kernel<P, UP, PR>, smem, ntiles);                                 \
+        cov_traj_fused_kernel<P, UP, PR><<<grid, COV_THREADS, smem, s>>>(xyz, n, poses, quats, W, K, C, minmax,     \
+                                                                         upstream, reward_index, rewards, acc,     \
+                                                                         seg_log2, prior);                         \
     }
+#define LAUNCH_FP(UP, PR) \
+    if (ppt_d == 4) LAUNCH_F(4, UP, PR) else if (ppt_d == 2) LAUNCH_F(2, UP, PR) else LAUNCH_F(1, UP, PR)
         if (upstream) {
-            if (ppt_d == 4) LAUNCH_F(4, true) else if (ppt_d == 2) LAUNCH_F(2, true) else LAUNCH_F(1, true)
+            if (prior) { LAUNCH_FP(true, true) } else { LAUNCH_FP(true, false) }
         } else {
-            if (ppt_d == 4) LAUNCH_F(4, false) else if (ppt_d == 2) LAUNCH_F(2, false) else LAUNCH_F(1, false)
+            if (prior) { LAUNCH_FP(false, true) } else { LAUNCH_FP(false, false) }
         }
+#undef LAUNCH_FP
 #undef LAUNCH_F
         return cov_check_launch("cov_traj_fused");
     }
@@ -1768,28 +1998,113 @@ extern "C" int cov_traj_fused(const float* xyz, int64_t n, const float* poses, c
     static_assert(ppt == 4 && tile_points(ppt) == kItemsPerTile * kItemPts, "tile = 8 items");
     const int64_t ntiles = (n + tile_points(ppt) - 1) / tile_points(ppt);
     const float4* boxes = boxes_for_call(xyz, n, boxes_dev, t, s);
-    cov_traj_table_kernel<<<(W + 63) / 64, 64, 0, s>>>(poses, quats, W, K, C, minmax, t.table, t.ctrl,
-                                                       (int)(t.ctrl_bytes / sizeof(int)), acc, 0.5 * (double)n);
+    if (prior) {
+        cov_traj_table_kernel<true><<<(W + 63) / 64, 64, 0, s>>>(poses, quats, W, K, C, minmax, t.table, t.ctrl,
+                                                                 (int)(t.ctrl_bytes / sizeof(int)), acc, 0.0, prior_sum);
+    } else {
+        cov_traj_table_kernel<false><<<(W + 63) / 64, 64, 0, s>>>(poses, quats, W, K, C, minmax, t.table, t.ctrl,
+                                                                  (int)(t.ctrl_bytes / sizeof(int)), acc, 0.5 * (double)n,
+                                                                  nullptr);
+    }
     const bool prefilled = opts && opts->rewards_prefilled;
-    if ((rc = launch_cull(boxes, ppt, ntiles, t, W, nullptr, 0.f, prefilled ? nullptr : rewards, n, s)) != COV_OK) return rc;
+    if ((rc = launch_cull(boxes, ppt, ntiles, t, W, nullptr, 0.f, prefilled ? nullptr : rewards, n, s, prior)) != COV_OK)
+        return rc;
     // persistent warps: as many blocks as are resident; every warp draws 128-point items from a ticket counter
-    const auto tiles_kern = upstream ? cov_traj_fused_tiles_kernel<true> : cov_traj_fused_tiles_kernel<false>;
+    const auto tiles_kern = upstream ? (prior ? cov_traj_fused_tiles_kernel<true, true> : cov_traj_fused_tiles_kernel<true, false>)
+                                     : (prior ? cov_traj_fused_tiles_kernel<false, true> : cov_traj_fused_tiles_kernel<false, false>);
     tiles_kern<<<persistent_grid(tiles_kern, 0, ntiles), COV_THREADS, 0, s>>>(
         xyz, n, t.table, W, C, upstream, reward_index, rewards, acc, boxes, t.amask, mask_stride_words(W), t.worklist,
-        t.ctrl, ntiles, opts ? opts->stats_dev : nullptr);
+        t.ctrl, ntiles, opts ? opts->stats_dev : nullptr, prior);
     return cov_check_launch("cov_traj_fused");
 }
 
-extern "C" int cov_sweep_rewards(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
-                                 int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
-                                 const float* minmax, double* sum_rewards, const cov_traj_opts* opts, void* ws,
-                                 size_t ws_bytes, void* stream) {
+extern "C" int cov_traj_fused(const float* xyz, int64_t n, const float* poses, const float* quats, int W,
+                              const float* K, const cov_camera* cam, const float* boxes_dev, const float* minmax,
+                              const float* upstream, const int32_t* reward_index, float* rewards, double* acc,
+                              const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+    return traj_fused_impl(xyz, n, poses, quats, W, K, cam, boxes_dev, minmax, upstream, reward_index, rewards, acc,
+                           nullptr, nullptr, opts, ws, ws_bytes, stream);
+}
+
+extern "C" int cov_traj_fused_prior(const float* xyz, int64_t n, const float* poses, const float* quats, int W,
+                                    const float* K, const cov_camera* cam, const float* boxes_dev, const float* minmax,
+                                    const float* upstream, const int32_t* reward_index, float* rewards, double* acc,
+                                    const float* prior, const double* prior_sum, const cov_traj_opts* opts, void* ws,
+                                    size_t ws_bytes, void* stream) {
+    const int rc = check_prior("cov_traj_fused_prior", prior, prior_sum, true);
+    if (rc) return rc;
+    return traj_fused_impl(xyz, n, poses, quats, W, K, cam, boxes_dev, minmax, upstream, reward_index, rewards, acc,
+                           prior, prior_sum, opts, ws, ws_bytes, stream);
+}
+
+extern "C" int cov_prior_reward_sum(const float* prior, int64_t n, double* sum_out, void* stream) {
+    if (!prior || !sum_out || n < 0) {
+        cov_set_error("cov_prior_reward_sum: null pointer or negative size (n=%lld)", (long long)n);
+        return COV_ERR_ARG;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaMemsetAsync(sum_out, 0, sizeof(double), s);
+    if (n > 0) {
+        const int grid = (int)std::min<int64_t>((n + 255) / 256, (int64_t)cov_sm_count_cached() * 8);
+        cov_prior_sum_kernel<<<grid, 256, 0, s>>>(prior, n, sum_out);
+    }
+    return cov_check_launch("cov_prior_reward_sum");
+}
+
+extern "C" int cov_traj_logodds(const float* xyz, int64_t n, const float* poses, const float* quats, int W,
+                                const float* K, const cov_camera* cam, const float* boxes_dev, const float* minmax,
+                                const int32_t* reward_index, float* logodds, const cov_traj_opts* opts, void* ws,
+                                size_t ws_bytes, void* stream) {
+    const bool prune = !(opts && opts->dense) && n >= kDenseBelow;
+    int rc = check_traj_args("cov_traj_logodds", xyz, n, poses, quats, W, K, cam, ws, ws_bytes, prune);
+    if (rc) return rc;
+    if (!minmax || !logodds) {
+        cov_set_error("cov_traj_logodds: null minmax/logodds");
+        return COV_ERR_ARG;
+    }
+    if ((boxes_dev && (((uintptr_t)boxes_dev) & 15)) || (reward_index && (((uintptr_t)reward_index) & 15))) {
+        cov_set_error("cov_traj_logodds: boxes and reward_index must be 16-byte aligned");
+        return COV_ERR_ALIGN;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    const CovConst C = cov_make_const(cam);
+    if (!prune) {
+        constexpr int ppt_d = 4;
+        const size_t smem = (size_t)W * COV_ROW_F4 * sizeof(float4);
+        if (smem > kSmemCap) {
+            cov_set_error("cov_traj_logodds: %d poses do not fit in shared memory", W);
+            return COV_ERR_UNSUPPORTED;
+        }
+        const int64_t ntiles = (n + COV_THREADS * ppt_d - 1) / (COV_THREADS * ppt_d);
+        const int grid = grid_for(cov_traj_logodds_kernel<ppt_d>, smem, ntiles);
+        cov_traj_logodds_kernel<ppt_d><<<grid, COV_THREADS, smem, s>>>(xyz, n, poses, quats, W, K, C, minmax, reward_index,
+                                                                       logodds);
+        return cov_check_launch("cov_traj_logodds");
+    }
+    // pruned: pass B's table and cull (no accumulators, no pre-fill), then its forward over the listed tiles
+    constexpr int ppt = 4;
+    const int64_t ntiles = (n + tile_points(ppt) - 1) / tile_points(ppt);
+    const TrajWorkspace t = carve_workspace(ws, n, W);
+    const float4* boxes = boxes_for_call(xyz, n, boxes_dev, t, s);
+    cov_traj_table_kernel<false><<<(W + 63) / 64, 64, 0, s>>>(poses, quats, W, K, C, minmax, t.table, t.ctrl,
+                                                              (int)(t.ctrl_bytes / sizeof(int)), nullptr, 0.0, nullptr);
+    if ((rc = launch_cull(boxes, ppt, ntiles, t, W, nullptr, 0.f, nullptr, 0, s)) != COV_OK) return rc;
+    cov_traj_logodds_tiles_kernel<<<persistent_grid(cov_traj_logodds_tiles_kernel, 0, ntiles), COV_THREADS, 0, s>>>(
+        xyz, n, t.table, W, C, reward_index, logodds, boxes, t.amask, mask_stride_words(W), t.worklist, t.ctrl);
+    return cov_check_launch("cov_traj_logodds");
+}
+
+static int sweep_rewards_impl(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
+                              int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
+                              const float* minmax, double* sum_rewards, const float* prior, const double* prior_sum,
+                              const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
     if (!xyz || n <= 0 || !poses || !quats || n_traj <= 0 || per_traj <= 0 || !K || !cam || !minmax || !sum_rewards) {
         cov_set_error("cov_sweep_rewards: bad argument");
         return COV_ERR_ARG;
     }
     if (opts && opts->dense)
-        return cov_sweep_rewards_dense(xyz, n, poses, quats, n_traj, per_traj, K, cam, minmax, sum_rewards, stream);
+        return cov_sweep_rewards_dense(xyz, n, poses, quats, n_traj, per_traj, K, cam, minmax, sum_rewards, prior,
+                                       prior_sum, stream);
     // trajectories per launch: as many as the per-tile pose mask holds (32 * kMaskWords poses); the pose table stays in
     // global memory, the block keeps one fp64 total per trajectory in shared memory
     if (per_traj > 32 * kMaskWords) {
@@ -1817,14 +2132,36 @@ extern "C" int cov_sweep_rewards(const float* xyz, int64_t n, const float* poses
         const int w0 = t0 * per_traj, Wn = nt * per_traj;
         cudaMemcpyAsync(mm, minmax + w0, (size_t)Wn * sizeof(float), cudaMemcpyDeviceToDevice, s);
         cudaMemcpyAsync(mm + Wn, minmax + W + w0, (size_t)Wn * sizeof(float), cudaMemcpyDeviceToDevice, s);
-        cov_traj_table_kernel<<<(Wn + 63) / 64, 64, 0, s>>>(poses + 3 * (size_t)w0, quats + 4 * (size_t)w0, Wn, K, C, mm, t.table,
-                                                            t.ctrl, (int)(t.ctrl_bytes / sizeof(int)), nullptr, 0.0);
+        cov_traj_table_kernel<false><<<(Wn + 63) / 64, 64, 0, s>>>(poses + 3 * (size_t)w0, quats + 4 * (size_t)w0, Wn, K, C, mm,
+                                                                   t.table, t.ctrl, (int)(t.ctrl_bytes / sizeof(int)), nullptr,
+                                                                   0.0, nullptr);
         if (launch_cull(boxes, ppt, ntiles, t, Wn, nullptr, 0.f, nullptr, 0, s) != COV_OK) return COV_ERR_UNSUPPORTED;
         const size_t smem = (size_t)nt * sizeof(double);
-        cov_sweep_tiles_kernel<<<persistent_grid(cov_sweep_tiles_kernel, smem, ntiles), COV_THREADS, smem, s>>>(
-            xyz, n, t.table, Wn, per_traj, nt, C, boxes, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, sum_rewards + t0);
+        const auto kern = prior ? cov_sweep_tiles_kernel<true> : cov_sweep_tiles_kernel<false>;
+        kern<<<persistent_grid(kern, smem, ntiles), COV_THREADS, smem, s>>>(
+            xyz, n, t.table, Wn, per_traj, nt, C, boxes, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, sum_rewards + t0,
+            prior, prior_sum);
     }
     return cov_check_launch("cov_sweep_rewards");
+}
+
+extern "C" int cov_sweep_rewards(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
+                                 int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
+                                 const float* minmax, double* sum_rewards, const cov_traj_opts* opts, void* ws,
+                                 size_t ws_bytes, void* stream) {
+    return sweep_rewards_impl(xyz, n, poses, quats, n_traj, per_traj, K, cam, boxes_dev, minmax, sum_rewards, nullptr,
+                              nullptr, opts, ws, ws_bytes, stream);
+}
+
+extern "C" int cov_sweep_rewards_prior(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
+                                       int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
+                                       const float* minmax, double* sum_rewards, const float* prior,
+                                       const double* prior_sum, const cov_traj_opts* opts, void* ws, size_t ws_bytes,
+                                       void* stream) {
+    const int rc = check_prior("cov_sweep_rewards_prior", prior, prior_sum, true);
+    if (rc) return rc;
+    return sweep_rewards_impl(xyz, n, poses, quats, n_traj, per_traj, K, cam, boxes_dev, minmax, sum_rewards, prior,
+                              prior_sum, opts, ws, ws_bytes, stream);
 }
 
 extern "C" size_t cov_sweep_workspace_bytes(int64_t n, int n_traj, int per_traj) {
@@ -1851,10 +2188,10 @@ extern "C" size_t cov_sweep_fused_workspace_bytes(int64_t n, int n_traj, int per
     return sweep_fused_prunes(n, opts) ? cov_sweep_workspace_bytes(n, n_traj, per_traj) : sweep_fused_dense_bytes(n, per_traj);
 }
 
-extern "C" int cov_sweep_fused(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
-                               int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
-                               const float* minmax, double* acc, const cov_traj_opts* opts, void* ws, size_t ws_bytes,
-                               void* stream) {
+static int sweep_fused_impl(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
+                            int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
+                            const float* minmax, double* acc, const float* prior, const double* prior_sum,
+                            const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
     if (!xyz || n <= 0 || !poses || !quats || n_traj <= 0 || per_traj <= 0 || !K || !cam || !minmax || !acc || !ws) {
         cov_set_error("cov_sweep_fused: null pointer, empty cloud or no poses (n=%lld, n_traj=%d, poses_per_traj=%d)",
                       (long long)n, n_traj, per_traj);
@@ -1895,8 +2232,9 @@ extern "C" int cov_sweep_fused(const float* xyz, int64_t n, const float* poses, 
             const size_t w0 = (size_t)t * per_traj;
             cudaMemcpyAsync(mm, minmax + w0, (size_t)per_traj * sizeof(float), cudaMemcpyDeviceToDevice, s);
             cudaMemcpyAsync(mm + per_traj, minmax + TP + w0, (size_t)per_traj * sizeof(float), cudaMemcpyDeviceToDevice, s);
-            const int rc = cov_traj_fused(xyz, n, poses + 3 * w0, quats + 4 * w0, per_traj, K, cam, nullptr, mm, nullptr,
-                                          nullptr, rewards, acc + (size_t)t * block, &dense, ws, tws, stream);
+            const int rc = traj_fused_impl(xyz, n, poses + 3 * w0, quats + 4 * w0, per_traj, K, cam, nullptr, mm, nullptr,
+                                           nullptr, rewards, acc + (size_t)t * block, prior, prior_sum, &dense, ws, tws,
+                                           stream);
             if (rc) return rc;
         }
         return COV_OK;
@@ -1913,7 +2251,8 @@ extern "C" int cov_sweep_fused(const float* xyz, int64_t n, const float* poses, 
     {
         const int64_t count = (int64_t)n_traj * (int64_t)block;
         const int grid = (int)std::min<int64_t>((count + 255) / 256, (int64_t)cov_sm_count_cached() * 8);
-        cov_sweep_acc_init_kernel<<<grid, 256, 0, s>>>(acc, count, (int64_t)block, 0.5 * (double)n);
+        if (prior) cov_sweep_acc_init_dev_kernel<<<grid, 256, 0, s>>>(acc, count, (int64_t)block, prior_sum);
+        else cov_sweep_acc_init_kernel<<<grid, 256, 0, s>>>(acc, count, (int64_t)block, 0.5 * (double)n);
     }
     unsigned long long* stats = opts ? opts->stats_dev : nullptr;
     for (int t0 = 0; t0 < n_traj; t0 += chunk) {
@@ -1921,15 +2260,35 @@ extern "C" int cov_sweep_fused(const float* xyz, int64_t n, const float* poses, 
         const int w0 = t0 * per_traj, Wn = nt * per_traj;
         cudaMemcpyAsync(mm, minmax + w0, (size_t)Wn * sizeof(float), cudaMemcpyDeviceToDevice, s);
         cudaMemcpyAsync(mm + Wn, minmax + TP + w0, (size_t)Wn * sizeof(float), cudaMemcpyDeviceToDevice, s);
-        cov_traj_table_kernel<<<(Wn + 63) / 64, 64, 0, s>>>(poses + 3 * (size_t)w0, quats + 4 * (size_t)w0, Wn, K, C, mm,
-                                                            t.table, t.ctrl, (int)(t.ctrl_bytes / sizeof(int)), nullptr, 0.0);
+        cov_traj_table_kernel<false><<<(Wn + 63) / 64, 64, 0, s>>>(poses + 3 * (size_t)w0, quats + 4 * (size_t)w0, Wn, K, C,
+                                                                   mm, t.table, t.ctrl, (int)(t.ctrl_bytes / sizeof(int)),
+                                                                   nullptr, 0.0, nullptr);
         int rc = launch_cull(boxes, ppt, ntiles, t, Wn, nullptr, 0.f, nullptr, 0, s);
         if (rc != COV_OK) return rc;
-        cov_sweep_fused_tiles_kernel<<<persistent_grid(cov_sweep_fused_tiles_kernel, 0, ntiles), COV_THREADS, 0, s>>>(
+        const auto kern = prior ? cov_sweep_fused_tiles_kernel<true> : cov_sweep_fused_tiles_kernel<false>;
+        kern<<<persistent_grid(kern, 0, ntiles), COV_THREADS, 0, s>>>(
             xyz, n, t.table, Wn, per_traj, C, boxes, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, ntiles,
-            acc + (size_t)t0 * block, stats);
+            acc + (size_t)t0 * block, stats, prior);
     }
     return cov_check_launch("cov_sweep_fused");
+}
+
+extern "C" int cov_sweep_fused(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
+                               int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
+                               const float* minmax, double* acc, const cov_traj_opts* opts, void* ws, size_t ws_bytes,
+                               void* stream) {
+    return sweep_fused_impl(xyz, n, poses, quats, n_traj, per_traj, K, cam, boxes_dev, minmax, acc, nullptr, nullptr, opts,
+                            ws, ws_bytes, stream);
+}
+
+extern "C" int cov_sweep_fused_prior(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
+                                     int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
+                                     const float* minmax, double* acc, const float* prior, const double* prior_sum,
+                                     const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+    const int rc = check_prior("cov_sweep_fused_prior", prior, prior_sum, true);
+    if (rc) return rc;
+    return sweep_fused_impl(xyz, n, poses, quats, n_traj, per_traj, K, cam, boxes_dev, minmax, acc, prior, prior_sum, opts,
+                            ws, ws_bytes, stream);
 }
 
 extern "C" int cov_sweep_epilogue(const double* acc, const float* minmax, const float* quats, int n_traj, int per_traj,

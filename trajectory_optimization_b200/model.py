@@ -178,7 +178,55 @@ def _wps_quotient(poses0, vis_wps_dist):
 class _OrderedCloudModel(nn.Module):
     """What ModelTraj, ModelTrajBatch and ModelPoseBatch share: the Morton-ordered copy of `self.points` with its permutation and tile
     boxes (made once per state of the cloud), the kept workspace, and the release of the last autograd graph.
-    Subclasses set `points`, `spatial_sort`, `_pts32`, `_perm`, `_boxes`, `_ws` and `_mean` in their constructor."""
+    Subclasses set `points`, `spatial_sort`, `_pts32`, `_perm`, `_boxes`, `_ws` and `_mean` in their constructor.
+    ModelTraj and ModelTrajBatch also keep the prior log-odds (`_init_prior`)."""
+
+    _prior_in_cloud_order = False   # the kernels read the prior in the cloud's (Morton) order, not in that of `points`
+
+    def _init_prior(self, prior_logodds):
+        # The kernels read the model's own copy of the prior (`_prior`, in the order they index it) and sum_j sigmoid(
+        # prior_j) on the device (`_prior_sum`).  Like the cloud cache, both belong to ONE state of `prior_logodds`: keyed
+        # on identity and torch's version counter, rebuilt on the next forward when either changes.
+        self.prior_logodds = None if prior_logodds is None else torch.as_tensor(prior_logodds).to(self.device)
+        self._prior = None
+        self._prior_sum = None
+        self._prior_key = None
+
+    def _prior_state_key(self):
+        p = self.prior_logodds
+        return (id(p), p._version, id(self.points), self.points._version)
+
+    @torch.no_grad()
+    def _write_prior(self):
+        # into the same buffers when the shape allows (captured CUDA graphs hold their addresses)
+        pts = self._cloud()
+        q = ops._check_prior(self.prior_logodds, pts.shape[0], pts.device)
+        if not bool(torch.isfinite(q).all()):   # once per prior state (one host synchronisation)
+            raise ValueError("prior_logodds must be finite (clamp it, OctoMap-style, before handing it to the model)")
+        if self._prior_in_cloud_order and self._perm is not None:
+            q = q.index_select(0, self._perm.long())
+        if self._prior is None or self._prior.shape != q.shape or self._prior.device != q.device:
+            self._prior = torch.empty_like(q)
+            self._prior_sum = torch.empty(1, dtype=torch.float64, device=q.device)
+        self._prior.copy_(q)
+        self._prior_sum.copy_(ops._BACKEND.prior_sum(self._prior))
+        self._prior_key = self._prior_state_key()
+
+    def _prior_args(self):
+        """(prior as the kernels index it, sum_j sigmoid(prior_j) (1,) fp64), or (None, None) without a prior."""
+        if self.prior_logodds is None:
+            return None, None
+        if self._prior is None or self._prior_key != self._prior_state_key():
+            self._write_prior()
+        return self._prior, self._prior_sum
+
+    def set_prior_logodds(self, prior_logodds):
+        """Replace the prior log-odds (None: an empty map), (N,) fp32 in the order of `self.points`.  The model's copies
+        are rewritten now, at the same addresses when the shape is unchanged, so a CUDA graph captured WITH a prior
+        evaluates the new one on its next replay (a graph captured without a prior needs a new capture)."""
+        self.prior_logodds = None if prior_logodds is None else prior_logodds.to(self.device)
+        if self.prior_logodds is not None and self._prior is not None:
+            self._write_prior()
 
     def _cloud(self):
         # The ordered copy, its permutation and the tile boxes belong to ONE state of `self.points`: the cache is keyed
@@ -230,6 +278,8 @@ class _OrderedCloudModel(nn.Module):
         if self._boxes is not None and new_boxes is not None:
             self._boxes.copy_(new_boxes)
         self._pts32_key = (id(self.points), self.points._version)
+        if getattr(self, "prior_logodds", None) is not None and self._prior is not None:
+            self._write_prior()   # the prior copy follows the new permutation, in place
 
     def _kept_workspace(self, cloud, need):
         # one workspace per (cloud, size), kept across steps: nothing in it outlives a call
@@ -243,7 +293,7 @@ class _OrderedCloudModel(nn.Module):
 class ModelTraj(_OrderedCloudModel):
     def __init__(self, points, wps_poses, wps_quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0,
                  smoothness_weight=14.0, traj_length_weight=0.02, device=torch.device("cuda"), group=None,
-                 n_total=None, spatial_sort=True, fused_regularizers=False):
+                 n_total=None, spatial_sort=True, fused_regularizers=False, prior_logodds=None):
         super().__init__()
         assert wps_poses.dim() == wps_quats.dim()
         assert wps_poses.size()[1] == 3
@@ -283,6 +333,9 @@ class ModelTraj(_OrderedCloudModel):
         self._perm = None
         self._boxes = None
         self._ws = None
+        # Map memory: (N,) fp32 log-odds of what earlier paths observed, in the order of `self.points` (indexed like
+        # `rewards`); rewards_j = sigmoid(prior_j + sum_w lo_jw).  Folding an executed path in: `observed_logodds()`.
+        self._init_prior(prior_logodds)
         self.to(self.device)
 
     def _workspace(self, cloud):
@@ -302,11 +355,12 @@ class ModelTraj(_OrderedCloudModel):
         wps_step = self._wps_step(vis_wps_dist)
         # waypoints range(0, N_wps, wps_step) (src/model.py:217); the others get no visibility gradient
         cloud = self._cloud()
-        rewards, mean = ops.coverage_traj(cloud, self.poses[::wps_step], self.quats[::wps_step], self.K,
-                                          self.img_width, self.img_height, self.pc_clip_limits[0],
-                                          self.pc_clip_limits[1], self.eps, n_total=self.n_total, group=self.group,
-                                          reward_index=self._perm, boxes=self._boxes,
-                                          dense=None if self.spatial_sort else True, workspace=self._workspace(cloud))
+        prior, prior_sum = self._prior_args()
+        cam = ops._lib.camera(self.img_width, self.img_height, self.pc_clip_limits[0], self.pc_clip_limits[1], self.eps)
+        rewards, mean = ops.CoverageTrajFn.apply(cloud, self.poses[::wps_step], self.quats[::wps_step], self.K, cam,
+                                                 self.n_total, self.group, self._perm, self._boxes,
+                                                 None if self.spatial_sort else True, self._workspace(cloud), prior,
+                                                 prior_sum)
         self.rewards = rewards
         self._mean = mean
         if debug:
@@ -318,6 +372,19 @@ class ModelTraj(_OrderedCloudModel):
         if debug:
             print(f"Loss calculation took {1000 * (time() - t1)} msec")
         return loss
+
+    @torch.no_grad()
+    def observed_logodds(self, vis_wps_dist=0.5):
+        """prior_j + sum_w lo_jw over the waypoints forward() evaluates at this `vis_wps_dist`, (N,) fp32 in the order of
+        `self.points`, without gradients: sigmoid of it is `self.rewards`.  After executing the path,
+        `model.set_prior_logodds(model.observed_logodds())` folds what it saw into the map; clamping is the caller's."""
+        wps_step = self._wps_step(vis_wps_dist)
+        cloud = self._cloud()
+        prior, _ = self._prior_args()
+        return ops.traj_logodds(cloud, self.poses[::wps_step], self.quats[::wps_step], self.K, self.img_width,
+                                self.img_height, self.pc_clip_limits[0], self.pc_clip_limits[1], self.eps,
+                                prior_logodds=prior, reward_index=self._perm, boxes=self._boxes, group=self.group,
+                                dense=None if self.spatial_sort else True, workspace=self._workspace(cloud))
 
     def criterion(self, rewards):
         # src/model.py:244-260
@@ -347,11 +414,14 @@ class ModelTrajBatch(_OrderedCloudModel):
     and their gradients come from one differentiable sweep (ops.coverage_sweep) instead of T coverage_traj calls.
     Parameters `poses` (T, W, 3) and `quats` (T, W, 4); `forward()` returns sum_t loss_t, where loss_t is
     ModelTraj.criterion's loss of trajectory t.  The per-trajectory terms are kept as (T,) tensors in `self.losses`
-    ("vis", "l2", "smooth", "length"), the (T,) mean rewards in `self.means`."""
+    ("vis", "l2", "smooth", "length"), the (T,) mean rewards in `self.means`.  `prior_logodds` (N,) fp32, in the order
+    of `points`: the map memory every trajectory is scored on top of (see ModelTraj)."""
+
+    _prior_in_cloud_order = True    # the sweeps index the prior like the (Morton-ordered) cloud
 
     def __init__(self, points, wps_poses, wps_quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0,
                  smoothness_weight=14.0, traj_length_weight=0.02, device=torch.device("cuda"), group=None,
-                 n_total=None, spatial_sort=True):
+                 n_total=None, spatial_sort=True, prior_logodds=None):
         super().__init__()
         wps_poses = torch.as_tensor(wps_poses, dtype=torch.float32)
         wps_quats = torch.as_tensor(wps_quats, dtype=torch.float32)
@@ -383,6 +453,7 @@ class ModelTrajBatch(_OrderedCloudModel):
         self._perm = None
         self._boxes = None
         self._ws = None
+        self._init_prior(prior_logodds)
         self.to(self.device)
 
     def _wps_step(self, vis_wps_dist):
@@ -400,12 +471,19 @@ class ModelTrajBatch(_OrderedCloudModel):
     def forward(self, vis_wps_dist=0.5):
         wps_step = self._wps_step(vis_wps_dist)
         cloud = self._cloud()
+        prior, prior_sum = self._prior_args()
         P, Q = self.poses[:, ::wps_step], self.quats[:, ::wps_step]
         with ops.evaluation(dense=None if self.spatial_sort else True):
             ws = self._kept_workspace(cloud, ops._BACKEND.sweep_fused_workspace_bytes(cloud, P.shape[0], P.shape[1]))
-            means = ops.coverage_sweep(cloud, P, Q, self.K, self.img_width, self.img_height, self.pc_clip_limits[0],
-                                       self.pc_clip_limits[1], self.eps, n_total=self.n_total, group=self.group,
-                                       boxes=self._boxes, presorted=True, workspace=ws)
+            if prior is None:
+                means = ops.coverage_sweep(cloud, P, Q, self.K, self.img_width, self.img_height, self.pc_clip_limits[0],
+                                           self.pc_clip_limits[1], self.eps, n_total=self.n_total, group=self.group,
+                                           boxes=self._boxes, presorted=True, workspace=ws)
+            else:   # the kept sum_j sigmoid(prior_j): no reduction over the prior per step
+                cam = ops._lib.camera(self.img_width, self.img_height, self.pc_clip_limits[0], self.pc_clip_limits[1],
+                                      self.eps)
+                means = ops.CoverageSweepFn.apply(cloud, P, Q, self.K, cam, int(self.n_total or cloud.shape[0]),
+                                                  self.group, self._boxes, "points", ws, prior, prior_sum)
         self.means = means
         return self.criterion(means)
 

@@ -93,6 +93,27 @@ def _ptr(t):
     return ctypes.c_void_p(t.data_ptr() if t is not None else 0)
 
 
+def _check_prior(prior, n, device, what="prior_logodds"):
+    """A per-point prior log-odds tensor as the kernels take it: fp32, shape (n,), on the cloud's device; made contiguous
+    and 16-byte aligned (a copy only when it has to).  Shape, dtype and device errors raise ValueError naming `what`."""
+    if prior is None:
+        return None
+    if not isinstance(prior, torch.Tensor):
+        raise ValueError(f"{what} must be a torch.Tensor, got {type(prior).__name__}")
+    if prior.dtype != torch.float32:
+        raise ValueError(f"{what} must be float32, got {prior.dtype}")
+    if tuple(prior.shape) != (n,):
+        raise ValueError(f"{what} must have shape ({n},) (one log-odds per point), got {tuple(prior.shape)}")
+    if prior.device != device:
+        raise ValueError(f"{what} is on {prior.device}, the cloud on {device}")
+    prior = prior.detach()
+    if not prior.is_contiguous():
+        prior = prior.contiguous()
+    if prior.is_cuda and prior.data_ptr() % 16:
+        prior = prior.clone()
+    return prior
+
+
 def _all_reduce(t, op, group):
     if group is not None:
         import torch.distributed as dist
@@ -252,25 +273,50 @@ class CudaBackend:
         opts = _opts(dense)
         return bool(_lib.lib().cov_traj_prefill_applies(pts.shape[0], ctypes.byref(opts)))
 
-    def traj_minmax(self, pts, P, Q, Kd, cam, boxes=None, ws=None, dense=None, prefill=None):
+    def prior_sum(self, prior):
+        """sum_j sigmoid(prior_j) in fp64 on the device, (1,) (cov_prior_reward_sum): the reward-sum base of a prior."""
+        out = torch.empty(1, dtype=torch.float64, device=prior.device)
+        _call("cov_prior_reward_sum", prior, _ptr(prior), prior.shape[0], _ptr(out))
+        return out
+
+    def traj_minmax(self, pts, P, Q, Kd, cam, boxes=None, ws=None, dense=None, prefill=None, prior=None):
+        """`prior` (indexed like `prefill`): the pre-fill writes sigmoid(prior_i) instead of 1/2."""
         W = P.shape[0]
         minmax = torch.empty(2 * W, dtype=torch.float32, device=pts.device)
         ws = self.traj_workspace(pts, W) if ws is None else ws
         opts = _opts(dense, prefill=prefill)
+        if prior is not None and prefill is not None:
+            _call("cov_traj_minmax_prior", pts, _ptr(pts), pts.shape[0], _ptr(P), _ptr(Q), W, _ptr(Kd), ctypes.byref(cam),
+                  _ptr(boxes), _ptr(minmax), _ptr(prior), ctypes.byref(opts), _ptr(ws), ws.numel())
+            return minmax
         _call("cov_traj_minmax", pts, _ptr(pts), pts.shape[0], _ptr(P), _ptr(Q), W, _ptr(Kd), ctypes.byref(cam),
               _ptr(boxes), _ptr(minmax), ctypes.byref(opts), _ptr(ws), ws.numel())
         return minmax
 
     def traj_fused(self, pts, P, Q, Kd, cam, minmax, upstream, rewards, reward_index=None, boxes=None, ws=None,
-                   dense=None, prefilled=False):
+                   dense=None, prefilled=False, prior=None, prior_sum=None):
         W, n = P.shape[0], pts.shape[0]
         acc = torch.empty(W * _lib.ACC_STRIDE + 1, dtype=torch.float64, device=pts.device)
         ws = self.traj_workspace(pts, W) if ws is None else ws
         opts = _opts(dense, rewards_prefilled=prefilled)
+        if prior is not None:
+            _call("cov_traj_fused_prior", pts, _ptr(pts), n, _ptr(P), _ptr(Q), W, _ptr(Kd), ctypes.byref(cam), _ptr(boxes),
+                  _ptr(minmax), _ptr(upstream), _ptr(reward_index), _ptr(rewards), _ptr(acc), _ptr(prior), _ptr(prior_sum),
+                  ctypes.byref(opts), _ptr(ws), ws.numel())
+            return acc
         _call("cov_traj_fused", pts, _ptr(pts), n, _ptr(P), _ptr(Q), W, _ptr(Kd), ctypes.byref(cam), _ptr(boxes),
               _ptr(minmax), _ptr(upstream), _ptr(reward_index), _ptr(rewards), _ptr(acc), ctypes.byref(opts), _ptr(ws),
               ws.numel())
         return acc
+
+    def traj_logodds(self, pts, P, Q, Kd, cam, minmax, out, reward_index=None, boxes=None, ws=None, dense=None):
+        """out (pre-filled with the prior, indexed like the rewards) += L_j where L_j != 0 (cov_traj_logodds)."""
+        W, n = P.shape[0], pts.shape[0]
+        ws = self.traj_workspace(pts, W) if ws is None else ws
+        opts = _opts(dense)
+        _call("cov_traj_logodds", pts, _ptr(pts), n, _ptr(P), _ptr(Q), W, _ptr(Kd), ctypes.byref(cam), _ptr(boxes),
+              _ptr(minmax), _ptr(reward_index), _ptr(out), ctypes.byref(opts), _ptr(ws), ws.numel())
+        return out
 
     def sweep_minmax(self, pts, P, Q, Kd, cam, boxes=None):
         """Per-pose minima and maxima of all T*P poses of a sweep (pass A, one pose-table-full at a time)."""
@@ -290,14 +336,18 @@ class CudaBackend:
             minmax[W + w0:W + w1] = mm[w1 - w0:]
         return minmax
 
-    def sweep_sums(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax):
-        """sum_j rewards_j(t) over this cloud for every trajectory t (fp64)."""
+    def sweep_sums(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior=None, prior_sum=None):
+        """sum_j rewards_j(t) over this cloud for every trajectory t (fp64); `prior` in the cloud's order."""
         L = _lib.lib()
         n, dev = pts.shape[0], pts.device
         ws_bytes = L.cov_sweep_workspace_bytes(n, T, Pn)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         sums = torch.zeros(T, dtype=torch.float64, device=dev)
         opts = _opts()
+        if prior is not None:
+            _call("cov_sweep_rewards_prior", pts, _ptr(pts), n, _ptr(P), _ptr(Q), T, Pn, _ptr(Kd), ctypes.byref(cam),
+                  _ptr(boxes), _ptr(minmax), _ptr(sums), _ptr(prior), _ptr(prior_sum), ctypes.byref(opts), _ptr(ws), ws_bytes)
+            return sums
         _call("cov_sweep_rewards", pts, _ptr(pts), n, _ptr(P), _ptr(Q), T, Pn, _ptr(Kd), ctypes.byref(cam), _ptr(boxes),
               _ptr(minmax), _ptr(sums), ctypes.byref(opts), _ptr(ws), ws_bytes)
         return sums
@@ -313,14 +363,20 @@ class CudaBackend:
         opts = _opts(dense)
         return _lib.lib().cov_sweep_fused_workspace_bytes(pts.shape[0], T, Pn, ctypes.byref(opts))
 
-    def sweep_fused(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, ws=None):
-        """This cloud's pass-B accumulators of every trajectory: T blocks of 22 Pn + 1 doubles (cov_sweep_fused)."""
+    def sweep_fused(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, ws=None, prior=None, prior_sum=None):
+        """This cloud's pass-B accumulators of every trajectory: T blocks of 22 Pn + 1 doubles (cov_sweep_fused);
+        `prior` in the cloud's order."""
         n, dev = pts.shape[0], pts.device
         ws_bytes = self.sweep_fused_workspace_bytes(pts, T, Pn)
         if ws is None or ws.numel() < ws_bytes or ws.device != dev:
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         acc = torch.empty(T * (Pn * _lib.ACC_STRIDE + 1), dtype=torch.float64, device=dev)
         opts = _opts()
+        if prior is not None:
+            _call("cov_sweep_fused_prior", pts, _ptr(pts), n, _ptr(P), _ptr(Q), T, Pn, _ptr(Kd), ctypes.byref(cam),
+                  _ptr(boxes), _ptr(minmax), _ptr(acc), _ptr(prior), _ptr(prior_sum), ctypes.byref(opts), _ptr(ws),
+                  ws.numel())
+            return acc
         _call("cov_sweep_fused", pts, _ptr(pts), n, _ptr(P), _ptr(Q), T, Pn, _ptr(Kd), ctypes.byref(cam), _ptr(boxes),
               _ptr(minmax), _ptr(acc), ctypes.byref(opts), _ptr(ws), ws.numel())
         return acc
@@ -418,7 +474,9 @@ class CoverageTrajFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, points, poses, quats, K, cam, n_total, group, reward_index=None, boxes=None, dense=None,
-                workspace=None):
+                workspace=None, prior=None, prior_sum=None):
+        # prior / prior_sum: the checked (N,) prior log-odds in the order of the rewards and sum_j sigmoid(prior_j) of
+        # this shard ((1,) fp64 on the device), or None
         B = _BACKEND
         dev = points.device
         pts = B.prepare(points, what="points")
@@ -439,12 +497,15 @@ class CoverageTrajFn(torch.autograd.Function):
         rewards = torch.empty(n, dtype=torch.float32, device=dev)
         # the pruned pass A pre-fills pass B's rewards with 1/2 under its idle memory bandwidth
         prefill = rewards if B.prefill_applies(pts, dense) else None
-        minmax = B.traj_minmax(pts, P, Q, Kd, cam, boxes, ws, dense, prefill)   # pass A on this shard
+        if prior is None:
+            minmax = B.traj_minmax(pts, P, Q, Kd, cam, boxes, ws, dense, prefill)   # pass A on this shard
+        else:   # the pre-fill writes sigmoid(prior_i)
+            minmax = B.traj_minmax(pts, P, Q, Kd, cam, boxes, ws, dense, prefill, prior)
         _all_reduce_minmax(minmax, W, group)                 # global normalisers: W minima, W maxima
         out = CoverageTrajFn._run(pts, P, Q, Kd, cam, minmax, None, rewards, n_total, group, reward_index, boxes, ws,
-                                  dense, prefill is not None)
+                                  dense, prefill is not None, prior, prior_sum)
         ctx.cam, ctx.group, ctx.n_total, ctx.reward_index, ctx.boxes = cam, group, n_total, reward_index, boxes
-        ctx.dense = dense
+        ctx.dense, ctx.prior, ctx.prior_sum = dense, prior, prior_sum
         ctx.shapes = (poses.shape, quats.shape)
         ctx.save_for_backward(pts, P, Q, Kd, minmax, out)
         ctx.set_materialize_grads(False)
@@ -452,9 +513,13 @@ class CoverageTrajFn(torch.autograd.Function):
 
     @staticmethod
     def _run(pts, P, Q, Kd, cam, minmax, upstream, rewards, n_total, group, reward_index=None, boxes=None, ws=None,
-             dense=None, prefilled=False):
-        acc = _BACKEND.traj_fused(pts, P, Q, Kd, cam, minmax, upstream, rewards, reward_index, boxes, ws, dense,
-                                  prefilled)   # pass B
+             dense=None, prefilled=False, prior=None, prior_sum=None):
+        if prior is None:
+            acc = _BACKEND.traj_fused(pts, P, Q, Kd, cam, minmax, upstream, rewards, reward_index, boxes, ws, dense,
+                                      prefilled)   # pass B
+        else:
+            acc = _BACKEND.traj_fused(pts, P, Q, Kd, cam, minmax, upstream, rewards, reward_index, boxes, ws, dense,
+                                      prefilled, prior, prior_sum)
         _all_reduce_acc(acc, P.shape[0], group)
         return _BACKEND.traj_epilogue(acc, minmax, Q, n_total, 0 if upstream is None else 1)
 
@@ -470,12 +535,12 @@ class CoverageTrajFn(torch.autograd.Function):
             up = _BACKEND.prepare(g_rewards, pts.device, "grad_rewards").reshape(-1)
             scratch = torch.empty(pts.shape[0], dtype=torch.float32, device=pts.device)
             o2 = CoverageTrajFn._run(pts, P, Q, Kd, ctx.cam, minmax, up, scratch, ctx.n_total, ctx.group,
-                                     ctx.reward_index, ctx.boxes, None, ctx.dense)
+                                     ctx.reward_index, ctx.boxes, None, ctx.dense, False, ctx.prior, ctx.prior_sum)
             g_p = o2[1:1 + 3 * W] if g_p is None else g_p + o2[1:1 + 3 * W]
             g_q = o2[1 + 3 * W:] if g_q is None else g_q + o2[1 + 3 * W:]
         ps, qs = ctx.shapes
         return (None, None if g_p is None else g_p.reshape(ps), None if g_q is None else g_q.reshape(qs),
-                None, None, None, None, None, None, None, None)
+                None, None, None, None, None, None, None, None, None, None)
 
 
 class CoverageSweepFn(torch.autograd.Function):
@@ -483,7 +548,7 @@ class CoverageSweepFn(torch.autograd.Function):
     CoverageTrajFn evaluates them, and d means_t / d (poses_t, quats_t) from the same pass (cov_sweep_fused)."""
 
     @staticmethod
-    def forward(ctx, pts, poses, quats, K, cam, n_total, group, boxes, shard, workspace):
+    def forward(ctx, pts, poses, quats, K, cam, n_total, group, boxes, shard, workspace, prior=None, prior_sum=None):
         B = _BACKEND
         dev = pts.device
         T, Pn = poses.shape[0], poses.shape[1]
@@ -498,7 +563,8 @@ class CoverageSweepFn(torch.autograd.Function):
             nt = t1 - t0
             mine = torch.zeros(per * (1 + 7 * Pn), dtype=torch.float32, device=dev)
             if nt > 0:
-                o = CoverageSweepFn._run(pts, poses[t0:t1], quats[t0:t1], Kd, cam, n_total, None, boxes, workspace)
+                o = CoverageSweepFn._run(pts, poses[t0:t1], quats[t0:t1], Kd, cam, n_total, None, boxes, workspace, prior,
+                                         prior_sum)
                 mine[:nt] = o[:nt]
                 mine[per:per + 3 * nt * Pn] = o[nt:nt + 3 * nt * Pn]
                 mine[per + 3 * per * Pn:per + 3 * per * Pn + 4 * nt * Pn] = o[nt + 3 * nt * Pn:]
@@ -508,13 +574,13 @@ class CoverageSweepFn(torch.autograd.Function):
             out = torch.cat([every[:, :per].reshape(-1)[:T], every[:, per:per + 3 * per * Pn].reshape(-1)[:3 * T * Pn],
                              every[:, per + 3 * per * Pn:].reshape(-1)[:4 * T * Pn]])
         else:
-            out = CoverageSweepFn._run(pts, poses, quats, Kd, cam, n_total, group, boxes, workspace)
+            out = CoverageSweepFn._run(pts, poses, quats, Kd, cam, n_total, group, boxes, workspace, prior, prior_sum)
         ctx.shapes = (poses.shape, quats.shape)
         ctx.save_for_backward(out)
         return out[:T].clone()
 
     @staticmethod
-    def _run(pts, poses, quats, Kd, cam, n_total, group, boxes, workspace):
+    def _run(pts, poses, quats, Kd, cam, n_total, group, boxes, workspace, prior=None, prior_sum=None):
         B = _BACKEND
         dev = pts.device
         T, Pn = poses.shape[0], poses.shape[1]
@@ -522,7 +588,10 @@ class CoverageSweepFn(torch.autograd.Function):
         Q = B.prepare(quats, dev, "quats").reshape(-1, 4)
         minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)     # pass A on this shard, (2, T Pn)
         _all_reduce_minmax(minmax, T * Pn, group)
-        acc = B.sweep_fused(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, workspace)
+        if prior is None:
+            acc = B.sweep_fused(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, workspace)
+        else:
+            acc = B.sweep_fused(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, workspace, prior, prior_sum)
         if group is not None:
             # plain all-reduce: the in-kernel exchange buffers are sized for the 22 W + 1 doubles of one trajectory
             _all_reduce(acc, _reduce_ops()[2], group)
@@ -536,7 +605,7 @@ class CoverageSweepFn(torch.autograd.Function):
         g = g_means.reshape(T, 1).to(out.dtype)
         g_p = (g * out[T:T + 3 * T * Pn].reshape(T, 3 * Pn)).reshape(ps)
         g_q = (g * out[T + 3 * T * Pn:].reshape(T, 4 * Pn)).reshape(qs)
-        return None, g_p, g_q, None, None, None, None, None, None, None
+        return None, g_p, g_q, None, None, None, None, None, None, None, None, None
 
 
 class TrajRegularizersFn(torch.autograd.Function):
@@ -609,14 +678,56 @@ def coverage_pose_batch(points, trans, quats, intrins, img_width, img_height, mi
 
 
 def coverage_traj(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
-                  n_total=None, group=None, reward_index=None, boxes=None, dense=None, workspace=None):
+                  n_total=None, group=None, reward_index=None, boxes=None, dense=None, workspace=None,
+                  prior_logodds=None):
     """Fused ModelTraj visibility term over the W poses given.  Returns (rewards (N,), mean(rewards)).
     `reward_index` (int32, from `spatial_sort`): `points` is a reordered copy of the caller's cloud and
     rewards come back in the caller's order.  `boxes` (from `tile_boxes(points)`): built once per cloud so the
     pruned kernels do not rebuild them on every call.  `dense=True`: evaluate every pair (no pruning; what an unordered
-    cloud should ask for).  `workspace`: a uint8 CUDA tensor kept by the caller across calls (one per cloud)."""
+    cloud should ask for).  `workspace`: a uint8 CUDA tensor kept by the caller across calls (one per cloud).
+    `prior_logodds` (N,) fp32: what earlier paths observed (map memory, e.g. `traj_logodds` of an executed path);
+    rewards_j = sigmoid(prior_j + sum_w lo_jw), indexed like the rewards (the caller's order when `reward_index` is
+    given).  With a `group` it is this rank's slice.  None = an empty map (exactly the rewards of a zero prior)."""
     cam = _lib.camera(img_width, img_height, min_dist, max_dist, eps)
-    return CoverageTrajFn.apply(points, poses, quats, intrins, cam, n_total, group, reward_index, boxes, dense, workspace)
+    prior = psum = None
+    if prior_logodds is not None:
+        pts = _BACKEND.prepare(points, what="points")
+        prior = _check_prior(prior_logodds, pts.shape[0], pts.device)
+        psum = _BACKEND.prior_sum(prior)
+    return CoverageTrajFn.apply(points, poses, quats, intrins, cam, n_total, group, reward_index, boxes, dense, workspace,
+                                prior, psum)
+
+
+@torch.no_grad()
+def traj_logodds(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
+                 prior_logodds=None, reward_index=None, boxes=None, group=None, dense=None, workspace=None):
+    """The fused log-odds prior_j + sum_w lo_jw of the W poses given, (N,) fp32 in the caller's order (as `rewards` of
+    `coverage_traj`), without gradients: sigmoid of it is `coverage_traj(..., prior_logodds=prior_logodds)`'s rewards,
+    bit for bit.  Folding an executed path into the map is `prior = traj_logodds(..., prior_logodds=prior)`; clamping
+    (OctoMap's thresholds) is the caller's, in torch.  Arguments as for `coverage_traj`; with a `group`, `points` and
+    `prior_logodds` are this rank's slices (the normalisers are all-reduced) and so is the result."""
+    B = _BACKEND
+    pts = B.prepare(points, what="points")
+    dev, n = pts.device, pts.shape[0]
+    if reward_index is not None and (reward_index.dtype != torch.int32 or reward_index.shape[0] != n
+                                     or reward_index.device != dev or not reward_index.is_contiguous()):
+        raise ValueError("reward_index must be a contiguous int32 tensor with one entry per point, on the cloud's device")
+    prior = _check_prior(prior_logodds, n, dev)
+    P = B.prepare(poses, dev, "poses").reshape(-1, 3)
+    Q = B.prepare(quats, dev, "quats").reshape(-1, 4)
+    Kd = B.prepare(intrins, dev, "intrins").reshape(9)
+    W = P.shape[0]
+    if Q.shape[0] != W:
+        raise ValueError("poses and quats disagree on the number of waypoints")
+    cam = _lib.camera(img_width, img_height, min_dist, max_dist, eps)
+    dense = _MODE.dense if dense is None else bool(dense)
+    ws = workspace
+    if ws is None or ws.numel() < B.traj_workspace_bytes(pts, W) or ws.device != dev:
+        ws = B.traj_workspace(pts, W)
+    minmax = B.traj_minmax(pts, P, Q, Kd, cam, boxes, ws, dense)
+    _all_reduce_minmax(minmax, W, group)
+    out = torch.zeros(n, dtype=torch.float32, device=dev) if prior is None else prior.clone()
+    return B.traj_logodds(pts, P, Q, Kd, cam, minmax, out, reward_index, boxes, ws, dense)
 
 
 @torch.no_grad()
@@ -666,9 +777,24 @@ def sort_pairs(keys, vals, begin_bit=0, end_bit=32):
     return k, v
 
 
+def _order_with_prior(B, pts, prior, boxes, presorted):
+    """The sweeps' cloud ordering (Morton order unless `presorted` or `boxes`), the prior permuted with the cloud."""
+    if not presorted and boxes is None and pts.shape[0] > 0:
+        pts, perm, boxes = B.order_cloud(pts, True)
+        if prior is not None and perm is not None:
+            prior = _check_prior(prior.index_select(0, perm.long()), pts.shape[0], pts.device)   # prior[j] of point perm[j]
+    return pts, prior, boxes
+
+
+def _sweep_sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum):
+    if prior is None:
+        return B.sweep_sums(pts, P, Q, T, Pn, Kd, cam, boxes, minmax)
+    return B.sweep_sums(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum)
+
+
 @torch.no_grad()
 def sweep_rewards(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
-                  n_total=None, group=None, boxes=None, presorted=False, shard="points"):
+                  n_total=None, group=None, boxes=None, presorted=False, shard="points", prior_logodds=None):
     """Forward-only mean reward of many candidate trajectories: poses (T, P, 3), quats (T, P, 4) -> (T,) fp64
     (semantics: ModelTraj.forward per trajectory with every pose evaluated, reference src/model.py:217-237).
     The cloud is Morton-ordered first (no per-point output exists, so the order is free) unless `presorted`;
@@ -679,13 +805,19 @@ def sweep_rewards(points, poses, quats, intrins, img_width, img_height, min_dist
                             2 T P floats) and the per-trajectory sums are all-reduced (SUM of T doubles);
       shard="trajectories"  every rank holds the WHOLE cloud (it fits: 50 M points = 600 MB) and evaluates its own
                             contiguous block of T / world trajectories — no collective on the data path, one all-gather
-                            of T doubles at the end.  The choice when the cloud fits one GPU."""
+                            of T doubles at the end.  The choice when the cloud fits one GPU.
+
+    `prior_logodds` (N,) fp32: per-point prior log-odds (map memory), shared by every trajectory: each trajectory's
+    rewards are sigmoid(prior_j + sum_w lo_jw).  In the order of `points` as passed (permuted with the cloud when the
+    call orders it; with `presorted`, already in the cloud's order); shard="points": this rank's slice,
+    shard="trajectories": the whole prior on every rank."""
     B = _BACKEND
     if shard not in ("points", "trajectories"):
         raise ValueError("shard must be 'points' or 'trajectories'")
     pts = B.prepare(points, what="points")
-    if not presorted and boxes is None and pts.shape[0] > 0:
-        pts, _, boxes = B.order_cloud(pts, True)
+    prior = _check_prior(prior_logodds, pts.shape[0], pts.device)
+    pts, prior, boxes = _order_with_prior(B, pts, prior, boxes, presorted)
+    psum = None if prior is None else B.prior_sum(prior)
     dev = pts.device
     T, Pn = poses.shape[0], poses.shape[1]
     n = pts.shape[0]
@@ -701,7 +833,7 @@ def sweep_rewards(points, poses, quats, intrins, img_width, img_height, min_dist
             P = B.prepare(poses[t0:t1], dev, "poses").reshape(-1, 3)
             Q = B.prepare(quats[t0:t1], dev, "quats").reshape(-1, 4)
             minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)
-            mine[:t1 - t0] = B.sweep_sums(pts, P, Q, t1 - t0, Pn, Kd, cam, boxes, minmax)
+            mine[:t1 - t0] = _sweep_sums(B, pts, P, Q, t1 - t0, Pn, Kd, cam, boxes, minmax, prior, psum)
         out = torch.empty(world * per, dtype=torch.float64, device=dev)
         dist.all_gather_into_tensor(out, mine, group=group)
         return out[:T] / float(n)
@@ -709,14 +841,15 @@ def sweep_rewards(points, poses, quats, intrins, img_width, img_height, min_dist
     Q = B.prepare(quats, dev, "quats").reshape(-1, 4)
     minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)
     _all_reduce_minmax(minmax, T * Pn, group)
-    sums = B.sweep_sums(pts, P, Q, T, Pn, Kd, cam, boxes, minmax)
+    sums = _sweep_sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum)
     if group is not None:
         _all_reduce(sums, _reduce_ops()[2], group)
     return sums / float(n if n_total is None else n_total)
 
 
 def coverage_sweep(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
-                   n_total=None, group=None, boxes=None, presorted=False, shard="points", workspace=None):
+                   n_total=None, group=None, boxes=None, presorted=False, shard="points", workspace=None,
+                   prior_logodds=None):
     """Differentiable candidate sweep: poses (T, P, 3), quats (T, P, 4) -> means (T,) fp32, where means[t] is the mean
     reward of trajectory t as `coverage_traj(points, poses[t], quats[t])` computes it.  `means` is differentiable w.r.t.
     `poses` and `quats`; each trajectory's gradient comes from the same pass over the cloud (cov_sweep_fused), so a
@@ -725,7 +858,8 @@ def coverage_sweep(points, poses, quats, intrins, img_width, img_height, min_dis
     from `evaluation(dense=True)`.  No host synchronisation: capturable in a CUDA graph.  `workspace`: a uint8 CUDA tensor
     kept by the caller across calls (grown when too small).
     Sharding as in `sweep_rewards`: shard="points" (this rank's slice of the cloud; normalisers and accumulators are
-    all-reduced) or shard="trajectories" (the whole cloud on every rank; means and gradients are all-gathered)."""
+    all-reduced) or shard="trajectories" (the whole cloud on every rank; means and gradients are all-gathered).
+    `prior_logodds`: per-point prior log-odds shared by every trajectory, ordered and sharded as in `sweep_rewards`."""
     B = _BACKEND
     if shard not in ("points", "trajectories"):
         raise ValueError("shard must be 'points' or 'trajectories'")
@@ -735,11 +869,12 @@ def coverage_sweep(points, poses, quats, intrins, img_width, img_height, min_dis
         raise ValueError("coverage_sweep: poses must be (T, P, 3) and quats (T, P, 4) with the same T, P >= 1; got "
                          f"{tuple(getattr(poses, 'shape', ()))} and {tuple(getattr(quats, 'shape', ()))}")
     pts = B.prepare(points, what="points")
-    if not presorted and boxes is None and pts.shape[0] > 0:
-        pts, _, boxes = B.order_cloud(pts, True)
+    prior = _check_prior(prior_logodds, pts.shape[0], pts.device)
+    pts, prior, boxes = _order_with_prior(B, pts, prior, boxes, presorted)
+    psum = None if prior is None else B.prior_sum(prior)
     n_total = int(pts.shape[0] if n_total is None else n_total)
     cam = _lib.camera(img_width, img_height, min_dist, max_dist, eps)
-    return CoverageSweepFn.apply(pts, poses, quats, intrins, cam, n_total, group, boxes, shard, workspace)
+    return CoverageSweepFn.apply(pts, poses, quats, intrins, cam, n_total, group, boxes, shard, workspace, prior, psum)
 
 
 @torch.no_grad()
