@@ -223,6 +223,54 @@ int cov_sweep_fused_prior(const float* xyz_dev, int64_t n, const float* poses_de
                           const cov_traj_opts* opts, void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Point weights: what is worth seeing.  Weighted mean of the trajectory objective, mean_w = sum_j w_j r_j / sum_j w_j,
+ * and its pose gradients (pass B's backward with G_j = w_j r_j (1 - r_j)), in the same pass as the unweighted call.
+ * ref: no reference implementation.  The weight changes neither r_j nor the normalisers, the gate or the pruning: the
+ * rewards of cov_traj_fused_weighted are bit-identical to those of the call without a weight.  It composes with the prior
+ * (r_j = sigmoid(prior_j + L_j) as above).  A weight of all ones gives the unweighted sums up to the order of the fp64
+ * additions.  Nothing checks the values: they must be finite and >= 0 with sum_j w_j > 0 (NaN/inf propagate).
+ *   weight_dev       (n) fp32, 16-byte aligned, one per point, shared by every pose and trajectory of the call; indexed
+ *                    like prior_dev (cov_traj_*: like rewards_dev; cov_sweep_*: like xyz_dev).
+ *   prior_dev        NULL or the prior log-odds, as for the _prior entry points.  The weighted base below takes the
+ *                    place of prior_sum_dev.
+ *   weight_sums_dev  2 doubles from cov_weight_sums (once per weight and prior state), read on the device:
+ *                    [0] sum_j w_j r0_j with r0_j = sigmoid(prior_j), or 1/2 without a prior: the weighted reward sum of
+ *                        the points no listed pose reaches, where the accumulated sum starts;
+ *                    [1] sum_j w_j: the denominator of the weighted means (cov_*_epilogue_dev).
+ * Accumulators: the layouts of the unweighted calls, with sum_j w_j r_j in place of sum_j r_j.  Shard-additive: with a
+ * sharded cloud each rank passes its slices and its own sums; SUM the accumulators as before, and SUM [1] over the ranks
+ * (only [1]) before the epilogue.
+ * cov_traj_fused_weighted: cov_traj_fused without upstream (the gradient of the weighted mean).  Pre-fill, options,
+ *   workspace and paths as for cov_traj_fused (cov_traj_fused_prior with a prior).  The gradient through rewards_dev is
+ *   the unweighted call's with upstream_dev: the rewards do not depend on the weight.
+ * cov_sweep_rewards_weighted, cov_sweep_fused_weighted: the sweeps with sum_j w_j r_j(t) per trajectory; every path
+ *   (pruned, dense, the small-cloud path of cov_sweep_fused) weighs.  Workspace as for the unweighted calls.
+ * cov_traj_epilogue_dev, cov_sweep_epilogue_dev: cov_traj_epilogue (upstream_mode 0) and cov_sweep_epilogue with the
+ *   denominator *den_dev (fp64, on the device; weight_sums_dev + 1) in place of n_total; with *den_dev == n_total the
+ *   outputs are bit-identical to theirs.
+ * ------------------------------------------------------------------------------------------ */
+int cov_weight_sums(const float* weight_dev, const float* prior_dev, int64_t n, double* weight_sums_dev, void* stream);
+int cov_traj_fused_weighted(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev, int n_poses,
+                            const float* K_dev, const cov_camera* cam, const float* boxes_dev, const float* minmax_dev,
+                            const int32_t* reward_index_dev, float* rewards_dev, double* acc_dev, const float* prior_dev,
+                            const float* weight_dev, const double* weight_sums_dev, const cov_traj_opts* opts,
+                            void* workspace_dev, size_t workspace_bytes, void* stream);
+int cov_sweep_rewards_weighted(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev,
+                               int n_traj, int poses_per_traj, const float* K_dev, const cov_camera* cam,
+                               const float* boxes_dev, const float* minmax_dev, double* sum_rewards_dev,
+                               const float* prior_dev, const float* weight_dev, const double* weight_sums_dev,
+                               const cov_traj_opts* opts, void* workspace_dev, size_t workspace_bytes, void* stream);
+int cov_sweep_fused_weighted(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev, int n_traj,
+                             int poses_per_traj, const float* K_dev, const cov_camera* cam, const float* boxes_dev,
+                             const float* minmax_dev, double* acc_dev, const float* prior_dev, const float* weight_dev,
+                             const double* weight_sums_dev, const cov_traj_opts* opts, void* workspace_dev,
+                             size_t workspace_bytes, void* stream);
+int cov_traj_epilogue_dev(const double* acc_dev, const float* minmax_dev, const float* quats_dev, int n_poses,
+                          const double* den_dev, float* out_dev, void* stream);
+int cov_sweep_epilogue_dev(const double* acc_dev, const float* minmax_dev, const float* quats_dev, int n_traj,
+                           int poses_per_traj, const double* den_dev, float* out_dev, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Batched ModelPose: K candidate poses (t_k, q~_k) on one cloud, for every k the COV_POSE_ACC sums cov_pose_fused
  * computes for pose k alone ([0] sum m, [1..3] F, [4..6] T, [7] 0), in one pass over the cloud per chunk of poses.
  * ref: src/model.py:98-127 per pose (multi-start pose optimisation, scoring of candidate views); no per-point output.

@@ -21,12 +21,14 @@ size_t sweep_smem_bytes(int n_traj, int ppt_poses) {
 
 // HAS_PRIOR: sum_j (sigmoid(prior_j + L_j) - sigmoid(prior_j)) per trajectory (the prior indexed like xyz), and
 // *prior_sum = sum_j sigmoid(prior_j) in place of 0.5 * n.
-template <int PPT, bool HAS_PRIOR>
+// HAS_W: each point's term times its weight w_j (indexed like xyz), and *prior_sum is the weighted base
+// sum_j w_j r0_j (cov_weight_sums).
+template <int PPT, bool HAS_PRIOR, bool HAS_W = false>
 __global__ void __launch_bounds__(COV_THREADS, 2)
 cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restrict__ poses,
                  const float* __restrict__ quats, int n_traj, int per_traj, const float* __restrict__ K9, CovConst C,
                  const float* __restrict__ mins, const float* __restrict__ maxs, double* __restrict__ sum_out,
-                 const float* __restrict__ prior, const double* __restrict__ prior_sum) {
+                 const float* __restrict__ prior, const double* __restrict__ prior_sum, const float* __restrict__ weight) {
     extern __shared__ float4 smem4[];
     float4* ptab = smem4;
     const int W = n_traj * per_traj;
@@ -42,7 +44,7 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
     constexpr int T = COV_THREADS * PPT;
     const int64_t ntiles = (n + T - 1) / T;
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        float px[PPT], py[PPT], pz[PPT], pr[PPT], r0[PPT];
+        float px[PPT], py[PPT], pz[PPT], pr[PPT], r0[PPT], wt[PPT];
         bool valid[PPT];
 #pragma unroll
         for (int s = 0; s < PPT; ++s) {
@@ -56,6 +58,7 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
                 pr[s] = __ldg(prior + j);
                 r0[s] = cov_sigmoid(pr[s]);
             }
+            if (HAS_W) wt[s] = __ldg(weight + j);
         }
         for (int t = 0; t < n_traj; ++t) {
             float L[PPT];
@@ -86,7 +89,12 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
             if (__any_sync(kFull, any_nz)) {
 #pragma unroll
                 for (int s = 0; s < PPT; ++s) {
-                    if (HAS_PRIOR) {
+                    if (HAS_W) {
+                        if (valid[s] && L[s] != 0.f) {
+                            const float r = HAS_PRIOR ? cov_sigmoid(cov_fuse_prior(pr[s], L[s])) : 1.f / (1.f + expf(-L[s]));
+                            acc += wt[s] * (r - (HAS_PRIOR ? r0[s] : 0.5f));
+                        }
+                    } else if (HAS_PRIOR) {
                         if (valid[s] && L[s] != 0.f) acc += cov_sigmoid(cov_fuse_prior(pr[s], L[s])) - r0[s];
                     } else if (valid[s] && L[s] != 0.f) {
                         acc += 1.f / (1.f + expf(-L[s])) - 0.5f;
@@ -100,7 +108,7 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
     __syncthreads();
     for (int t = tid; t < n_traj; t += COV_THREADS) {
         double v = ssum[t];
-        if (blockIdx.x == 0) v += HAS_PRIOR ? *prior_sum : 0.5 * (double)n;
+        if (blockIdx.x == 0) v += (HAS_PRIOR || HAS_W) ? *prior_sum : 0.5 * (double)n;
         if (v != 0.0) atomicAdd(sum_out + t, v);
     }
 }
@@ -110,7 +118,8 @@ cov_sweep_kernel(const float* __restrict__ xyz, int64_t n, const float* __restri
 // Dense sweep (cov_traj_opts.dense); the pruned pipeline and the C entry point are in cov_traj.cu.
 int cov_sweep_rewards_dense(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
                             int per_traj, const float* K, const cov_camera* cam, const float* minmax,
-                            double* sum_rewards, const float* prior, const double* prior_sum, void* stream) {
+                            double* sum_rewards, const float* prior, const double* prior_sum, const float* weight,
+                            void* stream) {
     if (!xyz || n <= 0 || !poses || !quats || n_traj <= 0 || per_traj <= 0 || !K || !cam || !minmax || !sum_rewards) {
         cov_set_error("cov_sweep_rewards: bad argument");
         return COV_ERR_ARG;
@@ -127,7 +136,8 @@ int cov_sweep_rewards_dense(const float* xyz, int64_t n, const float* poses, con
     constexpr int T = COV_THREADS * kSweepPpt;
     const int64_t ntiles = (n + T - 1) / T;
     const size_t smem_max = sweep_smem_bytes(chunk, per_traj);
-    const auto kern = prior ? cov_sweep_kernel<kSweepPpt, true> : cov_sweep_kernel<kSweepPpt, false>;
+    const auto kern = weight ? (prior ? cov_sweep_kernel<kSweepPpt, true, true> : cov_sweep_kernel<kSweepPpt, false, true>)
+                             : (prior ? cov_sweep_kernel<kSweepPpt, true> : cov_sweep_kernel<kSweepPpt, false>);
     // always the same value: two host threads with different trajectory counts cannot race between set and launch
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - 256);
     int per_sm = 1;
@@ -141,7 +151,7 @@ int cov_sweep_rewards_dense(const float* xyz, int64_t n, const float* poses, con
         const int w0 = t0 * per_traj;
         kern<<<(unsigned)grid, COV_THREADS, sweep_smem_bytes(nt, per_traj), s>>>(
             xyz, n, poses + 3 * (size_t)w0, quats + 4 * (size_t)w0, nt, per_traj, K, C, minmax + w0, minmax + W + w0,
-            sum_rewards + t0, prior, prior_sum);
+            sum_rewards + t0, prior, prior_sum, weight);
     }
     return cov_check_launch("cov_sweep_rewards");
 }

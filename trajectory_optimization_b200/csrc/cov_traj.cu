@@ -1034,7 +1034,8 @@ __device__ __forceinline__ void fused_block_flush(const T* accs, int W, double* 
 
 // ---- dense ----
 // HAS_PRIOR: r_j = sigmoid(prior_j + L_j), prior indexed like `rewards` (through out_index).
-template <int PPT, bool HAS_UP, bool HAS_PRIOR>
+// WSUM (with HAS_UP): `upstream` is the point weight w_j; the reward sum is sum_j w_j r_j and G_j = w_j r_j (1 - r_j).
+template <int PPT, bool HAS_UP, bool HAS_PRIOR, bool WSUM = false>
 __global__ void __launch_bounds__(COV_THREADS, 2)
 cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __restrict__ poses,
                       const float* __restrict__ quats, int W, const float* __restrict__ K9, CovConst C,
@@ -1115,8 +1116,14 @@ cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __r
                 const int64_t j = tile * T + lbase + s * 32;
                 const int64_t jo = out_index ? (int64_t)out_index[j] : j;
                 rewards[jo] = r;
-                sum_r += (double)r;
-                if (HAS_UP) g *= upstream[jo];
+                if (WSUM) {
+                    const float wj = upstream[jo];
+                    sum_r += (double)wj * (double)r;
+                    g *= wj;
+                } else {
+                    sum_r += (double)r;
+                    if (HAS_UP) g *= upstream[jo];
+                }
             }
             Gs[lbase + s * 32] = g;
         }
@@ -1144,9 +1151,11 @@ cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __r
 // prior at the index its reward goes to (the gather HAS_UP makes for upstream_j), r_j = sigmoid(prior_j + L_j) is stored
 // where L_j != 0 and r_j - sigmoid(prior_j) is added.  G_j = r_j (1 - r_j) for every point, L_j = 0 included (a gated
 // pair with p exactly 1/2 adds nothing to L_j but still enters the backward).
+// WSUM (point weights, with HAS_UP): `upstream` is the weight w_j, gathered like upstream_j; w_j (r_j - r0_j) is added
+// (r0_j = 1/2 or sigmoid(prior_j)) to a sum that starts at sum_j w_j r0_j, and G_j = w_j r_j (1 - r_j).
 constexpr int kTilesMinBlocks = 3;            // resident blocks per SM the register allocation aims at
 
-template <bool HAS_UP, bool HAS_PRIOR>
+template <bool HAS_UP, bool HAS_PRIOR, bool WSUM = false>
 __global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
 cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, CovConst C,
                             const float* __restrict__ upstream, const int32_t* __restrict__ out_index,
@@ -1154,6 +1163,7 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
                             const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g, int mask_stride,
                             const int* __restrict__ worklist, int* __restrict__ ctrl, int64_t ntiles,
                             unsigned long long* __restrict__ stats, const float* __restrict__ prior) {
+    static_assert(HAS_UP || !WSUM, "the weight rides on the upstream gather");
     constexpr int PPT = kItemPpt;
     __shared__ unsigned wgate[kWarps][kMaskWords];   // per warp: poses with a gated pair among its points (this item)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1212,6 +1222,12 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
                     rewards[jo] = r;
                 }
                 G[s] = r * (1.f - r);
+                if (WSUM) {
+                    const float wj = upstream[jo];
+                    sum_r += (double)wj * (double)(r - r0);
+                    G[s] *= wj;
+                    continue;
+                }
                 sum_r += (double)(r - r0);
                 if (HAS_UP) G[s] *= upstream[jo];
                 continue;
@@ -1224,13 +1240,19 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
             }
             if (valid[s]) {
                 const int64_t j = item.j0 + s * 32 + lane;
-                sum_r += (double)(r - 0.5f);
+                if (!WSUM) sum_r += (double)(r - 0.5f);
                 const bool store = r != 0.5f;
                 int64_t jo = j;
                 if (out_index && (store || HAS_UP))
                     jo = item.whole ? (int64_t)item.perm[s * 32 + lane] : (int64_t)out_index[j];  // staged with the item
                 if (store) rewards[jo] = r;
-                if (HAS_UP) G[s] *= upstream[jo];
+                if (WSUM) {
+                    const float wj = upstream[jo];
+                    sum_r += (double)wj * (double)(r - 0.5f);
+                    G[s] *= wj;
+                } else if (HAS_UP) {
+                    G[s] *= upstream[jo];
+                }
             }
         }
         // ------------------------------ backward ------------------------------
@@ -1268,12 +1290,15 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
 // pose of which is listed for an item contribute exactly 1/2 per point: 0.5 * n is added once.
 // HAS_PRIOR: sum_j (sigmoid(prior_j + L_j) - sigmoid(prior_j)) at a flush (the item's 128 priors, in the cloud's order,
 // read there), and *prior_sum = sum_j sigmoid(prior_j) in place of 0.5 * n.
-template <bool HAS_PRIOR>
+// HAS_W: each point's term times its weight w_j (read next to the prior, in the cloud's order), and *prior_sum is the
+// weighted base sum_j w_j r0_j (cov_weight_sums).
+template <bool HAS_PRIOR, bool HAS_W = false>
 __global__ void __launch_bounds__(COV_THREADS, 3)
 cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, int per_traj,
                        int n_traj, CovConst C, const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g,
                        int mask_stride, const int* __restrict__ worklist, int* __restrict__ ctrl,
-                       double* __restrict__ sum_out, const float* __restrict__ prior, const double* __restrict__ prior_sum) {
+                       double* __restrict__ sum_out, const float* __restrict__ prior, const double* __restrict__ prior_sum,
+                       const float* __restrict__ weight) {
     constexpr int PPT = kItemPpt;
     extern __shared__ float4 smem4[];
     double* ssum = reinterpret_cast<double*>(smem4);   // per-trajectory totals of this block
@@ -1295,7 +1320,18 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
                 float a = 0.f;
 #pragma unroll
                 for (int s = 0; s < PPT; ++s) {
-                    if (HAS_PRIOR) {
+                    if (HAS_W) {
+                        if (valid[s] && L[s] != 0.f) {
+                            const int64_t j = item.j0 + s * 32 + lane;
+                            const float wj = __ldg(weight + j);
+                            if (HAS_PRIOR) {
+                                const float pr = __ldg(prior + j);
+                                a += wj * (cov_sigmoid(cov_fuse_prior(pr, L[s])) - cov_sigmoid(pr));
+                            } else {
+                                a += wj * (1.f / (1.f + expf(-L[s])) - 0.5f);
+                            }
+                        }
+                    } else if (HAS_PRIOR) {
                         if (valid[s] && L[s] != 0.f) {
                             const float pr = __ldg(prior + item.j0 + s * 32 + lane);
                             a += cov_sigmoid(cov_fuse_prior(pr, L[s])) - cov_sigmoid(pr);
@@ -1332,7 +1368,7 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
     __syncthreads();
     for (int t = tid; t < n_traj; t += COV_THREADS) {
         double v = ssum[t];
-        if (blockIdx.x == 0) v += HAS_PRIOR ? *prior_sum : 0.5 * (double)n;
+        if (blockIdx.x == 0) v += (HAS_PRIOR || HAS_W) ? *prior_sum : 0.5 * (double)n;
         if (v != 0.0) atomicAdd(sum_out + t, v);
     }
 }
@@ -1348,13 +1384,15 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
 // same box test), so its L, r_j and G_j — and the re-evaluated m of the backward — are bit-identical to pass B's.
 // HAS_PRIOR: at a flush r_j = sigmoid(prior_j + L_j) and r_j - sigmoid(prior_j) is added, with the item's 128 priors (in
 // the cloud's order) read there; the blocks start at sum_j sigmoid(prior_j) (cov_sweep_acc_init_kernel).
-template <bool HAS_PRIOR>
+// HAS_W: the item's 128 weights w_j (cloud's order) are read at a flush too; w_j (r_j - r0_j) is added and G_j is
+// multiplied by w_j before the backward; the blocks start at sum_j w_j r0_j (cov_weight_sums).
+template <bool HAS_PRIOR, bool HAS_W = false>
 __global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
 cov_sweep_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, int per_traj,
                              CovConst C, const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g,
                              int mask_stride, const int* __restrict__ worklist, int* __restrict__ ctrl, int64_t ntiles,
                              double* __restrict__ acc, unsigned long long* __restrict__ stats,
-                             const float* __restrict__ prior) {
+                             const float* __restrict__ prior, const float* __restrict__ weight) {
     constexpr int PPT = kItemPpt;
     __shared__ unsigned wgate[kWarps][kMaskWords];   // per warp: poses of the current trajectory with a gated pair
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1385,7 +1423,13 @@ cov_sweep_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
                     const float r0 = cov_sigmoid(pr);
                     const float r = L[s] != 0.f ? cov_sigmoid(cov_fuse_prior(pr, L[s])) : r0;
                     G[s] = r * (1.f - r);
-                    if (valid[s]) a += r - r0;
+                    if (HAS_W) {
+                        const float wj = valid[s] ? __ldg(weight + item.j0 + s * 32 + lane) : 0.f;
+                        G[s] *= wj;
+                        a += wj * (r - r0);
+                    } else if (valid[s]) {
+                        a += r - r0;
+                    }
                     continue;
                 }
                 float r = 0.5f;
@@ -1394,7 +1438,13 @@ cov_sweep_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
                     r = 1.f / (1.f + expf(-L[s]));
                     G[s] = r * (1.f - r);
                 }
-                if (valid[s]) a += r - 0.5f;
+                if (HAS_W) {
+                    const float wj = valid[s] ? __ldg(weight + item.j0 + s * 32 + lane) : 0.f;
+                    G[s] *= wj;
+                    a += wj * (r - 0.5f);
+                } else if (valid[s]) {
+                    a += r - 0.5f;
+                }
             }
             a = cov_warp_sum(a);
             if (lane == 0 && a != 0.f) atomicAdd(A + (size_t)per_traj * COV_ACC_STRIDE, (double)a);
@@ -1519,6 +1569,63 @@ __global__ void cov_sweep_epilogue_kernel(const double* __restrict__ acc, const 
     const int t = i / per_traj, k = i - t * per_traj;
     traj_epilogue_pose(acc + (size_t)t * block + (size_t)k * COV_ACC_STRIDE, minmax[i], minmax[TP + i], quats + 4 * (size_t)i,
                        1.0 / n_total, out + n_traj + 3 * (size_t)i, out + n_traj + 3 * (size_t)TP + 4 * (size_t)i);
+}
+
+// The epilogues of the point-weighted calls: the denominator is read on the device (sum_j w_j, cov_weight_sums) instead
+// of n_total.  With *den == n they compute what cov_traj_epilogue_kernel (upstream_mode 0) and cov_sweep_epilogue_kernel
+// compute, bit for bit.
+__global__ void cov_traj_epilogue_dev_kernel(const double* __restrict__ acc, const float* __restrict__ minmax,
+                                             const float* __restrict__ quats, int W, const double* __restrict__ den,
+                                             float* __restrict__ out) {
+    const int w = blockIdx.x * blockDim.x + threadIdx.x;
+    const double d = *den;
+    if (w == 0) out[0] = (float)(acc[(size_t)W * COV_ACC_STRIDE] / d);
+    if (w >= W) return;
+    traj_epilogue_pose(acc + (size_t)w * COV_ACC_STRIDE, minmax[w], minmax[W + w], quats + 4 * w, 1.0 / d, out + 1 + 3 * w,
+                       out + 1 + 3 * W + 4 * w);
+}
+
+__global__ void cov_sweep_epilogue_dev_kernel(const double* __restrict__ acc, const float* __restrict__ minmax,
+                                              const float* __restrict__ quats, int n_traj, int per_traj,
+                                              const double* __restrict__ den, float* __restrict__ out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;  // pose t * P + k
+    const int TP = n_traj * per_traj;
+    const size_t block = COV_SWEEP_ACC_BLOCK(per_traj);
+    const double d = *den;
+    if (i < n_traj) out[i] = (float)(acc[(size_t)i * block + (size_t)per_traj * COV_ACC_STRIDE] / d);
+    if (i >= TP) return;
+    const int t = i / per_traj, k = i - t * per_traj;
+    traj_epilogue_pose(acc + (size_t)t * block + (size_t)k * COV_ACC_STRIDE, minmax[i], minmax[TP + i], quats + 4 * (size_t)i,
+                       1.0 / d, out + n_traj + 3 * (size_t)i, out + n_traj + 3 * (size_t)TP + 4 * (size_t)i);
+}
+
+// ============================================== point weights ==============================================
+// [sum_j w_j r0_j, sum_j w_j] in fp64, r0_j = sigmoid(prior_j) (HAS_PRIOR) or 1/2: the reward-sum base of the weighted
+// calls and the denominator of their means.  Grid-stride, warp and block sums, two fp64 atomics per block into the
+// zeroed output.
+template <bool HAS_PRIOR>
+__global__ void __launch_bounds__(256) cov_weight_sums_kernel(const float* __restrict__ weight,
+                                                              const float* __restrict__ prior, int64_t n,
+                                                              double* __restrict__ out) {
+    __shared__ double red[2][8];
+    double base = 0.0, tot = 0.0;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const double w = (double)__ldg(weight + i);
+        base += w * (HAS_PRIOR ? (double)cov_sigmoid(__ldg(prior + i)) : 0.5);
+        tot += w;
+    }
+    base = cov_warp_sum(base);
+    tot = cov_warp_sum(tot);
+    if ((threadIdx.x & 31) == 0) {
+        red[0][threadIdx.x >> 5] = base;
+        red[1][threadIdx.x >> 5] = tot;
+    }
+    __syncthreads();
+    if (threadIdx.x < 2) {
+        double t = 0.0;
+        for (int i = 0; i < 8; ++i) t += red[threadIdx.x][i];
+        atomicAdd(out + threadIdx.x, t);
+    }
 }
 
 // ============================================ prior log-odds (map memory) ============================================
@@ -1867,6 +1974,19 @@ static int check_prior(const char* who, const float* prior, const double* prior_
     return COV_OK;
 }
 
+// The weight (16-byte aligned, indexed like the prior) and the 2-double sums of the _weighted entry points.
+static int check_weight(const char* who, const float* weight, const double* weight_sums, const float* prior) {
+    if (!weight || !weight_sums) {
+        cov_set_error("%s: null weight_dev or weight_sums_dev", who);
+        return COV_ERR_ARG;
+    }
+    if ((((uintptr_t)weight) & 15) || (((uintptr_t)prior) & 15)) {
+        cov_set_error("%s: weight_dev and prior_dev must be 16-byte aligned", who);
+        return COV_ERR_ALIGN;
+    }
+    return COV_OK;
+}
+
 static int traj_minmax_impl(const float* xyz, int64_t n, const float* poses, const float* quats, int W, const float* K,
                             const cov_camera* cam, const float* boxes_dev, float* minmax, const float* prior,
                             const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
@@ -1948,7 +2068,14 @@ extern "C" int cov_traj_minmax_prior(const float* xyz, int64_t n, const float* p
 static int traj_fused_impl(const float* xyz, int64_t n, const float* poses, const float* quats, int W, const float* K,
                            const cov_camera* cam, const float* boxes_dev, const float* minmax, const float* upstream,
                            const int32_t* reward_index, float* rewards, double* acc, const float* prior,
-                           const double* prior_sum, const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+                           const double* prior_sum, const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream,
+                           const float* weight = nullptr, const double* weight_sums = nullptr) {
+    // point weights ride on the upstream gather (WSUM); the reward sum starts at sum_j w_j r0_j instead
+    const bool wsum = weight != nullptr;
+    if (wsum) {
+        upstream = weight;
+        prior_sum = weight_sums;
+    }
     const bool prune = !(opts && opts->dense) && n >= kDenseBelow;
     int rc = check_traj_args("cov_traj_fused", xyz, n, poses, quats, W, K, cam, ws, ws_bytes, prune);
     if (rc) return rc;
@@ -1975,20 +2102,25 @@ static int traj_fused_impl(const float* xyz, int64_t n, const float* poses, cons
         // phase-2 parallelism: split each pose row over 2^seg_log2 lanes until there are >= 2 tasks per thread
         int seg_log2 = 0;
         while ((W << seg_log2) < 2 * COV_THREADS && (2 << seg_log2) <= bit_words(ppt_d) && seg_log2 < 5) ++seg_log2;
-#define LAUNCH_F(P, UP, PR)                                                                                        \
+#define LAUNCH_F(P, UP, PR, WS)                                                                                    \
     {                                                                                                              \
-        const int grid = grid_for(cov_traj_fused_kernel<P, UP, PR>, smem, ntiles);                                 \
-        cov_traj_fused_kernel<P, UP, PR><<<grid, COV_THREADS, smem, s>>>(xyz, n, poses, quats, W, K, C, minmax,     \
-                                                                         upstream, reward_index, rewards, acc,     \
-                                                                         seg_log2, prior);                         \
+        const int grid = grid_for(cov_traj_fused_kernel<P, UP, PR, WS>, smem, ntiles);                             \
+        cov_traj_fused_kernel<P, UP, PR, WS><<<grid, COV_THREADS, smem, s>>>(xyz, n, poses, quats, W, K, C, minmax, \
+                                                                             upstream, reward_index, rewards, acc, \
+                                                                             seg_log2, prior);                     \
     }
 #define LAUNCH_FP(UP, PR) \
-    if (ppt_d == 4) LAUNCH_F(4, UP, PR) else if (ppt_d == 2) LAUNCH_F(2, UP, PR) else LAUNCH_F(1, UP, PR)
-        if (upstream) {
+    if (ppt_d == 4) LAUNCH_F(4, UP, PR, false) else if (ppt_d == 2) LAUNCH_F(2, UP, PR, false) else LAUNCH_F(1, UP, PR, false)
+#define LAUNCH_FW(PR) \
+    if (ppt_d == 4) LAUNCH_F(4, true, PR, true) else if (ppt_d == 2) LAUNCH_F(2, true, PR, true) else LAUNCH_F(1, true, PR, true)
+        if (wsum) {
+            if (prior) { LAUNCH_FW(true) } else { LAUNCH_FW(false) }
+        } else if (upstream) {
             if (prior) { LAUNCH_FP(true, true) } else { LAUNCH_FP(true, false) }
         } else {
             if (prior) { LAUNCH_FP(false, true) } else { LAUNCH_FP(false, false) }
         }
+#undef LAUNCH_FW
 #undef LAUNCH_FP
 #undef LAUNCH_F
         return cov_check_launch("cov_traj_fused");
@@ -1998,7 +2130,7 @@ static int traj_fused_impl(const float* xyz, int64_t n, const float* poses, cons
     static_assert(ppt == 4 && tile_points(ppt) == kItemsPerTile * kItemPts, "tile = 8 items");
     const int64_t ntiles = (n + tile_points(ppt) - 1) / tile_points(ppt);
     const float4* boxes = boxes_for_call(xyz, n, boxes_dev, t, s);
-    if (prior) {
+    if (prior || wsum) {
         cov_traj_table_kernel<true><<<(W + 63) / 64, 64, 0, s>>>(poses, quats, W, K, C, minmax, t.table, t.ctrl,
                                                                  (int)(t.ctrl_bytes / sizeof(int)), acc, 0.0, prior_sum);
     } else {
@@ -2010,8 +2142,10 @@ static int traj_fused_impl(const float* xyz, int64_t n, const float* poses, cons
     if ((rc = launch_cull(boxes, ppt, ntiles, t, W, nullptr, 0.f, prefilled ? nullptr : rewards, n, s, prior)) != COV_OK)
         return rc;
     // persistent warps: as many blocks as are resident; every warp draws 128-point items from a ticket counter
-    const auto tiles_kern = upstream ? (prior ? cov_traj_fused_tiles_kernel<true, true> : cov_traj_fused_tiles_kernel<true, false>)
-                                     : (prior ? cov_traj_fused_tiles_kernel<false, true> : cov_traj_fused_tiles_kernel<false, false>);
+    const auto tiles_kern =
+        wsum ? (prior ? cov_traj_fused_tiles_kernel<true, true, true> : cov_traj_fused_tiles_kernel<true, false, true>)
+        : upstream ? (prior ? cov_traj_fused_tiles_kernel<true, true> : cov_traj_fused_tiles_kernel<true, false>)
+                   : (prior ? cov_traj_fused_tiles_kernel<false, true> : cov_traj_fused_tiles_kernel<false, false>);
     tiles_kern<<<persistent_grid(tiles_kern, 0, ntiles), COV_THREADS, 0, s>>>(
         xyz, n, t.table, W, C, upstream, reward_index, rewards, acc, boxes, t.amask, mask_stride_words(W), t.worklist,
         t.ctrl, ntiles, opts ? opts->stats_dev : nullptr, prior);
@@ -2035,6 +2169,32 @@ extern "C" int cov_traj_fused_prior(const float* xyz, int64_t n, const float* po
     if (rc) return rc;
     return traj_fused_impl(xyz, n, poses, quats, W, K, cam, boxes_dev, minmax, upstream, reward_index, rewards, acc,
                            prior, prior_sum, opts, ws, ws_bytes, stream);
+}
+
+extern "C" int cov_traj_fused_weighted(const float* xyz, int64_t n, const float* poses, const float* quats, int W,
+                                       const float* K, const cov_camera* cam, const float* boxes_dev, const float* minmax,
+                                       const int32_t* reward_index, float* rewards, double* acc, const float* prior,
+                                       const float* weight, const double* weight_sums, const cov_traj_opts* opts, void* ws,
+                                       size_t ws_bytes, void* stream) {
+    const int rc = check_weight("cov_traj_fused_weighted", weight, weight_sums, prior);
+    if (rc) return rc;
+    return traj_fused_impl(xyz, n, poses, quats, W, K, cam, boxes_dev, minmax, nullptr, reward_index, rewards, acc, prior,
+                           nullptr, opts, ws, ws_bytes, stream, weight, weight_sums);
+}
+
+extern "C" int cov_weight_sums(const float* weight, const float* prior, int64_t n, double* sums_out, void* stream) {
+    if (!weight || !sums_out || n < 0) {
+        cov_set_error("cov_weight_sums: null pointer or negative size (n=%lld)", (long long)n);
+        return COV_ERR_ARG;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaMemsetAsync(sums_out, 0, 2 * sizeof(double), s);
+    if (n > 0) {
+        const int grid = (int)std::min<int64_t>((n + 255) / 256, (int64_t)cov_sm_count_cached() * 8);
+        if (prior) cov_weight_sums_kernel<true><<<grid, 256, 0, s>>>(weight, prior, n, sums_out);
+        else cov_weight_sums_kernel<false><<<grid, 256, 0, s>>>(weight, nullptr, n, sums_out);
+    }
+    return cov_check_launch("cov_weight_sums");
 }
 
 extern "C" int cov_prior_reward_sum(const float* prior, int64_t n, double* sum_out, void* stream) {
@@ -2097,14 +2257,15 @@ extern "C" int cov_traj_logodds(const float* xyz, int64_t n, const float* poses,
 static int sweep_rewards_impl(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
                               int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
                               const float* minmax, double* sum_rewards, const float* prior, const double* prior_sum,
-                              const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+                              const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream,
+                              const float* weight = nullptr) {
     if (!xyz || n <= 0 || !poses || !quats || n_traj <= 0 || per_traj <= 0 || !K || !cam || !minmax || !sum_rewards) {
         cov_set_error("cov_sweep_rewards: bad argument");
         return COV_ERR_ARG;
     }
     if (opts && opts->dense)
         return cov_sweep_rewards_dense(xyz, n, poses, quats, n_traj, per_traj, K, cam, minmax, sum_rewards, prior,
-                                       prior_sum, stream);
+                                       prior_sum, weight, stream);
     // trajectories per launch: as many as the per-tile pose mask holds (32 * kMaskWords poses); the pose table stays in
     // global memory, the block keeps one fp64 total per trajectory in shared memory
     if (per_traj > 32 * kMaskWords) {
@@ -2137,10 +2298,11 @@ static int sweep_rewards_impl(const float* xyz, int64_t n, const float* poses, c
                                                                    0.0, nullptr);
         if (launch_cull(boxes, ppt, ntiles, t, Wn, nullptr, 0.f, nullptr, 0, s) != COV_OK) return COV_ERR_UNSUPPORTED;
         const size_t smem = (size_t)nt * sizeof(double);
-        const auto kern = prior ? cov_sweep_tiles_kernel<true> : cov_sweep_tiles_kernel<false>;
+        const auto kern = weight ? (prior ? cov_sweep_tiles_kernel<true, true> : cov_sweep_tiles_kernel<false, true>)
+                                 : (prior ? cov_sweep_tiles_kernel<true> : cov_sweep_tiles_kernel<false>);
         kern<<<persistent_grid(kern, smem, ntiles), COV_THREADS, smem, s>>>(
             xyz, n, t.table, Wn, per_traj, nt, C, boxes, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, sum_rewards + t0,
-            prior, prior_sum);
+            prior, prior_sum, weight);
     }
     return cov_check_launch("cov_sweep_rewards");
 }
@@ -2162,6 +2324,18 @@ extern "C" int cov_sweep_rewards_prior(const float* xyz, int64_t n, const float*
     if (rc) return rc;
     return sweep_rewards_impl(xyz, n, poses, quats, n_traj, per_traj, K, cam, boxes_dev, minmax, sum_rewards, prior,
                               prior_sum, opts, ws, ws_bytes, stream);
+}
+
+extern "C" int cov_sweep_rewards_weighted(const float* xyz, int64_t n, const float* poses, const float* quats,
+                                          int n_traj, int per_traj, const float* K, const cov_camera* cam,
+                                          const float* boxes_dev, const float* minmax, double* sum_rewards,
+                                          const float* prior, const float* weight, const double* weight_sums,
+                                          const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+    const int rc = check_weight("cov_sweep_rewards_weighted", weight, weight_sums, prior);
+    if (rc) return rc;
+    // the weighted base sum_j w_j r0_j takes the place of the prior's sum
+    return sweep_rewards_impl(xyz, n, poses, quats, n_traj, per_traj, K, cam, boxes_dev, minmax, sum_rewards, prior,
+                              weight_sums, opts, ws, ws_bytes, stream, weight);
 }
 
 extern "C" size_t cov_sweep_workspace_bytes(int64_t n, int n_traj, int per_traj) {
@@ -2191,7 +2365,8 @@ extern "C" size_t cov_sweep_fused_workspace_bytes(int64_t n, int n_traj, int per
 static int sweep_fused_impl(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
                             int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
                             const float* minmax, double* acc, const float* prior, const double* prior_sum,
-                            const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+                            const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream,
+                            const float* weight = nullptr, const double* weight_sums = nullptr) {
     if (!xyz || n <= 0 || !poses || !quats || n_traj <= 0 || per_traj <= 0 || !K || !cam || !minmax || !acc || !ws) {
         cov_set_error("cov_sweep_fused: null pointer, empty cloud or no poses (n=%lld, n_traj=%d, poses_per_traj=%d)",
                       (long long)n, n_traj, per_traj);
@@ -2234,7 +2409,7 @@ static int sweep_fused_impl(const float* xyz, int64_t n, const float* poses, con
             cudaMemcpyAsync(mm + per_traj, minmax + TP + w0, (size_t)per_traj * sizeof(float), cudaMemcpyDeviceToDevice, s);
             const int rc = traj_fused_impl(xyz, n, poses + 3 * w0, quats + 4 * w0, per_traj, K, cam, nullptr, mm, nullptr,
                                            nullptr, rewards, acc + (size_t)t * block, prior, prior_sum, &dense, ws, tws,
-                                           stream);
+                                           stream, weight, weight_sums);
             if (rc) return rc;
         }
         return COV_OK;
@@ -2251,7 +2426,8 @@ static int sweep_fused_impl(const float* xyz, int64_t n, const float* poses, con
     {
         const int64_t count = (int64_t)n_traj * (int64_t)block;
         const int grid = (int)std::min<int64_t>((count + 255) / 256, (int64_t)cov_sm_count_cached() * 8);
-        if (prior) cov_sweep_acc_init_dev_kernel<<<grid, 256, 0, s>>>(acc, count, (int64_t)block, prior_sum);
+        if (weight) cov_sweep_acc_init_dev_kernel<<<grid, 256, 0, s>>>(acc, count, (int64_t)block, weight_sums);
+        else if (prior) cov_sweep_acc_init_dev_kernel<<<grid, 256, 0, s>>>(acc, count, (int64_t)block, prior_sum);
         else cov_sweep_acc_init_kernel<<<grid, 256, 0, s>>>(acc, count, (int64_t)block, 0.5 * (double)n);
     }
     unsigned long long* stats = opts ? opts->stats_dev : nullptr;
@@ -2265,10 +2441,11 @@ static int sweep_fused_impl(const float* xyz, int64_t n, const float* poses, con
                                                                    nullptr, 0.0, nullptr);
         int rc = launch_cull(boxes, ppt, ntiles, t, Wn, nullptr, 0.f, nullptr, 0, s);
         if (rc != COV_OK) return rc;
-        const auto kern = prior ? cov_sweep_fused_tiles_kernel<true> : cov_sweep_fused_tiles_kernel<false>;
+        const auto kern = weight ? (prior ? cov_sweep_fused_tiles_kernel<true, true> : cov_sweep_fused_tiles_kernel<false, true>)
+                                 : (prior ? cov_sweep_fused_tiles_kernel<true> : cov_sweep_fused_tiles_kernel<false>);
         kern<<<persistent_grid(kern, 0, ntiles), COV_THREADS, 0, s>>>(
             xyz, n, t.table, Wn, per_traj, C, boxes, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, ntiles,
-            acc + (size_t)t0 * block, stats, prior);
+            acc + (size_t)t0 * block, stats, prior, weight);
     }
     return cov_check_launch("cov_sweep_fused");
 }
@@ -2289,6 +2466,17 @@ extern "C" int cov_sweep_fused_prior(const float* xyz, int64_t n, const float* p
     if (rc) return rc;
     return sweep_fused_impl(xyz, n, poses, quats, n_traj, per_traj, K, cam, boxes_dev, minmax, acc, prior, prior_sum, opts,
                             ws, ws_bytes, stream);
+}
+
+extern "C" int cov_sweep_fused_weighted(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
+                                        int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
+                                        const float* minmax, double* acc, const float* prior, const float* weight,
+                                        const double* weight_sums, const cov_traj_opts* opts, void* ws, size_t ws_bytes,
+                                        void* stream) {
+    const int rc = check_weight("cov_sweep_fused_weighted", weight, weight_sums, prior);
+    if (rc) return rc;
+    return sweep_fused_impl(xyz, n, poses, quats, n_traj, per_traj, K, cam, boxes_dev, minmax, acc, prior, nullptr, opts,
+                            ws, ws_bytes, stream, weight, weight_sums);
 }
 
 extern "C" int cov_sweep_epilogue(const double* acc, const float* minmax, const float* quats, int n_traj, int per_traj,
@@ -2314,4 +2502,27 @@ extern "C" int cov_traj_epilogue(const double* acc, const float* minmax, const f
     cov_traj_epilogue_kernel<<<(W + 127) / 128, 128, 0, (cudaStream_t)stream>>>(acc, minmax, quats, W, (double)n_total,
                                                                                upstream_mode, out);
     return cov_check_launch("cov_traj_epilogue");
+}
+
+extern "C" int cov_traj_epilogue_dev(const double* acc, const float* minmax, const float* quats, int W,
+                                     const double* den_dev, float* out, void* stream) {
+    if (!acc || !minmax || !quats || !den_dev || !out || W <= 0) {
+        cov_set_error("cov_traj_epilogue_dev: bad argument");
+        return COV_ERR_ARG;
+    }
+    cov_traj_epilogue_dev_kernel<<<(W + 127) / 128, 128, 0, (cudaStream_t)stream>>>(acc, minmax, quats, W, den_dev, out);
+    return cov_check_launch("cov_traj_epilogue_dev");
+}
+
+extern "C" int cov_sweep_epilogue_dev(const double* acc, const float* minmax, const float* quats, int n_traj, int per_traj,
+                                      const double* den_dev, float* out, void* stream) {
+    if (!acc || !minmax || !quats || !den_dev || !out || n_traj <= 0 || per_traj <= 0 ||
+        (int64_t)n_traj * per_traj > INT32_MAX / 8) {
+        cov_set_error("cov_sweep_epilogue_dev: bad argument (n_traj=%d, poses_per_traj=%d)", n_traj, per_traj);
+        return COV_ERR_ARG;
+    }
+    const int TP = n_traj * per_traj;
+    cov_sweep_epilogue_dev_kernel<<<(TP + 127) / 128, 128, 0, (cudaStream_t)stream>>>(acc, minmax, quats, n_traj, per_traj,
+                                                                                     den_dev, out);
+    return cov_check_launch("cov_sweep_epilogue_dev");
 }

@@ -179,9 +179,9 @@ class _OrderedCloudModel(nn.Module):
     """What ModelTraj, ModelTrajBatch and ModelPoseBatch share: the Morton-ordered copy of `self.points` with its permutation and tile
     boxes (made once per state of the cloud), the kept workspace, and the release of the last autograd graph.
     Subclasses set `points`, `spatial_sort`, `_pts32`, `_perm`, `_boxes`, `_ws` and `_mean` in their constructor.
-    ModelTraj and ModelTrajBatch also keep the prior log-odds (`_init_prior`)."""
+    ModelTraj and ModelTrajBatch also keep the prior log-odds (`_init_prior`) and the point weight (`_init_weight`)."""
 
-    _prior_in_cloud_order = False   # the kernels read the prior in the cloud's (Morton) order, not in that of `points`
+    _prior_in_cloud_order = False   # the kernels read the prior and the weight in the cloud's (Morton) order, not in that of `points`
 
     def _init_prior(self, prior_logodds):
         # The kernels read the model's own copy of the prior (`_prior`, in the order they index it) and sum_j sigmoid(
@@ -227,6 +227,61 @@ class _OrderedCloudModel(nn.Module):
         self.prior_logodds = None if prior_logodds is None else prior_logodds.to(self.device)
         if self.prior_logodds is not None and self._prior is not None:
             self._write_prior()
+        if getattr(self, "point_weight", None) is not None and self._weight is not None:
+            self._write_weight()   # its reward-sum base is sum_j w_j sigmoid(prior_j)
+
+    def _init_weight(self, point_weight):
+        # Like the prior: the kernels read the model's copy (`_weight`, in the order they index it), this shard's
+        # cov_weight_sums (`_weight_sums`, whose base depends on the prior) and sum_j w_j over every rank (`_weight_den`),
+        # all belonging to ONE state of `point_weight`, of the cloud and of the prior.
+        self.point_weight = None if point_weight is None else torch.as_tensor(point_weight).to(self.device)
+        self._weight = None
+        self._weight_sums = None
+        self._weight_den = None
+        self._weight_key = None
+
+    def _weight_state_key(self):
+        w, p = self.point_weight, self.prior_logodds
+        return (id(w), w._version, id(self.points), self.points._version, None if p is None else (id(p), p._version))
+
+    @torch.no_grad()
+    def _write_weight(self):
+        # into the same buffers when the shape allows (captured CUDA graphs hold their addresses)
+        pts = self._cloud()
+        w = ops._check_weight(self.point_weight, pts.shape[0], pts.device, what="point_weight")
+        if bool((~torch.isfinite(w) | (w < 0)).any()):   # once per weight state (one host synchronisation)
+            raise ValueError("point_weight must be finite and >= 0")
+        if self._prior_in_cloud_order and self._perm is not None:
+            w = w.index_select(0, self._perm.long())
+        prior, _ = self._prior_args()
+        if self._weight is None or self._weight.shape != w.shape or self._weight.device != w.device:
+            self._weight = torch.empty_like(w)
+            self._weight_sums = torch.empty(2, dtype=torch.float64, device=w.device)
+            self._weight_den = torch.empty(1, dtype=torch.float64, device=w.device)
+        self._weight.copy_(w)
+        self._weight_sums.copy_(ops._BACKEND.weight_sums(self._weight, prior))
+        self._weight_den.copy_(self._weight_sums[1:])
+        ops._all_reduce(self._weight_den, ops._reduce_ops()[2], self.group)   # one double per weight state
+        if not float(self._weight_den[0]) > 0.0:
+            raise ValueError("point_weight must have a positive sum")
+        self._weight_key = self._weight_state_key()
+
+    def _weight_args(self):
+        """(weight as the kernels index it, this shard's cov_weight_sums (2,), global sum_j w_j (1,)), or Nones."""
+        if self.point_weight is None:
+            return None, None, None
+        if self._weight is None or self._weight_key != self._weight_state_key():
+            self._write_weight()
+        return self._weight, self._weight_sums, self._weight_den
+
+    def set_point_weight(self, point_weight):
+        """Replace the point weight (None: every point counts the same), (N,) fp32 in the order of `self.points`, finite,
+        >= 0, with a positive sum.  The model's copies are rewritten now, at the same addresses when the shape is unchanged,
+        so a CUDA graph captured WITH a weight evaluates the new one on its next replay (a graph captured without a weight
+        needs a new capture)."""
+        self.point_weight = None if point_weight is None else torch.as_tensor(point_weight).to(self.device)
+        if self.point_weight is not None and self._weight is not None:
+            self._write_weight()
 
     def _cloud(self):
         # The ordered copy, its permutation and the tile boxes belong to ONE state of `self.points`: the cache is keyed
@@ -280,6 +335,8 @@ class _OrderedCloudModel(nn.Module):
         self._pts32_key = (id(self.points), self.points._version)
         if getattr(self, "prior_logodds", None) is not None and self._prior is not None:
             self._write_prior()   # the prior copy follows the new permutation, in place
+        if getattr(self, "point_weight", None) is not None and self._weight is not None:
+            self._write_weight()   # so does the weight copy (and its sums)
 
     def _kept_workspace(self, cloud, need):
         # one workspace per (cloud, size), kept across steps: nothing in it outlives a call
@@ -293,7 +350,7 @@ class _OrderedCloudModel(nn.Module):
 class ModelTraj(_OrderedCloudModel):
     def __init__(self, points, wps_poses, wps_quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0,
                  smoothness_weight=14.0, traj_length_weight=0.02, device=torch.device("cuda"), group=None,
-                 n_total=None, spatial_sort=True, fused_regularizers=False, prior_logodds=None):
+                 n_total=None, spatial_sort=True, fused_regularizers=False, prior_logodds=None, point_weight=None):
         super().__init__()
         assert wps_poses.dim() == wps_quats.dim()
         assert wps_poses.size()[1] == 3
@@ -336,6 +393,9 @@ class ModelTraj(_OrderedCloudModel):
         # Map memory: (N,) fp32 log-odds of what earlier paths observed, in the order of `self.points` (indexed like
         # `rewards`); rewards_j = sigmoid(prior_j + sum_w lo_jw).  Folding an executed path in: `observed_logodds()`.
         self._init_prior(prior_logodds)
+        # What is worth seeing: (N,) fp32 importance per point, in the order of `self.points`; the visibility term then
+        # uses the weighted mean sum_j w_j r_j / sum_j w_j (the rewards themselves do not change).
+        self._init_weight(point_weight)
         self.to(self.device)
 
     def _workspace(self, cloud):
@@ -356,11 +416,12 @@ class ModelTraj(_OrderedCloudModel):
         # waypoints range(0, N_wps, wps_step) (src/model.py:217); the others get no visibility gradient
         cloud = self._cloud()
         prior, prior_sum = self._prior_args()
+        weight, wsums, wden = self._weight_args()
         cam = ops._lib.camera(self.img_width, self.img_height, self.pc_clip_limits[0], self.pc_clip_limits[1], self.eps)
         rewards, mean = ops.CoverageTrajFn.apply(cloud, self.poses[::wps_step], self.quats[::wps_step], self.K, cam,
                                                  self.n_total, self.group, self._perm, self._boxes,
                                                  None if self.spatial_sort else True, self._workspace(cloud), prior,
-                                                 prior_sum)
+                                                 prior_sum, weight, wsums, wden)
         self.rewards = rewards
         self._mean = mean
         if debug:
@@ -387,8 +448,14 @@ class ModelTraj(_OrderedCloudModel):
                                 dense=None if self.spatial_sort else True, workspace=self._workspace(cloud))
 
     def criterion(self, rewards):
-        # src/model.py:244-260
-        mean = self._mean if (rewards is self.rewards and self._mean is not None) else torch.mean(rewards)
+        # src/model.py:244-260; with a point weight the weighted mean (fp64 sums), also for rewards from elsewhere
+        if rewards is self.rewards and self._mean is not None:
+            mean = self._mean
+        elif self.point_weight is not None:
+            w = self._weight_args()[0].to(torch.float64)
+            mean = ((w * rewards.to(torch.float64)).sum() / w.sum()).to(rewards.dtype)
+        else:
+            mean = torch.mean(rewards)
         self.loss["vis"] = 1.0 / (mean + self.eps)
         if self.fused_regularizers and self.poses.is_cuda and self.poses.shape[0] >= 3:
             # the three O(W) regularisers and their gradients in one launch (same formulas, fp64 inside)
@@ -415,13 +482,14 @@ class ModelTrajBatch(_OrderedCloudModel):
     Parameters `poses` (T, W, 3) and `quats` (T, W, 4); `forward()` returns sum_t loss_t, where loss_t is
     ModelTraj.criterion's loss of trajectory t.  The per-trajectory terms are kept as (T,) tensors in `self.losses`
     ("vis", "l2", "smooth", "length"), the (T,) mean rewards in `self.means`.  `prior_logodds` (N,) fp32, in the order
-    of `points`: the map memory every trajectory is scored on top of (see ModelTraj)."""
+    of `points`: the map memory every trajectory is scored on top of (see ModelTraj).  `point_weight` (N,) fp32, in the
+    order of `points`: per-point importance; the means are then weighted means (see ModelTraj)."""
 
     _prior_in_cloud_order = True    # the sweeps index the prior like the (Morton-ordered) cloud
 
     def __init__(self, points, wps_poses, wps_quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0,
                  smoothness_weight=14.0, traj_length_weight=0.02, device=torch.device("cuda"), group=None,
-                 n_total=None, spatial_sort=True, prior_logodds=None):
+                 n_total=None, spatial_sort=True, prior_logodds=None, point_weight=None):
         super().__init__()
         wps_poses = torch.as_tensor(wps_poses, dtype=torch.float32)
         wps_quats = torch.as_tensor(wps_quats, dtype=torch.float32)
@@ -454,6 +522,7 @@ class ModelTrajBatch(_OrderedCloudModel):
         self._boxes = None
         self._ws = None
         self._init_prior(prior_logodds)
+        self._init_weight(point_weight)
         self.to(self.device)
 
     def _wps_step(self, vis_wps_dist):
@@ -472,18 +541,20 @@ class ModelTrajBatch(_OrderedCloudModel):
         wps_step = self._wps_step(vis_wps_dist)
         cloud = self._cloud()
         prior, prior_sum = self._prior_args()
+        weight, wsums, wden = self._weight_args()
         P, Q = self.poses[:, ::wps_step], self.quats[:, ::wps_step]
         with ops.evaluation(dense=None if self.spatial_sort else True):
             ws = self._kept_workspace(cloud, ops._BACKEND.sweep_fused_workspace_bytes(cloud, P.shape[0], P.shape[1]))
-            if prior is None:
+            if prior is None and weight is None:
                 means = ops.coverage_sweep(cloud, P, Q, self.K, self.img_width, self.img_height, self.pc_clip_limits[0],
                                            self.pc_clip_limits[1], self.eps, n_total=self.n_total, group=self.group,
                                            boxes=self._boxes, presorted=True, workspace=ws)
-            else:   # the kept sum_j sigmoid(prior_j): no reduction over the prior per step
+            else:   # the kept sums of the prior and the weight: no reduction over them per step
                 cam = ops._lib.camera(self.img_width, self.img_height, self.pc_clip_limits[0], self.pc_clip_limits[1],
                                       self.eps)
                 means = ops.CoverageSweepFn.apply(cloud, P, Q, self.K, cam, int(self.n_total or cloud.shape[0]),
-                                                  self.group, self._boxes, "points", ws, prior, prior_sum)
+                                                  self.group, self._boxes, "points", ws, prior, prior_sum, weight, wsums,
+                                                  wden)
         self.means = means
         return self.criterion(means)
 

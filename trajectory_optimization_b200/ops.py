@@ -93,9 +93,10 @@ def _ptr(t):
     return ctypes.c_void_p(t.data_ptr() if t is not None else 0)
 
 
-def _check_prior(prior, n, device, what="prior_logodds"):
-    """A per-point prior log-odds tensor as the kernels take it: fp32, shape (n,), on the cloud's device; made contiguous
-    and 16-byte aligned (a copy only when it has to).  Shape, dtype and device errors raise ValueError naming `what`."""
+def _check_prior(prior, n, device, what="prior_logodds", unit="log-odds"):
+    """A per-point prior log-odds tensor (or point weight) as the kernels take it: fp32, shape (n,), on the cloud's
+    device; made contiguous and 16-byte aligned (a copy only when it has to).  Shape, dtype and device errors raise
+    ValueError naming `what`."""
     if prior is None:
         return None
     if not isinstance(prior, torch.Tensor):
@@ -103,7 +104,7 @@ def _check_prior(prior, n, device, what="prior_logodds"):
     if prior.dtype != torch.float32:
         raise ValueError(f"{what} must be float32, got {prior.dtype}")
     if tuple(prior.shape) != (n,):
-        raise ValueError(f"{what} must have shape ({n},) (one log-odds per point), got {tuple(prior.shape)}")
+        raise ValueError(f"{what} must have shape ({n},) (one {unit} per point), got {tuple(prior.shape)}")
     if prior.device != device:
         raise ValueError(f"{what} is on {prior.device}, the cloud on {device}")
     prior = prior.detach()
@@ -112,6 +113,12 @@ def _check_prior(prior, n, device, what="prior_logodds"):
     if prior.is_cuda and prior.data_ptr() % 16:
         prior = prior.clone()
     return prior
+
+
+def _check_weight(weight, n, device, what="weight"):
+    """A per-point weight as the kernels take it (see _check_prior), or None.  Values are not checked here (that would
+    synchronise with the host): finite, >= 0 and a positive sum are the caller's to ensure."""
+    return _check_prior(weight, n, device, what, unit="weight")
 
 
 def _all_reduce(t, op, group):
@@ -279,6 +286,13 @@ class CudaBackend:
         _call("cov_prior_reward_sum", prior, _ptr(prior), prior.shape[0], _ptr(out))
         return out
 
+    def weight_sums(self, weight, prior=None):
+        """[sum_j w_j r0_j, sum_j w_j] in fp64 on the device, (2,) (cov_weight_sums); r0_j = sigmoid(prior_j) or 1/2: the
+        reward-sum base and the denominator of the weighted calls."""
+        out = torch.empty(2, dtype=torch.float64, device=weight.device)
+        _call("cov_weight_sums", weight, _ptr(weight), _ptr(prior), weight.shape[0], _ptr(out))
+        return out
+
     def traj_minmax(self, pts, P, Q, Kd, cam, boxes=None, ws=None, dense=None, prefill=None, prior=None):
         """`prior` (indexed like `prefill`): the pre-fill writes sigmoid(prior_i) instead of 1/2."""
         W = P.shape[0]
@@ -294,11 +308,17 @@ class CudaBackend:
         return minmax
 
     def traj_fused(self, pts, P, Q, Kd, cam, minmax, upstream, rewards, reward_index=None, boxes=None, ws=None,
-                   dense=None, prefilled=False, prior=None, prior_sum=None):
+                   dense=None, prefilled=False, prior=None, prior_sum=None, weight=None, wsums=None):
+        """`weight` (with `wsums` from weight_sums): the weighted sums of cov_traj_fused_weighted (no upstream)."""
         W, n = P.shape[0], pts.shape[0]
         acc = torch.empty(W * _lib.ACC_STRIDE + 1, dtype=torch.float64, device=pts.device)
         ws = self.traj_workspace(pts, W) if ws is None else ws
         opts = _opts(dense, rewards_prefilled=prefilled)
+        if weight is not None:
+            _call("cov_traj_fused_weighted", pts, _ptr(pts), n, _ptr(P), _ptr(Q), W, _ptr(Kd), ctypes.byref(cam),
+                  _ptr(boxes), _ptr(minmax), _ptr(reward_index), _ptr(rewards), _ptr(acc), _ptr(prior), _ptr(weight),
+                  _ptr(wsums), ctypes.byref(opts), _ptr(ws), ws.numel())
+            return acc
         if prior is not None:
             _call("cov_traj_fused_prior", pts, _ptr(pts), n, _ptr(P), _ptr(Q), W, _ptr(Kd), ctypes.byref(cam), _ptr(boxes),
                   _ptr(minmax), _ptr(upstream), _ptr(reward_index), _ptr(rewards), _ptr(acc), _ptr(prior), _ptr(prior_sum),
@@ -336,14 +356,20 @@ class CudaBackend:
             minmax[W + w0:W + w1] = mm[w1 - w0:]
         return minmax
 
-    def sweep_sums(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior=None, prior_sum=None):
-        """sum_j rewards_j(t) over this cloud for every trajectory t (fp64); `prior` in the cloud's order."""
+    def sweep_sums(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior=None, prior_sum=None, weight=None, wsums=None):
+        """sum_j rewards_j(t) over this cloud for every trajectory t (fp64); `prior` in the cloud's order.  `weight` (cloud's
+        order, with `wsums`): sum_j w_j rewards_j(t)."""
         L = _lib.lib()
         n, dev = pts.shape[0], pts.device
         ws_bytes = L.cov_sweep_workspace_bytes(n, T, Pn)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         sums = torch.zeros(T, dtype=torch.float64, device=dev)
         opts = _opts()
+        if weight is not None:
+            _call("cov_sweep_rewards_weighted", pts, _ptr(pts), n, _ptr(P), _ptr(Q), T, Pn, _ptr(Kd), ctypes.byref(cam),
+                  _ptr(boxes), _ptr(minmax), _ptr(sums), _ptr(prior), _ptr(weight), _ptr(wsums), ctypes.byref(opts),
+                  _ptr(ws), ws_bytes)
+            return sums
         if prior is not None:
             _call("cov_sweep_rewards_prior", pts, _ptr(pts), n, _ptr(P), _ptr(Q), T, Pn, _ptr(Kd), ctypes.byref(cam),
                   _ptr(boxes), _ptr(minmax), _ptr(sums), _ptr(prior), _ptr(prior_sum), ctypes.byref(opts), _ptr(ws), ws_bytes)
@@ -352,9 +378,14 @@ class CudaBackend:
               _ptr(minmax), _ptr(sums), ctypes.byref(opts), _ptr(ws), ws_bytes)
         return sums
 
-    def traj_epilogue(self, acc, minmax, Q, n_total, upstream_mode):
+    def traj_epilogue(self, acc, minmax, Q, n_total, upstream_mode, den=None):
+        """`den` ((1,) fp64 on the device, sum_j w_j): the weighted mean's epilogue (cov_traj_epilogue_dev) in place of
+        n_total."""
         W = Q.shape[0]
         out = torch.empty(1 + 7 * W, dtype=torch.float32, device=acc.device)
+        if den is not None:
+            _call("cov_traj_epilogue_dev", acc, _ptr(acc), _ptr(minmax), _ptr(Q), W, _ptr(den), _ptr(out))
+            return out
         _call("cov_traj_epilogue", acc, _ptr(acc), _ptr(minmax), _ptr(Q), W, n_total, upstream_mode, _ptr(out))
         return out
 
@@ -363,15 +394,21 @@ class CudaBackend:
         opts = _opts(dense)
         return _lib.lib().cov_sweep_fused_workspace_bytes(pts.shape[0], T, Pn, ctypes.byref(opts))
 
-    def sweep_fused(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, ws=None, prior=None, prior_sum=None):
+    def sweep_fused(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, ws=None, prior=None, prior_sum=None, weight=None,
+                    wsums=None):
         """This cloud's pass-B accumulators of every trajectory: T blocks of 22 Pn + 1 doubles (cov_sweep_fused);
-        `prior` in the cloud's order."""
+        `prior` in the cloud's order; `weight` (cloud's order, with `wsums`): cov_sweep_fused_weighted."""
         n, dev = pts.shape[0], pts.device
         ws_bytes = self.sweep_fused_workspace_bytes(pts, T, Pn)
         if ws is None or ws.numel() < ws_bytes or ws.device != dev:
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         acc = torch.empty(T * (Pn * _lib.ACC_STRIDE + 1), dtype=torch.float64, device=dev)
         opts = _opts()
+        if weight is not None:
+            _call("cov_sweep_fused_weighted", pts, _ptr(pts), n, _ptr(P), _ptr(Q), T, Pn, _ptr(Kd), ctypes.byref(cam),
+                  _ptr(boxes), _ptr(minmax), _ptr(acc), _ptr(prior), _ptr(weight), _ptr(wsums), ctypes.byref(opts),
+                  _ptr(ws), ws.numel())
+            return acc
         if prior is not None:
             _call("cov_sweep_fused_prior", pts, _ptr(pts), n, _ptr(P), _ptr(Q), T, Pn, _ptr(Kd), ctypes.byref(cam),
                   _ptr(boxes), _ptr(minmax), _ptr(acc), _ptr(prior), _ptr(prior_sum), ctypes.byref(opts), _ptr(ws),
@@ -381,14 +418,29 @@ class CudaBackend:
               _ptr(minmax), _ptr(acc), ctypes.byref(opts), _ptr(ws), ws.numel())
         return acc
 
-    def sweep_epilogue(self, acc, minmax, Q, T, Pn, n_total):
-        """[T means | T Pn 3 d mean_t/d poses | T Pn 4 d mean_t/d quats] (fp32) from the summed accumulators."""
+    def sweep_epilogue(self, acc, minmax, Q, T, Pn, n_total, den=None):
+        """[T means | T Pn 3 d mean_t/d poses | T Pn 4 d mean_t/d quats] (fp32) from the summed accumulators; `den` ((1,)
+        fp64 on the device): the denominator in place of n_total (cov_sweep_epilogue_dev, weighted means)."""
         out = torch.empty(T * (1 + 7 * Pn), dtype=torch.float32, device=acc.device)
+        if den is not None:
+            _call("cov_sweep_epilogue_dev", acc, _ptr(acc), _ptr(minmax), _ptr(Q), T, Pn, _ptr(den), _ptr(out))
+            return out
         _call("cov_sweep_epilogue", acc, _ptr(acc), _ptr(minmax), _ptr(Q), T, Pn, n_total, _ptr(out))
         return out
 
 
 _BACKEND = CudaBackend()
+
+
+def _weight_sums(B, w, prior, group):
+    """(this shard's cov_weight_sums (2,), the denominator sum_j w_j over every rank (1,)): with a group the denominator
+    is all-reduced (SUM of one double); the base [0] stays per shard, the accumulators' all-reduce sums it."""
+    wsums = B.weight_sums(w, prior)
+    if group is None:
+        return wsums, wsums[1:]
+    den = wsums[1:].clone()
+    _all_reduce(den, _reduce_ops()[2], group)
+    return wsums, den
 
 
 class CoveragePoseFn(torch.autograd.Function):
@@ -474,9 +526,11 @@ class CoverageTrajFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, points, poses, quats, K, cam, n_total, group, reward_index=None, boxes=None, dense=None,
-                workspace=None, prior=None, prior_sum=None):
+                workspace=None, prior=None, prior_sum=None, weight=None, wsums=None, den=None):
         # prior / prior_sum: the checked (N,) prior log-odds in the order of the rewards and sum_j sigmoid(prior_j) of
-        # this shard ((1,) fp64 on the device), or None
+        # this shard ((1,) fp64 on the device), or None.  weight / wsums / den: the checked (N,) point weight in the same
+        # order, this shard's cov_weight_sums (2,) and the global sum_j w_j (1,): the mean is then the weighted mean
+        # (prior_sum may be None: only the gradient through the rewards needs it, and computes it then)
         B = _BACKEND
         dev = points.device
         pts = B.prepare(points, what="points")
@@ -503,7 +557,7 @@ class CoverageTrajFn(torch.autograd.Function):
             minmax = B.traj_minmax(pts, P, Q, Kd, cam, boxes, ws, dense, prefill, prior)
         _all_reduce_minmax(minmax, W, group)                 # global normalisers: W minima, W maxima
         out = CoverageTrajFn._run(pts, P, Q, Kd, cam, minmax, None, rewards, n_total, group, reward_index, boxes, ws,
-                                  dense, prefill is not None, prior, prior_sum)
+                                  dense, prefill is not None, prior, prior_sum, weight, wsums, den)
         ctx.cam, ctx.group, ctx.n_total, ctx.reward_index, ctx.boxes = cam, group, n_total, reward_index, boxes
         ctx.dense, ctx.prior, ctx.prior_sum = dense, prior, prior_sum
         ctx.shapes = (poses.shape, quats.shape)
@@ -513,14 +567,19 @@ class CoverageTrajFn(torch.autograd.Function):
 
     @staticmethod
     def _run(pts, P, Q, Kd, cam, minmax, upstream, rewards, n_total, group, reward_index=None, boxes=None, ws=None,
-             dense=None, prefilled=False, prior=None, prior_sum=None):
-        if prior is None:
+             dense=None, prefilled=False, prior=None, prior_sum=None, weight=None, wsums=None, den=None):
+        if weight is not None:   # pass B, weighted sums (never with an upstream)
+            acc = _BACKEND.traj_fused(pts, P, Q, Kd, cam, minmax, None, rewards, reward_index, boxes, ws, dense,
+                                      prefilled, prior=prior, weight=weight, wsums=wsums)
+        elif prior is None:
             acc = _BACKEND.traj_fused(pts, P, Q, Kd, cam, minmax, upstream, rewards, reward_index, boxes, ws, dense,
                                       prefilled)   # pass B
         else:
             acc = _BACKEND.traj_fused(pts, P, Q, Kd, cam, minmax, upstream, rewards, reward_index, boxes, ws, dense,
                                       prefilled, prior, prior_sum)
         _all_reduce_acc(acc, P.shape[0], group)
+        if weight is not None:
+            return _BACKEND.traj_epilogue(acc, minmax, Q, n_total, 0, den)
         return _BACKEND.traj_epilogue(acc, minmax, Q, n_total, 0 if upstream is None else 1)
 
     @staticmethod
@@ -534,13 +593,17 @@ class CoverageTrajFn(torch.autograd.Function):
         if g_rewards is not None:
             up = _BACKEND.prepare(g_rewards, pts.device, "grad_rewards").reshape(-1)
             scratch = torch.empty(pts.shape[0], dtype=torch.float32, device=pts.device)
+            # the rewards do not depend on the weight: the unweighted pass B with the upstream
+            psum = ctx.prior_sum
+            if ctx.prior is not None and psum is None:
+                psum = _BACKEND.prior_sum(ctx.prior)
             o2 = CoverageTrajFn._run(pts, P, Q, Kd, ctx.cam, minmax, up, scratch, ctx.n_total, ctx.group,
-                                     ctx.reward_index, ctx.boxes, None, ctx.dense, False, ctx.prior, ctx.prior_sum)
+                                     ctx.reward_index, ctx.boxes, None, ctx.dense, False, ctx.prior, psum)
             g_p = o2[1:1 + 3 * W] if g_p is None else g_p + o2[1:1 + 3 * W]
             g_q = o2[1 + 3 * W:] if g_q is None else g_q + o2[1 + 3 * W:]
         ps, qs = ctx.shapes
         return (None, None if g_p is None else g_p.reshape(ps), None if g_q is None else g_q.reshape(qs),
-                None, None, None, None, None, None, None, None, None, None)
+                None, None, None, None, None, None, None, None, None, None, None, None, None)
 
 
 class CoverageSweepFn(torch.autograd.Function):
@@ -548,7 +611,10 @@ class CoverageSweepFn(torch.autograd.Function):
     CoverageTrajFn evaluates them, and d means_t / d (poses_t, quats_t) from the same pass (cov_sweep_fused)."""
 
     @staticmethod
-    def forward(ctx, pts, poses, quats, K, cam, n_total, group, boxes, shard, workspace, prior=None, prior_sum=None):
+    def forward(ctx, pts, poses, quats, K, cam, n_total, group, boxes, shard, workspace, prior=None, prior_sum=None,
+                weight=None, wsums=None, den=None):
+        # weight / wsums / den (cloud's order): the checked point weight, cov_weight_sums of this rank's cloud and the
+        # denominator sum_j w_j of the whole cloud (shard="points": all-reduced; "trajectories": this rank's own)
         B = _BACKEND
         dev = pts.device
         T, Pn = poses.shape[0], poses.shape[1]
@@ -564,7 +630,7 @@ class CoverageSweepFn(torch.autograd.Function):
             mine = torch.zeros(per * (1 + 7 * Pn), dtype=torch.float32, device=dev)
             if nt > 0:
                 o = CoverageSweepFn._run(pts, poses[t0:t1], quats[t0:t1], Kd, cam, n_total, None, boxes, workspace, prior,
-                                         prior_sum)
+                                         prior_sum, weight, wsums, den)
                 mine[:nt] = o[:nt]
                 mine[per:per + 3 * nt * Pn] = o[nt:nt + 3 * nt * Pn]
                 mine[per + 3 * per * Pn:per + 3 * per * Pn + 4 * nt * Pn] = o[nt + 3 * nt * Pn:]
@@ -574,13 +640,15 @@ class CoverageSweepFn(torch.autograd.Function):
             out = torch.cat([every[:, :per].reshape(-1)[:T], every[:, per:per + 3 * per * Pn].reshape(-1)[:3 * T * Pn],
                              every[:, per + 3 * per * Pn:].reshape(-1)[:4 * T * Pn]])
         else:
-            out = CoverageSweepFn._run(pts, poses, quats, Kd, cam, n_total, group, boxes, workspace, prior, prior_sum)
+            out = CoverageSweepFn._run(pts, poses, quats, Kd, cam, n_total, group, boxes, workspace, prior, prior_sum,
+                                       weight, wsums, den)
         ctx.shapes = (poses.shape, quats.shape)
         ctx.save_for_backward(out)
         return out[:T].clone()
 
     @staticmethod
-    def _run(pts, poses, quats, Kd, cam, n_total, group, boxes, workspace, prior=None, prior_sum=None):
+    def _run(pts, poses, quats, Kd, cam, n_total, group, boxes, workspace, prior=None, prior_sum=None, weight=None,
+             wsums=None, den=None):
         B = _BACKEND
         dev = pts.device
         T, Pn = poses.shape[0], poses.shape[1]
@@ -588,13 +656,18 @@ class CoverageSweepFn(torch.autograd.Function):
         Q = B.prepare(quats, dev, "quats").reshape(-1, 4)
         minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)     # pass A on this shard, (2, T Pn)
         _all_reduce_minmax(minmax, T * Pn, group)
-        if prior is None:
+        if weight is not None:
+            acc = B.sweep_fused(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, workspace, prior=prior, weight=weight,
+                                wsums=wsums)
+        elif prior is None:
             acc = B.sweep_fused(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, workspace)
         else:
             acc = B.sweep_fused(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, workspace, prior, prior_sum)
         if group is not None:
             # plain all-reduce: the in-kernel exchange buffers are sized for the 22 W + 1 doubles of one trajectory
             _all_reduce(acc, _reduce_ops()[2], group)
+        if weight is not None:
+            return B.sweep_epilogue(acc, minmax, Q, T, Pn, n_total, den)
         return B.sweep_epilogue(acc, minmax, Q, T, Pn, n_total)
 
     @staticmethod
@@ -605,7 +678,7 @@ class CoverageSweepFn(torch.autograd.Function):
         g = g_means.reshape(T, 1).to(out.dtype)
         g_p = (g * out[T:T + 3 * T * Pn].reshape(T, 3 * Pn)).reshape(ps)
         g_q = (g * out[T + 3 * T * Pn:].reshape(T, 4 * Pn)).reshape(qs)
-        return None, g_p, g_q, None, None, None, None, None, None, None, None, None
+        return None, g_p, g_q, None, None, None, None, None, None, None, None, None, None, None, None
 
 
 class TrajRegularizersFn(torch.autograd.Function):
@@ -679,7 +752,7 @@ def coverage_pose_batch(points, trans, quats, intrins, img_width, img_height, mi
 
 def coverage_traj(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
                   n_total=None, group=None, reward_index=None, boxes=None, dense=None, workspace=None,
-                  prior_logodds=None):
+                  prior_logodds=None, weight=None):
     """Fused ModelTraj visibility term over the W poses given.  Returns (rewards (N,), mean(rewards)).
     `reward_index` (int32, from `spatial_sort`): `points` is a reordered copy of the caller's cloud and
     rewards come back in the caller's order.  `boxes` (from `tile_boxes(points)`): built once per cloud so the
@@ -687,15 +760,22 @@ def coverage_traj(points, poses, quats, intrins, img_width, img_height, min_dist
     cloud should ask for).  `workspace`: a uint8 CUDA tensor kept by the caller across calls (one per cloud).
     `prior_logodds` (N,) fp32: what earlier paths observed (map memory, e.g. `traj_logodds` of an executed path);
     rewards_j = sigmoid(prior_j + sum_w lo_jw), indexed like the rewards (the caller's order when `reward_index` is
-    given).  With a `group` it is this rank's slice.  None = an empty map (exactly the rewards of a zero prior)."""
+    given).  With a `group` it is this rank's slice.  None = an empty map (exactly the rewards of a zero prior).
+    `weight` (N,) fp32, finite and >= 0 with a positive sum (not checked: no host synchronisation): per-point importance,
+    indexed like the rewards.  The mean is then sum_j w_j r_j / sum_j w_j (its gradient from the same pass); the rewards
+    are unchanged.  With a `group` it is this rank's slice (the denominator is all-reduced); `n_total` is not used."""
     cam = _lib.camera(img_width, img_height, min_dist, max_dist, eps)
-    prior = psum = None
-    if prior_logodds is not None:
+    prior = psum = w = wsums = den = None
+    if prior_logodds is not None or weight is not None:
         pts = _BACKEND.prepare(points, what="points")
         prior = _check_prior(prior_logodds, pts.shape[0], pts.device)
-        psum = _BACKEND.prior_sum(prior)
+        w = _check_weight(weight, pts.shape[0], pts.device)
+        if w is not None:
+            wsums, den = _weight_sums(_BACKEND, w, prior, group)
+        elif prior is not None:
+            psum = _BACKEND.prior_sum(prior)
     return CoverageTrajFn.apply(points, poses, quats, intrins, cam, n_total, group, reward_index, boxes, dense, workspace,
-                                prior, psum)
+                                prior, psum, w, wsums, den)
 
 
 @torch.no_grad()
@@ -777,16 +857,22 @@ def sort_pairs(keys, vals, begin_bit=0, end_bit=32):
     return k, v
 
 
-def _order_with_prior(B, pts, prior, boxes, presorted):
-    """The sweeps' cloud ordering (Morton order unless `presorted` or `boxes`), the prior permuted with the cloud."""
+def _order_with_prior(B, pts, prior, boxes, presorted, weight=None):
+    """The sweeps' cloud ordering (Morton order unless `presorted` or `boxes`), the prior and the weight permuted with
+    the cloud."""
     if not presorted and boxes is None and pts.shape[0] > 0:
         pts, perm, boxes = B.order_cloud(pts, True)
-        if prior is not None and perm is not None:
-            prior = _check_prior(prior.index_select(0, perm.long()), pts.shape[0], pts.device)   # prior[j] of point perm[j]
-    return pts, prior, boxes
+        if perm is not None:
+            if prior is not None:   # prior[j] of point perm[j]
+                prior = _check_prior(prior.index_select(0, perm.long()), pts.shape[0], pts.device)
+            if weight is not None:
+                weight = _check_weight(weight.index_select(0, perm.long()), pts.shape[0], pts.device)
+    return pts, prior, boxes, weight
 
 
-def _sweep_sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum):
+def _sweep_sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum, w=None, wsums=None):
+    if w is not None:
+        return B.sweep_sums(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior=prior, weight=w, wsums=wsums)
     if prior is None:
         return B.sweep_sums(pts, P, Q, T, Pn, Kd, cam, boxes, minmax)
     return B.sweep_sums(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum)
@@ -794,7 +880,8 @@ def _sweep_sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum):
 
 @torch.no_grad()
 def sweep_rewards(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
-                  n_total=None, group=None, boxes=None, presorted=False, shard="points", prior_logodds=None):
+                  n_total=None, group=None, boxes=None, presorted=False, shard="points", prior_logodds=None,
+                  weight=None):
     """Forward-only mean reward of many candidate trajectories: poses (T, P, 3), quats (T, P, 4) -> (T,) fp64
     (semantics: ModelTraj.forward per trajectory with every pose evaluated, reference src/model.py:217-237).
     The cloud is Morton-ordered first (no per-point output exists, so the order is free) unless `presorted`;
@@ -810,14 +897,22 @@ def sweep_rewards(points, poses, quats, intrins, img_width, img_height, min_dist
     `prior_logodds` (N,) fp32: per-point prior log-odds (map memory), shared by every trajectory: each trajectory's
     rewards are sigmoid(prior_j + sum_w lo_jw).  In the order of `points` as passed (permuted with the cloud when the
     call orders it; with `presorted`, already in the cloud's order); shard="points": this rank's slice,
-    shard="trajectories": the whole prior on every rank."""
+    shard="trajectories": the whole prior on every rank.
+    `weight` (N,) fp32, finite and >= 0 with a positive sum (not checked): per-point importance shared by every
+    trajectory; each result is then sum_j w_j r_j(t) / sum_j w_j.  Ordered and sharded like `prior_logodds` (with
+    shard="points" the denominator is all-reduced); `n_total` is not used."""
     B = _BACKEND
     if shard not in ("points", "trajectories"):
         raise ValueError("shard must be 'points' or 'trajectories'")
     pts = B.prepare(points, what="points")
     prior = _check_prior(prior_logodds, pts.shape[0], pts.device)
-    pts, prior, boxes = _order_with_prior(B, pts, prior, boxes, presorted)
-    psum = None if prior is None else B.prior_sum(prior)
+    w = _check_weight(weight, pts.shape[0], pts.device)
+    pts, prior, boxes, w = _order_with_prior(B, pts, prior, boxes, presorted, w)
+    psum = wsums = den = None
+    if w is not None:
+        wsums, den = _weight_sums(B, w, prior, group if shard == "points" else None)
+    elif prior is not None:
+        psum = B.prior_sum(prior)
     dev = pts.device
     T, Pn = poses.shape[0], poses.shape[1]
     n = pts.shape[0]
@@ -833,23 +928,25 @@ def sweep_rewards(points, poses, quats, intrins, img_width, img_height, min_dist
             P = B.prepare(poses[t0:t1], dev, "poses").reshape(-1, 3)
             Q = B.prepare(quats[t0:t1], dev, "quats").reshape(-1, 4)
             minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)
-            mine[:t1 - t0] = _sweep_sums(B, pts, P, Q, t1 - t0, Pn, Kd, cam, boxes, minmax, prior, psum)
+            mine[:t1 - t0] = _sweep_sums(B, pts, P, Q, t1 - t0, Pn, Kd, cam, boxes, minmax, prior, psum, w, wsums)
         out = torch.empty(world * per, dtype=torch.float64, device=dev)
         dist.all_gather_into_tensor(out, mine, group=group)
-        return out[:T] / float(n)
+        return out[:T] / (float(n) if w is None else den)
     P = B.prepare(poses, dev, "poses").reshape(-1, 3)
     Q = B.prepare(quats, dev, "quats").reshape(-1, 4)
     minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)
     _all_reduce_minmax(minmax, T * Pn, group)
-    sums = _sweep_sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum)
+    sums = _sweep_sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum, w, wsums)
     if group is not None:
         _all_reduce(sums, _reduce_ops()[2], group)
+    if w is not None:
+        return sums / den
     return sums / float(n if n_total is None else n_total)
 
 
 def coverage_sweep(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
                    n_total=None, group=None, boxes=None, presorted=False, shard="points", workspace=None,
-                   prior_logodds=None):
+                   prior_logodds=None, weight=None):
     """Differentiable candidate sweep: poses (T, P, 3), quats (T, P, 4) -> means (T,) fp32, where means[t] is the mean
     reward of trajectory t as `coverage_traj(points, poses[t], quats[t])` computes it.  `means` is differentiable w.r.t.
     `poses` and `quats`; each trajectory's gradient comes from the same pass over the cloud (cov_sweep_fused), so a
@@ -859,7 +956,8 @@ def coverage_sweep(points, poses, quats, intrins, img_width, img_height, min_dis
     kept by the caller across calls (grown when too small).
     Sharding as in `sweep_rewards`: shard="points" (this rank's slice of the cloud; normalisers and accumulators are
     all-reduced) or shard="trajectories" (the whole cloud on every rank; means and gradients are all-gathered).
-    `prior_logodds`: per-point prior log-odds shared by every trajectory, ordered and sharded as in `sweep_rewards`."""
+    `prior_logodds`: per-point prior log-odds shared by every trajectory, ordered and sharded as in `sweep_rewards`.
+    `weight`: per-point importance as in `sweep_rewards`: means[t] = sum_j w_j r_j(t) / sum_j w_j and its gradient."""
     B = _BACKEND
     if shard not in ("points", "trajectories"):
         raise ValueError("shard must be 'points' or 'trajectories'")
@@ -870,11 +968,17 @@ def coverage_sweep(points, poses, quats, intrins, img_width, img_height, min_dis
                          f"{tuple(getattr(poses, 'shape', ()))} and {tuple(getattr(quats, 'shape', ()))}")
     pts = B.prepare(points, what="points")
     prior = _check_prior(prior_logodds, pts.shape[0], pts.device)
-    pts, prior, boxes = _order_with_prior(B, pts, prior, boxes, presorted)
-    psum = None if prior is None else B.prior_sum(prior)
+    w = _check_weight(weight, pts.shape[0], pts.device)
+    pts, prior, boxes, w = _order_with_prior(B, pts, prior, boxes, presorted, w)
+    psum = wsums = den = None
+    if w is not None:
+        wsums, den = _weight_sums(B, w, prior, group if shard == "points" else None)
+    elif prior is not None:
+        psum = B.prior_sum(prior)
     n_total = int(pts.shape[0] if n_total is None else n_total)
     cam = _lib.camera(img_width, img_height, min_dist, max_dist, eps)
-    return CoverageSweepFn.apply(pts, poses, quats, intrins, cam, n_total, group, boxes, shard, workspace, prior, psum)
+    return CoverageSweepFn.apply(pts, poses, quats, intrins, cam, n_total, group, boxes, shard, workspace, prior, psum, w,
+                                 wsums, den)
 
 
 @torch.no_grad()
