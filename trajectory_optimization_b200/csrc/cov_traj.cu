@@ -29,17 +29,19 @@
 //             the arg-max, adds logit(1/2) = 0 to the log-odds sum and nothing to the gradient.
 //   cov_traj_prepare_kernel (A) / cov_traj_table_kernel (B)   pose table; A also evaluates a strided sample of the
 //                        cloud (lower bounds of the maxima, which minima are exactly 0); B zeroes the accumulators
-//   cov_cull_kernel      one warp per group of 8 tiles: boxes against every pose -> per-tile pose bit mask, and the
-//                        ascending work list of the tiles with a non-empty mask, positions from a decoupled
-//                        look-back scan over the blocks' counts (deterministic; no second kernel); in pass B the
-//                        same blocks pre-fill the rewards with 1/2 (what every unlisted point gets, exactly)
-//   *_tiles_kernel       persistent WARPS (for_each_item): a warp draws 128-point items of the listed tiles from a
-//                        ticket counter; the next item's points, box and the tile's pose mask arrive by TMA bulk copy
-//                        in the warp's other stage (double-buffered, one mbarrier per stage) while it works on the
-//                        current one.  A warp evaluates a listed pose only if its own 128-point box (in pass A, then
-//                        also one of its points) passes the same test.  Pass B's backward re-evaluates: the warp walks
-//                        the poses it gated and recomputes m and dm/dx for its own points, with every lane busy.
-//   Tiles that are not listed are never read: their rewards are the pre-filled 1/2 (exact), their sum is 0.5 * count.
+//   cov_cull_kernel      one warp per group of 8 tiles of 1024 points: the group's box, then each tile's box, then each
+//                        128-point box against every pose -> a pose bit mask per listed box (a pose is listed for a
+//                        box when its tile's box and its own box pass the test), and the ascending work list of the
+//                        boxes with a non-empty mask, positions from a decoupled look-back scan over the blocks'
+//                        counts (deterministic; no second kernel); in pass B the same blocks pre-fill the rewards with
+//                        1/2 (what every unlisted point gets, exactly)
+//   *_tiles_kernel       persistent WARPS (for_each_item): a warp draws listed boxes (128-point items) from a ticket
+//                        counter; the next item's points and pose mask arrive by TMA bulk copy in the warp's other
+//                        stage (double-buffered, one mbarrier per stage) while it works on the current one.  Every
+//                        pose of the mask is evaluated (pass A first runs its per-point pre-filter).  Pass B's backward
+//                        re-evaluates: the warp walks the poses it gated and recomputes m and dm/dx for its own points,
+//                        with every lane busy.
+//   Boxes that are not listed are never read: their rewards are the pre-filled 1/2 (exact), their sum is 0.5 * count.
 //
 // CANDIDATE SWEEPS (many trajectories, one cloud; pose tables of up to 2048 trajectory-major poses per launch):
 //   cov_sweep_tiles_kernel        forward only: per-trajectory sum_j r_j
@@ -62,7 +64,7 @@ namespace {
 
 constexpr int kWarps = COV_THREADS / 32;
 constexpr unsigned kFull = 0xffffffffu;
-constexpr int kMaskWords = 64;   // pose bit mask of a tile: covers cov_traj_max_poses() <= 2048
+constexpr int kMaskWords = 64;   // pose bit mask of a box: covers cov_traj_max_poses() <= 2048
 constexpr int kBoxPts = COV_BOX_POINTS;  // points per precomputed bounding box
 
 __host__ __device__ constexpr int tile_points(int ppt) { return COV_THREADS * ppt; }
@@ -130,10 +132,6 @@ __device__ __forceinline__ float ord2f(unsigned u) {
 }
 
 // (box_q2lb, the box bound the pruned kernels test against, is in cov_common.cuh)
-__device__ __forceinline__ void box_union(float4& lo, float4& hi, const float4& lo2, const float4& hi2) {
-    lo.x = fminf(lo.x, lo2.x); lo.y = fminf(lo.y, lo2.y); lo.z = fminf(lo.z, lo2.z);
-    hi.x = fmaxf(hi.x, hi2.x); hi.y = fmaxf(hi.y, hi2.y); hi.z = fmaxf(hi.z, hi2.z);
-}
 // Pass-A cap on q2 from the extrema seen so far (as uints): +inf (evaluate everything) unless the minimum is known
 // to be exactly 0.  NaN propagates and every test against it evaluates.
 __device__ __forceinline__ float minmax_qcap(unsigned mn, unsigned mx, float inv_kd) {
@@ -234,8 +232,11 @@ __global__ void cov_minmax_init_kernel(unsigned* gmin, unsigned* gmax, int W) {
 // ============================================ pruned passes: set-up ============================================
 // Control words of one pruned call, at the head of the workspace (zeroed once per call: by a memset node in pass A,
 // by cov_traj_table_kernel in pass B):
-//   ctrl[0] work-list length   ctrl[1] some pose has min_j m > 0   ctrl[2] block ticket of the evaluation kernel
-//   ctrl[4..5] (tile, pose) pairs the cull listed (u64)
+//   ctrl[0] work-list length (listed boxes)   ctrl[1] some pose has min_j m > 0   ctrl[2] block ticket of the
+//   evaluation kernel   ctrl[3] its item ticket
+//   ctrl[4..5] (box, pose) pairs of the poses the cull listed per tile, all 8 boxes of a tile (u64; work counter [6])
+//   ctrl[6..7] the same over the boxes inside the cloud (u64; work counter [7])
+//   ctrl[8..9] boxes of listed tiles that no pose reaches at box level (u64)
 //   enc[0..W)  ~bits(min_j m)   enc[W..2W) bits(max_j m)   pass A's extrema in an encoding whose neutral element is 0:
 //              m >= +0, so the unsigned order of the bits is the float order; both are kept with atomicMax
 //   desc[c]    look-back descriptor of cull chunk c (status in the top two bits)
@@ -366,27 +367,90 @@ __global__ void __launch_bounds__(256) cov_tile_boxes_kernel(const float* __rest
     }
 }
 
-// Cull + work list.  mask[tile][c] bit i <=> pose 32c+i can matter for some point of the tile.  One warp per GROUP of 8
-// consecutive tiles: every pose is tested against the group's box first (one lane per pose), and only the few that
-// pass are tested against the 8 tile boxes (one lane per tile).  Pass A passes `enc` (after the prepare launch) and the
-// cap is derived here; pass B reads qthr from the table.
+// Cull + work list.  The work list holds the indices of the LISTED BOXES (128 points each) in ascending order, and
+// mask[b][c] bit i <=> pose 32c+i is to be evaluated on box b (masks are indexed by box and written for listed boxes
+// only).  The predicate is two-level: a pose is listed for a 1024-point tile when the tile's box passes the test, and
+// evaluated on a box of that tile when the box's own box passes it too (`!(box_q2lb(lo, hi, v3) > cap)`, a NaN cap
+// evaluates).  One warp per GROUP of 8 consecutive tiles (64 boxes): every pose is tested against the group's box
+// first (one lane per pose); for each pose that passes, lane l tests tile l & 7 (one ballot gives the 8 tiles' bits) and
+// its own two boxes, in-group boxes l and 32 + l (tiles l >> 3 and 4 + (l >> 3)), so a lane ends a pose word holding
+// that word of its two boxes' masks and stores it once the box is known to be listed.  Pass A passes `enc` (after the
+// prepare launch) and the cap is derived here; pass B reads qthr from the table.
 // A block iteration covers a CHUNK of 64 consecutive tiles; the block first culls ALL its chunks (warps independent, no
-// barrier), then appends each chunk's listed tiles to the work list in ascending order: the chunk's offset is the
+// barrier), then appends each chunk's listed boxes to the work list in ascending order: the chunk's offset is the
 // exclusive prefix sum of the chunks' counts, obtained with a decoupled look-back over per-chunk descriptors (publish
 // the own aggregates, then sum predecessors until one carries an inclusive prefix).  The list is a pure function of the
-// masks (deterministic).  Grid <= resident capacity, and every block publishes its aggregates before it waits for
-// anybody's, so every predecessor a block waits for has been (or is being) published.  `fill_dst` (pass B): the same
-// blocks write 1/2 to every reward (HAS_PRIOR: sigmoid(prior_i), with pass B's expression).
+// boxes and the caps (deterministic).  Grid <= resident capacity, and every block publishes its aggregates before it
+// waits for anybody's, so every predecessor a block waits for has been (or is being) published.  `fill_dst` (pass B):
+// the same blocks write 1/2 to every reward (HAS_PRIOR: sigmoid(prior_i), with pass B's expression).
+// Counts for the work counters (ctrl[4..9], u64 each): (box, pose) pairs of the poses listed per tile, over all 8 boxes
+// of the tile and over the boxes inside the cloud, and the boxes of listed tiles that no pose reaches.
 constexpr int kCullMaxIter = 32;  // chunks per block at most (the host sizes the grid accordingly)
+constexpr int kTileBoxes = 8;     // 128-point boxes per 1024-point tile of the pruned passes
+
+// One warp's group of 8 tiles as the cull sees it from lane l: its boxes l and 32 + l, the box of tile l & 7 and the
+// group's box.  Boxes of tiles past `ntiles` are empty and never listed.
+struct CullGroup {
+    float4 lo[2], hi[2];  // the lane's two boxes
+    float4 tlo, thi;      // the box of tile l & 7
+    float4 glo, ghi;      // the group's box
+    bool tile_ok;         // tile l & 7 is < ntiles
+    int tile_in;          // its boxes inside the cloud (0..8)
+};
+
+__device__ __forceinline__ void box_shfl_union(float4& lo, float4& hi, int o) {
+    lo.x = fminf(lo.x, __shfl_xor_sync(kFull, lo.x, o)); lo.y = fminf(lo.y, __shfl_xor_sync(kFull, lo.y, o));
+    lo.z = fminf(lo.z, __shfl_xor_sync(kFull, lo.z, o)); hi.x = fmaxf(hi.x, __shfl_xor_sync(kFull, hi.x, o));
+    hi.y = fmaxf(hi.y, __shfl_xor_sync(kFull, hi.y, o)); hi.z = fmaxf(hi.z, __shfl_xor_sync(kFull, hi.z, o));
+}
+
+__device__ __forceinline__ CullGroup cull_group_load(const float4* __restrict__ boxes, int64_t group, int64_t ntiles,
+                                                     int64_t n, int lane) {
+    const float inf = __uint_as_float(0x7f800000u);
+    CullGroup g;
+    float4 tlo[2], thi[2];
+#pragma unroll
+    for (int s = 0; s < 2; ++s) {
+        const int64_t box = group * (8 * kTileBoxes) + s * 32 + lane;
+        g.lo[s] = make_float4(inf, inf, inf, 0.f);
+        g.hi[s] = make_float4(-inf, -inf, -inf, 0.f);
+        if (box < ntiles * kTileBoxes) {
+            g.lo[s] = boxes[box * 2];
+            g.hi[s] = boxes[box * 2 + 1];
+        }
+        tlo[s] = g.lo[s];
+        thi[s] = g.hi[s];
+#pragma unroll
+        for (int o = 1; o < 8; o <<= 1) box_shfl_union(tlo[s], thi[s], o);  // lanes 8g..8g+7: tile g (s = 0), 4 + g (s = 1)
+    }
+    const int t = lane & 7, src = (t & 3) << 3;  // lane l takes tile l & 7 from lane 8 (t mod 4), slot t / 4
+    float4 a_lo, a_hi, b_lo, b_hi;
+    a_lo.x = __shfl_sync(kFull, tlo[0].x, src); a_lo.y = __shfl_sync(kFull, tlo[0].y, src); a_lo.z = __shfl_sync(kFull, tlo[0].z, src);
+    a_hi.x = __shfl_sync(kFull, thi[0].x, src); a_hi.y = __shfl_sync(kFull, thi[0].y, src); a_hi.z = __shfl_sync(kFull, thi[0].z, src);
+    b_lo.x = __shfl_sync(kFull, tlo[1].x, src); b_lo.y = __shfl_sync(kFull, tlo[1].y, src); b_lo.z = __shfl_sync(kFull, tlo[1].z, src);
+    b_hi.x = __shfl_sync(kFull, thi[1].x, src); b_hi.y = __shfl_sync(kFull, thi[1].y, src); b_hi.z = __shfl_sync(kFull, thi[1].z, src);
+    g.tlo = t < 4 ? a_lo : b_lo;
+    g.thi = t < 4 ? a_hi : b_hi;
+    g.tlo.w = g.thi.w = 0.f;
+    g.glo = g.tlo;
+    g.ghi = g.thi;
+#pragma unroll
+    for (int o = 1; o < 8; o <<= 1) box_shfl_union(g.glo, g.ghi, o);  // the 8 tiles
+    const int64_t tile = group * 8 + t;
+    g.tile_ok = tile < ntiles;
+    const int64_t rest = n - tile * (kTileBoxes * kBoxPts);
+    g.tile_in = rest <= 0 ? 0 : (rest >= kTileBoxes * kBoxPts ? kTileBoxes : (int)((rest + kBoxPts - 1) / kBoxPts));
+    return g;
+}
 
 template <bool HAS_PRIOR>
-__global__ void __launch_bounds__(256)
-cov_cull_kernel(const float4* __restrict__ boxes, int boxes_per_tile, int64_t ntiles, const float4* __restrict__ table,
+__global__ void __launch_bounds__(256, 5)
+cov_cull_kernel(const float4* __restrict__ boxes, int64_t n, int64_t ntiles, const float4* __restrict__ table,
                 int W, const unsigned* __restrict__ enc, float inv_kd, unsigned* __restrict__ amask_g, int mask_stride,
                 int* __restrict__ worklist, int* __restrict__ ctrl, unsigned long long* __restrict__ desc,
                 float* __restrict__ fill_dst, int64_t fill_n, const float* __restrict__ fill_prior) {
     extern __shared__ float4 v3s[];
-    __shared__ unsigned char listed_s[kCullMaxIter][8];  // per own chunk and warp: which of the warp's 8 tiles are listed
+    __shared__ unsigned long long listed_s[kCullMaxIter][8];  // per own chunk and warp: which of its 64 boxes are listed
     __shared__ int chunk_base[kCullMaxIter];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     for (int w = tid; w < W; w += blockDim.x) {
@@ -412,71 +476,68 @@ cov_cull_kernel(const float4* __restrict__ boxes, int boxes_per_tile, int64_t nt
         }
     }
     __syncthreads();
-    const float inf = __uint_as_float(0x7f800000u);
-    const int nwords = (W + 31) >> 5;
     const int64_t nchunks = (ntiles + kChunkTiles - 1) / kChunkTiles;
-    const int sub = lane >> 3, tl = lane & 7;  // box loads: lane = (pass-local box slot, tile of the group)
-    unsigned long long npairs = 0;
+    const int nwords = (W + 31) >> 5;
+    unsigned pairs_all = 0, pairs_in = 0, n_empty = 0;  // per lane: at most kCullMaxIter * 8 * 2048 pairs
     int it = 0;
     for (int64_t chunk = blockIdx.x; chunk < nchunks; chunk += gridDim.x, ++it) {
-        // lane -> tile tl of this warp's group; the 4 lanes with the same tl share the tile's boxes_per_tile boxes (<= 16)
-        const int64_t tile_l = (chunk * 8 + warp) * 8 + tl;
-        float4 lo = make_float4(inf, inf, inf, 0.f), hi = make_float4(-inf, -inf, -inf, 0.f);
-        if (tile_l < ntiles) {
-            for (int b = sub; b < boxes_per_tile; b += 4) {
-                const float4 l2 = boxes[(tile_l * boxes_per_tile + b) * 2], h2 = boxes[(tile_l * boxes_per_tile + b) * 2 + 1];
-                box_union(lo, hi, l2, h2);
-            }
-        }
-#pragma unroll
-        for (int o = 8; o < 32; o <<= 1) {  // join the 4 lanes of a tile: afterwards every lane holds ITS tile's box
-            lo.x = fminf(lo.x, __shfl_xor_sync(kFull, lo.x, o)); lo.y = fminf(lo.y, __shfl_xor_sync(kFull, lo.y, o));
-            lo.z = fminf(lo.z, __shfl_xor_sync(kFull, lo.z, o)); hi.x = fmaxf(hi.x, __shfl_xor_sync(kFull, hi.x, o));
-            hi.y = fmaxf(hi.y, __shfl_xor_sync(kFull, hi.y, o)); hi.z = fmaxf(hi.z, __shfl_xor_sync(kFull, hi.z, o));
-        }
-        float4 glo = lo, ghi = hi;  // the group's box: join the 8 tiles
-#pragma unroll
-        for (int o = 1; o < 8; o <<= 1) {
-            glo.x = fminf(glo.x, __shfl_xor_sync(kFull, glo.x, o)); glo.y = fminf(glo.y, __shfl_xor_sync(kFull, glo.y, o));
-            glo.z = fminf(glo.z, __shfl_xor_sync(kFull, glo.z, o)); ghi.x = fmaxf(ghi.x, __shfl_xor_sync(kFull, ghi.x, o));
-            ghi.y = fmaxf(ghi.y, __shfl_xor_sync(kFull, ghi.y, o)); ghi.z = fmaxf(ghi.z, __shfl_xor_sync(kFull, ghi.z, o));
-        }
-        unsigned any = 0u;  // lanes 0..7: number of poses listed for tile tl
+        const int64_t group = chunk * 8 + warp;
+        const CullGroup g = cull_group_load(boxes, group, ntiles, n, lane);
+        // the mask rows of the lane's two boxes: mrow and mrow + 32 * mask_stride
+        unsigned* mrow = amask_g + (size_t)(group * (8 * kTileBoxes) + lane) * mask_stride;
+        int first[2] = {-1, -1};  // first non-zero word of the box's mask: the box is listed, its words are stored
+        unsigned tany = 0u;       // lanes 0..7: poses listed for tile l & 7
         for (int c = 0; c < mask_stride; ++c) {
             const int w = c * 32 + lane;
             bool cand = false;
             if (c < nwords && w < W) {
                 const float4 v3 = v3s[w];
-                cand = !(box_q2lb(glo, ghi, v3) > v3.w);  // NaN cap: evaluate
+                cand = !(box_q2lb(g.glo, g.ghi, v3) > v3.w);  // NaN cap: evaluate
             }
             unsigned gword = __ballot_sync(kFull, cand);
-            unsigned mine = 0u;  // lanes 0..7: word c of tile tl's mask
+            unsigned bm[2] = {0u, 0u}, tm = 0u;
             while (gword) {
                 const int b = __ffs(gword) - 1;
                 gword &= gword - 1;
                 const float4 v3 = v3s[c * 32 + b];
-                const bool hit = !(box_q2lb(lo, hi, v3) > v3.w);  // an empty box (+inf, -inf) gives +inf: never hit
-                const unsigned tb = __ballot_sync(kFull, hit) & 0xffu;  // lanes 0..7 speak for the 8 tiles
-                if ((tb >> tl) & 1u) mine |= 1u << b;
+                const bool th = g.tile_ok && !(box_q2lb(g.tlo, g.thi, v3) > v3.w);  // an empty box gives +inf
+                const unsigned tb = __ballot_sync(kFull, th);  // bit t (t < 8): tile t lists the pose
+                tm |= (unsigned)th << b;
+                if (tb == 0u) continue;
+#pragma unroll
+                for (int s = 0; s < 2; ++s) {
+                    const bool hit = ((tb >> (s * 4 + (lane >> 3))) & 1u) && !(box_q2lb(g.lo[s], g.hi[s], v3) > v3.w);
+                    bm[s] |= (unsigned)hit << b;
+                }
             }
-            if (lane < 8 && tile_l < ntiles) {
-                amask_g[tile_l * mask_stride + c] = mine;
-                any += __popc(mine);
+#pragma unroll
+            for (int s = 0; s < 2; ++s) {
+                if (first[s] < 0 && bm[s] != 0u) first[s] = c;
+                if (first[s] >= 0) mrow[s * 32 * mask_stride + c] = bm[s];
+            }
+            if (lane < 8) {
+                pairs_all += (unsigned)kTileBoxes * __popc(tm);
+                pairs_in += (unsigned)g.tile_in * __popc(tm);
+                tany |= tm;
             }
         }
-        const bool listed = lane < 8 && tile_l < ntiles && any != 0u;
-        if (listed) npairs += any;
-        const unsigned listed8 = __ballot_sync(kFull, listed);
-        if (lane == 0) listed_s[it][warp] = (unsigned char)listed8;
+#pragma unroll
+        for (int s = 0; s < 2; ++s)
+            for (int c = 0; c < first[s]; ++c) mrow[s * 32 * mask_stride + c] = 0u;  // the words before the first non-zero one
+        const unsigned tl8 = __ballot_sync(kFull, lane < 8 && tany != 0u);  // listed tiles
+#pragma unroll
+        for (int s = 0; s < 2; ++s) n_empty += ((tl8 >> (s * 4 + (lane >> 3))) & 1u) && first[s] < 0;
+        const unsigned l0 = __ballot_sync(kFull, first[0] >= 0), l1 = __ballot_sync(kFull, first[1] >= 0);
+        if (lane == 0) listed_s[it][warp] = ((unsigned long long)l1 << 32) | l0;
     }
     const int n_it = it;
     __syncthreads();
     if (warp == 0) {
-        // own chunk `k` is chunk blockIdx.x + k * gridDim.x; lane l < 8 holds warp l's listed bits
+        // own chunk `k` is chunk blockIdx.x + k * gridDim.x; listed_s[k][q] = the listed boxes of its warp q
         for (int k = lane; k < n_it; k += 32) {  // publish every own aggregate first
             int total = 0;
 #pragma unroll
-            for (int q = 0; q < 8; ++q) total += __popc((unsigned)listed_s[k][q]);
+            for (int q = 0; q < 8; ++q) total += __popcll(listed_s[k][q]);
             const int64_t chunk = blockIdx.x + (int64_t)k * gridDim.x;
             if (chunk > 0) st_release_u64(desc + chunk, kDescAgg | (unsigned long long)total);
         }
@@ -485,7 +546,7 @@ cov_cull_kernel(const float4* __restrict__ boxes, int boxes_per_tile, int64_t nt
             const int64_t chunk = blockIdx.x + (int64_t)k * gridDim.x;
             unsigned long long total = 0ull;
 #pragma unroll
-            for (int q = 0; q < 8; ++q) total += (unsigned long long)__popc((unsigned)listed_s[k][q]);
+            for (int q = 0; q < 8; ++q) total += (unsigned long long)__popcll(listed_s[k][q]);
             unsigned long long excl = 0ull;
             if (chunk > 0) {
                 int64_t look = chunk - 1;
@@ -514,50 +575,58 @@ cov_cull_kernel(const float4* __restrict__ boxes, int boxes_per_tile, int64_t nt
         }
     }
     __syncthreads();
+    // the listed boxes of each own chunk at their list positions
     for (int k = 0; k < n_it; ++k) {
+        const unsigned long long listed = listed_s[k][warp];
+        if (listed == 0ull) continue;
         const int64_t chunk = blockIdx.x + (int64_t)k * gridDim.x;
-        const int64_t tile_l = (chunk * 8 + warp) * 8 + tl;
-        const unsigned listed8 = listed_s[k][warp];
-        int before = 0;  // listed tiles of the chunk in the warps ahead of this one
-        for (int q = 0; q < warp; ++q) before += __popc((unsigned)listed_s[k][q]);
-        if (lane < 8 && ((listed8 >> lane) & 1u))
-            worklist[chunk_base[k] + before + __popc(listed8 & ((1u << lane) - 1u))] = (int)tile_l;
+        int pos = chunk_base[k];  // listed boxes of the chunk in the warps ahead of this one
+        for (int q = 0; q < warp; ++q) pos += __popcll(listed_s[k][q]);
+        const unsigned below = (1u << lane) - 1u;
+        const unsigned l0 = (unsigned)listed, l1 = (unsigned)(listed >> 32);
+        const int64_t box0 = (chunk * 8 + warp) * (8 * kTileBoxes) + lane;
+        if ((l0 >> lane) & 1u) worklist[pos + __popc(l0 & below)] = (int)box0;
+        if ((l1 >> lane) & 1u) worklist[pos + __popc(l0) + __popc(l1 & below)] = (int)(box0 + 32);
     }
-    npairs = __reduce_add_sync(kFull, (unsigned)npairs);
-    if (lane == 0 && npairs) atomicAdd(reinterpret_cast<unsigned long long*>(ctrl + 4), npairs);
+    pairs_all = __reduce_add_sync(kFull, pairs_all);
+    pairs_in = __reduce_add_sync(kFull, pairs_in);
+    n_empty = __reduce_add_sync(kFull, n_empty);
+    if (lane == 0) {
+        if (pairs_all) atomicAdd(reinterpret_cast<unsigned long long*>(ctrl + 4), (unsigned long long)pairs_all);
+        if (pairs_in) atomicAdd(reinterpret_cast<unsigned long long*>(ctrl + 6), (unsigned long long)pairs_in);
+        if (n_empty) atomicAdd(reinterpret_cast<unsigned long long*>(ctrl + 8), (unsigned long long)n_empty);
+    }
 }
 
 // ================================= pruned evaluation: the persistent-warp item loop =================================
-// The three *_tiles_kernel below run persistent WARPS over the work list.  The unit of work is one box of 128
-// consecutive points (one eighth of a listed tile), taken by ONE WARP from a global ticket counter: warps never wait for
-// each other (no block barrier, no static assignment), so neither the uneven cost of neighbouring boxes nor a heavy tile
-// at the end of the list leaves lanes idle.  A warp keeps two private stages in shared memory; its lane 0 draws the next
-// ticket and issues the TMA bulk copies for it (points, the box, the tile's pose mask, and in pass B the slice of the
-// permutation — one mbarrier per stage) before the warp starts on the current item.  The pose table stays in global
-// memory (a box touches ~5 rows: L1 hits).
+// The *_tiles_kernel below run persistent WARPS over the work list.  The unit of work is one listed box of 128
+// consecutive points, taken by ONE WARP from a global ticket counter: warps never wait for each other (no block barrier,
+// no static assignment), so neither the uneven cost of neighbouring boxes nor a heavy box at the end of the list leaves
+// lanes idle.  A warp keeps two private stages in shared memory; its lane 0 draws the next ticket and issues the TMA bulk
+// copies for it (points, the box's pose mask, and in pass B the slice of the permutation — one mbarrier per stage)
+// before the warp starts on the current item.  Every pose of the mask is evaluated: the cull has already tested it
+// against the box.  The pose table stays in global memory (a box touches ~5 rows: L1 hits).
 constexpr int kItemPts = 128;                 // points per work item = one warp's registers = one precomputed box
-constexpr int kItemsPerTile = 8;              // a listed tile (1024 points) is eight items
 constexpr int kItemPpt = kItemPts / 32;
+static_assert(kItemPts == kBoxPts, "a work item is one box");
 
 // One work item as the loop body sees it: points [j0, j0 + 128) of the cloud.
 struct Item {
     int64_t j0;
     bool whole;             // j0 + 128 <= n: the points (and the permutation slice) were staged
     const float* pts;       // the staged points, xyz interleaved
-    const float4* box;      // the item's bounding box (lo, hi); the sweep copies it to registers once per item, the
-                            // two passes read it from the stage at each pose: the faster choice for each kernel
-    const unsigned* mask;   // the tile's pose mask
+    const unsigned* mask;   // the box's pose mask: the poses to evaluate
     const int32_t* perm;    // the staged slice of the permutation (WITH_PERM, whole, permutation given)
 };
 
 // Draws items until the work list is exhausted; `pre_wait(it)` runs after the next item was issued and before the wait
 // for the current one, `body(item)` once the current one has arrived.  Every lane of the warp calls it.
 template <bool WITH_PERM, typename PreWait, typename Body>
-__device__ __forceinline__ void for_each_item(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ boxes,
+__device__ __forceinline__ void for_each_item(const float* __restrict__ xyz, int64_t n,
                                               const unsigned* __restrict__ amask_g, int mask_stride,
                                               const int32_t* __restrict__ perm, const int* __restrict__ worklist,
                                               int n_items, int* ticket, PreWait pre_wait, Body body) {
-    constexpr int kStageWords = kItemPts * 3 + 8 + kMaskWords + (WITH_PERM ? kItemPts : 0);  // points|box|mask|perm
+    constexpr int kStageWords = kItemPts * 3 + kMaskWords + (WITH_PERM ? kItemPts : 0);  // points|mask|perm
     __shared__ __align__(128) float stages[kWarps][2][kStageWords];
     __shared__ __align__(8) unsigned long long mbar[kWarps][2];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -568,19 +637,18 @@ __device__ __forceinline__ void for_each_item(const float* __restrict__ xyz, int
         mbar_fence_init();
     }
     __syncwarp();
-    // lane 0: stage item `it` (tile = worklist[it / 8], box k = it % 8); a ragged item's points are loaded by hand
+    // lane 0: stage item `it` (box worklist[it] and its mask row); a ragged item's points are loaded by hand
     auto issue = [&](int it, int b) {
         if (it >= n_items) return;
-        const int64_t tile = worklist[it >> 3];
-        const int64_t j0 = tile * (kItemsPerTile * kItemPts) + (int64_t)(it & 7) * kItemPts;
+        const int64_t box = worklist[it];
+        const int64_t j0 = box * kItemPts;
         float* st = stages[warp][b];
         const bool whole = j0 + kItemPts <= n;
         const bool with_perm = WITH_PERM && whole && perm != nullptr;
-        mbar_expect_tx(&bar[b], (whole ? kItemPts * 12u : 0u) + 32u + (unsigned)mask_stride * 4u + (with_perm ? kItemPts * 4u : 0u));
+        mbar_expect_tx(&bar[b], (whole ? kItemPts * 12u : 0u) + (unsigned)mask_stride * 4u + (with_perm ? kItemPts * 4u : 0u));
         if (whole) tma_copy(st, xyz + j0 * 3, kItemPts * 12u, &bar[b]);
-        tma_copy(st + kItemPts * 3, boxes + (j0 / kBoxPts) * 2, 32u, &bar[b]);
-        tma_copy(st + kItemPts * 3 + 8, amask_g + tile * mask_stride, (unsigned)mask_stride * 4u, &bar[b]);
-        if (with_perm) tma_copy(st + kItemPts * 3 + 8 + kMaskWords, perm + j0, kItemPts * 4u, &bar[b]);
+        tma_copy(st + kItemPts * 3, amask_g + box * mask_stride, (unsigned)mask_stride * 4u, &bar[b]);
+        if (with_perm) tma_copy(st + kItemPts * 3 + kMaskWords, perm + j0, kItemPts * 4u, &bar[b]);
     };
     unsigned uses0 = 0, uses1 = 0;
     int cur = 0;
@@ -602,12 +670,11 @@ __device__ __forceinline__ void for_each_item(const float* __restrict__ xyz, int
         else mbar_wait(&bar[1], uses1++ & 1u);
         const float* st = stages[warp][buf];
         Item item;
-        item.j0 = (int64_t)worklist[cur >> 3] * (kItemsPerTile * kItemPts) + (int64_t)(cur & 7) * kItemPts;
+        item.j0 = (int64_t)worklist[cur] * kItemPts;
         item.whole = item.j0 + kItemPts <= n;
         item.pts = st;
-        item.box = reinterpret_cast<const float4*>(st + kItemPts * 3);
-        item.mask = reinterpret_cast<const unsigned*>(st + kItemPts * 3 + 8);
-        item.perm = reinterpret_cast<const int32_t*>(st + kItemPts * 3 + 8 + kMaskWords);
+        item.mask = reinterpret_cast<const unsigned*>(st + kItemPts * 3);
+        item.perm = reinterpret_cast<const int32_t*>(st + kItemPts * 3 + kMaskWords);
         body(item);
         __syncwarp();  // every lane is done with this stage before lane 0 refills it
         cur = nxt;
@@ -652,13 +719,14 @@ __device__ __forceinline__ void load_item_points(const Item& item, const float* 
 }
 
 // =============================================== pass A, pruned ===============================================
-// A listed pose is evaluated when the cap ball (from the seed's extrema; any later value is tighter and valid) meets
-// the warp's box and one of its points.  Extrema meet per block in shared memory, then in the zero-initialised encoded
-// arrays; the last block decodes them into the caller's floats.
+// A pose of the box's mask (the cull tested the cap ball from the seed's extrema against the box) is evaluated when the
+// cap ball meets one of the box's points; the cap is re-read from the extrema at start-up (any later value is tighter
+// and valid).  Extrema meet per block in shared memory, then in the zero-initialised encoded arrays; the last block
+// decodes them into the caller's floats.
 template <bool HAS_PRIOR>
 __global__ void __launch_bounds__(COV_THREADS, 3)
 cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, CovConst C,
-                             unsigned* __restrict__ enc, float* __restrict__ minmax_out, const float4* __restrict__ boxes,
+                             unsigned* __restrict__ enc, float* __restrict__ minmax_out,
                              const unsigned* __restrict__ amask_g, int mask_stride, const int* __restrict__ worklist,
                              int* __restrict__ ctrl, int64_t ntiles, unsigned long long* __restrict__ stats,
                              float* __restrict__ fill_dst, int64_t fill_n, const float* __restrict__ fill_prior) {
@@ -675,7 +743,7 @@ cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
         sqcap[w] = minmax_qcap(~enc[w], enc[W + w], inv_kd);  // from the seed (any later value is tighter and valid)
     }
     __syncthreads();
-    const int n_items = ctrl[0] * kItemsPerTile;
+    const int n_items = ctrl[0];
     const int nwords = (W + 31) >> 5;
     // Pre-fill of pass B's rewards with 1/2 under this kernel's idle memory bandwidth (cov_traj_opts.prefill_dev): the
     // warp that takes item i also writes slice i of the buffer (fire-and-forget streaming stores), in 16-byte units.
@@ -701,16 +769,16 @@ cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
         const int64_t per = (fill_q + nw - 1) / nw;
         fill_slice(gw * per, (gw + 1) * per);
     }
-    unsigned n_box = 0, n_pre = 0, n_full = 0;
+    unsigned n_pre = 0, n_full = 0;
     auto fill_item = [&](int it) {
         if (fill_dst) fill_slice((int64_t)it * fill_per_item, (int64_t)(it + 1) * fill_per_item);
     };
-    for_each_item<false>(xyz, n, boxes, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 3, fill_item,
+    for_each_item<false>(xyz, n, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 3, fill_item,
                          [&](const Item& item) {
         float px[PPT], py[PPT], pz[PPT];
         bool valid[PPT];
         load_item_points<true>(item, xyz, n, lane, px, py, pz, valid);
-        if (item.j0 >= n) return;  // a listed tile's items past the end of the cloud
+        if (item.j0 >= n) return;  // a listed box past the end of the cloud (an empty box under an infinite cap)
         for (int c = 0; c < nwords; ++c) {
             unsigned word = item.mask[c];
             while (word) {
@@ -719,8 +787,6 @@ cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
                 const float4* row = table + (size_t)w * COV_ROW_F4;
                 const float4 v3 = __ldg(row + 3);
                 const float cap = sqcap[w];
-                ++n_box;
-                if (box_q2lb(item.box[0], item.box[1], v3) > cap) continue;
                 ++n_pre;
                 float qmin = cov_q2(px[0], py[0], pz[0], v3);
 #pragma unroll
@@ -754,10 +820,12 @@ cov_traj_minmax_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
         }
     }
     if (stats && lane == 0) {
-        if (tid == 0 && blockIdx.x == 0) atomicAdd(stats + 2, (unsigned long long)ntiles * kWarps * W);
+        if (tid == 0 && blockIdx.x == 0) {
+            atomicAdd(stats + 2, (unsigned long long)ntiles * kWarps * W);
+            atomicAdd(stats + 7, *reinterpret_cast<const unsigned long long*>(ctrl + 6));  // counted by the cull
+        }
         atomicAdd(stats + 3, (unsigned long long)n_full);
         atomicAdd(stats + 5, (unsigned long long)n_pre);
-        atomicAdd(stats + 7, (unsigned long long)n_box);
     }
     // the last block to arrive decodes the extrema into the caller's floats (minima, then maxima)
     __shared__ int s_last;
@@ -1137,8 +1205,8 @@ cov_traj_fused_kernel(const float* __restrict__ xyz, int64_t n, const float* __r
 }
 
 // ---- pruned: persistent warps over the work list (for_each_item), per 128-point item ----
-//   forward   walk the tile's pose mask; a listed pose is evaluated when its qthr-ball meets the warp's box; gated lanes
-//             add their log-odds; the warp notes (one bit per pose) whether it had a gated pair.  Then r_j,
+//   forward   walk the box's pose mask (the poses whose qthr-ball meets the box) and evaluate each; gated lanes add their
+//             log-odds; the warp notes (one bit per pose) whether it had a gated pair.  Then r_j,
 //             G_j = r_j (1 - r_j) per point; rewards stored.
 //   backward  the warp walks its noted poses: m again for its points (bit-identical), the gate, dm/dx, the 8 weighted
 //             sums in registers; a fixed 9-shuffle tree reduces them over the warp and one lane per component adds the
@@ -1160,7 +1228,7 @@ __global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
 cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, CovConst C,
                             const float* __restrict__ upstream, const int32_t* __restrict__ out_index,
                             float* __restrict__ rewards, double* __restrict__ acc,
-                            const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g, int mask_stride,
+                            const unsigned* __restrict__ amask_g, int mask_stride,
                             const int* __restrict__ worklist, int* __restrict__ ctrl, int64_t ntiles,
                             unsigned long long* __restrict__ stats, const float* __restrict__ prior) {
     static_assert(HAS_UP || !WSUM, "the weight rides on the upstream gather");
@@ -1168,12 +1236,12 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
     __shared__ unsigned wgate[kWarps][kMaskWords];   // per warp: poses with a gated pair among its points (this item)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const bool check_amin = ctrl[1] != 0;  // some pose has min_j m > 0
-    const int n_items = ctrl[0] * kItemsPerTile;
+    const int n_items = ctrl[0];
     const int nwords = (W + 31) >> 5;
     unsigned* wg = wgate[warp];  // lane 0 rewrites it for the next item only after the closing __syncwarp of this one
     double sum_r = 0.0;
-    unsigned n_box = 0, n_full = 0, n_bwd = 0;
-    for_each_item<true>(xyz, n, boxes, amask_g, mask_stride, out_index, worklist, n_items, ctrl + 3, [](int) {},
+    unsigned n_full = 0, n_bwd = 0;
+    for_each_item<true>(xyz, n, amask_g, mask_stride, out_index, worklist, n_items, ctrl + 3, [](int) {},
                         [&](const Item& item) {
         // ------------------------------ forward ------------------------------
         float px[PPT], py[PPT], pz[PPT], L[PPT];
@@ -1191,10 +1259,8 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
                 word &= word - 1;
                 const float4* row = table + (size_t)w * COV_ROW_F4;
                 const float4 v3 = __ldg(row + 3);
-                ++n_box;
-                // the warp's own box against the pose's qthr-ball; no per-point pre-filter here: it rejected only 11 % of
-                // what the box test let through and cost a fifth of the evaluation it saved
-                if (box_q2lb(item.box[0], item.box[1], v3) > v3.w) continue;
+                // no per-point pre-filter here: it rejected only 11 % of what the cull's box test let through and cost a fifth
+                // of the evaluation it saved
                 ++n_full;
                 double* acc_row = acc + (size_t)w * COV_ACC_STRIDE;
                 const bool g = check_amin ? tiles_pose_iter<PPT, true>(row, v3, px, py, pz, L, C, acc_row)
@@ -1275,16 +1341,18 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
         if (lane == 0 && ws != 0.0) atomicAdd(acc + (size_t)W * COV_ACC_STRIDE, ws);
     }
     if (stats && lane == 0) {
-        if (threadIdx.x == 0 && blockIdx.x == 0) atomicAdd(stats + 0, (unsigned long long)ntiles * kWarps * W);
+        if (threadIdx.x == 0 && blockIdx.x == 0) {
+            atomicAdd(stats + 0, (unsigned long long)ntiles * kWarps * W);
+            atomicAdd(stats + 6, *reinterpret_cast<const unsigned long long*>(ctrl + 4));  // counted by the cull
+        }
         atomicAdd(stats + 1, (unsigned long long)n_full);
         atomicAdd(stats + 4, (unsigned long long)n_bwd);
-        atomicAdd(stats + 6, (unsigned long long)n_box);
     }
 }
 
 // ---- candidate sweep, pruned (BASELINE config 5): forward only, per-trajectory sum_j r_j ----
 // Persistent warps as in the two passes above (for_each_item).  Poses are trajectory-major (pose = traj * per_traj + i),
-// so walking a tile's pose mask in ascending order visits the trajectories one after the other: a warp keeps the log-odds
+// so walking a box's pose mask in ascending order visits the trajectories one after the other: a warp keeps the log-odds
 // sums of its points for the current trajectory, and when the trajectory changes it adds sum_j (sigmoid(L_j) - 1/2) to
 // that trajectory's total (fp64 shared atomic; the block adds its totals to the output at the end).  Trajectories no
 // pose of which is listed for an item contribute exactly 1/2 per point: 0.5 * n is added once.
@@ -1295,8 +1363,7 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
 template <bool HAS_PRIOR, bool HAS_W = false>
 __global__ void __launch_bounds__(COV_THREADS, 3)
 cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, int per_traj,
-                       int n_traj, CovConst C, const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g,
-                       int mask_stride, const int* __restrict__ worklist, int* __restrict__ ctrl,
+                       int n_traj, CovConst C, const unsigned* __restrict__ amask_g, int mask_stride, const int* __restrict__ worklist, int* __restrict__ ctrl,
                        double* __restrict__ sum_out, const float* __restrict__ prior, const double* __restrict__ prior_sum,
                        const float* __restrict__ weight) {
     constexpr int PPT = kItemPpt;
@@ -1305,14 +1372,13 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
     const int tid = threadIdx.x, lane = tid & 31;
     for (int t = tid; t < n_traj; t += COV_THREADS) ssum[t] = 0.0;
     __syncthreads();
-    const int n_items = ctrl[0] * kItemsPerTile;
+    const int n_items = ctrl[0];
     const int nwords = (W + 31) >> 5;
-    for_each_item<false>(xyz, n, boxes, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 3, [](int) {},
+    for_each_item<false>(xyz, n, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 3, [](int) {},
                          [&](const Item& item) {
         float px[PPT], py[PPT], pz[PPT], L[PPT];
         bool valid[PPT];
         load_item_points<false>(item, xyz, n, lane, px, py, pz, valid);
-        const float4 lo = item.box[0], hi = item.box[1];
         int cur = -1;      // trajectory whose log-odds sums are in L
         bool touched = false;
         auto flush = [&]() {
@@ -1351,7 +1417,6 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
                 word &= word - 1;
                 const float4* row = table + (size_t)w * COV_ROW_F4;
                 const float4 v3 = __ldg(row + 3);
-                if (box_q2lb(lo, hi, v3) > v3.w) continue;
                 const int t = w / per_traj;
                 if (t != cur) {
                     flush();
@@ -1380,8 +1445,8 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
 // expressions, adds sum_j (r_j - 1/2) to the trajectory's reward sum and runs pass B's backward (tiles_pose_backward) over
 // the noted poses, then clears the notes.  Pose w of trajectory t owns row (w - t P) of block t of the accumulators,
 // `acc + t * COV_SWEEP_ACC_BLOCK(P)`: the layout cov_traj_fused writes for that trajectory alone (rows, then sum_j r_j).
-// The forward of a trajectory visits the same poses in the same order as pass B with W = P on the same item (same cull,
-// same box test), so its L, r_j and G_j — and the re-evaluated m of the backward — are bit-identical to pass B's.
+// The forward of a trajectory visits the same poses in the same order as pass B with W = P on the same item (same cull),
+// so its L, r_j and G_j — and the re-evaluated m of the backward — are bit-identical to pass B's.
 // HAS_PRIOR: at a flush r_j = sigmoid(prior_j + L_j) and r_j - sigmoid(prior_j) is added, with the item's 128 priors (in
 // the cloud's order) read there; the blocks start at sum_j sigmoid(prior_j) (cov_sweep_acc_init_kernel).
 // HAS_W: the item's 128 weights w_j (cloud's order) are read at a flush too; w_j (r_j - r0_j) is added and G_j is
@@ -1389,22 +1454,21 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
 template <bool HAS_PRIOR, bool HAS_W = false>
 __global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
 cov_sweep_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, int per_traj,
-                             CovConst C, const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g,
-                             int mask_stride, const int* __restrict__ worklist, int* __restrict__ ctrl, int64_t ntiles,
+                             CovConst C, const unsigned* __restrict__ amask_g, int mask_stride, const int* __restrict__ worklist, int* __restrict__ ctrl, int64_t ntiles,
                              double* __restrict__ acc, unsigned long long* __restrict__ stats,
                              const float* __restrict__ prior, const float* __restrict__ weight) {
     constexpr int PPT = kItemPpt;
     __shared__ unsigned wgate[kWarps][kMaskWords];   // per warp: poses of the current trajectory with a gated pair
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const bool check_amin = ctrl[1] != 0;  // some pose has min_j m > 0
-    const int n_items = ctrl[0] * kItemsPerTile;
+    const int n_items = ctrl[0];
     const int nwords = (W + 31) >> 5;
     const size_t block = COV_SWEEP_ACC_BLOCK(per_traj);
     unsigned* wg = wgate[warp];
     for (int c = lane; c < kMaskWords; c += 32) wg[c] = 0u;  // afterwards every flush clears the words it walked
     __syncwarp();
-    unsigned n_box = 0, n_full = 0, n_bwd = 0;
-    for_each_item<false>(xyz, n, boxes, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 3, [](int) {},
+    unsigned n_full = 0, n_bwd = 0;
+    for_each_item<false>(xyz, n, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 3, [](int) {},
                          [&](const Item& item) {
         float px[PPT], py[PPT], pz[PPT], L[PPT];
         bool valid[PPT];
@@ -1473,8 +1537,6 @@ cov_sweep_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
                 word &= word - 1;
                 const float4* row = table + (size_t)w * COV_ROW_F4;
                 const float4 v3 = __ldg(row + 3);
-                ++n_box;
-                if (box_q2lb(item.box[0], item.box[1], v3) > v3.w) continue;
                 ++n_full;
                 const int t = w / per_traj;
                 if (t != cur) {
@@ -1496,10 +1558,12 @@ cov_sweep_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const flo
         flush();
     });
     if (stats && lane == 0) {
-        if (threadIdx.x == 0 && blockIdx.x == 0) atomicAdd(stats + 0, (unsigned long long)ntiles * kWarps * W);
+        if (threadIdx.x == 0 && blockIdx.x == 0) {
+            atomicAdd(stats + 0, (unsigned long long)ntiles * kWarps * W);
+            atomicAdd(stats + 6, *reinterpret_cast<const unsigned long long*>(ctrl + 4));  // counted by the cull
+        }
         atomicAdd(stats + 1, (unsigned long long)n_full);
         atomicAdd(stats + 4, (unsigned long long)n_bwd);
-        atomicAdd(stats + 6, (unsigned long long)n_box);
     }
 }
 
@@ -1647,19 +1711,19 @@ __global__ void __launch_bounds__(256) cov_prior_sum_kernel(const float* __restr
     }
 }
 
-// Fused log-odds output, pruned: pass B's forward (same work list, same box test, same pose order, hence the same L_j)
+// Fused log-odds output, pruned: pass B's forward (same work list and masks, same pose order, hence the same L_j)
 // without the backward; out[jo] = out[jo] + L_j for the points with L_j != 0 (the caller pre-filled `out` with the prior,
 // indexed like the rewards), the x that pass B's sigmoid takes.
 __global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
 cov_traj_logodds_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, CovConst C,
                               const int32_t* __restrict__ out_index, float* __restrict__ out,
-                              const float4* __restrict__ boxes, const unsigned* __restrict__ amask_g, int mask_stride,
+                              const unsigned* __restrict__ amask_g, int mask_stride,
                               const int* __restrict__ worklist, int* __restrict__ ctrl) {
     constexpr int PPT = kItemPpt;
     const int lane = threadIdx.x & 31;
-    const int n_items = ctrl[0] * kItemsPerTile;
+    const int n_items = ctrl[0];
     const int nwords = (W + 31) >> 5;
-    for_each_item<true>(xyz, n, boxes, amask_g, mask_stride, out_index, worklist, n_items, ctrl + 3, [](int) {},
+    for_each_item<true>(xyz, n, amask_g, mask_stride, out_index, worklist, n_items, ctrl + 3, [](int) {},
                         [&](const Item& item) {
         float px[PPT], py[PPT], pz[PPT], L[PPT];
         bool valid[PPT];
@@ -1672,9 +1736,7 @@ cov_traj_logodds_tiles_kernel(const float* __restrict__ xyz, int64_t n, const fl
                 const int w = c * 32 + __ffs(word) - 1;
                 word &= word - 1;
                 const float4* row = table + (size_t)w * COV_ROW_F4;
-                const float4 v3 = __ldg(row + 3);
-                if (box_q2lb(item.box[0], item.box[1], v3) > v3.w) continue;
-                tiles_pose_iter<PPT, false>(row, v3, px, py, pz, L, C, nullptr);
+                tiles_pose_iter<PPT, false>(row, __ldg(row + 3), px, py, pz, L, C, nullptr);
             }
         }
 #pragma unroll
@@ -1821,8 +1883,13 @@ int pick_ppt(int64_t n, int W, bool fused) {
 size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 int64_t boxes_padded(int64_t n) { return ((n + 2047) / 2048) * (2048 / kBoxPts); }
 
+// Work items the cull can list at most: every box of every 1024-point tile.
+int64_t list_capacity(int64_t n) { return ((n + 1023) / 1024) * kTileBoxes; }
+
 // Workspace of both passes (every region 256-byte aligned):
-//   [control: ctrl ints | encoded extrema 2W | look-back descriptors][pose table][work list][tile masks][boxes]
+//   [control: ctrl ints | encoded extrema 2W | look-back descriptors][pose table][work list][box masks][boxes]
+// The work list and the masks are sized for the worst case, every box listed: list_capacity entries, and as many mask
+// rows of mask_stride_words(W), indexed by box.  The cull writes the rows of the listed boxes only.
 struct TrajWorkspace {
     int* ctrl;
     unsigned* enc;
@@ -1835,8 +1902,9 @@ struct TrajWorkspace {
     size_t bytes;
 };
 TrajWorkspace carve_workspace(void* ws, int64_t n, int W) {
-    const int64_t nt = (n + 255) / 256;  // tiles at the smallest tile size
+    const int64_t nt = (n + 1023) / 1024;  // tiles of the pruned passes
     const int64_t nchunks = (nt + kChunkTiles - 1) / kChunkTiles;
+    const int64_t cap = list_capacity(n);
     char* p = reinterpret_cast<char*>(ws);
     size_t off = 0;
     TrajWorkspace t;
@@ -1849,8 +1917,8 @@ TrajWorkspace carve_workspace(void* ws, int64_t n, int W) {
     t.enc = reinterpret_cast<unsigned*>(c + enc_off);
     t.desc = reinterpret_cast<unsigned long long*>(c + desc_off);
     t.table = reinterpret_cast<float4*>(take((size_t)W * COV_ROW_F4 * sizeof(float4)));
-    t.worklist = reinterpret_cast<int*>(take((size_t)nt * sizeof(int)));
-    t.amask = reinterpret_cast<unsigned*>(take((size_t)nt * mask_stride_words(W) * sizeof(unsigned)));
+    t.worklist = reinterpret_cast<int*>(take((size_t)cap * sizeof(int)));
+    t.amask = reinterpret_cast<unsigned*>(take((size_t)cap * mask_stride_words(W) * sizeof(unsigned)));
     t.boxes = reinterpret_cast<float4*>(take((size_t)boxes_padded(n) * 2 * sizeof(float4)));
     t.bytes = off;
     return t;
@@ -1862,7 +1930,7 @@ int check_traj_args(const char* who, const float* xyz, int64_t n, const float* p
         cov_set_error("%s: null pointer, empty cloud or no poses (n=%lld, W=%d)", who, (long long)n, W);
         return COV_ERR_ARG;
     }
-    // the dense kernels keep the pose table in shared memory; the pruned ones only a bit per pose in the tile masks
+    // the dense kernels keep the pose table in shared memory; the pruned ones only a bit per pose in the box masks
     const int max_w = pruned ? cov_traj_max_poses_pruned() : cov_traj_max_poses();
     if (W > max_w) {
         cov_set_error("%s: %d poses exceed what one call takes on this path (max %d)", who, W, max_w);
@@ -1900,9 +1968,11 @@ const float4* boxes_for_call(const float* xyz, int64_t n, const float* boxes_dev
     return t.boxes;
 }
 
-// cull + work list in one launch; every block must be resident (the blocks wait on one another's descriptors)
-int launch_cull(const float4* boxes, int ppt, int64_t ntiles, const TrajWorkspace& t, int W, const unsigned* enc,
-                float inv_kd, float* fill_dst, int64_t fill_n, cudaStream_t s, const float* fill_prior = nullptr) {
+// cull + work list in one launch (1024-point tiles of n points); every block must be resident (the blocks wait on one
+// another's descriptors)
+int launch_cull(const float4* boxes, int64_t n, const TrajWorkspace& t, int W, const unsigned* enc, float inv_kd,
+                float* fill_dst, int64_t fill_n, cudaStream_t s, const float* fill_prior = nullptr) {
+    const int64_t ntiles = (n + tile_points(4) - 1) / tile_points(4);
     const size_t smem = (size_t)W * sizeof(float4);
     const auto cull = fill_prior ? cov_cull_kernel<true> : cov_cull_kernel<false>;
     const int64_t nchunks = (ntiles + kChunkTiles - 1) / kChunkTiles;
@@ -1916,8 +1986,8 @@ int launch_cull(const float4* boxes, int ppt, int64_t ntiles, const TrajWorkspac
         return COV_ERR_UNSUPPORTED;
     }
     const int grid = (int)g;
-    cull<<<grid, 256, smem, s>>>(boxes, tile_boxes(ppt), ntiles, t.table, W, enc, inv_kd, t.amask, mask_stride_words(W),
-                                 t.worklist, t.ctrl, t.desc, fill_dst, fill_n, fill_prior);
+    cull<<<grid, 256, smem, s>>>(boxes, n, ntiles, t.table, W, enc, inv_kd, t.amask, mask_stride_words(W), t.worklist,
+                                 t.ctrl, t.desc, fill_dst, fill_n, fill_prior);
     return COV_OK;
 }
 
@@ -2028,7 +2098,7 @@ static int traj_minmax_impl(const float* xyz, int64_t n, const float* poses, con
 #undef LAUNCH_DENSE
         return cov_check_launch("cov_traj_minmax");
     }
-    // pruned: pose table + seed on a strided sample, cull + work list, evaluation of the listed tiles: 3 launches
+    // pruned: pose table + seed on a strided sample, cull + work list, evaluation of the listed boxes: 3 launches
     const TrajWorkspace t = carve_workspace(ws, n, W);
     const float4* boxes = boxes_for_call(xyz, n, boxes_dev, t, s);
     constexpr int ppt_t = 4;  // tiles of 1024 points, eight 128-point items each (as pass B)
@@ -2040,12 +2110,12 @@ static int traj_minmax_impl(const float* xyz, int64_t n, const float* poses, con
         const dim3 sgrid((unsigned)((nsamples + COV_THREADS - 1) / COV_THREADS), (unsigned)((W + 31) / 32));
         cov_traj_prepare_kernel<<<sgrid, COV_THREADS, 0, s>>>(xyz, nsamples, stride, poses, quats, W, K, C, t.table, t.enc);
     }
-    if ((rc = launch_cull(boxes, ppt_t, ntiles_t, t, W, t.enc, 1.f / C.kd, nullptr, 0, s)) != COV_OK) return rc;
+    if ((rc = launch_cull(boxes, n, t, W, t.enc, 1.f / C.kd, nullptr, 0, s)) != COV_OK) return rc;
     const size_t smem_t = (size_t)W * 12;
     float* prefill = opts ? opts->prefill_dev : nullptr;
     const auto tiles_kern = (prior && prefill) ? cov_traj_minmax_tiles_kernel<true> : cov_traj_minmax_tiles_kernel<false>;
     tiles_kern<<<persistent_grid(tiles_kern, smem_t, ntiles_t), COV_THREADS, smem_t, s>>>(
-        xyz, n, t.table, W, C, t.enc, minmax, boxes, t.amask, mask_stride_words(W), t.worklist, t.ctrl, ntiles_t,
+        xyz, n, t.table, W, C, t.enc, minmax, t.amask, mask_stride_words(W), t.worklist, t.ctrl, ntiles_t,
         opts ? opts->stats_dev : nullptr, prefill, n, prior);
     return cov_check_launch("cov_traj_minmax");
 }
@@ -2125,9 +2195,9 @@ static int traj_fused_impl(const float* xyz, int64_t n, const float* poses, cons
 #undef LAUNCH_F
         return cov_check_launch("cov_traj_fused");
     }
-    // pruned: table (+ zeroing), cull + work list (+ rewards pre-fill), evaluation of the listed tiles: 3 launches
-    constexpr int ppt = kItemPpt * kItemsPerTile * 32 / COV_THREADS;  // tiles of 1024 points, eight 128-point items each
-    static_assert(ppt == 4 && tile_points(ppt) == kItemsPerTile * kItemPts, "tile = 8 items");
+    // pruned: table (+ zeroing), cull + work list (+ rewards pre-fill), evaluation of the listed boxes: 3 launches
+    constexpr int ppt = 4;  // tiles of 1024 points, eight 128-point boxes each
+    static_assert(tile_boxes(ppt) == kTileBoxes, "the cull's tiles");
     const int64_t ntiles = (n + tile_points(ppt) - 1) / tile_points(ppt);
     const float4* boxes = boxes_for_call(xyz, n, boxes_dev, t, s);
     if (prior || wsum) {
@@ -2139,7 +2209,7 @@ static int traj_fused_impl(const float* xyz, int64_t n, const float* poses, cons
                                                                   nullptr);
     }
     const bool prefilled = opts && opts->rewards_prefilled;
-    if ((rc = launch_cull(boxes, ppt, ntiles, t, W, nullptr, 0.f, prefilled ? nullptr : rewards, n, s, prior)) != COV_OK)
+    if ((rc = launch_cull(boxes, n, t, W, nullptr, 0.f, prefilled ? nullptr : rewards, n, s, prior)) != COV_OK)
         return rc;
     // persistent warps: as many blocks as are resident; every warp draws 128-point items from a ticket counter
     const auto tiles_kern =
@@ -2147,7 +2217,7 @@ static int traj_fused_impl(const float* xyz, int64_t n, const float* poses, cons
         : upstream ? (prior ? cov_traj_fused_tiles_kernel<true, true> : cov_traj_fused_tiles_kernel<true, false>)
                    : (prior ? cov_traj_fused_tiles_kernel<false, true> : cov_traj_fused_tiles_kernel<false, false>);
     tiles_kern<<<persistent_grid(tiles_kern, 0, ntiles), COV_THREADS, 0, s>>>(
-        xyz, n, t.table, W, C, upstream, reward_index, rewards, acc, boxes, t.amask, mask_stride_words(W), t.worklist,
+        xyz, n, t.table, W, C, upstream, reward_index, rewards, acc, t.amask, mask_stride_words(W), t.worklist,
         t.ctrl, ntiles, opts ? opts->stats_dev : nullptr, prior);
     return cov_check_launch("cov_traj_fused");
 }
@@ -2241,16 +2311,16 @@ extern "C" int cov_traj_logodds(const float* xyz, int64_t n, const float* poses,
                                                                        logodds);
         return cov_check_launch("cov_traj_logodds");
     }
-    // pruned: pass B's table and cull (no accumulators, no pre-fill), then its forward over the listed tiles
+    // pruned: pass B's table and cull (no accumulators, no pre-fill), then its forward over the listed boxes
     constexpr int ppt = 4;
     const int64_t ntiles = (n + tile_points(ppt) - 1) / tile_points(ppt);
     const TrajWorkspace t = carve_workspace(ws, n, W);
     const float4* boxes = boxes_for_call(xyz, n, boxes_dev, t, s);
     cov_traj_table_kernel<false><<<(W + 63) / 64, 64, 0, s>>>(poses, quats, W, K, C, minmax, t.table, t.ctrl,
                                                               (int)(t.ctrl_bytes / sizeof(int)), nullptr, 0.0, nullptr);
-    if ((rc = launch_cull(boxes, ppt, ntiles, t, W, nullptr, 0.f, nullptr, 0, s)) != COV_OK) return rc;
+    if ((rc = launch_cull(boxes, n, t, W, nullptr, 0.f, nullptr, 0, s)) != COV_OK) return rc;
     cov_traj_logodds_tiles_kernel<<<persistent_grid(cov_traj_logodds_tiles_kernel, 0, ntiles), COV_THREADS, 0, s>>>(
-        xyz, n, t.table, W, C, reward_index, logodds, boxes, t.amask, mask_stride_words(W), t.worklist, t.ctrl);
+        xyz, n, t.table, W, C, reward_index, logodds, t.amask, mask_stride_words(W), t.worklist, t.ctrl);
     return cov_check_launch("cov_traj_logodds");
 }
 
@@ -2266,7 +2336,7 @@ static int sweep_rewards_impl(const float* xyz, int64_t n, const float* poses, c
     if (opts && opts->dense)
         return cov_sweep_rewards_dense(xyz, n, poses, quats, n_traj, per_traj, K, cam, minmax, sum_rewards, prior,
                                        prior_sum, weight, stream);
-    // trajectories per launch: as many as the per-tile pose mask holds (32 * kMaskWords poses); the pose table stays in
+    // trajectories per launch: as many as the per-box pose mask holds (32 * kMaskWords poses); the pose table stays in
     // global memory, the block keeps one fp64 total per trajectory in shared memory
     if (per_traj > 32 * kMaskWords) {
         cov_set_error("cov_sweep_rewards: %d poses per trajectory exceed the pose mask (%d)", per_traj, 32 * kMaskWords);
@@ -2296,12 +2366,12 @@ static int sweep_rewards_impl(const float* xyz, int64_t n, const float* poses, c
         cov_traj_table_kernel<false><<<(Wn + 63) / 64, 64, 0, s>>>(poses + 3 * (size_t)w0, quats + 4 * (size_t)w0, Wn, K, C, mm,
                                                                    t.table, t.ctrl, (int)(t.ctrl_bytes / sizeof(int)), nullptr,
                                                                    0.0, nullptr);
-        if (launch_cull(boxes, ppt, ntiles, t, Wn, nullptr, 0.f, nullptr, 0, s) != COV_OK) return COV_ERR_UNSUPPORTED;
+        if (launch_cull(boxes, n, t, Wn, nullptr, 0.f, nullptr, 0, s) != COV_OK) return COV_ERR_UNSUPPORTED;
         const size_t smem = (size_t)nt * sizeof(double);
         const auto kern = weight ? (prior ? cov_sweep_tiles_kernel<true, true> : cov_sweep_tiles_kernel<false, true>)
                                  : (prior ? cov_sweep_tiles_kernel<true> : cov_sweep_tiles_kernel<false>);
         kern<<<persistent_grid(kern, smem, ntiles), COV_THREADS, smem, s>>>(
-            xyz, n, t.table, Wn, per_traj, nt, C, boxes, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, sum_rewards + t0,
+            xyz, n, t.table, Wn, per_traj, nt, C, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, sum_rewards + t0,
             prior, prior_sum, weight);
     }
     return cov_check_launch("cov_sweep_rewards");
@@ -2414,8 +2484,8 @@ static int sweep_fused_impl(const float* xyz, int64_t n, const float* poses, con
         }
         return COV_OK;
     }
-    // pruned: the chunking of cov_sweep_rewards (as many trajectories per launch as the tile pose mask holds); per chunk
-    // pose table, cull + work list, evaluation of the listed tiles
+    // pruned: the chunking of cov_sweep_rewards (as many trajectories per launch as the box pose mask holds); per chunk
+    // pose table, cull + work list, evaluation of the listed boxes
     const int chunk = std::min((32 * kMaskWords) / per_traj, n_traj);
     const CovConst C = cov_make_const(cam);
     const TrajWorkspace t = carve_workspace(ws, n, chunk * per_traj);
@@ -2439,12 +2509,12 @@ static int sweep_fused_impl(const float* xyz, int64_t n, const float* poses, con
         cov_traj_table_kernel<false><<<(Wn + 63) / 64, 64, 0, s>>>(poses + 3 * (size_t)w0, quats + 4 * (size_t)w0, Wn, K, C,
                                                                    mm, t.table, t.ctrl, (int)(t.ctrl_bytes / sizeof(int)),
                                                                    nullptr, 0.0, nullptr);
-        int rc = launch_cull(boxes, ppt, ntiles, t, Wn, nullptr, 0.f, nullptr, 0, s);
+        int rc = launch_cull(boxes, n, t, Wn, nullptr, 0.f, nullptr, 0, s);
         if (rc != COV_OK) return rc;
         const auto kern = weight ? (prior ? cov_sweep_fused_tiles_kernel<true, true> : cov_sweep_fused_tiles_kernel<false, true>)
                                  : (prior ? cov_sweep_fused_tiles_kernel<true> : cov_sweep_fused_tiles_kernel<false>);
         kern<<<persistent_grid(kern, 0, ntiles), COV_THREADS, 0, s>>>(
-            xyz, n, t.table, Wn, per_traj, C, boxes, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, ntiles,
+            xyz, n, t.table, Wn, per_traj, C, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, ntiles,
             acc + (size_t)t0 * block, stats, prior, weight);
     }
     return cov_check_launch("cov_sweep_fused");
