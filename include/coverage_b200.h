@@ -271,6 +271,31 @@ int cov_sweep_epilogue_dev(const double* acc_dev, const float* minmax_dev, const
                            int poses_per_traj, const double* den_dev, float* out_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Prefix sweep: the reward sum of every prefix of every candidate trajectory in one pass over the cloud per chunk of
+ * cov_traj_max_poses_pruned() poses (the chunking of cov_sweep_rewards).
+ * ref: no reference implementation; entry [t*P + i] is what cov_sweep_rewards (or its _prior / _weighted form, with the
+ * same prior and weight) returns for trajectory t cut after its pose i, i.e. poses_dev[t*P .. t*P + i], up to the order of
+ * the fp64 additions: sum_j w_j r_j(t, first i + 1 poses) over this shard, w_j = 1 without a weight.  Each row is
+ * non-decreasing in i up to the fp32 rounding of single terms.  A pose with 0/0 normalisers (it sees nothing) makes its
+ * prefix and every later one NaN, as it makes the truncated sweeps'.  With a multi-camera rig (pose index
+ * body*n_cams + cam) the prefix after body k is entry (k+1)*n_cams - 1.
+ *   prefix_sums_dev  n_traj * P doubles, OVERWRITTEN (the call zeroes them first).  Shard-additive: SUM over the ranks.
+ *   minmax_dev       (2, n_traj*P): the normalisers, as for cov_sweep_rewards.
+ *   prior_dev, weight_dev  NULL, or as for the _prior / _weighted sweeps; NULL pointers select the plain variant.
+ *   base_dev         NULL without prior and weight (the base is n/2); cov_prior_reward_sum's double with a prior alone;
+ *                    cov_weight_sums' two doubles with a weight (with or without a prior).  Anything else: COV_ERR_ARG.
+ *   opts             dense as for cov_sweep_rewards (no small-cloud threshold: the pruned path for any n unless dense);
+ *                    stats_dev is not used (cov_sweep_rewards counts nothing either).  The pruned path takes
+ *                    P <= cov_traj_max_poses_pruned() (else COV_ERR_UNSUPPORTED).
+ *   workspace_dev    cov_sweep_workspace_bytes(n, n_traj, P) bytes, 256-byte aligned.
+ * ------------------------------------------------------------------------------------------ */
+int cov_sweep_prefix_rewards(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev,
+                             int n_traj, int poses_per_traj, const float* K_dev, const cov_camera* cam,
+                             const float* boxes_dev, const float* minmax_dev, const float* prior_dev,
+                             const float* weight_dev, const double* base_dev, double* prefix_sums_dev,
+                             const cov_traj_opts* opts, void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Batched ModelPose: K candidate poses (t_k, q~_k) on one cloud, for every k the COV_POSE_ACC sums cov_pose_fused
  * computes for pose k alone ([0] sum m, [1..3] F, [4..6] T, [7] 0), in one pass over the cloud per chunk of poses.
  * ref: src/model.py:98-127 per pose (multi-start pose optimisation, scoring of candidate views); no per-point output.

@@ -360,4 +360,5 @@ CovConst cov_make_const(const struct cov_camera* cam);
 int cov_sm_count_cached();
 int cov_sweep_rewards_dense(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj, int per_traj,
                             const float* K, const struct cov_camera* cam, const float* minmax, double* sum_rewards,
-                            const float* prior, const double* prior_sum, const float* weight, void* stream);
+                            const float* prior, const double* prior_sum, const float* weight, void* stream,
+                            bool prefix = false);

@@ -1360,7 +1360,12 @@ cov_traj_fused_tiles_kernel(const float* __restrict__ xyz, int64_t n, const floa
 // read there), and *prior_sum = sum_j sigmoid(prior_j) in place of 0.5 * n.
 // HAS_W: each point's term times its weight w_j (read next to the prior, in the cloud's order), and *prior_sum is the
 // weighted base sum_j w_j r0_j (cov_weight_sums).
-template <bool HAS_PRIOR, bool HAS_W = false>
+// PREFIX (cov_sweep_prefix_rewards): one slot per pose instead of one per trajectory.  After each pose at which the warp
+// gated a pair, the item's flush value V (the same fp32 terms and warp sum) is what the sweep of the trajectory cut after
+// that pose would add at its end; the difference (double)V - (double)V_prev goes to the pose's slot (V_prev = 0 at the
+// trajectory's first pose).  Block 0 adds the base to slot 0 of each trajectory; the inclusive scan of a trajectory's
+// slots (cov_prefix_scan_kernel) is then the truncated sweep's sum, up to the order of fp64 additions.
+template <bool HAS_PRIOR, bool HAS_W = false, bool PREFIX = false>
 __global__ void __launch_bounds__(COV_THREADS, 3)
 cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, int per_traj,
                        int n_traj, CovConst C, const unsigned* __restrict__ amask_g, int mask_stride, const int* __restrict__ worklist, int* __restrict__ ctrl,
@@ -1368,9 +1373,10 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
                        const float* __restrict__ weight) {
     constexpr int PPT = kItemPpt;
     extern __shared__ float4 smem4[];
-    double* ssum = reinterpret_cast<double*>(smem4);   // per-trajectory totals of this block
+    double* ssum = reinterpret_cast<double*>(smem4);   // per-trajectory (PREFIX: per-pose) totals of this block
     const int tid = threadIdx.x, lane = tid & 31;
-    for (int t = tid; t < n_traj; t += COV_THREADS) ssum[t] = 0.0;
+    const int nslots = PREFIX ? W : n_traj;
+    for (int t = tid; t < nslots; t += COV_THREADS) ssum[t] = 0.0;
     __syncthreads();
     const int n_items = ctrl[0];
     const int nwords = (W + 31) >> 5;
@@ -1381,32 +1387,37 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
         load_item_points<false>(item, xyz, n, lane, px, py, pz, valid);
         int cur = -1;      // trajectory whose log-odds sums are in L
         bool touched = false;
+        float vprev = 0.f;  // PREFIX: the item's value after the last gated pose of `cur`
+        // the warp sum of the item's reward terms for the log-odds sums in L
+        auto value = [&]() {
+            float a = 0.f;
+#pragma unroll
+            for (int s = 0; s < PPT; ++s) {
+                if (HAS_W) {
+                    if (valid[s] && L[s] != 0.f) {
+                        const int64_t j = item.j0 + s * 32 + lane;
+                        const float wj = __ldg(weight + j);
+                        if (HAS_PRIOR) {
+                            const float pr = __ldg(prior + j);
+                            a += wj * (cov_sigmoid(cov_fuse_prior(pr, L[s])) - cov_sigmoid(pr));
+                        } else {
+                            a += wj * (1.f / (1.f + expf(-L[s])) - 0.5f);
+                        }
+                    }
+                } else if (HAS_PRIOR) {
+                    if (valid[s] && L[s] != 0.f) {
+                        const float pr = __ldg(prior + item.j0 + s * 32 + lane);
+                        a += cov_sigmoid(cov_fuse_prior(pr, L[s])) - cov_sigmoid(pr);
+                    }
+                } else if (valid[s] && L[s] != 0.f) {
+                    a += 1.f / (1.f + expf(-L[s])) - 0.5f;
+                }
+            }
+            return cov_warp_sum(a);
+        };
         auto flush = [&]() {
             if (cur >= 0 && touched) {
-                float a = 0.f;
-#pragma unroll
-                for (int s = 0; s < PPT; ++s) {
-                    if (HAS_W) {
-                        if (valid[s] && L[s] != 0.f) {
-                            const int64_t j = item.j0 + s * 32 + lane;
-                            const float wj = __ldg(weight + j);
-                            if (HAS_PRIOR) {
-                                const float pr = __ldg(prior + j);
-                                a += wj * (cov_sigmoid(cov_fuse_prior(pr, L[s])) - cov_sigmoid(pr));
-                            } else {
-                                a += wj * (1.f / (1.f + expf(-L[s])) - 0.5f);
-                            }
-                        }
-                    } else if (HAS_PRIOR) {
-                        if (valid[s] && L[s] != 0.f) {
-                            const float pr = __ldg(prior + item.j0 + s * 32 + lane);
-                            a += cov_sigmoid(cov_fuse_prior(pr, L[s])) - cov_sigmoid(pr);
-                        }
-                    } else if (valid[s] && L[s] != 0.f) {
-                        a += 1.f / (1.f + expf(-L[s])) - 0.5f;
-                    }
-                }
-                a = cov_warp_sum(a);
+                const float a = value();
                 if (lane == 0 && a != 0.f) atomicAdd(ssum + cur, (double)a);
             }
         };
@@ -1419,22 +1430,53 @@ cov_sweep_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* _
                 const float4 v3 = __ldg(row + 3);
                 const int t = w / per_traj;
                 if (t != cur) {
-                    flush();
+                    if (!PREFIX) flush();
                     cur = t;
                     touched = false;
+                    vprev = 0.f;
 #pragma unroll
                     for (int s = 0; s < PPT; ++s) L[s] = 0.f;
                 }
-                touched |= tiles_pose_iter<PPT, false>(row, v3, px, py, pz, L, C, nullptr);
+                const bool g = tiles_pose_iter<PPT, false>(row, v3, px, py, pz, L, C, nullptr);
+                if (PREFIX) {
+                    if (g) {  // warp-uniform
+                        const float v = value();
+                        if (lane == 0 && v != vprev) atomicAdd(ssum + w, (double)v - (double)vprev);
+                        vprev = v;
+                    }
+                } else {
+                    touched |= g;
+                }
             }
         }
-        flush();
+        if (!PREFIX) flush();
     });
     __syncthreads();
-    for (int t = tid; t < n_traj; t += COV_THREADS) {
+    for (int t = tid; t < nslots; t += COV_THREADS) {
         double v = ssum[t];
-        if (blockIdx.x == 0) v += (HAS_PRIOR || HAS_W) ? *prior_sum : 0.5 * (double)n;
+        if (blockIdx.x == 0 && (!PREFIX || t % per_traj == 0)) v += (HAS_PRIOR || HAS_W) ? *prior_sum : 0.5 * (double)n;
         if (v != 0.0) atomicAdd(sum_out + t, v);
+    }
+}
+
+// Inclusive prefix sums of each trajectory's P slots, in place: one warp per trajectory, 32 slots at a time (a fixed
+// shuffle tree, then the carry of the previous 32), so the result is a deterministic function of the slots.
+__global__ void __launch_bounds__(256) cov_prefix_scan_kernel(double* __restrict__ sums, int n_traj, int per_traj) {
+    const int t = (int)((blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (t >= n_traj) return;
+    double* row = sums + (size_t)t * per_traj;
+    double carry = 0.0;
+    for (int i0 = 0; i0 < per_traj; i0 += 32) {
+        const int i = i0 + lane;
+        double v = i < per_traj ? row[i] : 0.0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const double u = __shfl_up_sync(kFull, v, o);
+            if (lane >= o) v += u;
+        }
+        v += carry;
+        if (i < per_traj) row[i] = v;
+        carry = __shfl_sync(kFull, v, 31);
     }
 }
 
@@ -2324,29 +2366,31 @@ extern "C" int cov_traj_logodds(const float* xyz, int64_t n, const float* poses,
     return cov_check_launch("cov_traj_logodds");
 }
 
+// prefix: the per-pose slots of cov_sweep_prefix_rewards (sum_rewards holds n_traj * per_traj doubles; the caller scans)
 static int sweep_rewards_impl(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
                               int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
                               const float* minmax, double* sum_rewards, const float* prior, const double* prior_sum,
                               const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream,
-                              const float* weight = nullptr) {
+                              const float* weight = nullptr, bool prefix = false) {
+    const char* who = prefix ? "cov_sweep_prefix_rewards" : "cov_sweep_rewards";
     if (!xyz || n <= 0 || !poses || !quats || n_traj <= 0 || per_traj <= 0 || !K || !cam || !minmax || !sum_rewards) {
-        cov_set_error("cov_sweep_rewards: bad argument");
+        cov_set_error("%s: bad argument", who);
         return COV_ERR_ARG;
     }
     if (opts && opts->dense)
         return cov_sweep_rewards_dense(xyz, n, poses, quats, n_traj, per_traj, K, cam, minmax, sum_rewards, prior,
-                                       prior_sum, weight, stream);
+                                       prior_sum, weight, stream, prefix);
     // trajectories per launch: as many as the per-box pose mask holds (32 * kMaskWords poses); the pose table stays in
-    // global memory, the block keeps one fp64 total per trajectory in shared memory
+    // global memory, the block keeps one fp64 total per trajectory (prefix: per pose) in shared memory
     if (per_traj > 32 * kMaskWords) {
-        cov_set_error("cov_sweep_rewards: %d poses per trajectory exceed the pose mask (%d)", per_traj, 32 * kMaskWords);
+        cov_set_error("%s: %d poses per trajectory exceed the pose mask (%d)", who, per_traj, 32 * kMaskWords);
         return COV_ERR_UNSUPPORTED;
     }
     int chunk = (32 * kMaskWords) / per_traj;
     if (chunk > n_traj) chunk = n_traj;
     const int Wc = chunk * per_traj;
     if (!ws || ws_bytes < cov_sweep_workspace_bytes(n, n_traj, per_traj) || (((uintptr_t)ws) & 255) || (((uintptr_t)xyz) & 15)) {
-        cov_set_error("cov_sweep_rewards: workspace missing, misaligned or smaller than cov_sweep_workspace_bytes(n, %d, %d) = %zu",
+        cov_set_error("%s: workspace missing, misaligned or smaller than cov_sweep_workspace_bytes(n, %d, %d) = %zu", who,
                       n_traj, per_traj, cov_sweep_workspace_bytes(n, n_traj, per_traj));
         return COV_ERR_WORKSPACE;
     }
@@ -2367,14 +2411,17 @@ static int sweep_rewards_impl(const float* xyz, int64_t n, const float* poses, c
                                                                    t.table, t.ctrl, (int)(t.ctrl_bytes / sizeof(int)), nullptr,
                                                                    0.0, nullptr);
         if (launch_cull(boxes, n, t, Wn, nullptr, 0.f, nullptr, 0, s) != COV_OK) return COV_ERR_UNSUPPORTED;
-        const size_t smem = (size_t)nt * sizeof(double);
-        const auto kern = weight ? (prior ? cov_sweep_tiles_kernel<true, true> : cov_sweep_tiles_kernel<false, true>)
-                                 : (prior ? cov_sweep_tiles_kernel<true> : cov_sweep_tiles_kernel<false>);
+        const size_t smem = (size_t)(prefix ? Wn : nt) * sizeof(double);
+        const auto kern =
+            prefix ? (weight ? (prior ? cov_sweep_tiles_kernel<true, true, true> : cov_sweep_tiles_kernel<false, true, true>)
+                             : (prior ? cov_sweep_tiles_kernel<true, false, true> : cov_sweep_tiles_kernel<false, false, true>))
+                   : (weight ? (prior ? cov_sweep_tiles_kernel<true, true> : cov_sweep_tiles_kernel<false, true>)
+                             : (prior ? cov_sweep_tiles_kernel<true> : cov_sweep_tiles_kernel<false>));
         kern<<<persistent_grid(kern, smem, ntiles), COV_THREADS, smem, s>>>(
-            xyz, n, t.table, Wn, per_traj, nt, C, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl, sum_rewards + t0,
-            prior, prior_sum, weight);
+            xyz, n, t.table, Wn, per_traj, nt, C, t.amask, mask_stride_words(Wn), t.worklist, t.ctrl,
+            sum_rewards + (prefix ? w0 : t0), prior, prior_sum, weight);
     }
-    return cov_check_launch("cov_sweep_rewards");
+    return cov_check_launch(who);
 }
 
 extern "C" int cov_sweep_rewards(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
@@ -2406,6 +2453,34 @@ extern "C" int cov_sweep_rewards_weighted(const float* xyz, int64_t n, const flo
     // the weighted base sum_j w_j r0_j takes the place of the prior's sum
     return sweep_rewards_impl(xyz, n, poses, quats, n_traj, per_traj, K, cam, boxes_dev, minmax, sum_rewards, prior,
                               weight_sums, opts, ws, ws_bytes, stream, weight);
+}
+
+extern "C" int cov_sweep_prefix_rewards(const float* xyz, int64_t n, const float* poses, const float* quats, int n_traj,
+                                        int per_traj, const float* K, const cov_camera* cam, const float* boxes_dev,
+                                        const float* minmax, const float* prior, const float* weight, const double* base,
+                                        double* prefix_sums, const cov_traj_opts* opts, void* ws, size_t ws_bytes,
+                                        void* stream) {
+    // base: NULL (n / 2) without prior and weight, cov_prior_reward_sum with a prior alone, cov_weight_sums with a weight
+    int rc = COV_OK;
+    if (weight) rc = check_weight("cov_sweep_prefix_rewards", weight, base, prior);
+    else if (prior) rc = check_prior("cov_sweep_prefix_rewards", prior, base, true);
+    else if (base) {
+        cov_set_error("cov_sweep_prefix_rewards: base_dev must be NULL without prior_dev and weight_dev");
+        rc = COV_ERR_ARG;
+    }
+    if (rc) return rc;
+    if (!prefix_sums || n_traj <= 0 || per_traj <= 0 || (int64_t)n_traj * per_traj > INT32_MAX) {
+        cov_set_error("cov_sweep_prefix_rewards: bad argument (prefix_sums_dev %p, n_traj=%d, poses_per_traj=%d)",
+                      (void*)prefix_sums, n_traj, per_traj);
+        return COV_ERR_ARG;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaMemsetAsync(prefix_sums, 0, (size_t)n_traj * per_traj * sizeof(double), s);
+    rc = sweep_rewards_impl(xyz, n, poses, quats, n_traj, per_traj, K, cam, boxes_dev, minmax, prefix_sums, prior, base,
+                            opts, ws, ws_bytes, stream, weight, true);
+    if (rc) return rc;
+    cov_prefix_scan_kernel<<<(unsigned)(((int64_t)n_traj * 32 + 255) / 256), 256, 0, s>>>(prefix_sums, n_traj, per_traj);
+    return cov_check_launch("cov_sweep_prefix_rewards");
 }
 
 extern "C" size_t cov_sweep_workspace_bytes(int64_t n, int n_traj, int per_traj) {

@@ -558,6 +558,23 @@ class ModelTrajBatch(_OrderedCloudModel):
         self.means = means
         return self.criterion(means)
 
+    @torch.no_grad()
+    def prefix_means(self, vis_wps_dist=0.5):
+        """(T, P') fp64 mean rewards of every prefix of every trajectory over the waypoints `forward()` evaluates
+        (`[:, ::wps_step]`): [t, i] is the mean of trajectory t cut after its i-th evaluated waypoint, and [:, -1] is
+        `self.means` of a forward at the same poses (ops.sweep_prefix_rewards).  With the model's cloud, prior, weight
+        and group; without gradients."""
+        wps_step = self._wps_step(vis_wps_dist)
+        cloud = self._cloud()
+        prior, prior_sum = self._prior_args()
+        weight, wsums, wden = self._weight_args()
+        P, Q = self.poses[:, ::wps_step], self.quats[:, ::wps_step]
+        cam = ops._lib.camera(self.img_width, self.img_height, self.pc_clip_limits[0], self.pc_clip_limits[1], self.eps)
+        with ops.evaluation(dense=None if self.spatial_sort else True):
+            out = ops._sweep_run(ops._prefix_sums, P.shape[1], cloud, P, Q, self.K, cam, self.n_total, self.group,
+                                 self._boxes, "points", prior, prior_sum, weight, wsums, wden)
+        return out.reshape(P.shape[0], P.shape[1])
+
     def criterion(self, means):
         # ModelTraj.criterion per trajectory; length_calc and mean_angle_calc restated over the batch dimension
         p, p0 = self.poses, self.poses0

@@ -378,6 +378,21 @@ class CudaBackend:
               _ptr(minmax), _ptr(sums), ctypes.byref(opts), _ptr(ws), ws_bytes)
         return sums
 
+    def sweep_prefix_sums(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior=None, base=None, weight=None):
+        """(T Pn,) fp64: entry t Pn + i = sweep_sums of trajectory t cut after its pose i, over this cloud
+        (cov_sweep_prefix_rewards).  `base`: prior_sum(prior) with a prior alone, weight_sums(weight, prior) with a
+        weight, else None."""
+        L = _lib.lib()
+        n, dev = pts.shape[0], pts.device
+        ws_bytes = L.cov_sweep_workspace_bytes(n, T, Pn)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        out = torch.empty(T * Pn, dtype=torch.float64, device=dev)
+        opts = _opts()
+        _call("cov_sweep_prefix_rewards", pts, _ptr(pts), n, _ptr(P), _ptr(Q), T, Pn, _ptr(Kd), ctypes.byref(cam),
+              _ptr(boxes), _ptr(minmax), _ptr(prior), _ptr(weight), _ptr(base), _ptr(out), ctypes.byref(opts), _ptr(ws),
+              ws_bytes)
+        return out
+
     def traj_epilogue(self, acc, minmax, Q, n_total, upstream_mode, den=None):
         """`den` ((1,) fp64 on the device, sum_j w_j): the weighted mean's epilogue (cov_traj_epilogue_dev) in place of
         n_total."""
@@ -878,6 +893,65 @@ def _sweep_sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum, w=None
     return B.sweep_sums(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum)
 
 
+def _prefix_sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum, w=None, wsums=None):
+    return B.sweep_prefix_sums(pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior=prior,
+                               base=psum if w is None else wsums, weight=w)
+
+
+def _sweep_forward(sums, k, points, poses, quats, intrins, cam, n_total, group, boxes, presorted, shard, prior_logodds,
+                   weight):
+    """The forward-only sweeps around one backend sum `sums` (`_sweep_sums`, `_prefix_sums`) that gives k fp64 values
+    per trajectory: the cloud ordered, the prior and the weight checked and permuted with it, their sums, then
+    `_sweep_run`."""
+    B = _BACKEND
+    if shard not in ("points", "trajectories"):
+        raise ValueError("shard must be 'points' or 'trajectories'")
+    pts = B.prepare(points, what="points")
+    prior = _check_prior(prior_logodds, pts.shape[0], pts.device)
+    w = _check_weight(weight, pts.shape[0], pts.device)
+    pts, prior, boxes, w = _order_with_prior(B, pts, prior, boxes, presorted, w)
+    psum = wsums = den = None
+    if w is not None:
+        wsums, den = _weight_sums(B, w, prior, group if shard == "points" else None)
+    elif prior is not None:
+        psum = B.prior_sum(prior)
+    return _sweep_run(sums, k, pts, poses, quats, intrins, cam, n_total, group, boxes, shard, prior, psum, w, wsums, den)
+
+
+def _sweep_run(sums, k, pts, poses, quats, intrins, cam, n_total, group, boxes, shard, prior, psum, w, wsums, den):
+    """(T k,) fp64 means of the ordered cloud `pts` with its prior, weight and their sums: pass A, `sums`, the
+    collectives of `shard` and the division by the point count or the weighted denominator `den`."""
+    B = _BACKEND
+    dev = pts.device
+    T, Pn = poses.shape[0], poses.shape[1]
+    n = pts.shape[0]
+    Kd = B.prepare(intrins, dev, "intrins").reshape(9)
+    if group is not None and shard == "trajectories":
+        import torch.distributed as dist
+        world, rank = dist.get_world_size(group), dist.get_rank(group)
+        per = (T + world - 1) // world
+        t0, t1 = min(T, rank * per), min(T, (rank + 1) * per)
+        mine = torch.zeros(per * k, dtype=torch.float64, device=dev)
+        if t1 > t0:
+            P = B.prepare(poses[t0:t1], dev, "poses").reshape(-1, 3)
+            Q = B.prepare(quats[t0:t1], dev, "quats").reshape(-1, 4)
+            minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)
+            mine[:(t1 - t0) * k] = sums(B, pts, P, Q, t1 - t0, Pn, Kd, cam, boxes, minmax, prior, psum, w, wsums)
+        out = torch.empty(world * per * k, dtype=torch.float64, device=dev)
+        dist.all_gather_into_tensor(out, mine, group=group)
+        return out[:T * k] / (float(n) if w is None else den)
+    P = B.prepare(poses, dev, "poses").reshape(-1, 3)
+    Q = B.prepare(quats, dev, "quats").reshape(-1, 4)
+    minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)
+    _all_reduce_minmax(minmax, T * Pn, group)
+    out = sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum, w, wsums)
+    if group is not None:
+        _all_reduce(out, _reduce_ops()[2], group)
+    if w is not None:
+        return out / den
+    return out / float(n if n_total is None else n_total)
+
+
 @torch.no_grad()
 def sweep_rewards(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
                   n_total=None, group=None, boxes=None, presorted=False, shard="points", prior_logodds=None,
@@ -901,47 +975,35 @@ def sweep_rewards(points, poses, quats, intrins, img_width, img_height, min_dist
     `weight` (N,) fp32, finite and >= 0 with a positive sum (not checked): per-point importance shared by every
     trajectory; each result is then sum_j w_j r_j(t) / sum_j w_j.  Ordered and sharded like `prior_logodds` (with
     shard="points" the denominator is all-reduced); `n_total` is not used."""
-    B = _BACKEND
-    if shard not in ("points", "trajectories"):
-        raise ValueError("shard must be 'points' or 'trajectories'")
-    pts = B.prepare(points, what="points")
-    prior = _check_prior(prior_logodds, pts.shape[0], pts.device)
-    w = _check_weight(weight, pts.shape[0], pts.device)
-    pts, prior, boxes, w = _order_with_prior(B, pts, prior, boxes, presorted, w)
-    psum = wsums = den = None
-    if w is not None:
-        wsums, den = _weight_sums(B, w, prior, group if shard == "points" else None)
-    elif prior is not None:
-        psum = B.prior_sum(prior)
-    dev = pts.device
-    T, Pn = poses.shape[0], poses.shape[1]
-    n = pts.shape[0]
-    Kd = B.prepare(intrins, dev, "intrins").reshape(9)
     cam = _lib.camera(img_width, img_height, min_dist, max_dist, eps)
-    if group is not None and shard == "trajectories":
-        import torch.distributed as dist
-        world, rank = dist.get_world_size(group), dist.get_rank(group)
-        per = (T + world - 1) // world
-        t0, t1 = min(T, rank * per), min(T, (rank + 1) * per)
-        mine = torch.zeros(per, dtype=torch.float64, device=dev)
-        if t1 > t0:
-            P = B.prepare(poses[t0:t1], dev, "poses").reshape(-1, 3)
-            Q = B.prepare(quats[t0:t1], dev, "quats").reshape(-1, 4)
-            minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)
-            mine[:t1 - t0] = _sweep_sums(B, pts, P, Q, t1 - t0, Pn, Kd, cam, boxes, minmax, prior, psum, w, wsums)
-        out = torch.empty(world * per, dtype=torch.float64, device=dev)
-        dist.all_gather_into_tensor(out, mine, group=group)
-        return out[:T] / (float(n) if w is None else den)
-    P = B.prepare(poses, dev, "poses").reshape(-1, 3)
-    Q = B.prepare(quats, dev, "quats").reshape(-1, 4)
-    minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes)
-    _all_reduce_minmax(minmax, T * Pn, group)
-    sums = _sweep_sums(B, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior, psum, w, wsums)
-    if group is not None:
-        _all_reduce(sums, _reduce_ops()[2], group)
-    if w is not None:
-        return sums / den
-    return sums / float(n if n_total is None else n_total)
+    return _sweep_forward(_sweep_sums, 1, points, poses, quats, intrins, cam, n_total, group, boxes, presorted, shard,
+                          prior_logodds, weight)
+
+
+@torch.no_grad()
+def sweep_prefix_rewards(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
+                         n_total=None, group=None, boxes=None, presorted=False, shard="points", prior_logodds=None,
+                         weight=None):
+    """The mean reward of every prefix of every candidate trajectory: poses (T, P, 3), quats (T, P, 4) -> (T, P) fp64,
+    where [t, i] is what `sweep_rewards(points, poses[:, :i+1], quats[:, :i+1], ...)` returns for trajectory t, with the
+    same prior and weight, up to the order of fp64 additions; [:, P-1] is `sweep_rewards`'s result.  One pass over the
+    cloud per chunk of poses, as `sweep_rewards` (cov_sweep_prefix_rewards), in place of P sweeps.
+    Rows are non-decreasing (up to the fp32 rounding of single terms).  Uses: how far along a candidate to commit
+    (receding horizon), gain per path cost at every node of a branch, and candidates of different lengths: pad each to P
+    (e.g. by repeating its last pose) and read column len_t - 1.  With a multi-camera rig (pose index body * n_cams +
+    cam, `multicam`) the prefix after waypoint k is column (k + 1) * n_cams - 1.  A pose that sees nothing has 0/0
+    normalisers: its prefix and every later one of its trajectory are NaN, as the truncated sweeps are.
+    Arguments, ordering, prior, weight and sharding as for `sweep_rewards` (shard="points": the T P sums are
+    all-reduced; "trajectories": the rank blocks are all-gathered).  Without gradients."""
+    if (not isinstance(poses, torch.Tensor) or not isinstance(quats, torch.Tensor) or poses.dim() != 3
+            or quats.dim() != 3 or poses.shape[2] != 3 or quats.shape[2] != 4 or poses.shape[:2] != quats.shape[:2]
+            or poses.shape[0] == 0 or poses.shape[1] == 0):
+        raise ValueError("sweep_prefix_rewards: poses must be (T, P, 3) and quats (T, P, 4) with the same T, P >= 1; got "
+                         f"{tuple(getattr(poses, 'shape', ()))} and {tuple(getattr(quats, 'shape', ()))}")
+    T, Pn = poses.shape[0], poses.shape[1]
+    cam = _lib.camera(img_width, img_height, min_dist, max_dist, eps)
+    return _sweep_forward(_prefix_sums, Pn, points, poses, quats, intrins, cam, n_total, group, boxes, presorted, shard,
+                          prior_logodds, weight).reshape(T, Pn)
 
 
 def coverage_sweep(points, poses, quats, intrins, img_width, img_height, min_dist=1.0, max_dist=5.0, eps=1e-6,
