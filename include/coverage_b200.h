@@ -271,6 +271,47 @@ int cov_sweep_epilogue_dev(const double* acc_dev, const float* minmax_dev, const
                            int poses_per_traj, const double* den_dev, float* out_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Long trajectories: the trajectory objective, its gradients and the log-odds fold for any number of poses W (one
+ * cov_traj_fused call takes at most cov_traj_max_poses_pruned()).  The poses run in chunks of pose_chunk; the fused
+ * log-odds L_j = sum_w lo_jw (fp32, ascending pose order) is carried between chunks in fp32, so the outputs are those
+ * of one cov_traj_fused / cov_traj_logodds call over all W poses, had it existed: normalisers, every reward and
+ * sigmoid(logodds) bit for bit, the accumulators up to the order of the fp64 additions; the variants, index conventions
+ * and tie accumulators are pass B's.  The pruned kernels run on every cloud size (they are exact on any point order).
+ * ref: src/model.py:217-237 over all waypoints, with no pose limit.
+ *   pose_chunk   0 = cov_traj_max_poses_pruned(); else 1 .. that (COV_ERR_ARG otherwise).  Results do not depend on it;
+ *                smaller chunks need more workspace (one box mask row per chunk) and more launches.
+ *   acc_dev      22 * W + 1 doubles, the layout of cov_traj_fused: the SUM all-reduce and the epilogues are unchanged.
+ *   prior_dev, weight_dev, base_dev  NULL pointers select the variant: no prior and weight (base_dev NULL), a prior alone
+ *                (base_dev = cov_prior_reward_sum), a weight with or without a prior (base_dev = cov_weight_sums; then
+ *                upstream_dev must be NULL).  Indexed like rewards_dev, as for the _prior / _weighted entry points.
+ *   opts         rewards_prefilled and stats_dev as for cov_traj_fused (stats: counters [0], [1], [4], [6], summed over
+ *                the chunks to what one call would count).  dense != 0: one dense cov_traj_fused (cov_traj_logodds)
+ *                call when W <= cov_traj_max_poses(), COV_ERR_UNSUPPORTED above that (there is no dense long path).
+ *   workspace    cov_traj_long_workspace_bytes(n, W, pose_chunk) bytes, 256-byte aligned; it never grows with pose_chunk
+ *                and also serves the per-chunk pass A below.  It grows with W: one mask row per listed 128-point box per
+ *                chunk (up to 2 n bytes per chunk of 2048 poses) next to 4 n bytes of carried log-odds.
+ * Pass A runs per chunk through cov_traj_minmax (the normalisers are per pose) into the W-wide layout.  For C callers:
+ *   for each chunk [w0, w1) of at most cov_traj_max_poses_pruned() poses (cov_traj_max_poses() when n < 65536 or dense):
+ *     cov_traj_minmax(.., poses + 3 w0, quats + 4 w0, w1 - w0, .., mm, opts, ws, ..)   (opts.prefill_dev = rewards on
+ *     the first chunk only; cov_traj_minmax_prior with a prior), then copy mm[0, w1-w0) to minmax[w0, w1) and
+ *     mm[w1-w0, 2(w1-w0)) to minmax[W + w0, W + w1);
+ *   MIN/MAX all-reduce of minmax over the ranks (sharded clouds);
+ *   cov_traj_fused_long(.., minmax, .., acc, .., opts.rewards_prefilled = cov_traj_prefill_applies(n, opts), ..);
+ *   SUM all-reduce of acc; cov_traj_epilogue (cov_traj_epilogue_dev with a weight).
+ * cov_traj_logodds_long: cov_traj_logodds over all W poses (logodds_dev holds the prior or zeros on entry).
+ * ------------------------------------------------------------------------------------------ */
+size_t cov_traj_long_workspace_bytes(int64_t n, int n_poses, int pose_chunk);
+int cov_traj_fused_long(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev, int n_poses,
+                        const float* K_dev, const cov_camera* cam, const float* boxes_dev, const float* minmax_dev,
+                        const float* upstream_dev, const int32_t* reward_index_dev, float* rewards_dev, double* acc_dev,
+                        const float* prior_dev, const double* base_dev, const float* weight_dev, int pose_chunk,
+                        const cov_traj_opts* opts, void* workspace_dev, size_t workspace_bytes, void* stream);
+int cov_traj_logodds_long(const float* xyz_dev, int64_t n, const float* poses_dev, const float* quats_dev, int n_poses,
+                          const float* K_dev, const cov_camera* cam, const float* boxes_dev, const float* minmax_dev,
+                          const int32_t* reward_index_dev, float* logodds_dev, int pose_chunk, const cov_traj_opts* opts,
+                          void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Prefix sweep: the reward sum of every prefix of every candidate trajectory in one pass over the cloud per chunk of
  * cov_traj_max_poses_pruned() poses (the chunking of cov_sweep_rewards).
  * ref: no reference implementation; entry [t*P + i] is what cov_sweep_rewards (or its _prior / _weighted form, with the

@@ -86,6 +86,10 @@ PROTOTYPES = {
     "cov_sweep_epilogue_dev": (_int, [_vp, _vp, _vp, _int, _int, _vp, _vp, _vp]),
     "cov_sweep_prefix_rewards": (_int, [_vp, _i64, _vp, _vp, _int, _int, _vp, _cam, _vp, _vp, _vp, _vp, _vp, _vp, _opts,
                                         _vp, _sz, _vp]),
+    "cov_traj_long_workspace_bytes": (_sz, [_i64, _int, _int]),
+    "cov_traj_fused_long": (_int, [_vp, _i64, _vp, _vp, _int, _vp, _cam, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int,
+                                   _opts, _vp, _sz, _vp]),
+    "cov_traj_logodds_long": (_int, [_vp, _i64, _vp, _vp, _int, _vp, _cam, _vp, _vp, _vp, _vp, _int, _opts, _vp, _sz, _vp]),
     "cov_peer_region_bytes": (_sz, [_int, _i64, _int]),
     "cov_peer_allreduce": (_int, [_int, _vp, _i64, C.POINTER(Peers), _sz, _vp]),
     "cov_rig_poses": (_int, [_vp, _int, _vp, _int, _vp, _vp, _vp]),

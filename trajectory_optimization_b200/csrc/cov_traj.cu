@@ -48,6 +48,10 @@
 //   cov_sweep_fused_tiles_kernel  per trajectory, pass B's accumulators (its forward and its backward, shared with the
 //                                 pass B kernel through tiles_pose_iter and tiles_pose_backward)
 //
+// LONG TRAJECTORIES (more poses than one box mask holds): pass B per pose chunk, the fused log-odds carried between the
+//   chunks in fp32 (cov_traj_logodds_tiles_kernel<CARRY>), one finalise pass over the cloud, then the backward per chunk
+//   over the kept work lists (cov_traj_long_backward_kernel).
+//
 // Block accumulators are added to the caller's fp64 accumulator rows with fp64 atomics (the order of those additions is
 // the only thing that differs between runs: ~1e-16 relative).  The arg-max / arg-min tie sets of the normalisation
 // backward are rare (one point per pose unless the minimum underflowed to 0, in which case their gradient is exactly
@@ -308,30 +312,33 @@ cov_traj_prepare_kernel(const float* __restrict__ xyz, int64_t nsamples, int64_t
 // some pose has min_j m > 0; every block builds 64 rows of the pose table with the normalisation constants:
 // v3.w = qthr, v4 = (b/2, b, 1/b, a), v5.w = thr.
 // SUM_DEV: the sum starts at *sum_base_dev instead (sum_j sigmoid(prior_j), cov_prior_reward_sum).
-template <bool SUM_DEV>
+// LONG (cov_traj_fused_long): the W poses are the chunk [w0, w0 + W) of a call over w_all poses; `poses`, `quats`, `table`
+// and `acc` point at the chunk's first pose, `minmax` is the call's [w_all minima | w_all maxima].  Only the chunk's
+// accumulator rows are zeroed, and the reward-sum slot acc[(w_all - w0) * STRIDE] is set by the chunk with w0 = 0 alone.
+template <bool SUM_DEV, bool LONG = false>
 __global__ void __launch_bounds__(64)
 cov_traj_table_kernel(const float* __restrict__ poses, const float* __restrict__ quats, int W,
                       const float* __restrict__ K9, CovConst C, const float* __restrict__ minmax,
                       float4* __restrict__ table, int* __restrict__ ctrl, int ctrl_words, double* __restrict__ acc,
-                      double sum_base, const double* __restrict__ sum_base_dev) {
+                      double sum_base, const double* __restrict__ sum_base_dev, int w0 = 0, int w_all = 0) {
     const int tid = threadIdx.x;
     if (blockIdx.x == 0) {
         int amin = 0;
-        for (int w = tid; w < W; w += blockDim.x) amin |= minmax[w] > 0.f;
+        for (int w = tid; w < W; w += blockDim.x) amin |= (LONG ? minmax[w0 + w] : minmax[w]) > 0.f;
         amin = __syncthreads_or(amin);
         for (int i = tid; i < ctrl_words; i += blockDim.x) ctrl[i] = (i == 1) ? amin : 0;
         if (acc) {
             for (int i = tid; i < W * COV_ACC_STRIDE; i += blockDim.x) acc[i] = 0.0;
-            if (tid == 0) acc[(size_t)W * COV_ACC_STRIDE] = SUM_DEV ? *sum_base_dev : sum_base;
+            if (tid == 0 && (!LONG || w0 == 0)) acc[(size_t)(LONG ? w_all : W) * COV_ACC_STRIDE] = SUM_DEV ? *sum_base_dev : sum_base;
         }
     }
     const int w = blockIdx.x * blockDim.x + tid;
     if (w >= W) return;
     float4 row[COV_ROW_F4];
     cov_pose_row(poses + 3 * w, quats + 4 * w, K9, C, row);
-    const float a = minmax[w];
+    const float a = LONG ? minmax[w0 + w] : minmax[w];
     float thr;
-    cov_norm_row(row, a, minmax[W + w], thr);
+    cov_norm_row(row, a, LONG ? minmax[w_all + w0 + w] : minmax[W + w], thr);
     row[5].w = thr;
     // q2 above qthr cannot reach thr (thr <= 0 or NaN, or a > 0 — arg-min points carry gradient: never prune)
     row[3].w = (thr > 0.f && !(a > 0.f)) ? (float)((1e-4 - log2((double)thr)) / (double)C.kd * 1.000001)
@@ -1756,40 +1763,214 @@ __global__ void __launch_bounds__(256) cov_prior_sum_kernel(const float* __restr
 // Fused log-odds output, pruned: pass B's forward (same work list and masks, same pose order, hence the same L_j)
 // without the backward; out[jo] = out[jo] + L_j for the points with L_j != 0 (the caller pre-filled `out` with the prior,
 // indexed like the rewards), the x that pass B's sigmoid takes.
+// CARRY (one pose chunk of the long path, cov_traj_fused_long / cov_traj_logodds_long): L_j starts from carry[j] (cloud
+// order; zeroed once per call) instead of 0 and, when the warp gated a pair, is stored back there, so that after the last
+// chunk carry[j] holds the fp32 sum of every chunk's terms in ascending pose order: the L_j of one call over all poses, bit
+// for bit.  A point of such an item whose sum is still 0 is stored as -0 (a marker the finalise kernel reads: the point may
+// enter the backward; -0 + x = x for every term x, so the sums are unchanged).  With `acc` (the chunk's rows) the arg-max
+// and arg-min tie accumulators go there as in pass B's forward; with `gate_out` lane 0 overwrites the item's mask row
+// with the poses at which the warp gated a pair: the poses pass B's backward walks for it (cov_traj_long_backward_kernel).
+template <bool CARRY = false>
 __global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
 cov_traj_logodds_tiles_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, CovConst C,
                               const int32_t* __restrict__ out_index, float* __restrict__ out,
                               const unsigned* __restrict__ amask_g, int mask_stride,
-                              const int* __restrict__ worklist, int* __restrict__ ctrl) {
+                              const int* __restrict__ worklist, int* __restrict__ ctrl, double* __restrict__ acc = nullptr,
+                              float* __restrict__ carry = nullptr, unsigned* __restrict__ gate_out = nullptr,
+                              int64_t ntiles = 0, unsigned long long* __restrict__ stats = nullptr) {
     constexpr int PPT = kItemPpt;
     const int lane = threadIdx.x & 31;
     const int n_items = ctrl[0];
     const int nwords = (W + 31) >> 5;
-    for_each_item<true>(xyz, n, amask_g, mask_stride, out_index, worklist, n_items, ctrl + 3, [](int) {},
-                        [&](const Item& item) {
-        float px[PPT], py[PPT], pz[PPT], L[PPT];
+    if constexpr (CARRY) {
+        const bool check_amin = acc && ctrl[1] != 0;  // some pose of the chunk has min_j m > 0
+        unsigned n_full = 0;
+        for_each_item<false>(xyz, n, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 3, [](int) {},
+                             [&](const Item& item) {
+            float px[PPT], py[PPT], pz[PPT], L[PPT];
+            bool valid[PPT];
+            load_item_points<false>(item, xyz, n, lane, px, py, pz, valid);
+#pragma unroll
+            for (int s = 0; s < PPT; ++s) L[s] = valid[s] ? carry[item.j0 + s * 32 + lane] : 0.f;
+            bool warp_gated = false;
+            unsigned* grow = gate_out ? gate_out + (size_t)(item.j0 / kItemPts) * mask_stride : nullptr;
+            for (int c = 0; c < nwords; ++c) {
+                unsigned word = item.mask[c];
+                unsigned gbits = 0u;
+                while (word) {
+                    const int b = __ffs(word) - 1;
+                    const int w = c * 32 + b;
+                    word &= word - 1;
+                    const float4* row = table + (size_t)w * COV_ROW_F4;
+                    const float4 v3 = __ldg(row + 3);
+                    ++n_full;
+                    double* acc_row = acc ? acc + (size_t)w * COV_ACC_STRIDE : nullptr;
+                    const bool g = check_amin ? tiles_pose_iter<PPT, true>(row, v3, px, py, pz, L, C, acc_row)
+                                              : tiles_pose_iter<PPT, false>(row, v3, px, py, pz, L, C, acc_row);
+                    if (g) gbits |= 1u << b;
+                }
+                if (grow && lane == 0) grow[c] = gbits;
+                warp_gated |= gbits != 0u;
+            }
+            if (warp_gated) {
+#pragma unroll
+                for (int s = 0; s < PPT; ++s)
+                    if (valid[s]) carry[item.j0 + s * 32 + lane] = L[s] != 0.f ? L[s] : -0.f;
+            }
+        });
+        if (stats && lane == 0) {
+            if (threadIdx.x == 0 && blockIdx.x == 0) {
+                atomicAdd(stats + 0, (unsigned long long)ntiles * kWarps * W);
+                atomicAdd(stats + 6, *reinterpret_cast<const unsigned long long*>(ctrl + 4));  // counted by the cull
+            }
+            atomicAdd(stats + 1, (unsigned long long)n_full);
+        }
+    } else {
+        for_each_item<true>(xyz, n, amask_g, mask_stride, out_index, worklist, n_items, ctrl + 3, [](int) {},
+                            [&](const Item& item) {
+            float px[PPT], py[PPT], pz[PPT], L[PPT];
+            bool valid[PPT];
+            load_item_points<false>(item, xyz, n, lane, px, py, pz, valid);
+#pragma unroll
+            for (int s = 0; s < PPT; ++s) L[s] = 0.f;
+            for (int c = 0; c < nwords; ++c) {
+                unsigned word = item.mask[c];
+                while (word) {
+                    const int w = c * 32 + __ffs(word) - 1;
+                    word &= word - 1;
+                    const float4* row = table + (size_t)w * COV_ROW_F4;
+                    tiles_pose_iter<PPT, false>(row, __ldg(row + 3), px, py, pz, L, C, nullptr);
+                }
+            }
+#pragma unroll
+            for (int s = 0; s < PPT; ++s) {
+                if (valid[s] && L[s] != 0.f) {
+                    const int64_t j = item.j0 + s * 32 + lane;
+                    const int64_t jo = out_index ? (item.whole ? (int64_t)item.perm[s * 32 + lane] : (int64_t)out_index[j]) : j;
+                    out[jo] = cov_fuse_prior(out[jo], L[s]);
+                }
+            }
+        });
+    }
+}
+
+// The long path after the last chunk's forward: one grid-stride pass over the cloud order.  carry[j] = +0 (bits 0): no
+// chunk gated a pair in the point's item, so r_j = r0_j and the point enters no backward: nothing to do.  Otherwise
+// L_j = carry[j] (-0 for 0) gives r_j with pass B's expressions: r_j is stored in the caller's order where L_j != 0,
+// sum_j (r_j - r0_j) (WSUM: w_j (r_j - r0_j)) is added to the reward-sum slot, and carry[j] becomes G_j = r_j (1 - r_j)
+// (times w_j or upstream_j), the dr/dL the backward reads.  FOLD (cov_traj_logodds_long): out[jo] = cov_fuse_prior(out[jo],
+// L_j) where L_j != 0, as cov_traj_logodds_tiles_kernel writes it.
+template <bool FOLD, bool HAS_UP, bool HAS_PRIOR, bool WSUM>
+__global__ void __launch_bounds__(256)
+cov_traj_long_finalise_kernel(int64_t n, float* __restrict__ carry, const int32_t* __restrict__ out_index,
+                              float* __restrict__ out, const float* __restrict__ upstream,
+                              const float* __restrict__ prior, double* __restrict__ sum_slot) {
+    static_assert(HAS_UP || !WSUM, "the weight rides on the upstream gather");
+    double sum_r = 0.0;
+    const int64_t nq = (n + 3) / 4;
+    for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < nq; q += (int64_t)gridDim.x * blockDim.x) {
+        const bool whole = q * 4 + 4 <= n;
+        float v[4];
+        if (whole) {
+            const float4 f = reinterpret_cast<const float4*>(carry)[q];
+            v[0] = f.x; v[1] = f.y; v[2] = f.z; v[3] = f.w;
+        } else {
+            for (int k = 0; k < 4; ++k) v[k] = q * 4 + k < n ? carry[q * 4 + k] : 0.f;
+        }
+        if ((__float_as_uint(v[0]) | __float_as_uint(v[1]) | __float_as_uint(v[2]) | __float_as_uint(v[3])) == 0u) continue;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            if (__float_as_uint(v[k]) == 0u) continue;
+            const float L = v[k];
+            const int64_t j = q * 4 + k;
+            const int64_t jo = out_index ? (int64_t)out_index[j] : j;
+            if (FOLD) {
+                if (L != 0.f) out[jo] = cov_fuse_prior(out[jo], L);
+                continue;
+            }
+            float r, G;
+            if (HAS_PRIOR) {
+                const float pr = __ldg(prior + jo);
+                const float r0 = cov_sigmoid(pr);
+                r = r0;
+                if (L != 0.f) {
+                    r = cov_sigmoid(cov_fuse_prior(pr, L));
+                    out[jo] = r;
+                }
+                G = r * (1.f - r);
+                if (WSUM) {
+                    const float wj = upstream[jo];
+                    sum_r += (double)wj * (double)(r - r0);
+                    G *= wj;
+                } else {
+                    sum_r += (double)(r - r0);
+                    if (HAS_UP) G *= upstream[jo];
+                }
+            } else {
+                r = 0.5f;
+                G = 0.25f;  // exactly what the formulas below give for L = 0
+                if (L != 0.f) {
+                    r = 1.f / (1.f + expf(-L));
+                    G = r * (1.f - r);
+                    out[jo] = r;
+                }
+                if (WSUM) {
+                    const float wj = upstream[jo];
+                    sum_r += (double)wj * (double)(r - 0.5f);
+                    G *= wj;
+                } else {
+                    sum_r += (double)(r - 0.5f);
+                    if (HAS_UP) G *= upstream[jo];
+                }
+            }
+            v[k] = G;
+        }
+        if (FOLD) continue;
+        if (whole) reinterpret_cast<float4*>(carry)[q] = make_float4(v[0], v[1], v[2], v[3]);
+        else for (int k = 0; k < 4 && q * 4 + k < n; ++k) carry[q * 4 + k] = v[k];
+    }
+    if (!FOLD) {
+        const double ws = cov_warp_sum(sum_r);
+        if ((threadIdx.x & 31) == 0 && ws != 0.0) atomicAdd(sum_slot, ws);
+    }
+}
+
+// The long path's backward of one pose chunk: persistent warps over the chunk's kept work list (for_each_item), each item
+// with the mask row its forward rewrote (the poses at which the warp gated a pair) and the 128 G_j of its points (cloud
+// order, from the finalise kernel).  tiles_pose_backward for every pose of the mask: the (box, pose) pairs, m and terms of
+// pass B's backward.  The item ticket is ctrl[2] (the forward drew ctrl[3]).
+__global__ void __launch_bounds__(COV_THREADS, kTilesMinBlocks)
+cov_traj_long_backward_kernel(const float* __restrict__ xyz, int64_t n, const float4* __restrict__ table, int W, CovConst C,
+                              const float* __restrict__ G_dev, double* __restrict__ acc,
+                              const unsigned* __restrict__ amask_g, int mask_stride, const int* __restrict__ worklist,
+                              int* __restrict__ ctrl, unsigned long long* __restrict__ stats) {
+    constexpr int PPT = kItemPpt;
+    const int lane = threadIdx.x & 31;
+    const int n_items = ctrl[0];
+    const int nwords = (W + 31) >> 5;
+    unsigned n_bwd = 0;
+    for_each_item<false>(xyz, n, amask_g, mask_stride, nullptr, worklist, n_items, ctrl + 2, [](int) {},
+                         [&](const Item& item) {
+        unsigned any = 0u;
+        for (int c = 0; c < nwords; ++c) any |= item.mask[c];
+        if (any == 0u) return;
+        float px[PPT], py[PPT], pz[PPT], G[PPT];
         bool valid[PPT];
         load_item_points<false>(item, xyz, n, lane, px, py, pz, valid);
 #pragma unroll
-        for (int s = 0; s < PPT; ++s) L[s] = 0.f;
+        for (int s = 0; s < PPT; ++s) G[s] = valid[s] ? __ldg(G_dev + item.j0 + s * 32 + lane) : 0.f;
         for (int c = 0; c < nwords; ++c) {
             unsigned word = item.mask[c];
             while (word) {
                 const int w = c * 32 + __ffs(word) - 1;
                 word &= word - 1;
-                const float4* row = table + (size_t)w * COV_ROW_F4;
-                tiles_pose_iter<PPT, false>(row, __ldg(row + 3), px, py, pz, L, C, nullptr);
-            }
-        }
-#pragma unroll
-        for (int s = 0; s < PPT; ++s) {
-            if (valid[s] && L[s] != 0.f) {
-                const int64_t j = item.j0 + s * 32 + lane;
-                const int64_t jo = out_index ? (item.whole ? (int64_t)item.perm[s * 32 + lane] : (int64_t)out_index[j]) : j;
-                out[jo] = cov_fuse_prior(out[jo], L[s]);
+                ++n_bwd;
+                tiles_pose_backward<PPT>(table + (size_t)w * COV_ROW_F4, px, py, pz, G, C, acc + (size_t)w * COV_ACC_STRIDE,
+                                         lane);
             }
         }
     });
+    if (stats && lane == 0) atomicAdd(stats + 4, (unsigned long long)n_bwd);
 }
 
 // Fused log-odds output, dense: every (point, pose) pair, the pose rows (with the normalisers, cov_norm_row) in shared
@@ -2031,6 +2212,55 @@ int launch_cull(const float4* boxes, int64_t n, const TrajWorkspace& t, int W, c
     cull<<<grid, 256, smem, s>>>(boxes, n, ntiles, t.table, W, enc, inv_kd, t.amask, mask_stride_words(W), t.worklist,
                                  t.ctrl, t.desc, fill_dst, fill_n, fill_prior);
     return COV_OK;
+}
+
+// ---- the long path (cov_traj_fused_long, cov_traj_logodds_long): poses in chunks, the fused log-odds carried ----
+// Workspace: [boxes][carry: n floats][pose table: W rows][K chunk regions], every region 256-byte aligned.  A chunk region
+// is [ctrl ints | look-back descriptors][work list][box masks of mask_stride_words(chunk) words]: pass B's control words,
+// list and masks of one chunk, kept from its forward to its backward.
+int long_chunk(int pose_chunk) { return pose_chunk > 0 ? pose_chunk : 32 * kMaskWords; }
+
+TrajWorkspace carve_long_region(char* p, int64_t n, int Wc, float4* table) {
+    const int64_t nt = (n + 1023) / 1024;
+    const int64_t nchunks = (nt + kChunkTiles - 1) / kChunkTiles;
+    const int64_t cap = list_capacity(n);
+    size_t off = 0;
+    auto take = [&](size_t bytes) { char* q = p + off; off += align256(bytes); return q; };
+    TrajWorkspace t;
+    t.ctrl_bytes = kCtrlInts * sizeof(int) + (size_t)nchunks * sizeof(unsigned long long);
+    char* c = take(t.ctrl_bytes);
+    t.ctrl = reinterpret_cast<int*>(c);
+    t.enc = nullptr;
+    t.desc = reinterpret_cast<unsigned long long*>(c + kCtrlInts * sizeof(int));
+    t.table = table;
+    t.worklist = reinterpret_cast<int*>(take((size_t)cap * sizeof(int)));
+    t.amask = reinterpret_cast<unsigned*>(take((size_t)cap * mask_stride_words(Wc) * sizeof(unsigned)));
+    t.boxes = nullptr;
+    t.bytes = off;
+    return t;
+}
+
+struct LongWorkspace {
+    float4* boxes;
+    float* carry;
+    float4* table;
+    char* regions;
+    size_t region_bytes;
+    size_t bytes;
+};
+LongWorkspace carve_long(void* ws, int64_t n, int W, int chunk) {
+    char* p = reinterpret_cast<char*>(ws);
+    size_t off = 0;
+    auto take = [&](size_t bytes) { char* q = p + off; off += align256(bytes); return q; };
+    LongWorkspace l;
+    l.boxes = reinterpret_cast<float4*>(take((size_t)boxes_padded(n) * 2 * sizeof(float4)));
+    l.carry = reinterpret_cast<float*>(take((size_t)n * sizeof(float)));
+    l.table = reinterpret_cast<float4*>(take((size_t)W * COV_ROW_F4 * sizeof(float4)));
+    l.region_bytes = carve_long_region(nullptr, n, std::min(chunk, W), nullptr).bytes;
+    const int64_t k = (W + chunk - 1) / chunk;
+    l.regions = take((size_t)k * l.region_bytes);
+    l.bytes = off;
+    return l;
 }
 
 }  // namespace
@@ -2361,9 +2591,164 @@ extern "C" int cov_traj_logodds(const float* xyz, int64_t n, const float* poses,
     cov_traj_table_kernel<false><<<(W + 63) / 64, 64, 0, s>>>(poses, quats, W, K, C, minmax, t.table, t.ctrl,
                                                               (int)(t.ctrl_bytes / sizeof(int)), nullptr, 0.0, nullptr);
     if ((rc = launch_cull(boxes, n, t, W, nullptr, 0.f, nullptr, 0, s)) != COV_OK) return rc;
-    cov_traj_logodds_tiles_kernel<<<persistent_grid(cov_traj_logodds_tiles_kernel, 0, ntiles), COV_THREADS, 0, s>>>(
+    cov_traj_logodds_tiles_kernel<><<<persistent_grid(cov_traj_logodds_tiles_kernel<>, 0, ntiles), COV_THREADS, 0, s>>>(
         xyz, n, t.table, W, C, reward_index, logodds, t.amask, mask_stride_words(W), t.worklist, t.ctrl);
     return cov_check_launch("cov_traj_logodds");
+}
+
+extern "C" size_t cov_traj_long_workspace_bytes(int64_t n, int W, int pose_chunk) {
+    if (n < 1) n = 1;
+    if (W < 1) W = 1;
+    const int max_chunk = 32 * kMaskWords;
+    const int c0 = (pose_chunk < 1 || pose_chunk > max_chunk) ? max_chunk : pose_chunk;
+    // the largest layout of any chunk >= c0, so that the size never grows with the chunk (a workspace sized for one
+    // chunk serves every larger one); and at least the single-call workspace pass A runs its chunks in
+    size_t bytes = cov_traj_workspace_bytes(n, std::min(W, max_chunk));
+    for (int c = c0; c <= std::max(c0, std::min(W, max_chunk)); ++c) bytes = std::max(bytes, carve_long(nullptr, n, W, c).bytes);
+    return bytes;
+}
+
+// The long path.  FOLD: cov_traj_logodds_long (out = the log-odds buffer; no accumulators, no backward).
+static int traj_long_impl(const char* who, const float* xyz, int64_t n, const float* poses, const float* quats, int W,
+                          const float* K, const cov_camera* cam, const float* boxes_dev, const float* minmax,
+                          const float* upstream, const int32_t* reward_index, float* out, double* acc, const float* prior,
+                          const double* base, const float* weight, int pose_chunk, const cov_traj_opts* opts, void* ws,
+                          size_t ws_bytes, void* stream, bool fold) {
+    if (!xyz || n <= 0 || !poses || !quats || W <= 0 || !K || !cam || !minmax || !out || (!fold && !acc)) {
+        cov_set_error("%s: null pointer, empty cloud or no poses (n=%lld, W=%d)", who, (long long)n, W);
+        return COV_ERR_ARG;
+    }
+    if (pose_chunk < 0 || pose_chunk > 32 * kMaskWords) {
+        cov_set_error("%s: pose_chunk %d outside 0 .. %d", who, pose_chunk, 32 * kMaskWords);
+        return COV_ERR_ARG;
+    }
+    int rc = COV_OK;
+    if (!fold) {  // base: NULL without prior and weight, cov_prior_reward_sum with a prior alone, cov_weight_sums with a weight
+        if (weight && upstream) {
+            cov_set_error("%s: weight_dev and upstream_dev are never given together", who);
+            return COV_ERR_ARG;
+        }
+        if (weight) rc = check_weight(who, weight, base, prior);
+        else if (prior) rc = check_prior(who, prior, base, true);
+        else if (base) {
+            cov_set_error("%s: base_dev must be NULL without prior_dev and weight_dev", who);
+            rc = COV_ERR_ARG;
+        }
+        if (rc) return rc;
+    }
+    if (opts && opts->dense) {  // no dense long path: what one dense call takes, it takes
+        if (W > cov_traj_max_poses()) {
+            cov_set_error("%s: %d poses exceed what one call takes on this path (max %d)", who, W, cov_traj_max_poses());
+            return COV_ERR_UNSUPPORTED;
+        }
+        if (fold)
+            return cov_traj_logodds(xyz, n, poses, quats, W, K, cam, boxes_dev, minmax, reward_index, out, opts, ws, ws_bytes,
+                                    stream);
+        return traj_fused_impl(xyz, n, poses, quats, W, K, cam, boxes_dev, minmax, upstream, reward_index, out, acc, prior,
+                               weight ? nullptr : base, opts, ws, ws_bytes, stream, weight, weight ? base : nullptr);
+    }
+    if (n >= ((int64_t)1 << 31) * 256) {
+        cov_set_error("%s: %lld points exceed the int32 tile index range", who, (long long)n);
+        return COV_ERR_UNSUPPORTED;
+    }
+    if (!ws) {
+        cov_set_error("%s: null workspace", who);
+        return COV_ERR_ARG;
+    }
+    const size_t need = cov_traj_long_workspace_bytes(n, W, pose_chunk);
+    if (ws_bytes < need) {
+        cov_set_error("%s: workspace %zu < cov_traj_long_workspace_bytes(n, %d, %d) = %zu", who, ws_bytes, W, pose_chunk,
+                      need);
+        return COV_ERR_WORKSPACE;
+    }
+    if ((((uintptr_t)ws) & 255) || (((uintptr_t)xyz) & 15) || (boxes_dev && (((uintptr_t)boxes_dev) & 15)) ||
+        (reward_index && (((uintptr_t)reward_index) & 15))) {
+        cov_set_error("%s: workspace must be 256-byte aligned, the cloud, boxes and reward_index 16-byte aligned", who);
+        return COV_ERR_ALIGN;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    const CovConst C = cov_make_const(cam);
+    const int chunk = long_chunk(pose_chunk);
+    const LongWorkspace l = carve_long(ws, n, W, chunk);
+    const float4* boxes = boxes_dev ? reinterpret_cast<const float4*>(boxes_dev) : l.boxes;
+    if (!boxes_dev) launch_tile_boxes(xyz, n, l.boxes, s);
+    constexpr int ppt = 4;  // tiles of 1024 points, eight 128-point boxes each
+    const int64_t ntiles = (n + tile_points(ppt) - 1) / tile_points(ppt);
+    unsigned long long* stats = (opts && !fold) ? opts->stats_dev : nullptr;
+    const bool prefilled = opts && opts->rewards_prefilled;
+    const bool sum_dev = prior || weight;
+    const int nk = (W + chunk - 1) / chunk;
+    auto region = [&](int k) {
+        return carve_long_region(l.regions + (size_t)k * l.region_bytes, n, std::min(chunk, W),
+                                 l.table + (size_t)k * chunk * COV_ROW_F4);
+    };
+    cudaMemsetAsync(l.carry, 0, (size_t)n * sizeof(float), s);
+    // forward, chunk by chunk: pass B's table (chunk rows of the accumulators zeroed), cull + work list (the first also
+    // pre-fills the rewards), then the CARRY forward over the listed boxes
+    const auto fwd = cov_traj_logodds_tiles_kernel<true>;
+    for (int k = 0; k < nk; ++k) {
+        const int w0 = k * chunk, Wc = std::min(chunk, W - w0);
+        const TrajWorkspace t = region(k);
+        double* acc_k = fold ? nullptr : acc + (size_t)w0 * COV_ACC_STRIDE;
+        const int ctrl_words = (int)(t.ctrl_bytes / sizeof(int));
+        if (sum_dev)
+            cov_traj_table_kernel<true, true><<<(Wc + 63) / 64, 64, 0, s>>>(poses + 3 * (size_t)w0, quats + 4 * (size_t)w0,
+                                                                           Wc, K, C, minmax, t.table, t.ctrl, ctrl_words,
+                                                                           acc_k, 0.0, base, w0, W);
+        else
+            cov_traj_table_kernel<false, true><<<(Wc + 63) / 64, 64, 0, s>>>(poses + 3 * (size_t)w0, quats + 4 * (size_t)w0,
+                                                                            Wc, K, C, minmax, t.table, t.ctrl, ctrl_words,
+                                                                            acc_k, 0.5 * (double)n, nullptr, w0, W);
+        const bool fill = k == 0 && !fold && !prefilled;
+        if ((rc = launch_cull(boxes, n, t, Wc, nullptr, 0.f, fill ? out : nullptr, n, s, fill ? prior : nullptr)) != COV_OK)
+            return rc;
+        fwd<<<persistent_grid(fwd, 0, ntiles), COV_THREADS, 0, s>>>(xyz, n, t.table, Wc, C, nullptr, nullptr, t.amask,
+                                                                     mask_stride_words(Wc), t.worklist, t.ctrl, acc_k,
+                                                                     l.carry, fold ? nullptr : t.amask, ntiles, stats);
+    }
+    // finalise: r_j, the reward sum and G_j (FOLD: the fused log-odds) from the carried L_j
+    {
+        const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((n / 4 + 255) / 256, (int64_t)cov_sm_count_cached() * 8));
+        double* sum_slot = fold ? nullptr : acc + (size_t)W * COV_ACC_STRIDE;
+        const float* up = weight ? weight : upstream;
+#define LAUNCH_FIN(FO, UP, PR, WS) \
+    cov_traj_long_finalise_kernel<FO, UP, PR, WS><<<grid, 256, 0, s>>>(n, l.carry, reward_index, out, up, prior, sum_slot)
+        if (fold) LAUNCH_FIN(true, false, false, false);
+        else if (weight) { if (prior) LAUNCH_FIN(false, true, true, true); else LAUNCH_FIN(false, true, false, true); }
+        else if (upstream) { if (prior) LAUNCH_FIN(false, true, true, false); else LAUNCH_FIN(false, true, false, false); }
+        else if (prior) LAUNCH_FIN(false, false, true, false);
+        else LAUNCH_FIN(false, false, false, false);
+#undef LAUNCH_FIN
+    }
+    if (fold) return cov_check_launch(who);
+    // backward, chunk by chunk, over the kept work lists and rewritten masks
+    const auto bwd = cov_traj_long_backward_kernel;
+    for (int k = 0; k < nk; ++k) {
+        const int w0 = k * chunk, Wc = std::min(chunk, W - w0);
+        const TrajWorkspace t = region(k);
+        bwd<<<persistent_grid(bwd, 0, ntiles), COV_THREADS, 0, s>>>(xyz, n, t.table, Wc, C, l.carry,
+                                                                     acc + (size_t)w0 * COV_ACC_STRIDE, t.amask,
+                                                                     mask_stride_words(Wc), t.worklist, t.ctrl, stats);
+    }
+    return cov_check_launch(who);
+}
+
+extern "C" int cov_traj_fused_long(const float* xyz, int64_t n, const float* poses, const float* quats, int W,
+                                   const float* K, const cov_camera* cam, const float* boxes_dev, const float* minmax,
+                                   const float* upstream, const int32_t* reward_index, float* rewards, double* acc,
+                                   const float* prior, const double* base, const float* weight, int pose_chunk,
+                                   const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+    return traj_long_impl("cov_traj_fused_long", xyz, n, poses, quats, W, K, cam, boxes_dev, minmax, upstream, reward_index,
+                          rewards, acc, prior, base, weight, pose_chunk, opts, ws, ws_bytes, stream, false);
+}
+
+extern "C" int cov_traj_logodds_long(const float* xyz, int64_t n, const float* poses, const float* quats, int W,
+                                     const float* K, const cov_camera* cam, const float* boxes_dev, const float* minmax,
+                                     const int32_t* reward_index, float* logodds, int pose_chunk,
+                                     const cov_traj_opts* opts, void* ws, size_t ws_bytes, void* stream) {
+    return traj_long_impl("cov_traj_logodds_long", xyz, n, poses, quats, W, K, cam, boxes_dev, minmax, nullptr,
+                          reward_index, logodds, nullptr, nullptr, nullptr, nullptr, pose_chunk, opts, ws, ws_bytes, stream,
+                          true);
 }
 
 // prefix: the per-pose slots of cov_sweep_prefix_rewards (sum_rewards holds n_traj * per_traj doubles; the caller scans)

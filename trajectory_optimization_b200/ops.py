@@ -93,6 +93,15 @@ def _ptr(t):
     return ctypes.c_void_p(t.data_ptr() if t is not None else 0)
 
 
+def _max_poses_pruned():
+    """Poses one pruned call takes (cov_traj_max_poses_pruned); trajectory calls with more take the long path."""
+    return _lib.lib().cov_traj_max_poses_pruned()
+
+
+def _takes_long_path(W, dense):
+    return not dense and W > _max_poses_pruned()
+
+
 def _check_prior(prior, n, device, what="prior_logodds", unit="log-odds"):
     """A per-point prior log-odds tensor (or point weight) as the kernels take it: fp32, shape (n,), on the cloud's
     device; made contiguous and 16-byte aligned (a copy only when it has to).  Shape, dtype and device errors raise
@@ -270,6 +279,9 @@ class CudaBackend:
         return out
 
     def traj_workspace_bytes(self, pts, W):
+        """Workspace of both passes of a W-pose call; above cov_traj_max_poses_pruned() poses, of the long path."""
+        if W > _max_poses_pruned():
+            return _lib.lib().cov_traj_long_workspace_bytes(pts.shape[0], W, 0)
         return _lib.lib().cov_traj_workspace_bytes(pts.shape[0], W)
 
     def traj_workspace(self, pts, W):
@@ -338,23 +350,58 @@ class CudaBackend:
               _ptr(minmax), _ptr(reward_index), _ptr(out), ctypes.byref(opts), _ptr(ws), ws.numel())
         return out
 
-    def sweep_minmax(self, pts, P, Q, Kd, cam, boxes=None):
-        """Per-pose minima and maxima of all T*P poses of a sweep (pass A, one pose-table-full at a time)."""
+    def sweep_minmax(self, pts, P, Q, Kd, cam, boxes=None, ws=None, dense=None, prefill=None, prior=None):
+        """Per-pose minima and maxima of all T*P poses of a sweep, or of the W poses of a long trajectory (pass A, one
+        pose-table-full at a time).  `ws`: a kept workspace of at least cov_traj_workspace_bytes(n, chunk) bytes;
+        `prefill` (with `prior`, indexed like it): the first chunk pre-fills it as traj_minmax does."""
         L = _lib.lib()
         W, n, dev = P.shape[0], pts.shape[0], pts.device
         minmax = torch.empty(2 * W, dtype=torch.float32, device=dev)
-        chunk = L.cov_traj_max_poses_pruned() if self.prefill_applies(pts) else L.cov_traj_max_poses()
+        chunk = L.cov_traj_max_poses_pruned() if self.prefill_applies(pts, dense) else L.cov_traj_max_poses()
         ws_bytes = L.cov_traj_workspace_bytes(n, min(W, chunk))
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        opts = _opts()
+        if ws is None or ws.numel() < ws_bytes:
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         for w0 in range(0, W, chunk):
             w1 = min(W, w0 + chunk)
             mm = torch.empty(2 * (w1 - w0), dtype=torch.float32, device=dev)
-            _call("cov_traj_minmax", pts, _ptr(pts), n, _ptr(P[w0:w1]), _ptr(Q[w0:w1]), w1 - w0, _ptr(Kd),
-                  ctypes.byref(cam), _ptr(boxes), _ptr(mm), ctypes.byref(opts), _ptr(ws), ws_bytes)
+            fill = prefill if w0 == 0 else None
+            opts = _opts(dense, prefill=fill)
+            if prior is not None and fill is not None:
+                _call("cov_traj_minmax_prior", pts, _ptr(pts), n, _ptr(P[w0:w1]), _ptr(Q[w0:w1]), w1 - w0, _ptr(Kd),
+                      ctypes.byref(cam), _ptr(boxes), _ptr(mm), _ptr(prior), ctypes.byref(opts), _ptr(ws), ws.numel())
+            else:
+                _call("cov_traj_minmax", pts, _ptr(pts), n, _ptr(P[w0:w1]), _ptr(Q[w0:w1]), w1 - w0, _ptr(Kd),
+                      ctypes.byref(cam), _ptr(boxes), _ptr(mm), ctypes.byref(opts), _ptr(ws), ws.numel())
             minmax[w0:w1] = mm[:w1 - w0]
             minmax[W + w0:W + w1] = mm[w1 - w0:]
         return minmax
+
+    def traj_fused_long(self, pts, P, Q, Kd, cam, minmax, upstream, rewards, reward_index=None, boxes=None, ws=None,
+                        prefilled=False, prior=None, base=None, weight=None, pose_chunk=0):
+        """traj_fused over any number of poses, in chunks of `pose_chunk` (0: cov_traj_max_poses_pruned()) with the fused
+        log-odds carried between them (cov_traj_fused_long).  `base`: prior_sum(prior) with a prior alone,
+        weight_sums(weight, prior) with a weight, else None."""
+        W, n = P.shape[0], pts.shape[0]
+        acc = torch.empty(W * _lib.ACC_STRIDE + 1, dtype=torch.float64, device=pts.device)
+        ws_bytes = _lib.lib().cov_traj_long_workspace_bytes(n, W, pose_chunk)
+        if ws is None or ws.numel() < ws_bytes or ws.device != pts.device:
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=pts.device)
+        opts = _opts(False, rewards_prefilled=prefilled)
+        _call("cov_traj_fused_long", pts, _ptr(pts), n, _ptr(P), _ptr(Q), W, _ptr(Kd), ctypes.byref(cam), _ptr(boxes),
+              _ptr(minmax), _ptr(upstream), _ptr(reward_index), _ptr(rewards), _ptr(acc), _ptr(prior), _ptr(base),
+              _ptr(weight), int(pose_chunk), ctypes.byref(opts), _ptr(ws), ws.numel())
+        return acc
+
+    def traj_logodds_long(self, pts, P, Q, Kd, cam, minmax, out, reward_index=None, boxes=None, ws=None, pose_chunk=0):
+        """traj_logodds over any number of poses, in chunks of `pose_chunk` (cov_traj_logodds_long)."""
+        W, n = P.shape[0], pts.shape[0]
+        ws_bytes = _lib.lib().cov_traj_long_workspace_bytes(n, W, pose_chunk)
+        if ws is None or ws.numel() < ws_bytes or ws.device != pts.device:
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=pts.device)
+        opts = _opts(False)
+        _call("cov_traj_logodds_long", pts, _ptr(pts), n, _ptr(P), _ptr(Q), W, _ptr(Kd), ctypes.byref(cam), _ptr(boxes),
+              _ptr(minmax), _ptr(reward_index), _ptr(out), int(pose_chunk), ctypes.byref(opts), _ptr(ws), ws.numel())
+        return out
 
     def sweep_sums(self, pts, P, Q, T, Pn, Kd, cam, boxes, minmax, prior=None, prior_sum=None, weight=None, wsums=None):
         """sum_j rewards_j(t) over this cloud for every trajectory t (fp64); `prior` in the cloud's order.  `weight` (cloud's
@@ -566,7 +613,9 @@ class CoverageTrajFn(torch.autograd.Function):
         rewards = torch.empty(n, dtype=torch.float32, device=dev)
         # the pruned pass A pre-fills pass B's rewards with 1/2 under its idle memory bandwidth
         prefill = rewards if B.prefill_applies(pts, dense) else None
-        if prior is None:
+        if _takes_long_path(W, dense):   # pass A one pose-table-full at a time (the first pre-fills)
+            minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes, ws, dense, prefill, prior)
+        elif prior is None:
             minmax = B.traj_minmax(pts, P, Q, Kd, cam, boxes, ws, dense, prefill)   # pass A on this shard
         else:   # the pre-fill writes sigmoid(prior_i)
             minmax = B.traj_minmax(pts, P, Q, Kd, cam, boxes, ws, dense, prefill, prior)
@@ -583,7 +632,10 @@ class CoverageTrajFn(torch.autograd.Function):
     @staticmethod
     def _run(pts, P, Q, Kd, cam, minmax, upstream, rewards, n_total, group, reward_index=None, boxes=None, ws=None,
              dense=None, prefilled=False, prior=None, prior_sum=None, weight=None, wsums=None, den=None):
-        if weight is not None:   # pass B, weighted sums (never with an upstream)
+        if _takes_long_path(P.shape[0], _MODE.dense if dense is None else dense):   # pass B in pose chunks
+            acc = _BACKEND.traj_fused_long(pts, P, Q, Kd, cam, minmax, upstream, rewards, reward_index, boxes, ws,
+                                           prefilled, prior, wsums if weight is not None else prior_sum, weight)
+        elif weight is not None:   # pass B, weighted sums (never with an upstream)
             acc = _BACKEND.traj_fused(pts, P, Q, Kd, cam, minmax, None, rewards, reward_index, boxes, ws, dense,
                                       prefilled, prior=prior, weight=weight, wsums=wsums)
         elif prior is None:
@@ -819,9 +871,13 @@ def traj_logodds(points, poses, quats, intrins, img_width, img_height, min_dist=
     ws = workspace
     if ws is None or ws.numel() < B.traj_workspace_bytes(pts, W) or ws.device != dev:
         ws = B.traj_workspace(pts, W)
-    minmax = B.traj_minmax(pts, P, Q, Kd, cam, boxes, ws, dense)
+    long = _takes_long_path(W, dense)
+    minmax = B.sweep_minmax(pts, P, Q, Kd, cam, boxes, ws, dense) if long else B.traj_minmax(pts, P, Q, Kd, cam, boxes,
+                                                                                           ws, dense)
     _all_reduce_minmax(minmax, W, group)
     out = torch.zeros(n, dtype=torch.float32, device=dev) if prior is None else prior.clone()
+    if long:
+        return B.traj_logodds_long(pts, P, Q, Kd, cam, minmax, out, reward_index, boxes, ws)
     return B.traj_logodds(pts, P, Q, Kd, cam, minmax, out, reward_index, boxes, ws, dense)
 
 
